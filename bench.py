@@ -3,9 +3,17 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                   [--workload arabidopsis|sorghum|maize|sugarcane|sample] [--no-extra] [--no-cpu-baseline]
+                  [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (PAM scan both strands + ordered compaction + Rule-Set-1
-scoring of every candidate) over one synthetic genome (tools/workloads.py).
+scoring of every candidate) over one synthetic genome (tools/workloads.py).  K steps are timed,
+after W >= 3 untimed ones; the end-to-end leg below times K steps of its own.
+
+  --dump-outputs DIR   after the timed steps, write what the last one computed as float64 .npy files
+          (dump_outputs below): the per-segment candidate counts, and of each strand stream a fixed,
+          seeded sample of at most 2^19 rows (row index, pos, fp64 x, packed 30-mer as two 32-bit
+          halves).  The inputs are seeded, so two builds run with the same arguments can be compared
+          file by file.
 
   N = 1   configs[1] (Arabidopsis-scale); the other single-GPU configs ride along as extra keys
   N > 1   STRONG scaling: ONE genome (configs[3], maize-scale; at N = 8 also configs[4], sugarcane-
@@ -263,9 +271,10 @@ class _ManyResults:
             r.free()
 
 
-def time_scans(engine, sh, steps, warmup, sampler_index=None):
-    """-> dict(ms mean of kernel(+collective) per step on this rank, kernel_ms, candidates, launches, wall_ms, clocks)"""
-    total_ms, kernel_ms, n_cand = [], [], 0
+def time_scans(engine, sh, steps, warmup, sampler_index=None, keep_last=False):
+    """-> dict(ms mean of kernel(+collective) per step on this rank, kernel_ms, candidates, launches, wall_ms, clocks,
+    last: the result of the last step if keep_last, else None; the caller frees it)"""
+    total_ms, kernel_ms, n_cand, last = [], [], 0, None
     launches0, sampler, t_wall0, relaunched = 0, None, 0.0, 0
     for i in range(warmup + steps):
         if i == warmup:
@@ -284,12 +293,44 @@ def time_scans(engine, sh, steps, warmup, sampler_index=None):
             kernel_ms.append(d["kernel_ms"])
             relaunched += d["launches"] - 1
         n_cand = res.n_plus + res.n_minus
-        res.free()
+        if keep_last and i == warmup + steps - 1:
+            last = res
+        else:
+            res.free()
     engine.comm_barrier()
     wall_ms = (time.perf_counter() - t_wall0) * 1e3 / steps
     return {"ms": float(np.mean(total_ms)), "kernel_ms": float(np.mean(kernel_ms)), "candidates": int(n_cand),
             "launches": engine.launch_count() - launches0, "wall_ms": wall_ms, "capacity_reruns": relaunched,
-            "sampler": sampler}
+            "sampler": sampler, "last": last}
+
+
+DUMP_ROWS = 1 << 19        # rows per strand, shared by all ranks: 2 strands x 5 float64 columns x 2^19 rows = 40 MiB
+
+
+def dump_outputs(res, out_dir, rank, world):
+    """What a caller of the scan gets back (ScanResult.fetch of both strands, per-segment counts), as float64
+    .npy files under out_dir: every count, and of each strand a sample of rows drawn with a fixed seed from
+    the row count alone, so two builds that agree on the counts sample the same rows.  Exact in float64:
+    pos and the two halves of the packed 30-mer are 32-bit integers.  Several ranks: files rank<r>_*.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    prefix = f"rank{rank}_" if world > 1 else ""
+    parts = res.results if isinstance(res, _ManyResults) else [res]
+
+    def save(name, a):
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), np.asarray(a, dtype=np.float64))
+
+    save("seg_counts", [np.concatenate([r.seg_plus for r in parts]), np.concatenate([r.seg_minus for r in parts])])
+    for strand, name in (("+", "plus"), ("-", "minus")):
+        rows = [r.fetch(strand) for r in parts]
+        pos, packed, x = (np.concatenate([f[k] for f in rows]) for k in ("pos", "packed", "x"))
+        n = len(pos)
+        keep = DUMP_ROWS // world
+        idx = np.arange(n) if n <= keep else np.sort(np.random.default_rng(20).choice(n, keep, replace=False))
+        save(f"{name}_row", idx)
+        save(f"{name}_pos", pos[idx])
+        save(f"{name}_x", x[idx])
+        save(f"{name}_packed_lo", packed[idx] & np.uint64(0xFFFFFFFF))
+        save(f"{name}_packed_hi", packed[idx] >> np.uint64(32))
 
 
 def roofline(my_bases, n_cand, kernel_ms, workload, world):
@@ -311,7 +352,13 @@ def main():
     ap.add_argument("--workload", default=None, choices=sorted(W.WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the ride-along workloads / single-GPU denominator")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup     # timing rule: W >= 3
 
     from cropsr_b200 import launch
@@ -332,7 +379,11 @@ def main():
 
     # ---- device-resident metric: kernel (+ all-gather of the counts for N > 1) between CUDA events
     # nvidia-smi is polled by rank 0 only: eight pollers at 10 Hz each take driver locks that every rank's CUDA calls need
-    t = time_scans(engine, sh, args.steps, args.warmup, sampler_index=local if rank == 0 else None)
+    t = time_scans(engine, sh, args.steps, args.warmup, sampler_index=local if rank == 0 else None,
+                   keep_last=args.dump_outputs is not None)
+    if t["last"] is not None:
+        dump_outputs(t["last"], args.dump_outputs, rank, world)
+        t["last"].free()
     sampler = t["sampler"]
     ms = float(engine.comm_max([t["ms"]])[0])                      # the slowest rank sets the step
     value = n_bases_total / (ms * 1e-3) / 1e9
@@ -346,7 +397,7 @@ def main():
     want = ("pos", "x")
     arena, e2e_ms, h2d, d2h = None, [], 0, 0
     e2e_warmup = max(args.warmup, 5)           # the block cache of the pipelined call settles within the first calls
-    for i in range(e2e_warmup + max(3, args.steps // 2)):
+    for i in range(e2e_warmup + args.steps):
         engine.comm_barrier()
         t0 = time.perf_counter()
         arena, n_plus, n_minus, _ = engine.scan_segments(segs, 20, flags=N.CRP_SCAN_LOGISTIC, arena=arena, want=want)
