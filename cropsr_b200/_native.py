@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # CROPSR_B200_LIB: another build of the same library (kernel experiments, tools/variants.sh)
 LIB_PATH = os.environ.get("CROPSR_B200_LIB") or os.path.join(_HERE, "libcropsr_b200.so")
 
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 CRP_SCAN_DEFAULT = 0
 CRP_SCAN_NO_SCORE = 1
@@ -25,6 +25,8 @@ CRP_CLASS_SINGLE = 2
 PACKED_IRREGULAR = 1 << 30
 PACKED_TRUNCATED = 1 << 31
 PACKED_UNSCORED = 1 << 62
+
+OFFTARGET_NO_COUNT = 0xFFFFFFFF     # counts of a candidate without a protospacer (crp_offtarget_count_candidates)
 
 
 class SegmentDesc(C.Structure):
@@ -127,6 +129,14 @@ SIGNATURES = {
     "crp_result_gathered_counts": (C.c_int, [C.c_void_p, C.c_void_p]),
     "crp_result_timing_detail": (C.c_int, [C.c_void_p, _f32p, _f32p, _u32p]),
     "crp_rs1_preactivation": (C.c_int, [C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "crp_offtarget_new": (C.c_int, [_vpp]),
+    "crp_offtarget_add_genome": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "crp_offtarget_num_sites": (C.c_int, [C.c_void_p, _u64p]),
+    "crp_offtarget_fetch_sites": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, _u64p]),
+    "crp_offtarget_count_candidates": (C.c_int, [C.c_void_p, C.c_void_p, C.c_char, C.c_uint32, C.c_void_p]),
+    "crp_offtarget_count_keys": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_void_p]),
+    "crp_offtarget_timing": (C.c_int, [C.c_void_p, _f32p, _f32p, _u64p]),
+    "crp_offtarget_free": (C.c_int, [C.c_void_p]),
 }
 COMM_ID_BYTES = 128
 

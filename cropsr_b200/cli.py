@@ -9,7 +9,8 @@ def build_parser():
     # the usage line is spelled out: with the reference's empty metavars argparse cannot wrap a usage
     # line of this length (its own consistency assertion fails), and --help would crash
     p = argparse.ArgumentParser(prog="CROPSR.py", usage="CROPSR.py [-h] -f FASTA [-g GFF] [-p TXT] [-o CSV] [-l 20] [-L 200] --cas9 [-v]\n"
-                                "                 [--device N | --devices 0-7] [--side-output TSV] [--blas-threads N]")
+                                "                 [--device N | --devices 0-7] [--side-output TSV] [--offtargets TSV [--mismatches K]]\n"
+                                "                 [--blas-threads N]")
     p.add_argument("-f", "--fasta", metavar="", required=True, dest="f",
                    help="[required] path to input file in FASTA format")
     p.add_argument("-g", "--gff", metavar="", dest="g", help="path to input file in GFF format")
@@ -34,6 +35,12 @@ def build_parser():
     p.add_argument("--side-output", metavar="", default=None,
                    help="also write a tab-separated table of opt-in per-candidate side outputs (GC, poly-T, "
                         "homopolymer, +-L flank window, GFF feature under the cut site); the CSV is unaffected")
+    p.add_argument("--offtargets", metavar="", default=None,
+                   help="also write a tab-separated table of off-target counts: per candidate its protospacer and the "
+                        "number of other NGG sites of the genome (both strands, any case) at exactly 0 .. K mismatches; "
+                        "-l 20 on one GPU only; the CSV is unaffected")
+    p.add_argument("--mismatches", metavar="", type=int, default=3,
+                   help="K of --offtargets: 0 to 3, default = 3")
     p.add_argument("--blas-threads", type=int, default=1,
                    help="emulate the float summation order of the reference running with this many "
                         "OpenBLAS threads (default 1 = OPENBLAS_NUM_THREADS=1)")
@@ -77,9 +84,16 @@ def main(argv=None):
         sys.exit("Please select at least one CRISPR system: Cas9")     # CROPSR.py:335-336
     if args.verbose:
         print(banner(args))
-    from . import engine, pipeline
     devices = parse_devices(args.devices) if args.devices else [args.device]
+    if args.offtargets is not None:
+        from .pipeline import check_offtarget_args
+        try:
+            check_offtarget_args(args.l, devices, args.mismatches)
+        except ValueError as e:
+            sys.exit(f"CROPSR.py: error: --offtargets: {e}")
+    from . import engine, pipeline
     engine.init(devices[0])
     pipeline.run_cas9(args.f, args.g, args.o, args.l, args.verbose, args.blas_threads,
-                      side_output=args.side_output, flank=args.L, annotation_info=args.p, devices=devices)
+                      side_output=args.side_output, flank=args.L, annotation_info=args.p, devices=devices,
+                      offtargets=args.offtargets, max_mismatches=args.mismatches)
     return 0

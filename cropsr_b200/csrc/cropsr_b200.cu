@@ -29,8 +29,9 @@
 #include "scan.cuh"
 #include "primers.cuh"
 #include "extras.cuh"
+#include "offtarget.cuh"
 
-#define CRP_ABI_VERSION 7
+#define CRP_ABI_VERSION 8
 
 static constexpr size_t kScanSmemFixed = (size_t)kStages * kRecBytes + 2 * (size_t)kListCap * sizeof(uint16_t);
 
@@ -2061,6 +2062,328 @@ int crp_rescore(const crp_genome *g, uint64_t n, const uint32_t *segment, const 
     dev_free(d_items, st);
     dev_free(d_x, st);
     return rc;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------ off-target counts (offtarget.cuh)
+
+struct crp_offtarget {
+    cudaStream_t st = nullptr;                 // own stream, ordered behind each genome's stream by an event
+    cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};   // sites start / end, count start / end, genome ready
+    std::vector<const crp_genome *> genomes;
+    unsigned long long *keys = nullptr;        // site keys of every genome added, any order
+    uint64_t n_sites = 0;
+    float ms_sites = 0.f, ms_count = 0.f;      // summed over add_genome / of the last count call
+    uint64_t comparisons = 0;
+};
+
+// Count every query of d_keys (n rows, kOtInvalid = no counts) against the index's sites into d_counts
+// ([n][k + 1], primed by the caller), on ix->st; waits for the result.
+static int ot_count(crp_offtarget *ix, const unsigned long long *d_keys, uint64_t n, uint32_t k, uint32_t *d_counts) {
+    cudaStream_t st = ix->st;
+    const size_t tbl = kOtBuckets + 1;
+    uint32_t *d_tbl = nullptr, *d_sites = nullptr;
+    uint2 *d_q = nullptr;
+    unsigned long long *d_misc = nullptr;      // [0] comparisons, [1] overflow flag
+    if (dev_alloc(&d_tbl, 7 * tbl * sizeof(uint32_t), st) != cudaSuccess ||
+        dev_alloc(&d_sites, (ix->n_sites + 8) * sizeof(uint32_t), st) != cudaSuccess ||
+        dev_alloc(&d_q, (n + 1) * sizeof(uint2), st) != cudaSuccess ||
+        dev_alloc(&d_misc, 2 * sizeof(unsigned long long), st) != cudaSuccess) {
+        cudaGetLastError();
+        dev_free(d_tbl, st);
+        dev_free(d_sites, st);
+        dev_free(d_q, st);
+        return fail(CRP_ERR_NOMEM, "cudaMalloc of the off-target work buffers failed");
+    }
+    uint32_t *hist_s = d_tbl, *hist_q = d_tbl + tbl;
+    OtScanArgs sa;
+    sa.hist[0] = hist_s;
+    sa.hist[1] = hist_q;
+    sa.off[0] = d_tbl + 2 * tbl;
+    sa.off[1] = d_tbl + 3 * tbl;
+    sa.cursor[0] = d_tbl + 4 * tbl;
+    sa.cursor[1] = d_tbl + 5 * tbl;
+    sa.item_off = d_tbl + 6 * tbl;
+    sa.comparisons = d_misc;
+    sa.overflow = reinterpret_cast<unsigned int *>(d_misc + 1);
+    OtCountArgs ca;
+    ca.sites = d_sites;
+    ca.queries = d_q;
+    ca.soff = sa.off[0];
+    ca.qoff = sa.off[1];
+    ca.item_off = sa.item_off;
+    ca.counts = d_counts;
+    ca.k = k;
+    auto grid = [](uint64_t items) { return (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((items + 255) / 256, (uint64_t)g_ctx.sm_count * 16)); };
+    int rc = 0;
+    unsigned long long misc[2] = {0, 0};
+    if (cudaMemsetAsync(d_misc, 0, 2 * sizeof(unsigned long long), st) != cudaSuccess ||
+        cudaEventRecord(ix->ev[2], st) != cudaSuccess)
+        rc = fail(CRP_ERR_CUDA, "off-target setup failed");
+    for (int p = 0; p < kOtPairs && !rc && n && ix->n_sites; ++p) {
+        int i = 0, j = 0;
+        ot_pair(p, i, j);
+        ca.jm1 = (uint32_t)(j - 1);
+        if (cudaMemsetAsync(d_tbl, 0, 2 * tbl * sizeof(uint32_t), st) != cudaSuccess) {
+            rc = fail(CRP_ERR_CUDA, "memset failed");
+            break;
+        }
+        k_ot_hist<<<grid(ix->n_sites), 256, 0, st>>>(ix->keys, ix->n_sites, i, j, hist_s);
+        k_ot_hist<<<grid(n), 256, 0, st>>>(d_keys, n, i, j, hist_q);
+        k_ot_scan<<<3, kOtScanThreads, 0, st>>>(sa);
+        k_ot_scatter<<<grid(ix->n_sites), 256, 0, st>>>(ix->keys, ix->n_sites, i, j, sa.cursor[0], d_sites, nullptr);
+        k_ot_scatter<<<grid(n), 256, 0, st>>>(d_keys, n, i, j, sa.cursor[1], nullptr, d_q);
+        k_ot_count<<<(unsigned)g_ctx.sm_count * 8, kOtThreads, 0, st>>>(ca);
+        g_ctx.launches += 6;
+        if (cudaGetLastError() != cudaSuccess) rc = fail(CRP_ERR_CUDA, "off-target launch failed");
+    }
+    if (!rc && (cudaEventRecord(ix->ev[3], st) != cudaSuccess ||
+                cudaMemcpyAsync(misc, d_misc, sizeof misc, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+                cudaStreamSynchronize(st) != cudaSuccess ||
+                cudaEventElapsedTime(&ix->ms_count, ix->ev[2], ix->ev[3]) != cudaSuccess))
+        rc = fail(CRP_ERR_CUDA, "off-target count failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (!rc && misc[1]) rc = fail(CRP_ERR_RANGE, "a part pair needs 2^32 work items or more");
+    if (!rc) ix->comparisons = misc[0];
+    dev_free(d_tbl, st);
+    dev_free(d_sites, st);
+    dev_free(d_q, st);
+    dev_free(d_misc, st);
+    return rc;
+}
+
+extern "C" {
+
+int crp_offtarget_new(crp_offtarget **ix) {
+    if (!ix) return fail(CRP_ERR_ARG, "ix is NULL");
+    if (int rc = need_ctx()) return rc;
+    crp_offtarget *o = new (std::nothrow) crp_offtarget();
+    if (!o) return fail(CRP_ERR_NOMEM, "out of host memory");
+    if (cudaStreamCreateWithFlags(&o->st, cudaStreamNonBlocking) != cudaSuccess) {
+        delete o;
+        return fail(CRP_ERR_CUDA, "cudaStreamCreate failed");
+    }
+    for (int i = 0; i < 5; ++i)
+        if (cudaEventCreateWithFlags(&o->ev[i], i == 4 ? cudaEventDisableTiming : cudaEventDefault) != cudaSuccess) {
+            crp_offtarget_free(o);
+            return fail(CRP_ERR_CUDA, "cudaEventCreate failed");
+        }
+    *ix = o;
+    return 0;
+}
+
+int crp_offtarget_add_genome(crp_offtarget *ix, const crp_genome *g) {
+    if (!ix || !g) return fail(CRP_ERR_ARG, "NULL argument");
+    if (int rc = need_ctx()) return rc;
+    if (!g->committed) return fail(CRP_ERR_STATE, "genome is not committed");
+    if (std::find(ix->genomes.begin(), ix->genomes.end(), g) != ix->genomes.end())
+        return fail(CRP_ERR_STATE, "genome already added to this index");
+    cudaStream_t st = ix->st;
+    CUDA_TRY(cudaEventRecord(ix->ev[4], stream_of(g)));        // the records are written on the genome's stream
+    CUDA_TRY(cudaStreamWaitEvent(st, ix->ev[4], 0));
+    const uint64_t items = (uint64_t)g->n_tiles * kTileWords;
+    unsigned long long *d_n = nullptr, *h_n = static_cast<unsigned long long *>(pinned_get(sizeof(unsigned long long)));
+    if (!h_n) return fail(CRP_ERR_NOMEM, "cudaHostAlloc failed");
+    CUDA_TRY(dev_alloc(&d_n, sizeof(unsigned long long), st));
+    OtSiteArgs a;
+    a.records = g->records;
+    a.n_tiles = g->n_tiles;
+    a.keys = nullptr;
+    a.base = ix->n_sites;
+    a.n = d_n;
+    int rc = 0;
+    *h_n = 0;
+    // pass 1 counts, pass 2 appends behind the sites already held (the key array grows by one copy)
+    if (cudaEventRecord(ix->ev[0], st) != cudaSuccess || cudaMemsetAsync(d_n, 0, sizeof *d_n, st) != cudaSuccess)
+        rc = fail(CRP_ERR_CUDA, "off-target setup failed");
+    if (!rc && items) {
+        k_ot_sites<<<(unsigned)((items + 255) / 256), 256, 0, st>>>(a);
+        g_ctx.launches++;
+    }
+    if (!rc && (cudaMemcpyAsync(h_n, d_n, sizeof *d_n, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+                cudaStreamSynchronize(st) != cudaSuccess))
+        rc = fail(CRP_ERR_CUDA, "site count failed: %s", cudaGetErrorString(cudaGetLastError()));
+    const uint64_t add = *h_n, total = ix->n_sites + add;
+    if (!rc && total > 0xFFFFFFFFull) rc = fail(CRP_ERR_RANGE, "%llu sites exceed 2^32 - 1", (unsigned long long)total);
+    if (!rc && add) {
+        unsigned long long *keys = nullptr;
+        if (dev_alloc(&keys, total * sizeof(unsigned long long), st) != cudaSuccess) {
+            cudaGetLastError();
+            rc = fail(CRP_ERR_NOMEM, "cudaMalloc of %llu site keys failed", (unsigned long long)total);
+        } else {
+            if (ix->n_sites && cudaMemcpyAsync(keys, ix->keys, ix->n_sites * sizeof(unsigned long long), cudaMemcpyDeviceToDevice,
+                                               st) != cudaSuccess)
+                rc = fail(CRP_ERR_CUDA, "copy of the site keys failed");
+            dev_free(ix->keys, st);
+            ix->keys = keys;
+            a.keys = keys;
+            if (!rc && cudaMemsetAsync(d_n, 0, sizeof *d_n, st) != cudaSuccess) rc = fail(CRP_ERR_CUDA, "memset failed");
+            if (!rc) {
+                k_ot_sites<<<(unsigned)((items + 255) / 256), 256, 0, st>>>(a);
+                g_ctx.launches++;
+            }
+            if (!rc && (cudaMemcpyAsync(h_n, d_n, sizeof *d_n, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+                        cudaEventRecord(ix->ev[1], st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess))
+                rc = fail(CRP_ERR_CUDA, "site keys failed: %s", cudaGetErrorString(cudaGetLastError()));
+            if (!rc && *h_n != add) rc = fail(CRP_ERR_STATE, "site passes disagree (%llu, %llu)", (unsigned long long)add, *h_n);
+            if (rc) {                          // the old keys went with the old array: the index is emptied
+                dev_free(ix->keys, st);
+                ix->keys = nullptr;
+                ix->n_sites = 0;
+                ix->genomes.clear();
+            }
+        }
+    } else if (!rc) {
+        rc = cudaEventRecord(ix->ev[1], st) == cudaSuccess && cudaEventSynchronize(ix->ev[1]) == cudaSuccess
+                 ? 0 : fail(CRP_ERR_CUDA, "event failed");
+    }
+    float ms = 0.f;
+    if (!rc && cudaEventElapsedTime(&ms, ix->ev[0], ix->ev[1]) == cudaSuccess) ix->ms_sites += ms;
+    if (!rc) {
+        ix->n_sites = total;
+        ix->genomes.push_back(g);
+    }
+    dev_free(d_n, st);
+    pinned_put(h_n);
+    return rc;
+}
+
+int crp_offtarget_num_sites(const crp_offtarget *ix, uint64_t *n) {
+    if (!ix || !n) return fail(CRP_ERR_ARG, "NULL argument");
+    *n = ix->n_sites;
+    return 0;
+}
+
+int crp_offtarget_fetch_sites(const crp_offtarget *ix, uint64_t capacity, uint64_t *keys, uint64_t *n) {
+    if (!ix || !n) return fail(CRP_ERR_ARG, "NULL argument");
+    *n = ix->n_sites;
+    if (capacity < ix->n_sites) return fail(CRP_ERR_RANGE, "%llu sites, room for %llu", (unsigned long long)ix->n_sites,
+                                            (unsigned long long)capacity);
+    if (!ix->n_sites) return 0;
+    if (!keys) return fail(CRP_ERR_ARG, "keys is NULL");
+    CUDA_TRY(cudaMemcpyAsync(keys, ix->keys, ix->n_sites * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->st));
+    CUDA_TRY(cudaStreamSynchronize(ix->st));
+    return 0;
+}
+
+int crp_offtarget_count_candidates(crp_offtarget *ix, const crp_result *res, char strand, uint32_t max_mm, uint32_t *counts) {
+    if (!ix || !res) return fail(CRP_ERR_ARG, "NULL argument");
+    if (int rc = need_ctx()) return rc;
+    if (strand != '+' && strand != '-') return fail(CRP_ERR_ARG, "strand must be '+' or '-'");
+    if (max_mm > 3) return fail(CRP_ERR_ARG, "max_mm %u: at most 3 mismatches", max_mm);
+    if (res->guide_len != 20) return fail(CRP_ERR_STATE, "off-target counts are defined for guide_len 20 only");
+    const crp_genome *g = res->g;
+    if (std::find(ix->genomes.begin(), ix->genomes.end(), g) == ix->genomes.end())
+        return fail(CRP_ERR_STATE, "the result's genome has not been added to the index");
+    const int s = strand == '+' ? 0 : 1;
+    const uint64_t n = s == 0 ? res->n_plus : res->n_minus;
+    if (n == 0) return 0;
+    if (!counts) return fail(CRP_ERR_ARG, "counts is NULL");
+    const std::vector<uint64_t> &cnt = s == 0 ? res->seg_plus : res->seg_minus;
+    const uint32_t n_seg = (uint32_t)cnt.size();
+    std::vector<uint32_t> seg(3 * (size_t)n_seg + 1);         // row offsets [n_seg + 1], first tiles, first positions
+    uint64_t row = 0;
+    for (uint32_t i = 0; i < n_seg; ++i) {
+        seg[i] = (uint32_t)row;
+        row += cnt[i];
+        seg[n_seg + 1 + i] = g->segs[i].first_tile;
+        seg[2 * (size_t)n_seg + 1 + i] = (uint32_t)g->segs[i].begin;
+    }
+    seg[n_seg] = (uint32_t)row;
+    cudaStream_t st = ix->st;
+    CUDA_TRY(cudaEventRecord(ix->ev[4], res->st));             // the candidate streams are written on the scan's stream
+    CUDA_TRY(cudaStreamWaitEvent(st, ix->ev[4], 0));
+    const uint32_t k1 = max_mm + 1;
+    uint32_t *d_seg = nullptr, *d_counts = nullptr;
+    unsigned long long *d_keys = nullptr;
+    if (dev_alloc(&d_seg, seg.size() * sizeof(uint32_t), st) != cudaSuccess ||
+        dev_alloc(&d_keys, n * sizeof(unsigned long long), st) != cudaSuccess ||
+        dev_alloc(&d_counts, n * k1 * sizeof(uint32_t), st) != cudaSuccess) {
+        cudaGetLastError();
+        dev_free(d_seg, st);
+        dev_free(d_keys, st);
+        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu query rows failed", (unsigned long long)n);
+    }
+    int rc = 0;
+    if (cudaMemcpyAsync(d_seg, seg.data(), seg.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
+        rc = fail(CRP_ERR_CUDA, "H2D of the segment table failed");
+    if (!rc) {
+        OtQueryArgs a;
+        a.records = g->records;
+        a.pos = res->pos[s];
+        a.n = n;
+        a.seg_row = d_seg;
+        a.seg_tile = d_seg + n_seg + 1;
+        a.seg_begin = d_seg + 2 * (size_t)n_seg + 1;
+        a.n_seg = n_seg;
+        a.k1 = k1;
+        a.minus = s;
+        a.keys = d_keys;
+        a.counts = d_counts;
+        k_ot_queries<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a);
+        g_ctx.launches++;
+        rc = ot_count(ix, d_keys, n, max_mm, d_counts);
+    }
+    if (!rc && (cudaMemcpyAsync(counts, d_counts, n * k1 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+                cudaStreamSynchronize(st) != cudaSuccess))
+        rc = fail(CRP_ERR_CUDA, "D2H of the off-target counts failed");
+    dev_free(d_seg, st);
+    dev_free(d_keys, st);
+    dev_free(d_counts, st);
+    return rc;
+}
+
+int crp_offtarget_count_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys, uint32_t max_mm, uint32_t *counts) {
+    if (!ix) return fail(CRP_ERR_ARG, "ix is NULL");
+    if (int rc = need_ctx()) return rc;
+    if (max_mm > 3) return fail(CRP_ERR_ARG, "max_mm %u: at most 3 mismatches", max_mm);
+    if (n == 0) return 0;
+    if (!keys || !counts) return fail(CRP_ERR_ARG, "NULL argument");
+    if (n > 0xFFFFFFFFull) return fail(CRP_ERR_RANGE, "at most 2^32 - 1 keys per call");
+    for (uint64_t i = 0; i < n; ++i)
+        if (keys[i] >> 40) return fail(CRP_ERR_ARG, "key %llu has bits above bit 39", (unsigned long long)i);
+    cudaStream_t st = ix->st;
+    const uint32_t k1 = max_mm + 1;
+    unsigned long long *d_keys = nullptr;
+    uint32_t *d_counts = nullptr;
+    if (dev_alloc(&d_keys, n * sizeof(unsigned long long), st) != cudaSuccess ||
+        dev_alloc(&d_counts, n * k1 * sizeof(uint32_t), st) != cudaSuccess) {
+        cudaGetLastError();
+        dev_free(d_keys, st);
+        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu keys failed", (unsigned long long)n);
+    }
+    int rc = 0;
+    if (cudaMemcpyAsync(d_keys, keys, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemsetAsync(d_counts, 0, n * k1 * sizeof(uint32_t), st) != cudaSuccess)
+        rc = fail(CRP_ERR_CUDA, "H2D of the keys failed");
+    if (!rc) rc = ot_count(ix, d_keys, n, max_mm, d_counts);
+    if (!rc && (cudaMemcpyAsync(counts, d_counts, n * k1 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+                cudaStreamSynchronize(st) != cudaSuccess))
+        rc = fail(CRP_ERR_CUDA, "D2H of the off-target counts failed");
+    dev_free(d_keys, st);
+    dev_free(d_counts, st);
+    return rc;
+}
+
+int crp_offtarget_timing(const crp_offtarget *ix, float *ms_sites, float *ms_count, uint64_t *comparisons) {
+    if (!ix) return fail(CRP_ERR_ARG, "ix is NULL");
+    if (ms_sites) *ms_sites = ix->ms_sites;
+    if (ms_count) *ms_count = ix->ms_count;
+    if (comparisons) *comparisons = ix->comparisons;
+    return 0;
+}
+
+int crp_offtarget_free(crp_offtarget *ix) {
+    if (!ix) return 0;
+    if (ix->st) {
+        dev_free(ix->keys, ix->st);
+        cudaStreamSynchronize(ix->st);
+    }
+    for (cudaEvent_t e : ix->ev)
+        if (e) cudaEventDestroy(e);
+    if (ix->st) cudaStreamDestroy(ix->st);
+    delete ix;
+    return 0;
 }
 
 }  // extern "C"

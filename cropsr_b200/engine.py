@@ -543,3 +543,88 @@ class ScanResult:
             self.free()
         except Exception:
             pass
+
+
+_GUIDE_CODE = np.full(256, 255, dtype=np.uint8)
+for _i, _c in enumerate(b"ATCG"):
+    _GUIDE_CODE[_c] = _GUIDE_CODE[_c | 0x20] = _i
+
+
+def guide_keys(guides):
+    """20-base guides (ACGTacgt, the orientation followed by NGG in the genome) -> uint64 keys:
+    base i (A0 T1 C2 G3) in bits 2i, 2i+1.  ValueError for anything else."""
+    keys = np.zeros(len(guides), dtype=np.uint64)
+    for n, g in enumerate(guides):
+        b = np.frombuffer(g.encode("ascii") if isinstance(g, str) else bytes(g), dtype=np.uint8)
+        code = _GUIDE_CODE[b]
+        if len(b) != 20 or (code == 255).any():
+            raise ValueError(f"guide {g!r}: 20 characters of ACGTacgt expected")
+        keys[n] = int((code.astype(np.uint64) << (2 * np.arange(20, dtype=np.uint64))).sum())
+    return keys
+
+
+class OffTargetIndex:
+    """NGG sites (both strands, case-insensitive) of one or more committed genomes, resident in HBM:
+    counts of sites within 0 .. k <= 3 mismatches of every scan candidate or of arbitrary guides
+    (semantics: include/cropsr_b200.h, csrc/offtarget.cuh)."""
+
+    NO_COUNT = N.OFFTARGET_NO_COUNT
+
+    def __init__(self, genomes=()):
+        if _device is None:
+            init(0)
+        self._h = C.c_void_p()
+        check(lib.crp_offtarget_new(C.byref(self._h)))
+        for g in genomes:
+            self.add_genome(g)
+
+    def add_genome(self, genome):
+        check(lib.crp_offtarget_add_genome(self._h, genome._h))
+
+    def num_sites(self):
+        n = C.c_uint64(0)
+        check(lib.crp_offtarget_num_sites(self._h, C.byref(n)))
+        return n.value
+
+    def sites(self):
+        """uint64 keys of every site, in no particular order"""
+        n = self.num_sites()
+        out = np.empty(n, dtype=np.uint64)
+        got = C.c_uint64(0)
+        check(lib.crp_offtarget_fetch_sites(self._h, n, out.ctypes.data if n else None, C.byref(got)))
+        return out
+
+    def count_candidates(self, result, strand, k=3):
+        """uint32[n_strand, k + 1]: sites at exactly d mismatches of every candidate of one strand stream
+        (stream order, the candidate's own site not counted); rows of NO_COUNT where the candidate has
+        no protospacer (cut off by the token end, or a byte outside ACGTacgt)."""
+        n = int(result.n_plus if strand == "+" else result.n_minus)
+        out = np.empty((n, int(k) + 1), dtype=np.uint32)
+        check(lib.crp_offtarget_count_candidates(self._h, result._h, strand.encode(), int(k),
+                                                 out.ctypes.data if n else None))
+        return out
+
+    def count_guides(self, guides, k=3):
+        """uint32[len(guides), k + 1] for 20-base guides in the protospacer orientation; nothing subtracted"""
+        keys = guide_keys(guides)
+        out = np.empty((len(keys), int(k) + 1), dtype=np.uint32)
+        if len(keys):
+            check(lib.crp_offtarget_count_keys(self._h, len(keys), keys.ctypes.data, int(k), out.ctypes.data))
+        return out
+
+    def timing(self):
+        """dict(ms_sites: every add_genome, ms_count and comparisons: the last count call)"""
+        a, b, n = C.c_float(0), C.c_float(0), C.c_uint64(0)
+        check(lib.crp_offtarget_timing(self._h, C.byref(a), C.byref(b), C.byref(n)))
+        return {"ms_sites": a.value, "ms_count": b.value, "comparisons": n.value}
+
+    def free(self):
+        if self._h:
+            check(lib.crp_offtarget_free(self._h))
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass

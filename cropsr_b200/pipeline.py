@@ -266,12 +266,79 @@ def write_gap_table(path, tokens, scan, min_len=10):
             w.writerows((key[1:], int(a), int(b)) for a, b in zip(start.tolist(), length.tolist()))
 
 
+_DNA = np.frombuffer(b"ATCG", dtype=np.uint8)
+
+
+def write_offtarget_table(path, tokens, scan, k=3):
+    """Opt-in off-target table (not part of the reference's output): one row per unique candidate in
+    reference order (token by token, '+' then '-', ascending t) with its protospacer as upper-case DNA
+    in the orientation followed by the PAM, and the numbers of OTHER NGG sites of the whole genome at
+    exactly 0 .. k mismatches (k_ot_* kernels; semantics in oracle/offtarget_oracle.py).  Protospacer
+    and counts are blank where the candidate has none (cut off by the token end, or a byte outside
+    ACGTacgt).  One index is built from every genome handle of the scan before anything is counted:
+    handles split at MAX_POSITIONS_PER_GENOME see each other's sites."""
+    import csv
+    import pandas as pd
+    keys = list(tokens.keys())
+    columns = ["chromosome", "strand", "pam_pos", "protospacer"] + [f"mm{d}" for d in range(k + 1)]
+    with open(path, "w", newline="") as f:
+        csv.writer(f, delimiter="\t").writerow(columns)
+    index = engine.OffTargetIndex([g for g, _, _, _ in scan.parts])
+    try:
+        for genome, result, first, cnt in scan.parts:
+            cols = {}
+            for strand, seg_cnt in (("+", result.seg_plus), ("-", result.seg_minus)):
+                seg_of = np.repeat(np.arange(cnt, dtype=np.int64), seg_cnt.astype(np.int64))
+                n = len(seg_of)
+                pos = result.fetch(strand, want=("pos",))["pos"]
+                counts = index.count_candidates(result, strand, k)
+                ok = counts[:, 0] != index.NO_COUNT if n else np.zeros(0, bool)
+                proto = np.full(n, "", dtype=object)
+                if ok.any():
+                    # the protospacer from the host token: '+' tok[t-20:t], '-' the reverse complement of tok[t+3:t+23]
+                    rows = []
+                    for s, t in zip(seg_of[ok].tolist(), pos[ok].tolist()):
+                        tok = scan.token_bytes[first + s]
+                        rows.append(tok[t - 20:t] if strand == "+" else tok[t + 3:t + 23][::-1])
+                    b = np.frombuffer(b"".join(rows), dtype=np.uint8).reshape(-1, 20) & 0xDF   # upper case
+                    if strand == "-":
+                        b = np.select([b == 65, b == 84, b == 67, b == 71], [84, 65, 71, 67]).astype(np.uint8)
+                    proto[ok] = b.view("S20").ravel().astype("U20").astype(object)
+                frame = {"chromosome": np.array([key[1:] for key in keys[first:first + cnt]], dtype=object)[seg_of]
+                         if n else np.empty(0, object),
+                         "strand": strand, "pam_pos": pos.astype(np.int64), "protospacer": proto}
+                for d in range(k + 1):
+                    frame[f"mm{d}"] = np.where(ok, counts[:, d].astype(np.int64).astype(str).astype(object), "") if n \
+                        else np.empty(0, object)
+                cols[strand] = (seg_of, pd.DataFrame(frame, columns=columns))
+            frame = pd.concat([cols["+"][1], cols["-"][1]], ignore_index=True)
+            order = np.argsort(np.concatenate((2 * cols["+"][0], 2 * cols["-"][0] + 1)), kind="stable")
+            frame.iloc[order].to_csv(path, sep="\t", mode="a", header=False, index=False, lineterminator="\r\n")
+    finally:
+        index.free()
+
+
+def check_offtarget_args(guide_len, devices, max_mismatches):
+    """The off-target table's limits, checked before any device work: ValueError with the reason."""
+    if int(guide_len) != 20:
+        raise ValueError(f"off-target counts are defined for 20-base guides, not -l {guide_len}")
+    if devices is not None and len(devices) > 1:
+        raise ValueError("off-target counts run on one GPU: the index needs every site of the genome on one device; "
+                         "run without --devices, or with one device")
+    if int(max_mismatches) not in (0, 1, 2, 3):
+        raise ValueError(f"--mismatches {max_mismatches}: 0 to 3 mismatches are supported")
+
+
 def run_cas9(fasta, gff, output="data.csv", guide_len=20, verbose=False, blas_threads=1,
              time_path="time.txt", out=print, side_output=None, flank=200, device_ingest=True, annotation_info=None,
-             chunk_rows=None, devices=None, handle_limit=None):
+             chunk_rows=None, devices=None, handle_limit=None, offtargets=None, max_mismatches=3):
     """devices: CUDA ordinals; more than one shards the genome over one process per GPU
     (cropsr_b200/multi.py) and writes the same CSV.  handle_limit: positions per genome handle
-    (tests shrink it to walk the several-handles path on small inputs)."""
+    (tests shrink it to walk the several-handles path on small inputs).  offtargets: path of the opt-in
+    off-target table (write_offtarget_table, guide length 20 on one GPU), written after the CSV with
+    counts at 0 .. max_mismatches."""
+    if offtargets is not None:
+        check_offtarget_args(guide_len, devices, max_mismatches)
     begin = time.time()
     timing = open(time_path, "w")                       # CROPSR.py:371
     multi_gpu = devices is not None and len(devices) > 1
@@ -324,6 +391,8 @@ def run_cas9(fasta, gff, output="data.csv", guide_len=20, verbose=False, blas_th
             formatted_path = ingest.needs_formatting(f.read())
         write_side_output(side_output, tokens, scan, gff_frame, flank, formatted_path, annotation_info)
         write_gap_table(side_output + ".gaps.tsv", tokens, scan)
+    if offtargets is not None:
+        write_offtarget_table(offtargets, tokens, scan, max_mismatches)
     stats = {"tokens": len(tokens), "candidates": len(table), "rows": rows_written,
              "scan_ms": scan.scan_ms(), **scan.timing()}
     t_plus = x_plus = t_minus = x_minus = None          # views into the scan's row arrays

@@ -337,6 +337,38 @@ int crp_rs1_score(uint64_t n, const uint8_t *rows, const uint8_t *cls, double *s
  * (a host that holds the tokens re-sums the few non-canonical rows of a slice without a genome handle). */
 int crp_rs1_preactivation(uint64_t n, const uint8_t *rows, const uint8_t *cls, double *x);
 
+/* ---- off-target counts (opt-in; the reference has none: its nearest relative is the bowtie2 call of
+ * /root/reference/prmrdsgn2.py:139-160, which aligns primers with an external aligner).  An index holds the
+ * 40-bit protospacer keys of every NGG site, both strands, case-insensitive, of every genome handle added
+ * to it; the counts of a query are the numbers of sites at exactly d = 0 .. max_mm mismatches (max_mm <= 3),
+ * found by exact pigeonhole filtering on the device.  Semantics in csrc/offtarget.cuh and
+ * oracle/offtarget_oracle.py:
+ *   site '+' at t   tok[t+1], tok[t+2] in {G, g}, tok[t-20 .. t) all of ACGTacgt; P = tok[t-20 .. t)
+ *   site '-' at t   tok[t], tok[t+1] in {C, c}, tok[t+3 .. t+23) all of ACGTacgt; P = revcomp(tok[t+3 .. t+23))
+ *   key             base P[i] (code A0 T1 C2 G3, case folded) in bits 2i, 2i+1; P[0] is the PAM-distal base
+ * Positions are token coordinates; the index is built on its own stream, ordered behind each genome's. */
+typedef struct crp_offtarget crp_offtarget;
+int crp_offtarget_new(crp_offtarget **ix);
+/* The genome must be committed; its site keys are copied (the genome may be freed afterwards, but a
+ * result of it can only be counted while both live).  CRP_ERR_RANGE beyond 2^32 - 1 sites in all. */
+int crp_offtarget_add_genome(crp_offtarget *ix, const crp_genome *g);
+int crp_offtarget_num_sites(const crp_offtarget *ix, uint64_t *n);
+/* All site keys, in no particular order; CRP_ERR_RANGE (and *n) if capacity is too small. */
+int crp_offtarget_fetch_sites(const crp_offtarget *ix, uint64_t capacity, uint64_t *keys, uint64_t *n);
+/* Counts of every candidate of one strand stream of a scan whose genome was added (CRP_ERR_STATE otherwise,
+ * and for guide_len != 20): counts[i * (max_mm + 1) + d], stream order, the candidate's own site not counted.
+ * A candidate whose protospacer is cut off by the token end or holds a byte outside ACGTacgt has no
+ * counts: max_mm + 1 times 0xFFFFFFFF. */
+int crp_offtarget_count_candidates(crp_offtarget *ix, const crp_result *res, char strand, uint32_t max_mm,
+                                   uint32_t *counts /* [n_strand][max_mm + 1] */);
+/* The same for arbitrary protospacer keys (< 2^40; user guides in the orientation followed by NGG in the
+ * genome); nothing is subtracted. */
+int crp_offtarget_count_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys, uint32_t max_mm, uint32_t *counts);
+/* ms_sites: device time of every add_genome; ms_count and comparisons (sum over the 10 part pairs and the
+ * 65,536 buckets of queries x sites) of the last count call. */
+int crp_offtarget_timing(const crp_offtarget *ix, float *ms_sites, float *ms_count, uint64_t *comparisons);
+int crp_offtarget_free(crp_offtarget *ix);
+
 /* Kernel timings (CUDA events on the library stream) of the last commit /
  * scan: milliseconds. */
 int crp_genome_timing(const crp_genome *g, float *ms_h2d, float *ms_pack);
