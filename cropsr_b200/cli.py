@@ -9,8 +9,8 @@ def build_parser():
     # the usage line is spelled out: with the reference's empty metavars argparse cannot wrap a usage
     # line of this length (its own consistency assertion fails), and --help would crash
     p = argparse.ArgumentParser(prog="CROPSR.py", usage="CROPSR.py [-h] -f FASTA [-g GFF] [-p TXT] [-o CSV] [-l 20] [-L 200] --cas9 [-v]\n"
-                                "                 [--device N | --devices 0-7] [--side-output TSV] [--offtargets TSV [--mismatches K]]\n"
-                                "                 [--blas-threads N]")
+                                "                 [--device N | --devices 0-7] [--side-output TSV] [--offtargets TSV] [--offtarget-sites TSV]\n"
+                                "                 [--mismatches K] [--max-sites N] [--blas-threads N]")
     p.add_argument("-f", "--fasta", metavar="", required=True, dest="f",
                    help="[required] path to input file in FASTA format")
     p.add_argument("-g", "--gff", metavar="", dest="g", help="path to input file in GFF format")
@@ -39,8 +39,16 @@ def build_parser():
                    help="also write a tab-separated table of off-target counts: per candidate its protospacer and the "
                         "number of other NGG sites of the genome (both strands, any case) at exactly 0 .. K mismatches; "
                         "-l 20 on one GPU only; the CSV is unaffected")
+    p.add_argument("--offtarget-sites", metavar="", default=None,
+                   help="also write a tab-separated table of off-target sites: one row per candidate and other NGG site "
+                        "of the genome within K mismatches, with the site's chromosome, strand, position and protospacer "
+                        "(differing bases in lower case); candidates with more than --max-sites such sites are left out "
+                        "(their counts are in --offtargets); -l 20 on one GPU only; the CSV is unaffected")
     p.add_argument("--mismatches", metavar="", type=int, default=3,
-                   help="K of --offtargets: 0 to 3, default = 3")
+                   help="K of --offtargets and --offtarget-sites: 0 to 3, default = 3")
+    p.add_argument("--max-sites", metavar="", type=int, default=1000,
+                   help="--offtarget-sites lists the candidates with at most this many other sites within K "
+                        "mismatches: at least 1, default = 1000")
     p.add_argument("--blas-threads", type=int, default=1,
                    help="emulate the float summation order of the reference running with this many "
                         "OpenBLAS threads (default 1 = OPENBLAS_NUM_THREADS=1)")
@@ -85,15 +93,18 @@ def main(argv=None):
     if args.verbose:
         print(banner(args))
     devices = parse_devices(args.devices) if args.devices else [args.device]
-    if args.offtargets is not None:
+    if args.offtargets is not None or args.offtarget_sites is not None:
         from .pipeline import check_offtarget_args
         try:
-            check_offtarget_args(args.l, devices, args.mismatches)
+            check_offtarget_args(args.l, devices, args.mismatches,
+                                 args.max_sites if args.offtarget_sites is not None else None)
         except ValueError as e:
-            sys.exit(f"CROPSR.py: error: --offtargets: {e}")
+            flag = "--offtargets" if args.offtarget_sites is None else "--offtarget-sites"
+            sys.exit(f"CROPSR.py: error: {flag}: {e}")
     from . import engine, pipeline
     engine.init(devices[0])
     pipeline.run_cas9(args.f, args.g, args.o, args.l, args.verbose, args.blas_threads,
                       side_output=args.side_output, flank=args.L, annotation_info=args.p, devices=devices,
-                      offtargets=args.offtargets, max_mismatches=args.mismatches)
+                      offtargets=args.offtargets, max_mismatches=args.mismatches,
+                      offtarget_sites=args.offtarget_sites, max_sites=args.max_sites)
     return 0

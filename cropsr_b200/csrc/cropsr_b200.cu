@@ -31,7 +31,7 @@
 #include "extras.cuh"
 #include "offtarget.cuh"
 
-#define CRP_ABI_VERSION 8
+#define CRP_ABI_VERSION 9
 
 static constexpr size_t kScanSmemFixed = (size_t)kStages * kRecBytes + 2 * (size_t)kListCap * sizeof(uint16_t);
 
@@ -2073,21 +2073,26 @@ struct crp_offtarget {
     cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};   // sites start / end, count start / end, genome ready
     std::vector<const crp_genome *> genomes;
     unsigned long long *keys = nullptr;        // site keys of every genome added, any order
+    unsigned long long *loci = nullptr;        // crp_offtarget_new_with_loci: the locus of every site, at its key's slot
+    bool with_loci = false;
     uint64_t n_sites = 0;
-    float ms_sites = 0.f, ms_count = 0.f;      // summed over add_genome / of the last count call
+    float ms_sites = 0.f, ms_count = 0.f;      // summed over add_genome / of the last count or list call
     uint64_t comparisons = 0;
 };
 
 // Count every query of d_keys (n rows, kOtInvalid = no counts) against the index's sites into d_counts
-// ([n][k + 1], primed by the caller), on ix->st; waits for the result.
-static int ot_count(crp_offtarget *ix, const unsigned long long *d_keys, uint64_t n, uint32_t k, uint32_t *d_counts) {
+// ([n][k + 1], primed by the caller), on ix->st; waits for the result.  list != NULL: list the pairs instead
+// (k_ot_list with the caller's own / first / cursor / out / overflow; the sites carry their index).
+static int ot_count(crp_offtarget *ix, const unsigned long long *d_keys, uint64_t n, uint32_t k, uint32_t *d_counts,
+                    const OtListArgs *list = nullptr) {
     cudaStream_t st = ix->st;
     const size_t tbl = kOtBuckets + 1;
     uint32_t *d_tbl = nullptr, *d_sites = nullptr;
     uint2 *d_q = nullptr;
     unsigned long long *d_misc = nullptr;      // [0] comparisons, [1] overflow flag
+    const size_t site_bytes = list ? sizeof(uint2) : sizeof(uint32_t);
     if (dev_alloc(&d_tbl, 7 * tbl * sizeof(uint32_t), st) != cudaSuccess ||
-        dev_alloc(&d_sites, (ix->n_sites + 8) * sizeof(uint32_t), st) != cudaSuccess ||
+        dev_alloc(&d_sites, (ix->n_sites + 8) * site_bytes, st) != cudaSuccess ||
         dev_alloc(&d_q, (n + 1) * sizeof(uint2), st) != cudaSuccess ||
         dev_alloc(&d_misc, 2 * sizeof(unsigned long long), st) != cudaSuccess) {
         cudaGetLastError();
@@ -2115,6 +2120,17 @@ static int ot_count(crp_offtarget *ix, const unsigned long long *d_keys, uint64_
     ca.item_off = sa.item_off;
     ca.counts = d_counts;
     ca.k = k;
+    OtListArgs la = {};
+    if (list) {
+        la = *list;
+        la.sites = reinterpret_cast<const uint2 *>(d_sites);
+        la.queries = d_q;
+        la.soff = sa.off[0];
+        la.qoff = sa.off[1];
+        la.item_off = sa.item_off;
+        la.loci = ix->loci;
+        la.k = k;
+    }
     auto grid = [](uint64_t items) { return (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((items + 255) / 256, (uint64_t)g_ctx.sm_count * 16)); };
     int rc = 0;
     unsigned long long misc[2] = {0, 0};
@@ -2132,9 +2148,18 @@ static int ot_count(crp_offtarget *ix, const unsigned long long *d_keys, uint64_
         k_ot_hist<<<grid(ix->n_sites), 256, 0, st>>>(ix->keys, ix->n_sites, i, j, hist_s);
         k_ot_hist<<<grid(n), 256, 0, st>>>(d_keys, n, i, j, hist_q);
         k_ot_scan<<<3, kOtScanThreads, 0, st>>>(sa);
-        k_ot_scatter<<<grid(ix->n_sites), 256, 0, st>>>(ix->keys, ix->n_sites, i, j, sa.cursor[0], d_sites, nullptr);
+        if (list)                              // {rest key, site index}: the query form of the scatter
+            k_ot_scatter<<<grid(ix->n_sites), 256, 0, st>>>(ix->keys, ix->n_sites, i, j, sa.cursor[0], nullptr,
+                                                             reinterpret_cast<uint2 *>(d_sites));
+        else
+            k_ot_scatter<<<grid(ix->n_sites), 256, 0, st>>>(ix->keys, ix->n_sites, i, j, sa.cursor[0], d_sites, nullptr);
         k_ot_scatter<<<grid(n), 256, 0, st>>>(d_keys, n, i, j, sa.cursor[1], nullptr, d_q);
-        k_ot_count<<<(unsigned)g_ctx.sm_count * 8, kOtThreads, 0, st>>>(ca);
+        if (list) {
+            la.jm1 = ca.jm1;
+            k_ot_list<<<(unsigned)g_ctx.sm_count * 8, kOtThreads, 0, st>>>(la);
+        } else {
+            k_ot_count<<<(unsigned)g_ctx.sm_count * 8, kOtThreads, 0, st>>>(ca);
+        }
         g_ctx.launches += 6;
         if (cudaGetLastError() != cudaSuccess) rc = fail(CRP_ERR_CUDA, "off-target launch failed");
     }
@@ -2172,12 +2197,22 @@ int crp_offtarget_new(crp_offtarget **ix) {
     return 0;
 }
 
+int crp_offtarget_new_with_loci(crp_offtarget **ix) {
+    if (int rc = crp_offtarget_new(ix)) return rc;
+    (*ix)->with_loci = true;
+    return 0;
+}
+
 int crp_offtarget_add_genome(crp_offtarget *ix, const crp_genome *g) {
     if (!ix || !g) return fail(CRP_ERR_ARG, "NULL argument");
     if (int rc = need_ctx()) return rc;
     if (!g->committed) return fail(CRP_ERR_STATE, "genome is not committed");
     if (std::find(ix->genomes.begin(), ix->genomes.end(), g) != ix->genomes.end())
         return fail(CRP_ERR_STATE, "genome already added to this index");
+    if (ix->with_loci && g->segs.size() >= kOtMaxSegments)
+        return fail(CRP_ERR_RANGE, "%zu segments: a locus holds 24 bits of segment index", g->segs.size());
+    if (ix->with_loci && ix->genomes.size() >= kOtMaxGenomes)
+        return fail(CRP_ERR_RANGE, "an index with loci takes at most %u genome handles", kOtMaxGenomes);
     cudaStream_t st = ix->st;
     CUDA_TRY(cudaEventRecord(ix->ev[4], stream_of(g)));        // the records are written on the genome's stream
     CUDA_TRY(cudaStreamWaitEvent(st, ix->ev[4], 0));
@@ -2191,13 +2226,15 @@ int crp_offtarget_add_genome(crp_offtarget *ix, const crp_genome *g) {
     a.keys = nullptr;
     a.base = ix->n_sites;
     a.n = d_n;
+    a.loci = nullptr;
+    a.genome = (uint32_t)ix->genomes.size();
     int rc = 0;
     *h_n = 0;
-    // pass 1 counts, pass 2 appends behind the sites already held (the key array grows by one copy)
+    // pass 1 counts, pass 2 appends behind the sites already held (the key and locus arrays grow by one copy)
     if (cudaEventRecord(ix->ev[0], st) != cudaSuccess || cudaMemsetAsync(d_n, 0, sizeof *d_n, st) != cudaSuccess)
         rc = fail(CRP_ERR_CUDA, "off-target setup failed");
     if (!rc && items) {
-        k_ot_sites<<<(unsigned)((items + 255) / 256), 256, 0, st>>>(a);
+        k_ot_sites<false><<<(unsigned)((items + 255) / 256), 256, 0, st>>>(a);
         g_ctx.launches++;
     }
     if (!rc && (cudaMemcpyAsync(h_n, d_n, sizeof *d_n, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
@@ -2206,20 +2243,31 @@ int crp_offtarget_add_genome(crp_offtarget *ix, const crp_genome *g) {
     const uint64_t add = *h_n, total = ix->n_sites + add;
     if (!rc && total > 0xFFFFFFFFull) rc = fail(CRP_ERR_RANGE, "%llu sites exceed 2^32 - 1", (unsigned long long)total);
     if (!rc && add) {
-        unsigned long long *keys = nullptr;
-        if (dev_alloc(&keys, total * sizeof(unsigned long long), st) != cudaSuccess) {
+        unsigned long long *keys = nullptr, *loci = nullptr;
+        if (dev_alloc(&keys, total * sizeof(unsigned long long), st) != cudaSuccess ||
+            (ix->with_loci && dev_alloc(&loci, total * sizeof(unsigned long long), st) != cudaSuccess)) {
             cudaGetLastError();
+            dev_free(keys, st);
             rc = fail(CRP_ERR_NOMEM, "cudaMalloc of %llu site keys failed", (unsigned long long)total);
         } else {
             if (ix->n_sites && cudaMemcpyAsync(keys, ix->keys, ix->n_sites * sizeof(unsigned long long), cudaMemcpyDeviceToDevice,
                                                st) != cudaSuccess)
                 rc = fail(CRP_ERR_CUDA, "copy of the site keys failed");
+            if (!rc && loci && ix->n_sites &&
+                cudaMemcpyAsync(loci, ix->loci, ix->n_sites * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, st) != cudaSuccess)
+                rc = fail(CRP_ERR_CUDA, "copy of the site loci failed");
             dev_free(ix->keys, st);
+            dev_free(ix->loci, st);
             ix->keys = keys;
+            ix->loci = loci;
             a.keys = keys;
+            a.loci = loci;
             if (!rc && cudaMemsetAsync(d_n, 0, sizeof *d_n, st) != cudaSuccess) rc = fail(CRP_ERR_CUDA, "memset failed");
             if (!rc) {
-                k_ot_sites<<<(unsigned)((items + 255) / 256), 256, 0, st>>>(a);
+                if (loci)
+                    k_ot_sites<true><<<(unsigned)((items + 255) / 256), 256, 0, st>>>(a);
+                else
+                    k_ot_sites<false><<<(unsigned)((items + 255) / 256), 256, 0, st>>>(a);
                 g_ctx.launches++;
             }
             if (!rc && (cudaMemcpyAsync(h_n, d_n, sizeof *d_n, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
@@ -2228,7 +2276,9 @@ int crp_offtarget_add_genome(crp_offtarget *ix, const crp_genome *g) {
             if (!rc && *h_n != add) rc = fail(CRP_ERR_STATE, "site passes disagree (%llu, %llu)", (unsigned long long)add, *h_n);
             if (rc) {                          // the old keys went with the old array: the index is emptied
                 dev_free(ix->keys, st);
+                dev_free(ix->loci, st);
                 ix->keys = nullptr;
+                ix->loci = nullptr;
                 ix->n_sites = 0;
                 ix->genomes.clear();
             }
@@ -2365,6 +2415,217 @@ int crp_offtarget_count_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys
     return rc;
 }
 
+int crp_offtarget_fetch_loci(const crp_offtarget *ix, uint64_t capacity, uint64_t *loci, uint64_t *n) {
+    if (!ix || !n) return fail(CRP_ERR_ARG, "NULL argument");
+    if (!ix->with_loci) return fail(CRP_ERR_STATE, "the index keeps no loci (crp_offtarget_new_with_loci)");
+    *n = ix->n_sites;
+    if (capacity < ix->n_sites) return fail(CRP_ERR_RANGE, "%llu sites, room for %llu", (unsigned long long)ix->n_sites,
+                                            (unsigned long long)capacity);
+    if (!ix->n_sites) return 0;
+    if (!loci) return fail(CRP_ERR_ARG, "loci is NULL");
+    CUDA_TRY(cudaMemcpyAsync(loci, ix->loci, ix->n_sites * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->st));
+    CUDA_TRY(cudaStreamSynchronize(ix->st));
+    return 0;
+}
+
+}  // extern "C"
+
+// The listing of n queries whose keys (and own-site loci, or NULL) are on the device: slices `first` [n + 1] on the
+// host, site indices into `sites` [first[n]] on the host.  CRP_ERR_STATE, with nothing copied, if a row finds a
+// number of sites other than its slice holds.
+static int ot_list(crp_offtarget *ix, const unsigned long long *d_keys, const unsigned long long *d_own, uint64_t n,
+                   uint32_t k, const uint64_t *first, uint32_t *sites) {
+    cudaStream_t st = ix->st;
+    const uint64_t total = first[n];
+    unsigned long long *d_first = nullptr;
+    uint32_t *d_cursor = nullptr, *d_out = nullptr;
+    unsigned int *d_flag = nullptr;
+    if (dev_alloc(&d_first, (n + 1) * sizeof(unsigned long long), st) != cudaSuccess ||
+        dev_alloc(&d_cursor, n * sizeof(uint32_t), st) != cudaSuccess ||
+        dev_alloc(&d_out, std::max<uint64_t>(total, 1) * sizeof(uint32_t), st) != cudaSuccess ||
+        dev_alloc(&d_flag, sizeof(unsigned int), st) != cudaSuccess) {
+        cudaGetLastError();
+        dev_free(d_first, st);
+        dev_free(d_cursor, st);
+        dev_free(d_out, st);
+        return fail(CRP_ERR_NOMEM, "cudaMalloc of a listing of %llu sites failed", (unsigned long long)total);
+    }
+    int rc = 0;
+    if (cudaMemcpyAsync(d_first, first, (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemsetAsync(d_cursor, 0, n * sizeof(uint32_t), st) != cudaSuccess ||
+        cudaMemsetAsync(d_flag, 0, sizeof(unsigned int), st) != cudaSuccess)
+        rc = fail(CRP_ERR_CUDA, "listing setup failed");
+    if (!rc) {
+        OtListArgs la = {};
+        la.own = d_own;
+        la.first = d_first;
+        la.cursor = d_cursor;
+        la.out = d_out;
+        la.overflow = d_flag;
+        rc = ot_count(ix, d_keys, n, k, nullptr, &la);
+    }
+    std::vector<uint32_t> found(rc ? 0 : n);
+    unsigned int flag = 0;
+    if (!rc && (cudaMemcpyAsync(found.data(), d_cursor, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+                cudaMemcpyAsync(&flag, d_flag, sizeof flag, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+                cudaStreamSynchronize(st) != cudaSuccess))
+        rc = fail(CRP_ERR_CUDA, "D2H of the listing cursors failed");
+    for (uint64_t i = 0; i < n && !rc; ++i)
+        if (found[i] != first[i + 1] - first[i])
+            rc = fail(CRP_ERR_STATE, "row %llu: %u sites found, its slice holds %llu", (unsigned long long)i, found[i],
+                      (unsigned long long)(first[i + 1] - first[i]));
+    if (!rc && flag) rc = fail(CRP_ERR_STATE, "a row found more sites than its slice holds");
+    if (!rc && total && (cudaMemcpyAsync(sites, d_out, total * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+                         cudaStreamSynchronize(st) != cudaSuccess))
+        rc = fail(CRP_ERR_CUDA, "D2H of the listing failed");
+    dev_free(d_first, st);
+    dev_free(d_cursor, st);
+    dev_free(d_out, st);
+    dev_free(d_flag, st);
+    return rc;
+}
+
+// first [n + 1] of a listing call: CRP_ERR_ARG unless it starts at 0 and never decreases
+static int ot_check_first(uint64_t n, const uint64_t *first) {
+    if (!first) return fail(CRP_ERR_ARG, "first is NULL");
+    if (first[0] != 0) return fail(CRP_ERR_ARG, "first[0] must be 0");
+    for (uint64_t i = 0; i < n; ++i)
+        if (first[i + 1] < first[i]) return fail(CRP_ERR_ARG, "first[%llu] < first[%llu]", (unsigned long long)i + 1,
+                                                 (unsigned long long)i);
+    return 0;
+}
+
+extern "C" {
+
+int crp_offtarget_list_candidates(crp_offtarget *ix, const crp_result *res, char strand, uint32_t max_mm, uint64_t n_rows,
+                                  const uint32_t *rows, const uint64_t *first, uint32_t *sites) {
+    if (!ix || !res) return fail(CRP_ERR_ARG, "NULL argument");
+    if (int rc = need_ctx()) return rc;
+    if (strand != '+' && strand != '-') return fail(CRP_ERR_ARG, "strand must be '+' or '-'");
+    if (max_mm > 3) return fail(CRP_ERR_ARG, "max_mm %u: at most 3 mismatches", max_mm);
+    if (!ix->with_loci) return fail(CRP_ERR_STATE, "listing needs an index with loci (crp_offtarget_new_with_loci)");
+    if (res->guide_len != 20) return fail(CRP_ERR_STATE, "off-target listings are defined for guide_len 20 only");
+    const crp_genome *g = res->g;
+    const auto gi = std::find(ix->genomes.begin(), ix->genomes.end(), g);
+    if (gi == ix->genomes.end()) return fail(CRP_ERR_STATE, "the result's genome has not been added to the index");
+    if (n_rows == 0) return 0;
+    if (!rows) return fail(CRP_ERR_ARG, "rows is NULL");
+    if (int rc = ot_check_first(n_rows, first)) return rc;
+    if (first[n_rows] && !sites) return fail(CRP_ERR_ARG, "sites is NULL");
+    const int s = strand == '+' ? 0 : 1;
+    const uint64_t n = s == 0 ? res->n_plus : res->n_minus;
+    for (uint64_t i = 0; i < n_rows; ++i)
+        if (rows[i] >= n || (i && rows[i] <= rows[i - 1]))
+            return fail(CRP_ERR_ARG, "rows[%llu] = %u: rows must be ascending, distinct and below %llu", (unsigned long long)i,
+                        rows[i], (unsigned long long)n);
+    const std::vector<uint64_t> &cnt = s == 0 ? res->seg_plus : res->seg_minus;
+    const uint32_t n_seg = (uint32_t)cnt.size();
+    std::vector<uint32_t> seg(3 * (size_t)n_seg + 1);         // as in crp_offtarget_count_candidates
+    uint64_t row = 0;
+    for (uint32_t i = 0; i < n_seg; ++i) {
+        seg[i] = (uint32_t)row;
+        row += cnt[i];
+        seg[n_seg + 1 + i] = g->segs[i].first_tile;
+        seg[2 * (size_t)n_seg + 1 + i] = (uint32_t)g->segs[i].begin;
+    }
+    seg[n_seg] = (uint32_t)row;
+    cudaStream_t st = ix->st;
+    CUDA_TRY(cudaEventRecord(ix->ev[4], res->st));
+    CUDA_TRY(cudaStreamWaitEvent(st, ix->ev[4], 0));
+    uint32_t *d_seg = nullptr, *d_scratch = nullptr, *d_rows = nullptr;
+    unsigned long long *d_keys = nullptr, *d_sel = nullptr;   // d_sel: [n_rows] keys, [n_rows] own loci
+    unsigned int *d_invalid = nullptr;
+    if (dev_alloc(&d_seg, seg.size() * sizeof(uint32_t), st) != cudaSuccess ||
+        dev_alloc(&d_keys, n * sizeof(unsigned long long), st) != cudaSuccess ||
+        dev_alloc(&d_scratch, n * sizeof(uint32_t), st) != cudaSuccess ||
+        dev_alloc(&d_rows, n_rows * sizeof(uint32_t), st) != cudaSuccess ||
+        dev_alloc(&d_sel, 2 * n_rows * sizeof(unsigned long long), st) != cudaSuccess ||
+        dev_alloc(&d_invalid, sizeof(unsigned int), st) != cudaSuccess) {
+        cudaGetLastError();
+        dev_free(d_seg, st);
+        dev_free(d_keys, st);
+        dev_free(d_scratch, st);
+        dev_free(d_rows, st);
+        dev_free(d_sel, st);
+        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu query rows failed", (unsigned long long)n);
+    }
+    int rc = 0;
+    unsigned int invalid = 0;
+    if (cudaMemcpyAsync(d_seg, seg.data(), seg.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemcpyAsync(d_rows, rows, n_rows * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemsetAsync(d_invalid, 0, sizeof(unsigned int), st) != cudaSuccess)
+        rc = fail(CRP_ERR_CUDA, "H2D of the listing rows failed");
+    if (!rc) {                                                 // every row's key, then the selected rows
+        OtQueryArgs a;
+        a.records = g->records;
+        a.pos = res->pos[s];
+        a.n = n;
+        a.seg_row = d_seg;
+        a.seg_tile = d_seg + n_seg + 1;
+        a.seg_begin = d_seg + 2 * (size_t)n_seg + 1;
+        a.n_seg = n_seg;
+        a.k1 = 1;
+        a.minus = s;
+        a.keys = d_keys;
+        a.counts = d_scratch;
+        k_ot_queries<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a);
+        OtGatherArgs ga;
+        ga.keys = d_keys;
+        ga.pos = res->pos[s];
+        ga.rows = d_rows;
+        ga.seg_row = d_seg;
+        ga.n = n_rows;
+        ga.n_seg = n_seg;
+        ga.genome = (uint32_t)(gi - ix->genomes.begin());
+        ga.minus = s;
+        ga.sel_keys = d_sel;
+        ga.own = d_sel + n_rows;
+        ga.invalid = d_invalid;
+        k_ot_gather<<<(unsigned)((n_rows + 255) / 256), 256, 0, st>>>(ga);
+        g_ctx.launches += 2;
+        if (cudaGetLastError() != cudaSuccess ||
+            cudaMemcpyAsync(&invalid, d_invalid, sizeof invalid, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+            cudaStreamSynchronize(st) != cudaSuccess)
+            rc = fail(CRP_ERR_CUDA, "off-target query keys failed: %s", cudaGetErrorString(cudaGetLastError()));
+    }
+    if (!rc && invalid) rc = fail(CRP_ERR_ARG, "a selected row has no protospacer (its counts are 0xFFFFFFFF)");
+    if (!rc) rc = ot_list(ix, d_sel, d_sel + n_rows, n_rows, max_mm, first, sites);
+    dev_free(d_seg, st);
+    dev_free(d_keys, st);
+    dev_free(d_scratch, st);
+    dev_free(d_rows, st);
+    dev_free(d_sel, st);
+    dev_free(d_invalid, st);
+    return rc;
+}
+
+int crp_offtarget_list_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys, uint32_t max_mm, const uint64_t *first,
+                            uint32_t *sites) {
+    if (!ix) return fail(CRP_ERR_ARG, "ix is NULL");
+    if (int rc = need_ctx()) return rc;
+    if (max_mm > 3) return fail(CRP_ERR_ARG, "max_mm %u: at most 3 mismatches", max_mm);
+    if (!ix->with_loci) return fail(CRP_ERR_STATE, "listing needs an index with loci (crp_offtarget_new_with_loci)");
+    if (n == 0) return 0;
+    if (!keys) return fail(CRP_ERR_ARG, "keys is NULL");
+    if (n > 0xFFFFFFFFull) return fail(CRP_ERR_RANGE, "at most 2^32 - 1 keys per call");
+    for (uint64_t i = 0; i < n; ++i)
+        if (keys[i] >> 40) return fail(CRP_ERR_ARG, "key %llu has bits above bit 39", (unsigned long long)i);
+    if (int rc = ot_check_first(n, first)) return rc;
+    if (first[n] && !sites) return fail(CRP_ERR_ARG, "sites is NULL");
+    cudaStream_t st = ix->st;
+    unsigned long long *d_keys = nullptr;
+    if (dev_alloc(&d_keys, n * sizeof(unsigned long long), st) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu keys failed", (unsigned long long)n);
+    }
+    int rc = 0;
+    if (cudaMemcpyAsync(d_keys, keys, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
+        rc = fail(CRP_ERR_CUDA, "H2D of the keys failed");
+    if (!rc) rc = ot_list(ix, d_keys, nullptr, n, max_mm, first, sites);
+    dev_free(d_keys, st);
+    return rc;
+}
+
 int crp_offtarget_timing(const crp_offtarget *ix, float *ms_sites, float *ms_count, uint64_t *comparisons) {
     if (!ix) return fail(CRP_ERR_ARG, "ix is NULL");
     if (ms_sites) *ms_sites = ix->ms_sites;
@@ -2377,6 +2638,7 @@ int crp_offtarget_free(crp_offtarget *ix) {
     if (!ix) return 0;
     if (ix->st) {
         dev_free(ix->keys, ix->st);
+        dev_free(ix->loci, ix->st);
         cudaStreamSynchronize(ix->st);
     }
     for (cudaEvent_t e : ix->ev)

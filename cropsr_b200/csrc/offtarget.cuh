@@ -25,6 +25,10 @@
 // 24 bits of the other three parts.  A (query, site) pair is counted only at the pair (i, j) formed by
 // its two LOWEST exactly matching parts, so every pair with d <= k is counted exactly once; that test
 // runs only on the rare path d <= k.  The hot loop is XOR / SHF / LOP3 / POPC / compare.
+//
+// Listing (an index built with loci): every site also has a 64-bit locus (ot_locus) at the slot of its key, and
+// k_ot_list walks the same work items as k_ot_count, storing the index of every site with d <= k in the query
+// row's slice of the output (sized by the caller from the counts) instead of counting it.
 #pragma once
 #include "scan.cuh"
 
@@ -35,6 +39,21 @@ static constexpr uint32_t kOtSiteTile = 2048;               // sites of a work i
 static constexpr uint32_t kOtNoCount = 0xFFFFFFFFu;         // counts of a candidate without a protospacer
 static constexpr unsigned long long kOtInvalid = 1ull << 63;   // query key: no protospacer
 static constexpr int kOtScanThreads = 1024;                 // k_ot_scan: 64 buckets per thread
+static constexpr uint32_t kOtMaxSegments = 1u << 24;        // segments of a genome handle an index with loci takes
+static constexpr uint32_t kOtMaxGenomes = 127;              // genome handles of an index with loci
+static constexpr unsigned long long kOtNoLocus = ~0ull;     // genome ordinal 127: never a site's locus
+
+// Locus of a site: t (token coordinates, as in the key's definition) in bits 0-31, the segment index in its genome
+// handle in bits 32-55, the ordinal of the add_genome call that added the handle in bits 56-62, strand in bit 63
+// (1 = '-').
+CRP_HD unsigned long long ot_locus(uint32_t t, uint32_t segment, uint32_t genome, bool minus) {
+    return (unsigned long long)t | (unsigned long long)(segment & 0xFFFFFFu) << 32 |
+           (unsigned long long)(genome & 0x7Fu) << 56 | (unsigned long long)minus << 63;
+}
+// the locus of the site at bit b of tile word kw of a record whose descriptor word is desc ({t_start, L, n, segment})
+CRP_HD unsigned long long ot_site_locus(uint4 desc, uint32_t kw, uint32_t b, uint32_t genome, bool minus) {
+    return ot_locus(desc.x + 32u * kw + b, desc.w, genome, minus);
+}
 
 // ------------------------------------------------------------------ keys (host and device: tests/offtarget_emu.cu)
 CRP_HD unsigned long long ot_spread20(uint32_t v) {         // bit i -> bit 2i
@@ -113,19 +132,26 @@ __device__ __forceinline__ uint32_t ot_lanemask_lt() {
 
 // Sites of a genome handle: one thread per tile word, reading the tile records as k_other_runs does (the halo
 // words cover the 20 positions to the left and the 23 to the right of every owned position).  keys == NULL:
-// count only.  Otherwise keys[base + slot] for an unordered slot per site.
+// count only.  Otherwise keys[base + slot] for an unordered slot per site, and with kLoci its locus at
+// loci[base + slot] (ot_site_locus: t and segment from the tile's descriptor word); the instantiation without loci reads
+// neither field.
 struct OtSiteArgs {
     const uint4 *records;
     uint32_t n_tiles;
     unsigned long long *keys;
     unsigned long long base;
     unsigned long long *n;              // counter
+    unsigned long long *loci;           // kLoci only
+    uint32_t genome;                    // kLoci only: ordinal of the genome handle in the index
 };
 
+template <bool kLoci>
 __global__ void __launch_bounds__(256) k_ot_sites(const OtSiteArgs a) {
     const uint64_t it = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const uint32_t lane = threadIdx.x & 31;
     uint32_t plus = 0, minus = 0;
+    uint4 desc = make_uint4(0, 0, 0, 0);   // kLoci: the tile's descriptor word
+    uint32_t kw = 0;                    // kLoci: the tile word
     uint4 prev = make_uint4(0, 0, 0, 0), cur = prev, next = prev;
     if (it < (uint64_t)a.n_tiles * kTileWords) {
         const uint32_t tile = (uint32_t)(it / kTileWords), k = (uint32_t)(it % kTileWords);
@@ -136,6 +162,10 @@ __global__ void __launch_bounds__(256) k_ot_sites(const OtSiteArgs a) {
             prev = rec[1 + k], cur = rec[2 + k], next = rec[3 + k];
             plus = ot_pam_plus(cur, next) & own;
             minus = ot_pam_minus(cur, next) & own;
+            if constexpr (kLoci) {
+                desc = rec[0];
+                kw = k;
+            }
         }
     }
     unsigned long long key;
@@ -153,10 +183,24 @@ __global__ void __launch_bounds__(256) k_ot_sites(const OtSiteArgs a) {
     slot = __shfl_sync(0xFFFFFFFFu, slot, 31) + incl - mine;
     if (!a.keys || !mine) return;
     unsigned long long *out = a.keys + a.base + slot;
-    for (uint32_t m = plus; m; m &= m - 1)
-        if (ot_key<false>(prev, cur, next, __ffs(m) - 1, key)) *out++ = key;
-    for (uint32_t m = minus; m; m &= m - 1)
-        if (ot_key<true>(prev, cur, next, __ffs(m) - 1, key)) *out++ = key;
+    if constexpr (kLoci) {
+        unsigned long long *lout = a.loci + a.base + slot;
+        for (uint32_t m = plus; m; m &= m - 1)
+            if (ot_key<false>(prev, cur, next, __ffs(m) - 1, key)) {
+                *out++ = key;
+                *lout++ = ot_site_locus(desc, kw, __ffs(m) - 1, a.genome, false);
+            }
+        for (uint32_t m = minus; m; m &= m - 1)
+            if (ot_key<true>(prev, cur, next, __ffs(m) - 1, key)) {
+                *out++ = key;
+                *lout++ = ot_site_locus(desc, kw, __ffs(m) - 1, a.genome, true);
+            }
+    } else {
+        for (uint32_t m = plus; m; m &= m - 1)
+            if (ot_key<false>(prev, cur, next, __ffs(m) - 1, key)) *out++ = key;
+        for (uint32_t m = minus; m; m &= m - 1)
+            if (ot_key<true>(prev, cur, next, __ffs(m) - 1, key)) *out++ = key;
+    }
 }
 
 // Query keys of one strand stream of a scan (rows in segment order): the protospacer is read from the tile
@@ -193,6 +237,36 @@ __global__ void k_ot_queries(const OtQueryArgs a) {
     uint32_t *c = a.counts + i * a.k1;
     c[0] = ok ? 0xFFFFFFFFu : kOtNoCount;
     for (uint32_t d = 1; d < a.k1; ++d) c[d] = ok ? 0u : kOtNoCount;
+}
+
+// Selected rows of a strand stream for listing (rows ascending): the query key k_ot_queries wrote for the row and
+// the locus of the row's own site, which the listing leaves out.  A selected row without a protospacer sets
+// `invalid`.
+struct OtGatherArgs {
+    const unsigned long long *keys;     // [stream rows], k_ot_queries
+    const uint32_t *pos, *rows;
+    const uint32_t *seg_row;            // [n_seg + 1] first row of every segment in the stream
+    uint64_t n;                         // selected rows
+    uint32_t n_seg, genome;
+    int minus;
+    unsigned long long *sel_keys, *own; // [n]
+    unsigned int *invalid;
+};
+
+__global__ void k_ot_gather(const OtGatherArgs a) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n) return;
+    const uint32_t r = a.rows[i];
+    uint32_t lo = 0, hi = a.n_seg;
+    while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (__ldg(a.seg_row + mid) <= r) lo = mid;
+        else hi = mid;
+    }
+    const unsigned long long key = a.keys[r];
+    if (key & kOtInvalid) atomicOr(a.invalid, 1u);
+    a.sel_keys[i] = key;
+    a.own[i] = ot_locus(a.pos[r], lo, a.genome, a.minus != 0);
 }
 
 // ---- counting sort by the bucket of part pair (i, j): histogram, scan, scatter.  Warps aggregate their
@@ -358,6 +432,76 @@ __global__ void __launch_bounds__(kOtThreads) k_ot_count(const OtCountArgs a) {
             if (c1) atomicAdd(c + 1, c1);
             if (c2) atomicAdd(c + 2, c2);
             if (c3) atomicAdd(c + 3, c3);
+        }
+        __syncthreads();                                                     // the tile is read before the next copy
+    }
+}
+
+// Listing: the work items of k_ot_count with {rest key, site index} in the site tile (16 KB).  On the rare path
+// d <= k a thread takes a slot of the query row's slice with one atomic on the row's cursor and stores the site
+// index; a slot beyond the slice is never written -- the overflow flag is raised instead.  The query's own site
+// (d = 0, same locus) is left out.
+struct OtListArgs {
+    const uint2 *sites;                 // {rest key, site index} in bucket order
+    const uint2 *queries;               // {rest key, row} in bucket order
+    const uint32_t *soff, *qoff, *item_off;   // [kOtBuckets + 1]
+    const unsigned long long *loci;     // [sites]
+    const unsigned long long *own;      // [rows] locus of the row's own site, kOtNoLocus for none; NULL: no row has one
+    const unsigned long long *first;    // [rows + 1] slice of every row in out
+    uint32_t *cursor;                   // [rows] zeroed: sites found per row
+    uint32_t *out;                      // [first[rows]] site indices
+    unsigned int *overflow;
+    uint32_t k, jm1;
+};
+
+__global__ void __launch_bounds__(kOtThreads) k_ot_list(const OtListArgs a) {
+    __shared__ __align__(16) uint2 s_sites[kOtSiteTile + 2];
+    __shared__ __align__(8) unsigned long long bar;
+    const uint32_t tid = threadIdx.x;
+    const uint32_t total = a.item_off[kOtBuckets];
+    if (tid == 0) {
+        mbar_init(&bar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+    uint32_t phase = 0;
+    for (uint32_t item = blockIdx.x; item < total; item += gridDim.x) {
+        uint32_t lo = 0, hi = kOtBuckets;      // bucket: last b with item_off[b] <= item
+        while (hi - lo > 1) {
+            const uint32_t mid = (lo + hi) >> 1;
+            if (__ldg(a.item_off + mid) <= item) lo = mid;
+            else hi = mid;
+        }
+        const uint32_t sb = __ldg(a.soff + lo), ns = __ldg(a.soff + lo + 1) - sb;
+        const uint32_t qb = __ldg(a.qoff + lo), nq = __ldg(a.qoff + lo + 1) - qb;
+        const uint32_t n_st = (ns + kOtSiteTile - 1) / kOtSiteTile, local = item - __ldg(a.item_off + lo);
+        const uint32_t qt = local / n_st, st = local % n_st;
+        const uint32_t s0 = sb + st * kOtSiteTile, ns_t = min(kOtSiteTile, ns - st * kOtSiteTile);
+        const uint32_t q0 = qb + qt * kOtThreads, nq_t = min((uint32_t)kOtThreads, nq - qt * kOtThreads);
+        const uint32_t a0 = s0 & ~1u;                                        // 16-byte aligned source
+        if (tid == 0) {
+            const uint32_t bytes = ((s0 + ns_t - a0) * 8u + 15u) & ~15u;
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // earlier generic reads of the tile come first
+            mbar_expect(&bar, bytes);
+            bulk_copy(s_sites, a.sites + a0, bytes, &bar);
+        }
+        const uint32_t g = kOtThreads / nq_t;                                // threads per query
+        const bool active = tid < nq_t * g;
+        const uint2 q = active ? a.queries[q0 + tid % nq_t] : make_uint2(0, 0);
+        mbar_wait(&bar, phase);
+        phase ^= 1u;
+        if (active) {
+            const uint2 *S = s_sites + (s0 - a0);
+            for (uint32_t s = tid / nq_t; s < ns_t; s += g) {
+                const uint2 site = S[s];
+                const int d = ot_rest_mismatches(q.x, site.x, a.k, a.jm1);
+                if (d < 0) continue;
+                if (d == 0 && a.own && __ldg(a.loci + site.y) == __ldg(a.own + q.y)) continue;
+                const unsigned long long b = __ldg(a.first + q.y), len = __ldg(a.first + q.y + 1) - b;
+                const uint32_t slot = atomicAdd(a.cursor + q.y, 1u);
+                if (slot < len) a.out[b + slot] = site.y;
+                else atomicOr(a.overflow, 1u);
+            }
         }
         __syncthreads();                                                     // the tile is read before the next copy
     }

@@ -563,18 +563,24 @@ def guide_keys(guides):
     return keys
 
 
+LIST_BATCH_SITES = 1 << 28       # site indices one listing call returns at most (1 GiB on the device and the host)
+
+
 class OffTargetIndex:
     """NGG sites (both strands, case-insensitive) of one or more committed genomes, resident in HBM:
-    counts of sites within 0 .. k <= 3 mismatches of every scan candidate or of arbitrary guides
-    (semantics: include/cropsr_b200.h, csrc/offtarget.cuh)."""
+    counts of sites within 0 .. k <= 3 mismatches of every scan candidate or of arbitrary guides, and with
+    loci=True the sites themselves (semantics: include/cropsr_b200.h, csrc/offtarget.cuh)."""
 
     NO_COUNT = N.OFFTARGET_NO_COUNT
 
-    def __init__(self, genomes=()):
+    def __init__(self, genomes=(), loci=False):
+        """loci=True: the index also keeps every site's locus (8 bytes per site more), which site_loci and the
+        listings (list_candidates, list_guides) need."""
         if _device is None:
             init(0)
         self._h = C.c_void_p()
-        check(lib.crp_offtarget_new(C.byref(self._h)))
+        self.loci = bool(loci)
+        check((lib.crp_offtarget_new_with_loci if self.loci else lib.crp_offtarget_new)(C.byref(self._h)))
         for g in genomes:
             self.add_genome(g)
 
@@ -612,8 +618,69 @@ class OffTargetIndex:
             check(lib.crp_offtarget_count_keys(self._h, len(keys), keys.ctypes.data, int(k), out.ctypes.data))
         return out
 
+    def site_loci(self):
+        """(genome, segment, t, strand) arrays in sites() order: the ordinal of the add_genome call that added
+        the site's handle, the segment index in that handle, t in token coordinates, and 0 for '+' / 1 for '-'"""
+        n = self.num_sites()
+        loci = np.empty(n, dtype=np.uint64)
+        got = C.c_uint64(0)
+        check(lib.crp_offtarget_fetch_loci(self._h, n, loci.ctypes.data if n else None, C.byref(got)))
+        return ((loci >> np.uint64(56) & np.uint64(0x7F)).astype(np.uint8),
+                (loci >> np.uint64(32) & np.uint64(0xFFFFFF)).astype(np.uint32),
+                (loci & np.uint64(0xFFFFFFFF)).astype(np.uint32),
+                (loci >> np.uint64(63)).astype(np.uint8))
+
+    def _list(self, n_rows, totals, call):
+        """Batches of consecutive rows whose listings hold at most LIST_BATCH_SITES indices (a row above that
+        goes alone): call(lo, hi, first, out) per batch -> (first [n_rows + 1] uint64, sites uint32)."""
+        totals = np.asarray(totals, dtype=np.uint64)
+        first = np.zeros(n_rows + 1, dtype=np.uint64)
+        np.cumsum(totals, out=first[1:])
+        sites = np.empty(int(first[-1]), dtype=np.uint32)
+        lo = 0
+        while lo < n_rows:
+            hi = int(np.searchsorted(first, first[lo] + np.uint64(LIST_BATCH_SITES), side="right")) - 1
+            hi = min(max(hi, lo + 1), n_rows)
+            f = first[lo:hi + 1] - first[lo]
+            out = sites[int(first[lo]):int(first[hi])]
+            call(lo, hi, f, out)
+            lo = hi
+        return first, sites
+
+    def list_candidates(self, result, strand, k=3, rows=None, counts=None):
+        """The other sites within k mismatches of candidates of one strand stream -> (rows, first, sites):
+        rows (uint32, ascending stream rows; default every row with a protospacer), first (uint64 [len(rows) + 1])
+        and sites (uint32 indices into sites() / site_loci() order): row rows[i] lists sites[first[i]:first[i + 1]],
+        in no particular order.  counts: count_candidates(result, strand, k), computed when not given."""
+        if counts is None:
+            counts = self.count_candidates(result, strand, k)
+        counts = np.asarray(counts)
+        if rows is None:
+            rows = np.nonzero(counts[:, 0] != self.NO_COUNT)[0] if len(counts) else np.zeros(0, np.int64)
+        rows = np.ascontiguousarray(rows, dtype=np.uint32)
+        totals = counts[rows.astype(np.int64), :int(k) + 1].astype(np.uint64).sum(axis=1) if len(rows) else []
+
+        def call(lo, hi, f, out):
+            r = np.ascontiguousarray(rows[lo:hi])
+            check(lib.crp_offtarget_list_candidates(self._h, result._h, strand.encode(), int(k), hi - lo, r.ctypes.data,
+                                                    f.ctypes.data, out.ctypes.data if len(out) else None))
+        first, sites = self._list(len(rows), totals, call)
+        return rows, first, sites
+
+    def list_guides(self, guides, k=3):
+        """(first, sites) of 20-base guides in the protospacer orientation: guide i lists the sites within k
+        mismatches, sites[first[i]:first[i + 1]]; nothing subtracted"""
+        keys = guide_keys(guides)
+        totals = self.count_guides(guides, k).astype(np.uint64).sum(axis=1) if len(keys) else []
+
+        def call(lo, hi, f, out):
+            kk = np.ascontiguousarray(keys[lo:hi])
+            check(lib.crp_offtarget_list_keys(self._h, hi - lo, kk.ctypes.data, int(k), f.ctypes.data,
+                                              out.ctypes.data if len(out) else None))
+        return self._list(len(keys), totals, call)
+
     def timing(self):
-        """dict(ms_sites: every add_genome, ms_count and comparisons: the last count call)"""
+        """dict(ms_sites: every add_genome, ms_count and comparisons: the last count or list call)"""
         a, b, n = C.c_float(0), C.c_float(0), C.c_uint64(0)
         check(lib.crp_offtarget_timing(self._h, C.byref(a), C.byref(b), C.byref(n)))
         return {"ms_sites": a.value, "ms_count": b.value, "comparisons": n.value}

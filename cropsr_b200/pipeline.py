@@ -269,29 +269,33 @@ def write_gap_table(path, tokens, scan, min_len=10):
 _DNA = np.frombuffer(b"ATCG", dtype=np.uint8)
 
 
-def write_offtarget_table(path, tokens, scan, k=3):
+def write_offtarget_table(path, tokens, scan, k=3, index=None, counts=None):
     """Opt-in off-target table (not part of the reference's output): one row per unique candidate in
     reference order (token by token, '+' then '-', ascending t) with its protospacer as upper-case DNA
     in the orientation followed by the PAM, and the numbers of OTHER NGG sites of the whole genome at
     exactly 0 .. k mismatches (k_ot_* kernels; semantics in oracle/offtarget_oracle.py).  Protospacer
     and counts are blank where the candidate has none (cut off by the token end, or a byte outside
     ACGTacgt).  One index is built from every genome handle of the scan before anything is counted:
-    handles split at MAX_POSITIONS_PER_GENOME see each other's sites."""
+    handles split at MAX_POSITIONS_PER_GENOME see each other's sites.  index: such an index, built by the
+    caller (and not freed here); counts: offtarget_counts(index, scan, k), computed here when not given."""
     import csv
     import pandas as pd
     keys = list(tokens.keys())
     columns = ["chromosome", "strand", "pam_pos", "protospacer"] + [f"mm{d}" for d in range(k + 1)]
     with open(path, "w", newline="") as f:
         csv.writer(f, delimiter="\t").writerow(columns)
-    index = engine.OffTargetIndex([g for g, _, _, _ in scan.parts])
+    own_index = index is None
+    if own_index:
+        index = engine.OffTargetIndex([g for g, _, _, _ in scan.parts])
+    given = counts
     try:
-        for genome, result, first, cnt in scan.parts:
+        for part, (genome, result, first, cnt) in enumerate(scan.parts):
             cols = {}
             for strand, seg_cnt in (("+", result.seg_plus), ("-", result.seg_minus)):
                 seg_of = np.repeat(np.arange(cnt, dtype=np.int64), seg_cnt.astype(np.int64))
                 n = len(seg_of)
                 pos = result.fetch(strand, want=("pos",))["pos"]
-                counts = index.count_candidates(result, strand, k)
+                counts = index.count_candidates(result, strand, k) if given is None else given[(part, strand)]
                 ok = counts[:, 0] != index.NO_COUNT if n else np.zeros(0, bool)
                 proto = np.full(n, "", dtype=object)
                 if ok.any():
@@ -315,11 +319,108 @@ def write_offtarget_table(path, tokens, scan, k=3):
             order = np.argsort(np.concatenate((2 * cols["+"][0], 2 * cols["-"][0] + 1)), kind="stable")
             frame.iloc[order].to_csv(path, sep="\t", mode="a", header=False, index=False, lineterminator="\r\n")
     finally:
-        index.free()
+        if own_index:
+            index.free()
 
 
-def check_offtarget_args(guide_len, devices, max_mismatches):
-    """The off-target table's limits, checked before any device work: ValueError with the reason."""
+def offtarget_counts(index, scan, k=3):
+    """{(part, strand): index.count_candidates} of every genome handle of the scan: both off-target tables
+    from one count per strand"""
+    return {(part, strand): index.count_candidates(result, strand, k)
+            for part, (_, result, _, _) in enumerate(scan.parts) for strand in "+-"}
+
+
+_UPPER_DNA = np.frombuffer(b"ATCG", dtype=np.uint8)
+_COMPLEMENT = np.arange(256, dtype=np.uint8)
+_COMPLEMENT[list(b"ATCG")] = list(b"TAGC")
+
+
+def write_offtarget_sites(path, tokens, scan, k=3, max_sites=1000, index=None, counts=None):
+    """Opt-in off-target sites table (not part of the reference's output): one row per (candidate, other NGG
+    site of the genome within k mismatches), candidates in the order of write_offtarget_table, and within a
+    candidate by mismatches, then the site's token (file order), site_pam_pos, '+' before '-'.  site_protospacer
+    is the site's 20 bases in the orientation followed by NGG, upper case, with the bases that differ from the
+    candidate's protospacer in lower case (semantics in oracle/offtarget_sites_oracle.py).  A candidate with no
+    other site, or with more than max_sites, writes no rows: its counts are in the --offtargets table.
+    index: an index with loci over the scan's genome handles in scan.parts order, built by the caller (and not
+    freed here); counts: offtarget_counts(index, scan, k).  Returns (pairs written, candidates left out by the cap)."""
+    import csv
+    import pandas as pd
+    keys = list(tokens.keys())
+    names = np.array([key[1:] for key in keys], dtype=object)
+    columns = ["chromosome", "strand", "pam_pos", "protospacer", "site_chromosome", "site_strand", "site_pam_pos",
+               "site_protospacer", "mismatches"]
+    with open(path, "w", newline="") as f:
+        csv.writer(f, delimiter="\t").writerow(columns)
+    own_index = index is None
+    if own_index:
+        index = engine.OffTargetIndex([g for g, _, _, _ in scan.parts], loci=True)
+    pairs = capped = 0
+    try:
+        site_keys = index.sites()
+        s_gen, s_seg, s_t, s_strand = index.site_loci()
+        part_first = np.array([first for _, _, first, _ in scan.parts], dtype=np.int64)
+        s_tok = part_first[s_gen.astype(np.int64)] + s_seg.astype(np.int64) if len(site_keys) else np.zeros(0, np.int64)
+        for part, (genome, result, first, cnt) in enumerate(scan.parts):
+            chunks = []
+            for si, (strand, seg_cnt) in enumerate((("+", result.seg_plus), ("-", result.seg_minus))):
+                seg_of = np.repeat(np.arange(cnt, dtype=np.int64), seg_cnt.astype(np.int64))
+                if not len(seg_of):
+                    continue
+                c = index.count_candidates(result, strand, k) if counts is None else counts[(part, strand)]
+                ok = c[:, 0] != index.NO_COUNT
+                total = np.where(ok, c[:, :k + 1].astype(np.int64).sum(axis=1), 0)
+                capped += int((total > max_sites).sum())
+                rows = np.nonzero((total > 0) & (total <= max_sites))[0]
+                if not len(rows):
+                    continue
+                rows, lfirst, sites = index.list_candidates(result, strand, k, rows=rows, counts=c)
+                rows = rows.astype(np.int64)
+                pos = result.fetch(strand, want=("pos",))["pos"].astype(np.int64)
+                # the candidate's protospacer from the host token, as write_offtarget_table reads it
+                proto = []
+                for s, t in zip(seg_of[rows].tolist(), pos[rows].tolist()):
+                    tok = scan.token_bytes[first + s]
+                    proto.append(tok[t - 20:t] if strand == "+" else tok[t + 3:t + 23][::-1])
+                cb = np.frombuffer(b"".join(proto), dtype=np.uint8).reshape(-1, 20) & 0xDF
+                if strand == "-":
+                    cb = _COMPLEMENT[cb]
+                per = np.diff(lfirst).astype(np.int64)
+                cand = np.repeat(np.arange(len(rows)), per)
+                sk = site_keys[sites]
+                sb = _UPPER_DNA[((sk[:, None] >> (2 * np.arange(20, dtype=np.uint64))) & np.uint64(3)).astype(np.intp)]
+                differ = sb != cb[cand]
+                sb = sb | (differ.astype(np.uint8) << 5)                  # lower case where the bases differ
+                mm = differ.sum(axis=1)
+                row = rows[cand]
+                site = sites.astype(np.int64)
+                chunks.append((seg_of[row], np.full(len(row), si), row, mm, s_tok[site], s_t[site].astype(np.int64),
+                               s_strand[site].astype(np.int64), pos, cb[cand], sb, strand))
+            if not chunks:
+                continue
+            frames, sort_keys = [], []
+            for seg, sidx, row, mm, tok_i, site_t, site_s, pos, cb, sb, strand in chunks:
+                frames.append(pd.DataFrame({
+                    "chromosome": names[first + seg], "strand": strand, "pam_pos": pos[row],
+                    "protospacer": cb.view("S20").ravel().astype("U20").astype(object),
+                    "site_chromosome": names[tok_i], "site_strand": np.array(["+", "-"], dtype=object)[site_s],
+                    "site_pam_pos": site_t, "site_protospacer": sb.view("S20").ravel().astype("U20").astype(object),
+                    "mismatches": mm}, columns=columns))
+                sort_keys.append(np.stack((seg, sidx, row, mm, tok_i, site_t, site_s)))
+            frame = pd.concat(frames, ignore_index=True)
+            key = np.concatenate(sort_keys, axis=1)
+            order = np.lexsort(key[::-1])
+            frame.iloc[order].to_csv(path, sep="\t", mode="a", header=False, index=False, lineterminator="\r\n")
+            pairs += len(frame)
+    finally:
+        if own_index:
+            index.free()
+    return pairs, capped
+
+
+def check_offtarget_args(guide_len, devices, max_mismatches, max_sites=None):
+    """The off-target tables' limits, checked before any device work: ValueError with the reason.
+    max_sites: the cap of the sites table (write_offtarget_sites), at least 1."""
     if int(guide_len) != 20:
         raise ValueError(f"off-target counts are defined for 20-base guides, not -l {guide_len}")
     if devices is not None and len(devices) > 1:
@@ -327,18 +428,23 @@ def check_offtarget_args(guide_len, devices, max_mismatches):
                          "run without --devices, or with one device")
     if int(max_mismatches) not in (0, 1, 2, 3):
         raise ValueError(f"--mismatches {max_mismatches}: 0 to 3 mismatches are supported")
+    if max_sites is not None and int(max_sites) < 1:
+        raise ValueError(f"--max-sites {max_sites}: at least 1")
 
 
 def run_cas9(fasta, gff, output="data.csv", guide_len=20, verbose=False, blas_threads=1,
              time_path="time.txt", out=print, side_output=None, flank=200, device_ingest=True, annotation_info=None,
-             chunk_rows=None, devices=None, handle_limit=None, offtargets=None, max_mismatches=3):
+             chunk_rows=None, devices=None, handle_limit=None, offtargets=None, max_mismatches=3,
+             offtarget_sites=None, max_sites=1000):
     """devices: CUDA ordinals; more than one shards the genome over one process per GPU
     (cropsr_b200/multi.py) and writes the same CSV.  handle_limit: positions per genome handle
     (tests shrink it to walk the several-handles path on small inputs).  offtargets: path of the opt-in
     off-target table (write_offtarget_table, guide length 20 on one GPU), written after the CSV with
-    counts at 0 .. max_mismatches."""
-    if offtargets is not None:
-        check_offtarget_args(guide_len, devices, max_mismatches)
+    counts at 0 .. max_mismatches.  offtarget_sites: path of the opt-in off-target sites table
+    (write_offtarget_sites: every other site within max_mismatches of every candidate with at most max_sites
+    of them); with both tables one index serves both and every strand is counted once."""
+    if offtargets is not None or offtarget_sites is not None:
+        check_offtarget_args(guide_len, devices, max_mismatches, max_sites if offtarget_sites is not None else None)
     begin = time.time()
     timing = open(time_path, "w")                       # CROPSR.py:371
     multi_gpu = devices is not None and len(devices) > 1
@@ -391,10 +497,25 @@ def run_cas9(fasta, gff, output="data.csv", guide_len=20, verbose=False, blas_th
             formatted_path = ingest.needs_formatting(f.read())
         write_side_output(side_output, tokens, scan, gff_frame, flank, formatted_path, annotation_info)
         write_gap_table(side_output + ".gaps.tsv", tokens, scan)
-    if offtargets is not None:
+    ot_stats = {}
+    if offtarget_sites is not None:
+        index = engine.OffTargetIndex([g for g, _, _, _ in scan.parts], loci=True)
+        try:
+            counts = offtarget_counts(index, scan, max_mismatches)
+            if offtargets is not None:
+                write_offtarget_table(offtargets, tokens, scan, max_mismatches, index=index, counts=counts)
+            pairs, capped = write_offtarget_sites(offtarget_sites, tokens, scan, max_mismatches, max_sites,
+                                                  index=index, counts=counts)
+        finally:
+            index.free()
+        ot_stats = {"offtarget_pairs": pairs, "offtarget_capped": capped}
+        if verbose:
+            out(f"{pairs:n} off-target sites listed in {offtarget_sites}; {capped:n} candidates with more than "
+                f"{max_sites:n} left out")
+    elif offtargets is not None:
         write_offtarget_table(offtargets, tokens, scan, max_mismatches)
     stats = {"tokens": len(tokens), "candidates": len(table), "rows": rows_written,
-             "scan_ms": scan.scan_ms(), **scan.timing()}
+             "scan_ms": scan.scan_ms(), **scan.timing(), **ot_stats}
     t_plus = x_plus = t_minus = x_minus = None          # views into the scan's row arrays
     scan.free()
     if verbose:

@@ -364,8 +364,34 @@ int crp_offtarget_count_candidates(crp_offtarget *ix, const crp_result *res, cha
 /* The same for arbitrary protospacer keys (< 2^40; user guides in the orientation followed by NGG in the
  * genome); nothing is subtracted. */
 int crp_offtarget_count_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys, uint32_t max_mm, uint32_t *counts);
+/* ---- off-target loci.  An index made by crp_offtarget_new_with_loci also keeps one uint64 LOCUS per site, at
+ * the slot of its key (8 more bytes per site of device memory):
+ *   bits 0-31   t, token coordinates (the t of the definition above and of a candidate's pam_pos)
+ *   bits 32-55  the segment index in its genome handle
+ *   bits 56-62  the ordinal of the add_genome call that added the handle (0, 1, ...)
+ *   bit 63      strand, 1 = '-'
+ * add_genome of such an index answers CRP_ERR_RANGE for a handle of 2^24 segments or more and for a 128th
+ * handle.  An index made by crp_offtarget_new behaves as before and keeps no loci. */
+int crp_offtarget_new_with_loci(crp_offtarget **ix);
+/* The loci in crp_offtarget_fetch_sites order; CRP_ERR_STATE on an index without loci, CRP_ERR_RANGE (and *n)
+ * if capacity is too small. */
+int crp_offtarget_fetch_loci(const crp_offtarget *ix, uint64_t capacity, uint64_t *loci, uint64_t *n);
+/* LISTING: the sites that the counts of a row count, as site indices (positions in fetch_sites / fetch_loci
+ * order).  The caller sizes row i's slice from its counts: first[i + 1] - first[i] = sum of mm_d, d <= max_mm,
+ * first[0] = 0; the library writes the row's sites into sites[first[i] .. first[i + 1]) in no particular
+ * order and never outside the slice.  If a row finds another number of sites than its slice holds, the call
+ * answers CRP_ERR_STATE and nothing is copied to `sites`.  A candidate's own site (same locus) is left out.
+ * CRP_ERR_ARG: max_mm > 3, first not starting at 0 or decreasing, rows not ascending and distinct or beyond the
+ * stream, a selected row without a protospacer, a key >= 2^40.  CRP_ERR_STATE: an index without loci, a genome
+ * not added, guide_len != 20. */
+int crp_offtarget_list_candidates(crp_offtarget *ix, const crp_result *res, char strand, uint32_t max_mm,
+                                  uint64_t n_rows, const uint32_t *rows,   /* stream rows, ascending, distinct */
+                                  const uint64_t *first,                   /* [n_rows + 1], first[0] = 0 */
+                                  uint32_t *sites);                        /* [first[n_rows]] site indices */
+int crp_offtarget_list_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys, uint32_t max_mm,
+                            const uint64_t *first, uint32_t *sites);
 /* ms_sites: device time of every add_genome; ms_count and comparisons (sum over the 10 part pairs and the
- * 65,536 buckets of queries x sites) of the last count call. */
+ * 65,536 buckets of queries x sites) of the last count or list call. */
 int crp_offtarget_timing(const crp_offtarget *ix, float *ms_sites, float *ms_count, uint64_t *comparisons);
 int crp_offtarget_free(crp_offtarget *ix);
 
