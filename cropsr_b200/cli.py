@@ -101,6 +101,12 @@ def main(argv=None):
         except ValueError as e:
             flag = "--offtargets" if args.offtarget_sites is None else "--offtarget-sites"
             sys.exit(f"CROPSR.py: error: {flag}: {e}")
+    if args.side_output is not None:
+        from .pipeline import check_side_output_args
+        try:
+            check_side_output_args(args.L)
+        except ValueError as e:
+            sys.exit(f"CROPSR.py: error: --side-output: {e}")
     from . import engine, pipeline
     engine.init(devices[0])
     pipeline.run_cas9(args.f, args.g, args.o, args.l, args.verbose, args.blas_threads,

@@ -55,7 +55,7 @@ __global__ void k_extras(const ExtrasArgs a) {
     if (a.run) a.run[i] = (uint8_t)run;
     if (a.cut) a.cut[i] = cut;
     if (a.flank_lo) a.flank_lo[i] = cut > a.flank ? cut - a.flank : 0u;
-    if (a.flank_hi) a.flank_hi[i] = cut + a.flank < a.L ? cut + a.flank : a.L;
+    if (a.flank_hi) a.flank_hi[i] = a.flank >= a.L - cut ? a.L : cut + a.flank;     // cut < L: no 32-bit wrap
 }
 
 // Intervals sorted by start, inclusive [start, end]; maxend[j] = max(end[0..j]).  One thread

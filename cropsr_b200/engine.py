@@ -416,6 +416,15 @@ class Genome:
             pass
 
 
+def _flank(flank):
+    """The flank half-width as the library takes it (uint32): ValueError outside 0 <= flank < 2**32, which a
+    ctypes uint32 would wrap silently (-1 -> 2**32 - 1, 2**32 + 200 -> 200)."""
+    f = int(flank)
+    if not 0 <= f < 1 << 32:
+        raise ValueError(f"flank {flank}: 0 <= flank < 2**32 expected")
+    return f
+
+
 class ScanResult:
     """Two ordered candidate streams ('+', '-') resident in HBM."""
 
@@ -484,22 +493,24 @@ class ScanResult:
 
     def extras(self, seg, strand, flank=200):
         """Opt-in side outputs of one segment's candidates (never in the parity CSV):
-        dict(gc, flags, run: uint8[]; cut, flank_lo, flank_hi: uint32[])."""
+        dict(gc, flags, run: uint8[]; cut, flank_lo, flank_hi: uint32[]).  flank: 0 <= flank < 2**32."""
+        flank = _flank(flank)
         n = int((self.seg_plus if strand == "+" else self.seg_minus)[seg])
         out = {k: np.empty(n, np.uint8) for k in ("gc", "flags", "run")}
         out.update({k: np.empty(n, np.uint32) for k in ("cut", "flank_lo", "flank_hi")})
         ptr = lambda a: a.ctypes.data if len(a) else None
-        check(lib.crp_result_extras(self._h, int(seg), strand.encode(), int(flank), ptr(out["gc"]), ptr(out["flags"]),
+        check(lib.crp_result_extras(self._h, int(seg), strand.encode(), flank, ptr(out["gc"]), ptr(out["flags"]),
                                     ptr(out["run"]), ptr(out["cut"]), ptr(out["flank_lo"]), ptr(out["flank_hi"])))
         return out
 
     def extras_strand(self, strand, flank=200):
         """extras() of every candidate of one strand stream (all segments), in stream order"""
+        flank = _flank(flank)
         n = int(self.n_plus if strand == "+" else self.n_minus)
         out = {k: np.empty(n, np.uint8) for k in ("gc", "flags", "run")}
         out.update({k: np.empty(n, np.uint32) for k in ("cut", "flank_lo", "flank_hi")})
         ptr = lambda a: a.ctypes.data if len(a) else None
-        check(lib.crp_result_extras_strand(self._h, strand.encode(), int(flank), ptr(out["gc"]), ptr(out["flags"]),
+        check(lib.crp_result_extras_strand(self._h, strand.encode(), flank, ptr(out["gc"]), ptr(out["flags"]),
                                            ptr(out["run"]), ptr(out["cut"]), ptr(out["flank_lo"]), ptr(out["flank_hi"])))
         return out
 

@@ -432,6 +432,13 @@ def check_offtarget_args(guide_len, devices, max_mismatches, max_sites=None):
         raise ValueError(f"--max-sites {max_sites}: at least 1")
 
 
+def check_side_output_args(flank):
+    """The side output's limit, checked before any device work: ValueError unless 0 <= flank < 2**32 (the flank
+    window [cut - flank, cut + flank) is computed in 32-bit token coordinates)."""
+    if not 0 <= int(flank) < 1 << 32:
+        raise ValueError(f"-L {flank}: the flanking length must be 0 to 2**32 - 1")
+
+
 def run_cas9(fasta, gff, output="data.csv", guide_len=20, verbose=False, blas_threads=1,
              time_path="time.txt", out=print, side_output=None, flank=200, device_ingest=True, annotation_info=None,
              chunk_rows=None, devices=None, handle_limit=None, offtargets=None, max_mismatches=3,
@@ -445,6 +452,8 @@ def run_cas9(fasta, gff, output="data.csv", guide_len=20, verbose=False, blas_th
     of them); with both tables one index serves both and every strand is counted once."""
     if offtargets is not None or offtarget_sites is not None:
         check_offtarget_args(guide_len, devices, max_mismatches, max_sites if offtarget_sites is not None else None)
+    if side_output:
+        check_side_output_args(flank)
     begin = time.time()
     timing = open(time_path, "w")                       # CROPSR.py:371
     multi_gpu = devices is not None and len(devices) > 1
