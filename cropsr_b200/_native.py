@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # CROPSR_B200_LIB: another build of the same library (kernel experiments, tools/variants.sh)
 LIB_PATH = os.environ.get("CROPSR_B200_LIB") or os.path.join(_HERE, "libcropsr_b200.so")
 
-ABI_VERSION = 9
+ABI_VERSION = 10
 
 CRP_SCAN_DEFAULT = 0
 CRP_SCAN_NO_SCORE = 1
@@ -27,6 +27,8 @@ PACKED_TRUNCATED = 1 << 31
 PACKED_UNSCORED = 1 << 62
 
 OFFTARGET_NO_COUNT = 0xFFFFFFFF     # counts of a candidate without a protospacer (crp_offtarget_count_candidates)
+OFFTARGET_NO_SCORE = 0xFFFFFFFFFFFFFFFF   # score of a candidate without a protospacer (crp_offtarget_score_candidates)
+OFFTARGET_SCORE_SETS = 1351         # CRP_OT_SCORE_SETS: mismatch-position sets of size <= 3
 
 
 class SegmentDesc(C.Structure):
@@ -140,6 +142,8 @@ SIGNATURES = {
     "crp_offtarget_list_candidates": (C.c_int, [C.c_void_p, C.c_void_p, C.c_char, C.c_uint32, C.c_uint64, C.c_void_p,
                                                 C.c_void_p, C.c_void_p]),
     "crp_offtarget_list_keys": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]),
+    "crp_offtarget_score_candidates": (C.c_int, [C.c_void_p, C.c_void_p, C.c_char, C.c_uint32, C.c_void_p, C.c_void_p]),
+    "crp_offtarget_score_keys": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]),
     "crp_offtarget_timing": (C.c_int, [C.c_void_p, _f32p, _f32p, _u64p]),
     "crp_offtarget_free": (C.c_int, [C.c_void_p]),
 }

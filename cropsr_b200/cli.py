@@ -10,7 +10,7 @@ def build_parser():
     # line of this length (its own consistency assertion fails), and --help would crash
     p = argparse.ArgumentParser(prog="CROPSR.py", usage="CROPSR.py [-h] -f FASTA [-g GFF] [-p TXT] [-o CSV] [-l 20] [-L 200] --cas9 [-v]\n"
                                 "                 [--device N | --devices 0-7] [--side-output TSV] [--offtargets TSV] [--offtarget-sites TSV]\n"
-                                "                 [--mismatches K] [--max-sites N] [--blas-threads N]")
+                                "                 [--offtarget-scores TSV] [--mismatches K] [--max-sites N] [--blas-threads N]")
     p.add_argument("-f", "--fasta", metavar="", required=True, dest="f",
                    help="[required] path to input file in FASTA format")
     p.add_argument("-g", "--gff", metavar="", dest="g", help="path to input file in GFF format")
@@ -44,8 +44,14 @@ def build_parser():
                         "of the genome within K mismatches, with the site's chromosome, strand, position and protospacer "
                         "(differing bases in lower case); candidates with more than --max-sites such sites are left out "
                         "(their counts are in --offtargets); -l 20 on one GPU only; the CSV is unaffected")
+    p.add_argument("--offtarget-scores", metavar="", default=None,
+                   help="also write a tab-separated table of off-target scores: per candidate its protospacer, the sum "
+                        "of the MIT hit scores (Hsu et al. 2013, as CRISPOR computes them) of the other NGG sites of the "
+                        "genome within K mismatches, and the MIT specificity 100 / (100 + sum) * 100; CRISPOR also "
+                        "counts 4-mismatch and NAG/NGA sites, so its numbers differ; -l 20 on one GPU only; the CSV is "
+                        "unaffected")
     p.add_argument("--mismatches", metavar="", type=int, default=3,
-                   help="K of --offtargets and --offtarget-sites: 0 to 3, default = 3")
+                   help="K of --offtargets, --offtarget-sites and --offtarget-scores: 0 to 3, default = 3")
     p.add_argument("--max-sites", metavar="", type=int, default=1000,
                    help="--offtarget-sites lists the candidates with at most this many other sites within K "
                         "mismatches: at least 1, default = 1000")
@@ -93,13 +99,14 @@ def main(argv=None):
     if args.verbose:
         print(banner(args))
     devices = parse_devices(args.devices) if args.devices else [args.device]
-    if args.offtargets is not None or args.offtarget_sites is not None:
+    if args.offtargets is not None or args.offtarget_sites is not None or args.offtarget_scores is not None:
         from .pipeline import check_offtarget_args
         try:
             check_offtarget_args(args.l, devices, args.mismatches,
                                  args.max_sites if args.offtarget_sites is not None else None)
         except ValueError as e:
-            flag = "--offtargets" if args.offtarget_sites is None else "--offtarget-sites"
+            flag = ("--offtarget-sites" if args.offtarget_sites is not None else
+                    "--offtargets" if args.offtargets is not None else "--offtarget-scores")
             sys.exit(f"CROPSR.py: error: {flag}: {e}")
     if args.side_output is not None:
         from .pipeline import check_side_output_args
@@ -112,5 +119,6 @@ def main(argv=None):
     pipeline.run_cas9(args.f, args.g, args.o, args.l, args.verbose, args.blas_threads,
                       side_output=args.side_output, flank=args.L, annotation_info=args.p, devices=devices,
                       offtargets=args.offtargets, max_mismatches=args.mismatches,
-                      offtarget_sites=args.offtarget_sites, max_sites=args.max_sites)
+                      offtarget_sites=args.offtarget_sites, max_sites=args.max_sites,
+                      offtarget_scores=args.offtarget_scores)
     return 0

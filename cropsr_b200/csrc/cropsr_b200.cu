@@ -31,7 +31,7 @@
 #include "extras.cuh"
 #include "offtarget.cuh"
 
-#define CRP_ABI_VERSION 9
+#define CRP_ABI_VERSION 10
 
 static constexpr size_t kScanSmemFixed = (size_t)kStages * kRecBytes + 2 * (size_t)kListCap * sizeof(uint16_t);
 
@@ -2068,6 +2068,23 @@ int crp_rescore(const crp_genome *g, uint64_t n, const uint32_t *segment, const 
 
 // ------------------------------------------------------------------ off-target counts (offtarget.cuh)
 
+// k_ot_queries' segment table of one strand stream (s = 0 '+', 1 '-'): row offsets [n_seg + 1], first tiles [n_seg],
+// first positions [n_seg]
+static std::vector<uint32_t> ot_segment_table(const crp_result *res, int s) {
+    const std::vector<uint64_t> &cnt = s == 0 ? res->seg_plus : res->seg_minus;
+    const uint32_t n_seg = (uint32_t)cnt.size();
+    std::vector<uint32_t> seg(3 * (size_t)n_seg + 1);
+    uint64_t row = 0;
+    for (uint32_t i = 0; i < n_seg; ++i) {
+        seg[i] = (uint32_t)row;
+        row += cnt[i];
+        seg[n_seg + 1 + i] = res->g->segs[i].first_tile;
+        seg[2 * (size_t)n_seg + 1 + i] = (uint32_t)res->g->segs[i].begin;
+    }
+    seg[n_seg] = (uint32_t)row;
+    return seg;
+}
+
 struct crp_offtarget {
     cudaStream_t st = nullptr;                 // own stream, ordered behind each genome's stream by an event
     cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};   // sites start / end, count start / end, genome ready
@@ -2076,15 +2093,16 @@ struct crp_offtarget {
     unsigned long long *loci = nullptr;        // crp_offtarget_new_with_loci: the locus of every site, at its key's slot
     bool with_loci = false;
     uint64_t n_sites = 0;
-    float ms_sites = 0.f, ms_count = 0.f;      // summed over add_genome / of the last count or list call
+    float ms_sites = 0.f, ms_count = 0.f;      // summed over add_genome / of the last count, list or score call
     uint64_t comparisons = 0;
 };
 
 // Count every query of d_keys (n rows, kOtInvalid = no counts) against the index's sites into d_counts
 // ([n][k + 1], primed by the caller), on ix->st; waits for the result.  list != NULL: list the pairs instead
-// (k_ot_list with the caller's own / first / cursor / out / overflow; the sites carry their index).
+// (k_ot_list with the caller's own / first / cursor / out / overflow; the sites carry their index).  score != NULL:
+// sum the weights of the pairs instead (k_ot_score with the caller's weights / sums).
 static int ot_count(crp_offtarget *ix, const unsigned long long *d_keys, uint64_t n, uint32_t k, uint32_t *d_counts,
-                    const OtListArgs *list = nullptr) {
+                    const OtListArgs *list = nullptr, const OtScoreArgs *score = nullptr) {
     cudaStream_t st = ix->st;
     const size_t tbl = kOtBuckets + 1;
     uint32_t *d_tbl = nullptr, *d_sites = nullptr;
@@ -2131,6 +2149,16 @@ static int ot_count(crp_offtarget *ix, const unsigned long long *d_keys, uint64_
         la.loci = ix->loci;
         la.k = k;
     }
+    OtScoreArgs sc = {};
+    if (score) {
+        sc = *score;
+        sc.sites = d_sites;
+        sc.queries = d_q;
+        sc.soff = sa.off[0];
+        sc.qoff = sa.off[1];
+        sc.item_off = sa.item_off;
+        sc.k = k;
+    }
     auto grid = [](uint64_t items) { return (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((items + 255) / 256, (uint64_t)g_ctx.sm_count * 16)); };
     int rc = 0;
     unsigned long long misc[2] = {0, 0};
@@ -2157,6 +2185,11 @@ static int ot_count(crp_offtarget *ix, const unsigned long long *d_keys, uint64_
         if (list) {
             la.jm1 = ca.jm1;
             k_ot_list<<<(unsigned)g_ctx.sm_count * 8, kOtThreads, 0, st>>>(la);
+        } else if (score) {
+            sc.jm1 = ca.jm1;
+            sc.pi = i;
+            sc.pj = j;
+            k_ot_score<<<(unsigned)g_ctx.sm_count * 8, kOtThreads, 0, st>>>(sc);
         } else {
             k_ot_count<<<(unsigned)g_ctx.sm_count * 8, kOtThreads, 0, st>>>(ca);
         }
@@ -2329,17 +2362,8 @@ int crp_offtarget_count_candidates(crp_offtarget *ix, const crp_result *res, cha
     const uint64_t n = s == 0 ? res->n_plus : res->n_minus;
     if (n == 0) return 0;
     if (!counts) return fail(CRP_ERR_ARG, "counts is NULL");
-    const std::vector<uint64_t> &cnt = s == 0 ? res->seg_plus : res->seg_minus;
-    const uint32_t n_seg = (uint32_t)cnt.size();
-    std::vector<uint32_t> seg(3 * (size_t)n_seg + 1);         // row offsets [n_seg + 1], first tiles, first positions
-    uint64_t row = 0;
-    for (uint32_t i = 0; i < n_seg; ++i) {
-        seg[i] = (uint32_t)row;
-        row += cnt[i];
-        seg[n_seg + 1 + i] = g->segs[i].first_tile;
-        seg[2 * (size_t)n_seg + 1 + i] = (uint32_t)g->segs[i].begin;
-    }
-    seg[n_seg] = (uint32_t)row;
+    const uint32_t n_seg = (uint32_t)(s == 0 ? res->seg_plus : res->seg_minus).size();
+    const std::vector<uint32_t> seg = ot_segment_table(res, s);
     cudaStream_t st = ix->st;
     CUDA_TRY(cudaEventRecord(ix->ev[4], res->st));             // the candidate streams are written on the scan's stream
     CUDA_TRY(cudaStreamWaitEvent(st, ix->ev[4], 0));
@@ -2518,17 +2542,8 @@ int crp_offtarget_list_candidates(crp_offtarget *ix, const crp_result *res, char
         if (rows[i] >= n || (i && rows[i] <= rows[i - 1]))
             return fail(CRP_ERR_ARG, "rows[%llu] = %u: rows must be ascending, distinct and below %llu", (unsigned long long)i,
                         rows[i], (unsigned long long)n);
-    const std::vector<uint64_t> &cnt = s == 0 ? res->seg_plus : res->seg_minus;
-    const uint32_t n_seg = (uint32_t)cnt.size();
-    std::vector<uint32_t> seg(3 * (size_t)n_seg + 1);         // as in crp_offtarget_count_candidates
-    uint64_t row = 0;
-    for (uint32_t i = 0; i < n_seg; ++i) {
-        seg[i] = (uint32_t)row;
-        row += cnt[i];
-        seg[n_seg + 1 + i] = g->segs[i].first_tile;
-        seg[2 * (size_t)n_seg + 1 + i] = (uint32_t)g->segs[i].begin;
-    }
-    seg[n_seg] = (uint32_t)row;
+    const uint32_t n_seg = (uint32_t)(s == 0 ? res->seg_plus : res->seg_minus).size();
+    const std::vector<uint32_t> seg = ot_segment_table(res, s);
     cudaStream_t st = ix->st;
     CUDA_TRY(cudaEventRecord(ix->ev[4], res->st));
     CUDA_TRY(cudaStreamWaitEvent(st, ix->ev[4], 0));
@@ -2623,6 +2638,138 @@ int crp_offtarget_list_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys,
         rc = fail(CRP_ERR_CUDA, "H2D of the keys failed");
     if (!rc) rc = ot_list(ix, d_keys, nullptr, n, max_mm, first, sites);
     dev_free(d_keys, st);
+    return rc;
+}
+
+}  // extern "C"
+
+// The weight table of a score call, [kOtScoreSets]: CRP_ERR_ARG if NULL or if an entry of a set of size <= k is 2^31
+// or more (2^32 sites of weight < 2^31 cannot overflow a uint64 sum); the entries of larger sets are not read.
+static int ot_check_weights(uint32_t k, const uint32_t *weights) {
+    static const uint32_t used[4] = {1, 21, 211, kOtScoreSets};
+    if (!weights) return fail(CRP_ERR_ARG, "weights is NULL");
+    for (uint32_t r = 0; r < used[k]; ++r)
+        if (weights[r] >> 31) return fail(CRP_ERR_ARG, "weights[%u] = %u: at most 2^31 - 1", r, weights[r]);
+    return 0;
+}
+
+// Weight sums of n queries whose keys are on the device into d_sums [n] (primed by the caller), on ix->st.
+static int ot_score(crp_offtarget *ix, const unsigned long long *d_keys, uint64_t n, uint32_t k, const uint32_t *weights,
+                    unsigned long long *d_sums) {
+    cudaStream_t st = ix->st;
+    uint32_t *d_w = nullptr;
+    if (dev_alloc(&d_w, kOtScoreSets * sizeof(uint32_t), st) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(CRP_ERR_NOMEM, "cudaMalloc of the weight table failed");
+    }
+    int rc = 0;
+    if (cudaMemcpyAsync(d_w, weights, kOtScoreSets * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
+        rc = fail(CRP_ERR_CUDA, "H2D of the weight table failed");
+    if (!rc) {
+        OtScoreArgs sc = {};
+        sc.weights = d_w;
+        sc.sums = d_sums;
+        rc = ot_count(ix, d_keys, n, k, nullptr, nullptr, &sc);
+    }
+    dev_free(d_w, st);
+    return rc;
+}
+
+extern "C" {
+
+int crp_offtarget_score_candidates(crp_offtarget *ix, const crp_result *res, char strand, uint32_t max_mm,
+                                   const uint32_t *weights, uint64_t *sums) {
+    if (!ix || !res) return fail(CRP_ERR_ARG, "NULL argument");
+    if (int rc = need_ctx()) return rc;
+    if (strand != '+' && strand != '-') return fail(CRP_ERR_ARG, "strand must be '+' or '-'");
+    if (max_mm > 3) return fail(CRP_ERR_ARG, "max_mm %u: at most 3 mismatches", max_mm);
+    if (res->guide_len != 20) return fail(CRP_ERR_STATE, "off-target scores are defined for guide_len 20 only");
+    const crp_genome *g = res->g;
+    if (std::find(ix->genomes.begin(), ix->genomes.end(), g) == ix->genomes.end())
+        return fail(CRP_ERR_STATE, "the result's genome has not been added to the index");
+    if (int rc = ot_check_weights(max_mm, weights)) return rc;
+    const int s = strand == '+' ? 0 : 1;
+    const uint64_t n = s == 0 ? res->n_plus : res->n_minus;
+    if (n == 0) return 0;
+    if (!sums) return fail(CRP_ERR_ARG, "sums is NULL");
+    const uint32_t n_seg = (uint32_t)(s == 0 ? res->seg_plus : res->seg_minus).size();
+    const std::vector<uint32_t> seg = ot_segment_table(res, s);
+    cudaStream_t st = ix->st;
+    CUDA_TRY(cudaEventRecord(ix->ev[4], res->st));             // the candidate streams are written on the scan's stream
+    CUDA_TRY(cudaStreamWaitEvent(st, ix->ev[4], 0));
+    uint32_t *d_seg = nullptr, *d_scratch = nullptr;
+    unsigned long long *d_keys = nullptr, *d_sums = nullptr;
+    if (dev_alloc(&d_seg, seg.size() * sizeof(uint32_t), st) != cudaSuccess ||
+        dev_alloc(&d_keys, n * sizeof(unsigned long long), st) != cudaSuccess ||
+        dev_alloc(&d_scratch, n * sizeof(uint32_t), st) != cudaSuccess ||
+        dev_alloc(&d_sums, n * sizeof(unsigned long long), st) != cudaSuccess) {
+        cudaGetLastError();
+        dev_free(d_seg, st);
+        dev_free(d_keys, st);
+        dev_free(d_scratch, st);
+        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu query rows failed", (unsigned long long)n);
+    }
+    int rc = 0;
+    if (cudaMemcpyAsync(d_seg, seg.data(), seg.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
+        rc = fail(CRP_ERR_CUDA, "H2D of the segment table failed");
+    if (!rc) {                                                 // the query keys (counts to scratch), then the primed sums
+        OtQueryArgs a;
+        a.records = g->records;
+        a.pos = res->pos[s];
+        a.n = n;
+        a.seg_row = d_seg;
+        a.seg_tile = d_seg + n_seg + 1;
+        a.seg_begin = d_seg + 2 * (size_t)n_seg + 1;
+        a.n_seg = n_seg;
+        a.k1 = 1;
+        a.minus = s;
+        a.keys = d_keys;
+        a.counts = d_scratch;
+        k_ot_queries<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a);
+        k_ot_score_prime<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_keys, n, 0ull - weights[0], d_sums);
+        g_ctx.launches += 2;
+        if (cudaGetLastError() != cudaSuccess) rc = fail(CRP_ERR_CUDA, "off-target query keys failed");
+    }
+    if (!rc) rc = ot_score(ix, d_keys, n, max_mm, weights, d_sums);
+    if (!rc && (cudaMemcpyAsync(sums, d_sums, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+                cudaStreamSynchronize(st) != cudaSuccess))
+        rc = fail(CRP_ERR_CUDA, "D2H of the off-target scores failed");
+    dev_free(d_seg, st);
+    dev_free(d_keys, st);
+    dev_free(d_scratch, st);
+    dev_free(d_sums, st);
+    return rc;
+}
+
+int crp_offtarget_score_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys, uint32_t max_mm, const uint32_t *weights,
+                             uint64_t *sums) {
+    if (!ix) return fail(CRP_ERR_ARG, "ix is NULL");
+    if (int rc = need_ctx()) return rc;
+    if (max_mm > 3) return fail(CRP_ERR_ARG, "max_mm %u: at most 3 mismatches", max_mm);
+    if (int rc = ot_check_weights(max_mm, weights)) return rc;
+    if (n == 0) return 0;
+    if (!keys || !sums) return fail(CRP_ERR_ARG, "NULL argument");
+    if (n > 0xFFFFFFFFull) return fail(CRP_ERR_RANGE, "at most 2^32 - 1 keys per call");
+    for (uint64_t i = 0; i < n; ++i)
+        if (keys[i] >> 40) return fail(CRP_ERR_ARG, "key %llu has bits above bit 39", (unsigned long long)i);
+    cudaStream_t st = ix->st;
+    unsigned long long *d_keys = nullptr, *d_sums = nullptr;
+    if (dev_alloc(&d_keys, n * sizeof(unsigned long long), st) != cudaSuccess ||
+        dev_alloc(&d_sums, n * sizeof(unsigned long long), st) != cudaSuccess) {
+        cudaGetLastError();
+        dev_free(d_keys, st);
+        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu keys failed", (unsigned long long)n);
+    }
+    int rc = 0;
+    if (cudaMemcpyAsync(d_keys, keys, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemsetAsync(d_sums, 0, n * sizeof(unsigned long long), st) != cudaSuccess)
+        rc = fail(CRP_ERR_CUDA, "H2D of the keys failed");
+    if (!rc) rc = ot_score(ix, d_keys, n, max_mm, weights, d_sums);
+    if (!rc && (cudaMemcpyAsync(sums, d_sums, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+                cudaStreamSynchronize(st) != cudaSuccess))
+        rc = fail(CRP_ERR_CUDA, "D2H of the off-target scores failed");
+    dev_free(d_keys, st);
+    dev_free(d_sums, st);
     return rc;
 }
 

@@ -29,6 +29,19 @@
 // Listing (an index built with loci): every site also has a 64-bit locus (ot_locus) at the slot of its key, and
 // k_ot_list walks the same work items as k_ot_count, storing the index of every site with d <= k in the query
 // row's slice of the output (sized by the caller from the counts) instead of counting it.
+//
+// Scores (oracle/offtarget_score_oracle.py states the same): the pairs are exactly those the counts count.  The
+// mismatch positions of a pair (0 = P[0], PAM-distal, .. 19) form a set of size d <= 3, ranked colexicographically:
+//   rank({})        = 0
+//   rank({a})       = 1 + a
+//   rank({a<b})     = 21 + a + C(b,2)
+//   rank({a<b<c})   = 211 + a + C(b,2) + C(c,3)                       (1,351 sets, ranks 0 .. 1350)
+// A caller-given table w[1351] (uint32, < 2^31) gives each set a weight; the score of a query is the uint64 sum of
+// w[rank] over its pairs (the candidate's own site, rank 0, subtracted; nothing subtracted for guides).  With the
+// table of the MIT specificity score (Hsu et al. 2013, as CRISPOR's calcHitScore computes it: score1 * score2 *
+// score3 * 100 in IEEE double, stored as round(hit * 2^24)) the sum over a candidate's NGG sites within k <= 3
+// mismatches is H * 2^24, and its specificity 100 / (100 + H) * 100.  CRISPOR sums over 4 mismatches and NAG / NGA
+// sites as well, so its numbers are not these.  Integer atomics make the sum independent of the order of the pairs.
 #pragma once
 #include "scan.cuh"
 
@@ -42,6 +55,8 @@ static constexpr int kOtScanThreads = 1024;                 // k_ot_scan: 64 buc
 static constexpr uint32_t kOtMaxSegments = 1u << 24;        // segments of a genome handle an index with loci takes
 static constexpr uint32_t kOtMaxGenomes = 127;              // genome handles of an index with loci
 static constexpr unsigned long long kOtNoLocus = ~0ull;     // genome ordinal 127: never a site's locus
+static constexpr uint32_t kOtScoreSets = 1351;              // mismatch-position sets of size <= 3 (ot_mask_rank)
+static constexpr unsigned long long kOtNoScore = ~0ull;     // score of a candidate without a protospacer
 
 // Locus of a site: t (token coordinates, as in the key's definition) in bits 0-31, the segment index in its genome
 // handle in bits 32-55, the ordinal of the add_genome call that added the handle in bits 56-62, strand in bit 63
@@ -121,6 +136,22 @@ CRP_HD int ot_rest_mismatches(uint32_t q, uint32_t s, uint32_t k, uint32_t jm1) 
     for (uint32_t m = 0; m < jm1; ++m)
         if (!((y >> (8 * m)) & 0xFFu)) return -1;
     return (int)d;
+}
+// Colex rank (see the head of this file) of the protospacer positions of the mismatches of a pair of part pair
+// (i, j), from y = (x | x >> 1) & 0x555555 of the rest keys' XOR x: rest nucleotide m (bit 2m) is position 4p + m % 4
+// of the part p that rest byte m / 4 holds (the parts other than i and j, ascending).  At most 3 bits of y are set.
+CRP_HD uint32_t ot_mask_rank(uint32_t y, int i, int j) {
+    uint32_t rank = 0, n = 0;
+    for (; y; y &= y - 1) {
+        const uint32_t m = (uint32_t)crp_popc((y & (0u - y)) - 1u) >> 1;   // the lowest set bit, 2m
+        uint32_t p = m >> 2;
+        p += p >= (uint32_t)i;
+        p += p >= (uint32_t)j;
+        const uint32_t x = 4u * p + (m & 3u);
+        ++n;
+        rank += n == 1 ? x : n == 2 ? x * (x - 1u) / 2u : x * (x - 1u) * (x - 2u) / 6u;
+    }
+    return rank + (n == 0 ? 0u : n == 1 ? 1u : n == 2 ? 21u : 211u);
 }
 
 // ------------------------------------------------------------------ kernels
@@ -505,4 +536,79 @@ __global__ void __launch_bounds__(kOtThreads) k_ot_list(const OtListArgs a) {
         }
         __syncthreads();                                                     // the tile is read before the next copy
     }
+}
+
+// Scores: the work items and site tiles of k_ot_count, and a copy of the weight table (5.4 KB) in shared memory.  On
+// the rare path d <= k a thread adds w[rank] of the pair's mismatch-position set to a uint64 in a register; a
+// non-zero sum is flushed with one 64-bit atomic per thread and item.  Rows are primed by the caller: a candidate
+// with -w[0] (its own site adds w[0]), a candidate without a protospacer with kOtNoScore (it joins no bucket), a
+// guide with 0.
+struct OtScoreArgs {
+    const uint32_t *sites;              // rest keys in bucket order
+    const uint2 *queries;               // {rest key, row} in bucket order
+    const uint32_t *soff, *qoff, *item_off;   // [kOtBuckets + 1]
+    const uint32_t *weights;            // [kOtScoreSets], by ot_mask_rank
+    unsigned long long *sums;           // [rows]
+    uint32_t k, jm1;
+    int pi, pj;                         // the part pair
+};
+
+__global__ void __launch_bounds__(kOtThreads) k_ot_score(const OtScoreArgs a) {
+    __shared__ __align__(16) uint32_t s_sites[kOtSiteTile + 8];
+    __shared__ uint32_t s_w[kOtScoreSets];
+    __shared__ __align__(8) unsigned long long bar;
+    const uint32_t tid = threadIdx.x;
+    const uint32_t total = a.item_off[kOtBuckets];
+    for (uint32_t r = tid; r < kOtScoreSets; r += kOtThreads) s_w[r] = __ldg(a.weights + r);
+    if (tid == 0) {
+        mbar_init(&bar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+    uint32_t phase = 0;
+    for (uint32_t item = blockIdx.x; item < total; item += gridDim.x) {
+        uint32_t lo = 0, hi = kOtBuckets;      // bucket: last b with item_off[b] <= item
+        while (hi - lo > 1) {
+            const uint32_t mid = (lo + hi) >> 1;
+            if (__ldg(a.item_off + mid) <= item) lo = mid;
+            else hi = mid;
+        }
+        const uint32_t sb = __ldg(a.soff + lo), ns = __ldg(a.soff + lo + 1) - sb;
+        const uint32_t qb = __ldg(a.qoff + lo), nq = __ldg(a.qoff + lo + 1) - qb;
+        const uint32_t n_st = (ns + kOtSiteTile - 1) / kOtSiteTile, local = item - __ldg(a.item_off + lo);
+        const uint32_t qt = local / n_st, st = local % n_st;
+        const uint32_t s0 = sb + st * kOtSiteTile, ns_t = min(kOtSiteTile, ns - st * kOtSiteTile);
+        const uint32_t q0 = qb + qt * kOtThreads, nq_t = min((uint32_t)kOtThreads, nq - qt * kOtThreads);
+        const uint32_t a0 = s0 & ~3u;                                        // 16-byte aligned source
+        if (tid == 0) {
+            const uint32_t bytes = ((s0 + ns_t - a0) * 4u + 15u) & ~15u;
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // earlier generic reads of the tile come first
+            mbar_expect(&bar, bytes);
+            bulk_copy(s_sites, a.sites + a0, bytes, &bar);
+        }
+        const uint32_t g = kOtThreads / nq_t;                                // threads per query
+        const bool active = tid < nq_t * g;
+        const uint2 q = active ? a.queries[q0 + tid % nq_t] : make_uint2(0, 0);
+        mbar_wait(&bar, phase);
+        phase ^= 1u;
+        if (active) {
+            const uint32_t *S = s_sites + (s0 - a0);
+            unsigned long long sum = 0;
+            for (uint32_t s = tid / nq_t; s < ns_t; s += g) {
+                const uint32_t site = S[s];
+                if (ot_rest_mismatches(q.x, site, a.k, a.jm1) < 0) continue;
+                const uint32_t x = q.x ^ site;
+                sum += s_w[ot_mask_rank((x | x >> 1) & 0x555555u, a.pi, a.pj)];
+            }
+            if (sum) atomicAdd(a.sums + q.y, sum);
+        }
+        __syncthreads();                                                     // the tile is read before the next copy
+    }
+}
+
+// The score rows of a candidate stream from the query keys k_ot_queries wrote: `own` (= -w[0]) or kOtNoScore.
+__global__ void k_ot_score_prime(const unsigned long long *__restrict__ keys, uint64_t n, unsigned long long own,
+                                 unsigned long long *sums) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) sums[i] = keys[i] & kOtInvalid ? kOtNoScore : own;
 }

@@ -576,6 +576,59 @@ def guide_keys(guides):
 
 LIST_BATCH_SITES = 1 << 28       # site indices one listing call returns at most (1 GiB on the device and the host)
 
+# MIT specificity score (Hsu et al. 2013) as CRISPOR's calcHitScore / calcMitGuideScore compute it: the per-position
+# mismatch weights, position 0 PAM-distal
+MIT_M = (0, 0, 0.014, 0, 0, 0.395, 0.317, 0, 0.389, 0.079, 0.445, 0.508, 0.613, 0.851, 0.732, 0.828, 0.615, 0.804,
+         0.685, 0.583)
+SCORE_SETS = N.OFFTARGET_SCORE_SETS
+SCORE_ONE = 1 << 24              # fixed point of the weights: w = round(hit * 2**24)
+
+
+def score_sets():
+    """The mismatch-position sets of size <= 3 (ascending tuples) in rank order (include/cropsr_b200.h):
+    {}, then {a} by a, {a<b} by (b, a), {a<b<c} by (c, b, a) -- colexicographic within a size."""
+    from itertools import combinations
+    return [c for d in range(4) for c in sorted(combinations(range(20), d), key=lambda c: c[::-1])]
+
+
+def mit_hit(positions):
+    """CRISPOR's calcHitScore of one site from its ascending mismatch positions, in its IEEE operation order.  The
+    distance term uses the mean of CONSECUTIVE distances, as CRISPOR does (not the all-pairs mean of the paper)."""
+    score1 = 1.0
+    for p in positions:
+        score1 *= 1 - MIT_M[p]
+    n = len(positions)
+    if n < 2:
+        score2 = 1.0
+    else:
+        dists = [positions[i + 1] - positions[i] for i in range(n - 1)]
+        score2 = 1.0 / (((19 - sum(dists) / len(dists)) / 19.0) * 4 + 1)
+    score3 = 1.0 if n == 0 else 1.0 / (n ** 2)
+    return score1 * score2 * score3 * 100
+
+
+def mit_weights():
+    """uint32[SCORE_SETS]: round(mit_hit(set) * 2**24) (half to even; the product is exact) in rank order"""
+    return np.array([round(mit_hit(c) * SCORE_ONE) for c in score_sets()], dtype=np.uint32)
+
+
+def mit_specificity(sums):
+    """CRISPOR's calcMitGuideScore, int(round(100 / (100 + H) * 100)) with H = sum / 2**24, of score sums
+    (score_candidates / score_guides with the MIT weights) -> uint64, NO_SCORE passed through"""
+    sums = np.asarray(sums, dtype=np.uint64)
+    ok = sums != np.uint64(N.OFFTARGET_NO_SCORE)
+    h = sums[ok].astype(np.float64) / SCORE_ONE
+    out = np.full(sums.shape, N.OFFTARGET_NO_SCORE, dtype=np.uint64)
+    out[ok] = np.round(100 / (100 + h) * 100).astype(np.uint64)
+    return out
+
+
+def _weights(weights):
+    w = mit_weights() if weights is None else np.ascontiguousarray(weights, dtype=np.uint32)
+    if w.shape != (SCORE_SETS,):
+        raise ValueError(f"weights: {SCORE_SETS} entries expected, got shape {w.shape}")
+    return w
+
 
 class OffTargetIndex:
     """NGG sites (both strands, case-insensitive) of one or more committed genomes, resident in HBM:
@@ -583,6 +636,7 @@ class OffTargetIndex:
     loci=True the sites themselves (semantics: include/cropsr_b200.h, csrc/offtarget.cuh)."""
 
     NO_COUNT = N.OFFTARGET_NO_COUNT
+    NO_SCORE = N.OFFTARGET_NO_SCORE
 
     def __init__(self, genomes=(), loci=False):
         """loci=True: the index also keeps every site's locus (8 bytes per site more), which site_loci and the
@@ -690,8 +744,30 @@ class OffTargetIndex:
                                               out.ctypes.data if len(out) else None))
         return self._list(len(keys), totals, call)
 
+    def score_candidates(self, result, strand, k=3, weights=None):
+        """uint64[n_strand]: per candidate of one strand stream (stream order) the sum of weights[rank] over the
+        sites its counts count (its own site not included), rank being that of the pair's mismatch-position set
+        (score_sets order); NO_SCORE where the candidate has no protospacer.  weights: uint32[SCORE_SETS], each
+        < 2**31 (default mit_weights(): sums of MIT hit scores * 2**24 over NGG sites within k mismatches)."""
+        w = _weights(weights)
+        n = int(result.n_plus if strand == "+" else result.n_minus)
+        out = np.empty(n, dtype=np.uint64)
+        check(lib.crp_offtarget_score_candidates(self._h, result._h, strand.encode(), int(k), w.ctypes.data,
+                                                 out.ctypes.data if n else None))
+        return out
+
+    def score_guides(self, guides, k=3, weights=None):
+        """uint64[len(guides)] for 20-base guides in the protospacer orientation; nothing subtracted"""
+        w = _weights(weights)
+        keys = guide_keys(guides)
+        out = np.empty(len(keys), dtype=np.uint64)
+        if len(keys):
+            check(lib.crp_offtarget_score_keys(self._h, len(keys), keys.ctypes.data, int(k), w.ctypes.data,
+                                               out.ctypes.data))
+        return out
+
     def timing(self):
-        """dict(ms_sites: every add_genome, ms_count and comparisons: the last count or list call)"""
+        """dict(ms_sites: every add_genome, ms_count and comparisons: the last count, list or score call)"""
         a, b, n = C.c_float(0), C.c_float(0), C.c_uint64(0)
         check(lib.crp_offtarget_timing(self._h, C.byref(a), C.byref(b), C.byref(n)))
         return {"ms_sites": a.value, "ms_count": b.value, "comparisons": n.value}

@@ -278,16 +278,45 @@ def write_offtarget_table(path, tokens, scan, k=3, index=None, counts=None):
     ACGTacgt).  One index is built from every genome handle of the scan before anything is counted:
     handles split at MAX_POSITIONS_PER_GENOME see each other's sites.  index: such an index, built by the
     caller (and not freed here); counts: offtarget_counts(index, scan, k), computed here when not given."""
+    def values(index, part, result, strand):
+        c = index.count_candidates(result, strand, k) if counts is None else counts[(part, strand)]
+        ok = c[:, 0] != index.NO_COUNT
+        return ok, {f"mm{d}": c[:, d].astype(np.int64).astype(str).astype(object) for d in range(k + 1)}
+    _write_candidate_table(path, tokens, scan, [f"mm{d}" for d in range(k + 1)], values, index)
+
+
+def write_offtarget_scores(path, tokens, scan, k=3, index=None):
+    """Opt-in off-target score table (not part of the reference's output): the rows of write_offtarget_table, in
+    its order, with mit_hit_sum, the sum of the MIT hit scores (Hsu et al. 2013, CRISPOR's calcHitScore) of the
+    candidate's OTHER NGG sites within k mismatches (.6f), and mit_specificity, 100 / (100 + mit_hit_sum) * 100
+    rounded to an integer (CRISPOR's calcMitGuideScore); both blank where the candidate has no protospacer
+    (k_ot_score; semantics in oracle/offtarget_score_oracle.py).  CRISPOR also sums 4-mismatch and NAG / NGA sites,
+    so its numbers differ.  index: an index over the scan's genome handles, built by the caller (and not freed
+    here), else built here."""
+    weights = engine.mit_weights()
+
+    def values(index, part, result, strand):
+        sums = index.score_candidates(result, strand, k, weights)
+        ok = sums != np.uint64(index.NO_SCORE)
+        hit = np.zeros(len(sums), dtype=object)
+        hit[ok] = np.char.mod("%.6f", sums[ok].astype(np.float64) / engine.SCORE_ONE).astype(object)
+        return ok, {"mit_hit_sum": hit, "mit_specificity": engine.mit_specificity(sums).astype(str).astype(object)}
+    _write_candidate_table(path, tokens, scan, ["mit_hit_sum", "mit_specificity"], values, index)
+
+
+def _write_candidate_table(path, tokens, scan, value_columns, values, index=None):
+    """The per-candidate off-target tables: chromosome strand pam_pos protospacer, then value_columns from
+    values(index, part, result, strand) -> (ok, {column: object array}) per strand stream; protospacer and values
+    blank where not ok.  index None: one is built over every genome handle of the scan and freed here."""
     import csv
     import pandas as pd
     keys = list(tokens.keys())
-    columns = ["chromosome", "strand", "pam_pos", "protospacer"] + [f"mm{d}" for d in range(k + 1)]
+    columns = ["chromosome", "strand", "pam_pos", "protospacer"] + value_columns
     with open(path, "w", newline="") as f:
         csv.writer(f, delimiter="\t").writerow(columns)
     own_index = index is None
     if own_index:
         index = engine.OffTargetIndex([g for g, _, _, _ in scan.parts])
-    given = counts
     try:
         for part, (genome, result, first, cnt) in enumerate(scan.parts):
             cols = {}
@@ -295,8 +324,9 @@ def write_offtarget_table(path, tokens, scan, k=3, index=None, counts=None):
                 seg_of = np.repeat(np.arange(cnt, dtype=np.int64), seg_cnt.astype(np.int64))
                 n = len(seg_of)
                 pos = result.fetch(strand, want=("pos",))["pos"]
-                counts = index.count_candidates(result, strand, k) if given is None else given[(part, strand)]
-                ok = counts[:, 0] != index.NO_COUNT if n else np.zeros(0, bool)
+                ok, vals = values(index, part, result, strand)
+                if not n:
+                    ok = np.zeros(0, bool)
                 proto = np.full(n, "", dtype=object)
                 if ok.any():
                     # the protospacer from the host token: '+' tok[t-20:t], '-' the reverse complement of tok[t+3:t+23]
@@ -311,9 +341,8 @@ def write_offtarget_table(path, tokens, scan, k=3, index=None, counts=None):
                 frame = {"chromosome": np.array([key[1:] for key in keys[first:first + cnt]], dtype=object)[seg_of]
                          if n else np.empty(0, object),
                          "strand": strand, "pam_pos": pos.astype(np.int64), "protospacer": proto}
-                for d in range(k + 1):
-                    frame[f"mm{d}"] = np.where(ok, counts[:, d].astype(np.int64).astype(str).astype(object), "") if n \
-                        else np.empty(0, object)
+                for c in value_columns:
+                    frame[c] = np.where(ok, vals[c], "") if n else np.empty(0, object)
                 cols[strand] = (seg_of, pd.DataFrame(frame, columns=columns))
             frame = pd.concat([cols["+"][1], cols["-"][1]], ignore_index=True)
             order = np.argsort(np.concatenate((2 * cols["+"][0], 2 * cols["-"][0] + 1)), kind="stable")
@@ -442,15 +471,17 @@ def check_side_output_args(flank):
 def run_cas9(fasta, gff, output="data.csv", guide_len=20, verbose=False, blas_threads=1,
              time_path="time.txt", out=print, side_output=None, flank=200, device_ingest=True, annotation_info=None,
              chunk_rows=None, devices=None, handle_limit=None, offtargets=None, max_mismatches=3,
-             offtarget_sites=None, max_sites=1000):
+             offtarget_sites=None, max_sites=1000, offtarget_scores=None):
     """devices: CUDA ordinals; more than one shards the genome over one process per GPU
     (cropsr_b200/multi.py) and writes the same CSV.  handle_limit: positions per genome handle
     (tests shrink it to walk the several-handles path on small inputs).  offtargets: path of the opt-in
     off-target table (write_offtarget_table, guide length 20 on one GPU), written after the CSV with
     counts at 0 .. max_mismatches.  offtarget_sites: path of the opt-in off-target sites table
     (write_offtarget_sites: every other site within max_mismatches of every candidate with at most max_sites
-    of them); with both tables one index serves both and every strand is counted once."""
-    if offtargets is not None or offtarget_sites is not None:
+    of them); with both tables one index serves both and every strand is counted once.  offtarget_scores: path of
+    the opt-in off-target score table (write_offtarget_scores: MIT hit-score sum and specificity over the NGG sites
+    within max_mismatches); one index, with loci only when the sites table needs them, serves every table."""
+    if offtargets is not None or offtarget_sites is not None or offtarget_scores is not None:
         check_offtarget_args(guide_len, devices, max_mismatches, max_sites if offtarget_sites is not None else None)
     if side_output:
         check_side_output_args(flank)
@@ -507,22 +538,24 @@ def run_cas9(fasta, gff, output="data.csv", guide_len=20, verbose=False, blas_th
         write_side_output(side_output, tokens, scan, gff_frame, flank, formatted_path, annotation_info)
         write_gap_table(side_output + ".gaps.tsv", tokens, scan)
     ot_stats = {}
-    if offtarget_sites is not None:
-        index = engine.OffTargetIndex([g for g, _, _, _ in scan.parts], loci=True)
+    if offtargets is not None or offtarget_sites is not None or offtarget_scores is not None:
+        index = engine.OffTargetIndex([g for g, _, _, _ in scan.parts], loci=offtarget_sites is not None)
         try:
-            counts = offtarget_counts(index, scan, max_mismatches)
+            # with the sites table, each strand is counted once for both count-driven tables
+            counts = offtarget_counts(index, scan, max_mismatches) if offtarget_sites is not None else None
             if offtargets is not None:
                 write_offtarget_table(offtargets, tokens, scan, max_mismatches, index=index, counts=counts)
-            pairs, capped = write_offtarget_sites(offtarget_sites, tokens, scan, max_mismatches, max_sites,
-                                                  index=index, counts=counts)
+            if offtarget_sites is not None:
+                pairs, capped = write_offtarget_sites(offtarget_sites, tokens, scan, max_mismatches, max_sites,
+                                                      index=index, counts=counts)
+                ot_stats = {"offtarget_pairs": pairs, "offtarget_capped": capped}
+            if offtarget_scores is not None:
+                write_offtarget_scores(offtarget_scores, tokens, scan, max_mismatches, index=index)
         finally:
             index.free()
-        ot_stats = {"offtarget_pairs": pairs, "offtarget_capped": capped}
-        if verbose:
+        if verbose and offtarget_sites is not None:
             out(f"{pairs:n} off-target sites listed in {offtarget_sites}; {capped:n} candidates with more than "
                 f"{max_sites:n} left out")
-    elif offtargets is not None:
-        write_offtarget_table(offtargets, tokens, scan, max_mismatches)
     stats = {"tokens": len(tokens), "candidates": len(table), "rows": rows_written,
              "scan_ms": scan.scan_ms(), **scan.timing(), **ot_stats}
     t_plus = x_plus = t_minus = x_minus = None          # views into the scan's row arrays

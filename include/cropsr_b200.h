@@ -390,8 +390,24 @@ int crp_offtarget_list_candidates(crp_offtarget *ix, const crp_result *res, char
                                   uint32_t *sites);                        /* [first[n_rows]] site indices */
 int crp_offtarget_list_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys, uint32_t max_mm,
                             const uint64_t *first, uint32_t *sites);
+/* ---- off-target SCORES: per query the uint64 sum, over the pairs its counts count (NGG sites within d <= max_mm
+ * mismatches, the candidate's own site subtracted, nothing subtracted for keys), of weights[rank of the pair's
+ * mismatch-position set].  The positions are 0 .. 19 of P (0 = PAM-distal), and the sets of size <= 3 are ranked
+ * colexicographically:
+ *   rank({}) = 0   rank({a}) = 1 + a   rank({a<b}) = 21 + a + C(b,2)   rank({a<b<c}) = 211 + a + C(b,2) + C(c,3)
+ * Entries for sets larger than max_mm are not read; an entry >= 2^31 among the others is CRP_ERR_ARG, so that no sum
+ * can overflow.  A candidate without a protospacer gets CRP_OT_NO_SCORE.  The sum does not depend on the order in
+ * which pairs are found.  With round(hit * 2^24) of the MIT hit score (Hsu et al. 2013, CRISPOR's calcHitScore) as
+ * weights, sum / 2^24 is the MIT hit-score sum over NGG sites within max_mm <= 3 mismatches -- CRISPOR also sums
+ * 4-mismatch and NAG / NGA sites, so its score is not this one.  Other refusals as for the count calls. */
+#define CRP_OT_SCORE_SETS 1351
+#define CRP_OT_NO_SCORE 0xFFFFFFFFFFFFFFFFull
+int crp_offtarget_score_candidates(crp_offtarget *ix, const crp_result *res, char strand, uint32_t max_mm,
+                                   const uint32_t *weights /* [CRP_OT_SCORE_SETS] */, uint64_t *sums /* [n_strand] */);
+int crp_offtarget_score_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys, uint32_t max_mm,
+                             const uint32_t *weights, uint64_t *sums);
 /* ms_sites: device time of every add_genome; ms_count and comparisons (sum over the 10 part pairs and the
- * 65,536 buckets of queries x sites) of the last count or list call. */
+ * 65,536 buckets of queries x sites) of the last count, list or score call. */
 int crp_offtarget_timing(const crp_offtarget *ix, float *ms_sites, float *ms_count, uint64_t *comparisons);
 int crp_offtarget_free(crp_offtarget *ix);
 
