@@ -1496,6 +1496,20 @@ int crp_scan_segments(uint32_t n_segments, const crp_segment_desc *segments, int
     if (n_segments && (!segments || !n_plus || !n_minus)) return fail(CRP_ERR_ARG, "NULL argument");
     if (guide_len < 1 || guide_len > 1000000) return fail(CRP_ERR_ARG, "guide_len %d out of range", guide_len);
     const bool scored = guide_len == 20 && !(flags & CRP_SCAN_NO_SCORE);
+    // every descriptor is checked before the first group is enqueued: a bad one in the middle of the
+    // list must not leave the groups before it copied, packed and scanned (the rules of add_segment)
+    for (uint32_t k = 0; k < n_segments; ++k) n_plus[k] = n_minus[k] = 0;
+    for (uint32_t k = 0; k < n_segments; ++k) {
+        const crp_segment_desc &sd = segments[k];
+        if (!sd.token && sd.token_len) return fail(CRP_ERR_ARG, "segment %u: token is NULL", k);
+        if (sd.begin > sd.end || sd.end > sd.token_len)
+            return fail(CRP_ERR_ARG, "segment %u: [%llu,%llu) outside token of length %llu", k,
+                        (unsigned long long)sd.begin, (unsigned long long)sd.end, (unsigned long long)sd.token_len);
+        if (sd.begin % kAlign) return fail(CRP_ERR_ARG, "segment %u: begin must be a multiple of %u", k, kAlign);
+        if (sd.token_len >= (1ull << 31) - (1ull << 15))
+            return fail(CRP_ERR_ARG, "segment %u: token of %llu positions exceeds the 31-bit position range", k,
+                        (unsigned long long)sd.token_len);
+    }
     constexpr int kLanes = 3;
     if (!g_ctx.lanes[0])
         for (int i = 0; i < kLanes; ++i) CUDA_TRY(cudaStreamCreateWithFlags(&g_ctx.lanes[i], cudaStreamNonBlocking));
@@ -1518,9 +1532,8 @@ int crp_scan_segments(uint32_t n_segments, const crp_segment_desc *segments, int
     };
     std::vector<Piece> pieces;
     for (uint32_t k = 0; k < n_segments; ++k) {
-        const uint64_t end = segments[k].end ? segments[k].end : segments[k].token_len;
+        const uint64_t end = segments[k].end;
         uint64_t b0 = segments[k].begin;
-        n_plus[k] = n_minus[k] = 0;
         if (end <= b0) {
             pieces.push_back(Piece{k, b0, end});
             continue;

@@ -214,12 +214,17 @@ int crp_result_free(crp_result *res);
  * receive the per-segment counts.  Returns CRP_ERR_RANGE if an arena of
  * `capacity` rows per strand is too small (the counts are still filled in).
  * packed / x arenas may be NULL (and are ignored when guide_len != 20).
- * ms_device (optional) receives the summed device time of the scan kernels. */
+ * ms_device (optional) receives the summed device time of the scan kernels.
+ * [begin, end) is taken as given, exactly as by crp_genome_add_segment: there is
+ * no sentinel, so end = 0 (or end = begin) owns no position.  Every descriptor is
+ * checked before any device work: begin <= end <= token_len, begin % 128 == 0,
+ * token non-NULL when token_len > 0, token_len below 2^31 - 2^15.  A violation
+ * returns CRP_ERR_ARG with n_plus / n_minus zeroed. */
 typedef struct crp_segment_desc {
     uint32_t token_id;
     const uint8_t *token;       /* position 0 of the whole token */
     uint64_t token_len;
-    uint64_t begin, end;        /* positions of the token this call owns (begin % 128 == 0) */
+    uint64_t begin, end;        /* positions [begin, end) of the token this call owns */
 } crp_segment_desc;
 int crp_scan_segments(uint32_t n_segments, const crp_segment_desc *segments, int guide_len, uint32_t flags,
                       uint64_t capacity, uint32_t *pos_plus, uint64_t *packed_plus, double *x_plus,
