@@ -18,6 +18,7 @@
 #include <atomic>
 #include <mutex>
 #include <new>
+#include <type_traits>
 #include <utility>
 #include <vector>
 
@@ -2110,20 +2111,20 @@ struct crp_offtarget {
     uint64_t comparisons = 0;
 };
 
-// Count every query of d_keys (n rows, kOtInvalid = no counts) against the index's sites into d_counts
-// ([n][k + 1], primed by the caller), on ix->st; waits for the result.  list != NULL: list the pairs instead
-// (k_ot_list with the caller's own / first / cursor / out / overflow; the sites carry their index).  score != NULL:
-// sum the weights of the pairs instead (k_ot_score with the caller's weights / sums).
-static int ot_count(crp_offtarget *ix, const unsigned long long *d_keys, uint64_t n, uint32_t k, uint32_t *d_counts,
-                    const OtListArgs *list = nullptr, const OtScoreArgs *score = nullptr) {
+// Join every query of d_keys (n rows, kOtInvalid = no key) against the index's sites, part pair by part pair, with
+// k_ot_join<Op>: op takes every (query, site) pair within k mismatches into its outputs.  On ix->st; waits for the
+// result.
+template <class Op>
+static int ot_join(crp_offtarget *ix, const unsigned long long *d_keys, uint64_t n, uint32_t k, const Op &op) {
+    using Site = typename Op::Site;
     cudaStream_t st = ix->st;
     const size_t tbl = kOtBuckets + 1;
-    uint32_t *d_tbl = nullptr, *d_sites = nullptr;
+    uint32_t *d_tbl = nullptr;
+    Site *d_sites = nullptr;
     uint2 *d_q = nullptr;
     unsigned long long *d_misc = nullptr;      // [0] comparisons, [1] overflow flag
-    const size_t site_bytes = list ? sizeof(uint2) : sizeof(uint32_t);
     if (dev_alloc(&d_tbl, 7 * tbl * sizeof(uint32_t), st) != cudaSuccess ||
-        dev_alloc(&d_sites, (ix->n_sites + 8) * site_bytes, st) != cudaSuccess ||
+        dev_alloc(&d_sites, (ix->n_sites + 8) * sizeof(Site), st) != cudaSuccess ||
         dev_alloc(&d_q, (n + 1) * sizeof(uint2), st) != cudaSuccess ||
         dev_alloc(&d_misc, 2 * sizeof(unsigned long long), st) != cudaSuccess) {
         cudaGetLastError();
@@ -2143,35 +2144,13 @@ static int ot_count(crp_offtarget *ix, const unsigned long long *d_keys, uint64_
     sa.item_off = d_tbl + 6 * tbl;
     sa.comparisons = d_misc;
     sa.overflow = reinterpret_cast<unsigned int *>(d_misc + 1);
-    OtCountArgs ca;
-    ca.sites = d_sites;
-    ca.queries = d_q;
-    ca.soff = sa.off[0];
-    ca.qoff = sa.off[1];
-    ca.item_off = sa.item_off;
-    ca.counts = d_counts;
-    ca.k = k;
-    OtListArgs la = {};
-    if (list) {
-        la = *list;
-        la.sites = reinterpret_cast<const uint2 *>(d_sites);
-        la.queries = d_q;
-        la.soff = sa.off[0];
-        la.qoff = sa.off[1];
-        la.item_off = sa.item_off;
-        la.loci = ix->loci;
-        la.k = k;
-    }
-    OtScoreArgs sc = {};
-    if (score) {
-        sc = *score;
-        sc.sites = d_sites;
-        sc.queries = d_q;
-        sc.soff = sa.off[0];
-        sc.qoff = sa.off[1];
-        sc.item_off = sa.item_off;
-        sc.k = k;
-    }
+    OtJoin ja;
+    ja.sites = d_sites;
+    ja.queries = d_q;
+    ja.soff = sa.off[0];
+    ja.qoff = sa.off[1];
+    ja.item_off = sa.item_off;
+    ja.k = k;
     auto grid = [](uint64_t items) { return (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((items + 255) / 256, (uint64_t)g_ctx.sm_count * 16)); };
     int rc = 0;
     unsigned long long misc[2] = {0, 0};
@@ -2181,7 +2160,9 @@ static int ot_count(crp_offtarget *ix, const unsigned long long *d_keys, uint64_
     for (int p = 0; p < kOtPairs && !rc && n && ix->n_sites; ++p) {
         int i = 0, j = 0;
         ot_pair(p, i, j);
-        ca.jm1 = (uint32_t)(j - 1);
+        ja.jm1 = (uint32_t)(j - 1);
+        ja.pi = i;
+        ja.pj = j;
         if (cudaMemsetAsync(d_tbl, 0, 2 * tbl * sizeof(uint32_t), st) != cudaSuccess) {
             rc = fail(CRP_ERR_CUDA, "memset failed");
             break;
@@ -2189,23 +2170,12 @@ static int ot_count(crp_offtarget *ix, const unsigned long long *d_keys, uint64_
         k_ot_hist<<<grid(ix->n_sites), 256, 0, st>>>(ix->keys, ix->n_sites, i, j, hist_s);
         k_ot_hist<<<grid(n), 256, 0, st>>>(d_keys, n, i, j, hist_q);
         k_ot_scan<<<3, kOtScanThreads, 0, st>>>(sa);
-        if (list)                              // {rest key, site index}: the query form of the scatter
-            k_ot_scatter<<<grid(ix->n_sites), 256, 0, st>>>(ix->keys, ix->n_sites, i, j, sa.cursor[0], nullptr,
-                                                             reinterpret_cast<uint2 *>(d_sites));
+        if constexpr (std::is_same_v<Site, uint2>)   // {rest key, site index}: the query form of the scatter
+            k_ot_scatter<<<grid(ix->n_sites), 256, 0, st>>>(ix->keys, ix->n_sites, i, j, sa.cursor[0], nullptr, d_sites);
         else
             k_ot_scatter<<<grid(ix->n_sites), 256, 0, st>>>(ix->keys, ix->n_sites, i, j, sa.cursor[0], d_sites, nullptr);
         k_ot_scatter<<<grid(n), 256, 0, st>>>(d_keys, n, i, j, sa.cursor[1], nullptr, d_q);
-        if (list) {
-            la.jm1 = ca.jm1;
-            k_ot_list<<<(unsigned)g_ctx.sm_count * 8, kOtThreads, 0, st>>>(la);
-        } else if (score) {
-            sc.jm1 = ca.jm1;
-            sc.pi = i;
-            sc.pj = j;
-            k_ot_score<<<(unsigned)g_ctx.sm_count * 8, kOtThreads, 0, st>>>(sc);
-        } else {
-            k_ot_count<<<(unsigned)g_ctx.sm_count * 8, kOtThreads, 0, st>>>(ca);
-        }
+        k_ot_join<Op><<<(unsigned)g_ctx.sm_count * 8, kOtThreads, 0, st>>>(ja, op);
         g_ctx.launches += 6;
         if (cudaGetLastError() != cudaSuccess) rc = fail(CRP_ERR_CUDA, "off-target launch failed");
     }
@@ -2213,13 +2183,97 @@ static int ot_count(crp_offtarget *ix, const unsigned long long *d_keys, uint64_
                 cudaMemcpyAsync(misc, d_misc, sizeof misc, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
                 cudaStreamSynchronize(st) != cudaSuccess ||
                 cudaEventElapsedTime(&ix->ms_count, ix->ev[2], ix->ev[3]) != cudaSuccess))
-        rc = fail(CRP_ERR_CUDA, "off-target count failed: %s", cudaGetErrorString(cudaGetLastError()));
+        rc = fail(CRP_ERR_CUDA, "off-target join failed: %s", cudaGetErrorString(cudaGetLastError()));
     if (!rc && misc[1]) rc = fail(CRP_ERR_RANGE, "a part pair needs 2^32 work items or more");
     if (!rc) ix->comparisons = misc[0];
     dev_free(d_tbl, st);
     dev_free(d_sites, st);
     dev_free(d_q, st);
     dev_free(d_misc, st);
+    return rc;
+}
+
+// The checks of a *_candidates call, in this order: CRP_ERR_ARG for a NULL index or result, a strand other than '+' /
+// '-' or max_mm above 3; CRP_ERR_STATE if `loci` and the index keeps none, for a guide length other than 20, or if
+// the result's genome is not in the index.  `what` names the mode's output.
+static int ot_check_candidates(const crp_offtarget *ix, const crp_result *res, char strand, uint32_t max_mm,
+                               const char *what, bool loci) {
+    if (!ix || !res) return fail(CRP_ERR_ARG, "NULL argument");
+    if (int rc = need_ctx()) return rc;
+    if (strand != '+' && strand != '-') return fail(CRP_ERR_ARG, "strand must be '+' or '-'");
+    if (max_mm > 3) return fail(CRP_ERR_ARG, "max_mm %u: at most 3 mismatches", max_mm);
+    if (loci && !ix->with_loci) return fail(CRP_ERR_STATE, "listing needs an index with loci (crp_offtarget_new_with_loci)");
+    if (res->guide_len != 20) return fail(CRP_ERR_STATE, "off-target %s are defined for guide_len 20 only", what);
+    if (std::find(ix->genomes.begin(), ix->genomes.end(), res->g) == ix->genomes.end())
+        return fail(CRP_ERR_STATE, "the result's genome has not been added to the index");
+    return 0;
+}
+
+// The query keys of strand stream s of a checked result into *d_keys [n] (k_ot_queries), on ix->st behind the scan's
+// stream.  d_counts [n][k1], when not NULL, gets every row's primed counts.  *d_seg keeps the segment table
+// (ot_segment_table) for k_ot_gather.  The caller frees *d_keys and *d_seg, also after a failure.
+static int ot_candidate_keys(crp_offtarget *ix, const crp_result *res, int s, uint32_t *d_counts, uint32_t k1,
+                             unsigned long long **d_keys, uint32_t **d_seg) {
+    const uint64_t n = s == 0 ? res->n_plus : res->n_minus;
+    const uint32_t n_seg = (uint32_t)(s == 0 ? res->seg_plus : res->seg_minus).size();
+    const std::vector<uint32_t> seg = ot_segment_table(res, s);
+    cudaStream_t st = ix->st;
+    CUDA_TRY(cudaEventRecord(ix->ev[4], res->st));             // the candidate streams are written on the scan's stream
+    CUDA_TRY(cudaStreamWaitEvent(st, ix->ev[4], 0));
+    if (dev_alloc(d_seg, seg.size() * sizeof(uint32_t), st) != cudaSuccess ||
+        dev_alloc(d_keys, n * sizeof(unsigned long long), st) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu query rows failed", (unsigned long long)n);
+    }
+    if (cudaMemcpyAsync(*d_seg, seg.data(), seg.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "H2D of the segment table failed");
+    OtQueryArgs a;
+    a.records = res->g->records;
+    a.pos = res->pos[s];
+    a.n = n;
+    a.seg_row = *d_seg;
+    a.seg_tile = *d_seg + n_seg + 1;
+    a.seg_begin = *d_seg + 2 * (size_t)n_seg + 1;
+    a.n_seg = n_seg;
+    a.k1 = k1;
+    a.minus = s;
+    a.keys = *d_keys;
+    a.counts = d_counts;
+    k_ot_queries<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a);
+    g_ctx.launches++;
+    if (cudaGetLastError() != cudaSuccess) return fail(CRP_ERR_CUDA, "off-target query keys failed");
+    return 0;
+}
+
+// The keys of a *_keys call: CRP_ERR_ARG if NULL or if a key has bits above bit 39, CRP_ERR_RANGE for more than
+// 2^32 - 1 keys.
+static int ot_check_keys(uint64_t n, const uint64_t *keys) {
+    if (!keys) return fail(CRP_ERR_ARG, "keys is NULL");
+    if (n > 0xFFFFFFFFull) return fail(CRP_ERR_RANGE, "at most 2^32 - 1 keys per call");
+    for (uint64_t i = 0; i < n; ++i)
+        if (keys[i] >> 40) return fail(CRP_ERR_ARG, "key %llu has bits above bit 39", (unsigned long long)i);
+    return 0;
+}
+
+// Checked keys into *d_keys [n] on ix->st; the caller frees *d_keys, also after a failure.
+static int ot_upload_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys, unsigned long long **d_keys) {
+    if (dev_alloc(d_keys, n * sizeof(unsigned long long), ix->st) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu keys failed", (unsigned long long)n);
+    }
+    if (cudaMemcpyAsync(*d_keys, keys, n * sizeof(uint64_t), cudaMemcpyHostToDevice, ix->st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "H2D of the keys failed");
+    return 0;
+}
+
+// Counts of n queries whose keys are on the device: d_counts [n][k + 1], primed by the caller, to counts on the host.
+static int ot_count(crp_offtarget *ix, const unsigned long long *d_keys, uint64_t n, uint32_t k, uint32_t *d_counts,
+                    uint32_t *counts) {
+    cudaStream_t st = ix->st;
+    int rc = ot_join(ix, d_keys, n, k, OtCount{d_counts});
+    if (!rc && (cudaMemcpyAsync(counts, d_counts, n * (k + 1) * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+                cudaStreamSynchronize(st) != cudaSuccess))
+        rc = fail(CRP_ERR_CUDA, "D2H of the off-target counts failed");
     return rc;
 }
 
@@ -2363,57 +2417,22 @@ int crp_offtarget_fetch_sites(const crp_offtarget *ix, uint64_t capacity, uint64
 }
 
 int crp_offtarget_count_candidates(crp_offtarget *ix, const crp_result *res, char strand, uint32_t max_mm, uint32_t *counts) {
-    if (!ix || !res) return fail(CRP_ERR_ARG, "NULL argument");
-    if (int rc = need_ctx()) return rc;
-    if (strand != '+' && strand != '-') return fail(CRP_ERR_ARG, "strand must be '+' or '-'");
-    if (max_mm > 3) return fail(CRP_ERR_ARG, "max_mm %u: at most 3 mismatches", max_mm);
-    if (res->guide_len != 20) return fail(CRP_ERR_STATE, "off-target counts are defined for guide_len 20 only");
-    const crp_genome *g = res->g;
-    if (std::find(ix->genomes.begin(), ix->genomes.end(), g) == ix->genomes.end())
-        return fail(CRP_ERR_STATE, "the result's genome has not been added to the index");
+    if (int rc = ot_check_candidates(ix, res, strand, max_mm, "counts", false)) return rc;
     const int s = strand == '+' ? 0 : 1;
     const uint64_t n = s == 0 ? res->n_plus : res->n_minus;
     if (n == 0) return 0;
     if (!counts) return fail(CRP_ERR_ARG, "counts is NULL");
-    const uint32_t n_seg = (uint32_t)(s == 0 ? res->seg_plus : res->seg_minus).size();
-    const std::vector<uint32_t> seg = ot_segment_table(res, s);
     cudaStream_t st = ix->st;
-    CUDA_TRY(cudaEventRecord(ix->ev[4], res->st));             // the candidate streams are written on the scan's stream
-    CUDA_TRY(cudaStreamWaitEvent(st, ix->ev[4], 0));
     const uint32_t k1 = max_mm + 1;
     uint32_t *d_seg = nullptr, *d_counts = nullptr;
     unsigned long long *d_keys = nullptr;
-    if (dev_alloc(&d_seg, seg.size() * sizeof(uint32_t), st) != cudaSuccess ||
-        dev_alloc(&d_keys, n * sizeof(unsigned long long), st) != cudaSuccess ||
-        dev_alloc(&d_counts, n * k1 * sizeof(uint32_t), st) != cudaSuccess) {
-        cudaGetLastError();
-        dev_free(d_seg, st);
-        dev_free(d_keys, st);
-        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu query rows failed", (unsigned long long)n);
-    }
     int rc = 0;
-    if (cudaMemcpyAsync(d_seg, seg.data(), seg.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
-        rc = fail(CRP_ERR_CUDA, "H2D of the segment table failed");
-    if (!rc) {
-        OtQueryArgs a;
-        a.records = g->records;
-        a.pos = res->pos[s];
-        a.n = n;
-        a.seg_row = d_seg;
-        a.seg_tile = d_seg + n_seg + 1;
-        a.seg_begin = d_seg + 2 * (size_t)n_seg + 1;
-        a.n_seg = n_seg;
-        a.k1 = k1;
-        a.minus = s;
-        a.keys = d_keys;
-        a.counts = d_counts;
-        k_ot_queries<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a);
-        g_ctx.launches++;
-        rc = ot_count(ix, d_keys, n, max_mm, d_counts);
+    if (dev_alloc(&d_counts, n * k1 * sizeof(uint32_t), st) != cudaSuccess) {
+        cudaGetLastError();
+        rc = fail(CRP_ERR_NOMEM, "cudaMalloc of %llu query rows failed", (unsigned long long)n);
     }
-    if (!rc && (cudaMemcpyAsync(counts, d_counts, n * k1 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-                cudaStreamSynchronize(st) != cudaSuccess))
-        rc = fail(CRP_ERR_CUDA, "D2H of the off-target counts failed");
+    if (!rc) rc = ot_candidate_keys(ix, res, s, d_counts, k1, &d_keys, &d_seg);
+    if (!rc) rc = ot_count(ix, d_keys, n, max_mm, d_counts, counts);
     dev_free(d_seg, st);
     dev_free(d_keys, st);
     dev_free(d_counts, st);
@@ -2425,28 +2444,20 @@ int crp_offtarget_count_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys
     if (int rc = need_ctx()) return rc;
     if (max_mm > 3) return fail(CRP_ERR_ARG, "max_mm %u: at most 3 mismatches", max_mm);
     if (n == 0) return 0;
-    if (!keys || !counts) return fail(CRP_ERR_ARG, "NULL argument");
-    if (n > 0xFFFFFFFFull) return fail(CRP_ERR_RANGE, "at most 2^32 - 1 keys per call");
-    for (uint64_t i = 0; i < n; ++i)
-        if (keys[i] >> 40) return fail(CRP_ERR_ARG, "key %llu has bits above bit 39", (unsigned long long)i);
+    if (!counts) return fail(CRP_ERR_ARG, "counts is NULL");
+    if (int rc = ot_check_keys(n, keys)) return rc;
     cudaStream_t st = ix->st;
     const uint32_t k1 = max_mm + 1;
     unsigned long long *d_keys = nullptr;
     uint32_t *d_counts = nullptr;
-    if (dev_alloc(&d_keys, n * sizeof(unsigned long long), st) != cudaSuccess ||
-        dev_alloc(&d_counts, n * k1 * sizeof(uint32_t), st) != cudaSuccess) {
+    int rc = ot_upload_keys(ix, n, keys, &d_keys);
+    if (!rc && dev_alloc(&d_counts, n * k1 * sizeof(uint32_t), st) != cudaSuccess) {
         cudaGetLastError();
-        dev_free(d_keys, st);
-        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu keys failed", (unsigned long long)n);
+        rc = fail(CRP_ERR_NOMEM, "cudaMalloc of %llu keys failed", (unsigned long long)n);
     }
-    int rc = 0;
-    if (cudaMemcpyAsync(d_keys, keys, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemsetAsync(d_counts, 0, n * k1 * sizeof(uint32_t), st) != cudaSuccess)
-        rc = fail(CRP_ERR_CUDA, "H2D of the keys failed");
-    if (!rc) rc = ot_count(ix, d_keys, n, max_mm, d_counts);
-    if (!rc && (cudaMemcpyAsync(counts, d_counts, n * k1 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-                cudaStreamSynchronize(st) != cudaSuccess))
-        rc = fail(CRP_ERR_CUDA, "D2H of the off-target counts failed");
+    if (!rc && cudaMemsetAsync(d_counts, 0, n * k1 * sizeof(uint32_t), st) != cudaSuccess)
+        rc = fail(CRP_ERR_CUDA, "memset failed");
+    if (!rc) rc = ot_count(ix, d_keys, n, max_mm, d_counts, counts);
     dev_free(d_keys, st);
     dev_free(d_counts, st);
     return rc;
@@ -2492,15 +2503,7 @@ static int ot_list(crp_offtarget *ix, const unsigned long long *d_keys, const un
         cudaMemsetAsync(d_cursor, 0, n * sizeof(uint32_t), st) != cudaSuccess ||
         cudaMemsetAsync(d_flag, 0, sizeof(unsigned int), st) != cudaSuccess)
         rc = fail(CRP_ERR_CUDA, "listing setup failed");
-    if (!rc) {
-        OtListArgs la = {};
-        la.own = d_own;
-        la.first = d_first;
-        la.cursor = d_cursor;
-        la.out = d_out;
-        la.overflow = d_flag;
-        rc = ot_count(ix, d_keys, n, k, nullptr, &la);
-    }
+    if (!rc) rc = ot_join(ix, d_keys, n, k, OtList{ix->loci, d_own, d_first, d_cursor, d_out, d_flag});
     std::vector<uint32_t> found(rc ? 0 : n);
     unsigned int flag = 0;
     if (!rc && (cudaMemcpyAsync(found.data(), d_cursor, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
@@ -2536,15 +2539,7 @@ extern "C" {
 
 int crp_offtarget_list_candidates(crp_offtarget *ix, const crp_result *res, char strand, uint32_t max_mm, uint64_t n_rows,
                                   const uint32_t *rows, const uint64_t *first, uint32_t *sites) {
-    if (!ix || !res) return fail(CRP_ERR_ARG, "NULL argument");
-    if (int rc = need_ctx()) return rc;
-    if (strand != '+' && strand != '-') return fail(CRP_ERR_ARG, "strand must be '+' or '-'");
-    if (max_mm > 3) return fail(CRP_ERR_ARG, "max_mm %u: at most 3 mismatches", max_mm);
-    if (!ix->with_loci) return fail(CRP_ERR_STATE, "listing needs an index with loci (crp_offtarget_new_with_loci)");
-    if (res->guide_len != 20) return fail(CRP_ERR_STATE, "off-target listings are defined for guide_len 20 only");
-    const crp_genome *g = res->g;
-    const auto gi = std::find(ix->genomes.begin(), ix->genomes.end(), g);
-    if (gi == ix->genomes.end()) return fail(CRP_ERR_STATE, "the result's genome has not been added to the index");
+    if (int rc = ot_check_candidates(ix, res, strand, max_mm, "listings", true)) return rc;
     if (n_rows == 0) return 0;
     if (!rows) return fail(CRP_ERR_ARG, "rows is NULL");
     if (int rc = ot_check_first(n_rows, first)) return rc;
@@ -2555,62 +2550,36 @@ int crp_offtarget_list_candidates(crp_offtarget *ix, const crp_result *res, char
         if (rows[i] >= n || (i && rows[i] <= rows[i - 1]))
             return fail(CRP_ERR_ARG, "rows[%llu] = %u: rows must be ascending, distinct and below %llu", (unsigned long long)i,
                         rows[i], (unsigned long long)n);
-    const uint32_t n_seg = (uint32_t)(s == 0 ? res->seg_plus : res->seg_minus).size();
-    const std::vector<uint32_t> seg = ot_segment_table(res, s);
     cudaStream_t st = ix->st;
-    CUDA_TRY(cudaEventRecord(ix->ev[4], res->st));
-    CUDA_TRY(cudaStreamWaitEvent(st, ix->ev[4], 0));
-    uint32_t *d_seg = nullptr, *d_scratch = nullptr, *d_rows = nullptr;
+    uint32_t *d_seg = nullptr, *d_rows = nullptr;
     unsigned long long *d_keys = nullptr, *d_sel = nullptr;   // d_sel: [n_rows] keys, [n_rows] own loci
     unsigned int *d_invalid = nullptr;
-    if (dev_alloc(&d_seg, seg.size() * sizeof(uint32_t), st) != cudaSuccess ||
-        dev_alloc(&d_keys, n * sizeof(unsigned long long), st) != cudaSuccess ||
-        dev_alloc(&d_scratch, n * sizeof(uint32_t), st) != cudaSuccess ||
-        dev_alloc(&d_rows, n_rows * sizeof(uint32_t), st) != cudaSuccess ||
-        dev_alloc(&d_sel, 2 * n_rows * sizeof(unsigned long long), st) != cudaSuccess ||
-        dev_alloc(&d_invalid, sizeof(unsigned int), st) != cudaSuccess) {
+    int rc = ot_candidate_keys(ix, res, s, nullptr, 0, &d_keys, &d_seg);   // every row's key, then the selected rows
+    if (!rc && (dev_alloc(&d_rows, n_rows * sizeof(uint32_t), st) != cudaSuccess ||
+                dev_alloc(&d_sel, 2 * n_rows * sizeof(unsigned long long), st) != cudaSuccess ||
+                dev_alloc(&d_invalid, sizeof(unsigned int), st) != cudaSuccess)) {
         cudaGetLastError();
-        dev_free(d_seg, st);
-        dev_free(d_keys, st);
-        dev_free(d_scratch, st);
-        dev_free(d_rows, st);
-        dev_free(d_sel, st);
-        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu query rows failed", (unsigned long long)n);
+        rc = fail(CRP_ERR_NOMEM, "cudaMalloc of %llu selected rows failed", (unsigned long long)n_rows);
     }
-    int rc = 0;
-    unsigned int invalid = 0;
-    if (cudaMemcpyAsync(d_seg, seg.data(), seg.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemcpyAsync(d_rows, rows, n_rows * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemsetAsync(d_invalid, 0, sizeof(unsigned int), st) != cudaSuccess)
+    if (!rc && (cudaMemcpyAsync(d_rows, rows, n_rows * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+                cudaMemsetAsync(d_invalid, 0, sizeof(unsigned int), st) != cudaSuccess))
         rc = fail(CRP_ERR_CUDA, "H2D of the listing rows failed");
-    if (!rc) {                                                 // every row's key, then the selected rows
-        OtQueryArgs a;
-        a.records = g->records;
-        a.pos = res->pos[s];
-        a.n = n;
-        a.seg_row = d_seg;
-        a.seg_tile = d_seg + n_seg + 1;
-        a.seg_begin = d_seg + 2 * (size_t)n_seg + 1;
-        a.n_seg = n_seg;
-        a.k1 = 1;
-        a.minus = s;
-        a.keys = d_keys;
-        a.counts = d_scratch;
-        k_ot_queries<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a);
+    unsigned int invalid = 0;
+    if (!rc) {
         OtGatherArgs ga;
         ga.keys = d_keys;
         ga.pos = res->pos[s];
         ga.rows = d_rows;
         ga.seg_row = d_seg;
         ga.n = n_rows;
-        ga.n_seg = n_seg;
-        ga.genome = (uint32_t)(gi - ix->genomes.begin());
+        ga.n_seg = (uint32_t)(s == 0 ? res->seg_plus : res->seg_minus).size();
+        ga.genome = (uint32_t)(std::find(ix->genomes.begin(), ix->genomes.end(), res->g) - ix->genomes.begin());
         ga.minus = s;
         ga.sel_keys = d_sel;
         ga.own = d_sel + n_rows;
         ga.invalid = d_invalid;
         k_ot_gather<<<(unsigned)((n_rows + 255) / 256), 256, 0, st>>>(ga);
-        g_ctx.launches += 2;
+        g_ctx.launches++;
         if (cudaGetLastError() != cudaSuccess ||
             cudaMemcpyAsync(&invalid, d_invalid, sizeof invalid, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
             cudaStreamSynchronize(st) != cudaSuccess)
@@ -2620,7 +2589,6 @@ int crp_offtarget_list_candidates(crp_offtarget *ix, const crp_result *res, char
     if (!rc) rc = ot_list(ix, d_sel, d_sel + n_rows, n_rows, max_mm, first, sites);
     dev_free(d_seg, st);
     dev_free(d_keys, st);
-    dev_free(d_scratch, st);
     dev_free(d_rows, st);
     dev_free(d_sel, st);
     dev_free(d_invalid, st);
@@ -2634,23 +2602,13 @@ int crp_offtarget_list_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys,
     if (max_mm > 3) return fail(CRP_ERR_ARG, "max_mm %u: at most 3 mismatches", max_mm);
     if (!ix->with_loci) return fail(CRP_ERR_STATE, "listing needs an index with loci (crp_offtarget_new_with_loci)");
     if (n == 0) return 0;
-    if (!keys) return fail(CRP_ERR_ARG, "keys is NULL");
-    if (n > 0xFFFFFFFFull) return fail(CRP_ERR_RANGE, "at most 2^32 - 1 keys per call");
-    for (uint64_t i = 0; i < n; ++i)
-        if (keys[i] >> 40) return fail(CRP_ERR_ARG, "key %llu has bits above bit 39", (unsigned long long)i);
+    if (int rc = ot_check_keys(n, keys)) return rc;
     if (int rc = ot_check_first(n, first)) return rc;
     if (first[n] && !sites) return fail(CRP_ERR_ARG, "sites is NULL");
-    cudaStream_t st = ix->st;
     unsigned long long *d_keys = nullptr;
-    if (dev_alloc(&d_keys, n * sizeof(unsigned long long), st) != cudaSuccess) {
-        cudaGetLastError();
-        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu keys failed", (unsigned long long)n);
-    }
-    int rc = 0;
-    if (cudaMemcpyAsync(d_keys, keys, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
-        rc = fail(CRP_ERR_CUDA, "H2D of the keys failed");
+    int rc = ot_upload_keys(ix, n, keys, &d_keys);
     if (!rc) rc = ot_list(ix, d_keys, nullptr, n, max_mm, first, sites);
-    dev_free(d_keys, st);
+    dev_free(d_keys, ix->st);
     return rc;
 }
 
@@ -2666,9 +2624,9 @@ static int ot_check_weights(uint32_t k, const uint32_t *weights) {
     return 0;
 }
 
-// Weight sums of n queries whose keys are on the device into d_sums [n] (primed by the caller), on ix->st.
+// Weight sums of n queries whose keys are on the device: d_sums [n], primed by the caller, to sums on the host.
 static int ot_score(crp_offtarget *ix, const unsigned long long *d_keys, uint64_t n, uint32_t k, const uint32_t *weights,
-                    unsigned long long *d_sums) {
+                    unsigned long long *d_sums, uint64_t *sums) {
     cudaStream_t st = ix->st;
     uint32_t *d_w = nullptr;
     if (dev_alloc(&d_w, kOtScoreSets * sizeof(uint32_t), st) != cudaSuccess) {
@@ -2678,12 +2636,10 @@ static int ot_score(crp_offtarget *ix, const unsigned long long *d_keys, uint64_
     int rc = 0;
     if (cudaMemcpyAsync(d_w, weights, kOtScoreSets * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
         rc = fail(CRP_ERR_CUDA, "H2D of the weight table failed");
-    if (!rc) {
-        OtScoreArgs sc = {};
-        sc.weights = d_w;
-        sc.sums = d_sums;
-        rc = ot_count(ix, d_keys, n, k, nullptr, nullptr, &sc);
-    }
+    if (!rc) rc = ot_join(ix, d_keys, n, k, OtScore{d_w, d_sums});
+    if (!rc && (cudaMemcpyAsync(sums, d_sums, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+                cudaStreamSynchronize(st) != cudaSuccess))
+        rc = fail(CRP_ERR_CUDA, "D2H of the off-target scores failed");
     dev_free(d_w, st);
     return rc;
 }
@@ -2692,64 +2648,29 @@ extern "C" {
 
 int crp_offtarget_score_candidates(crp_offtarget *ix, const crp_result *res, char strand, uint32_t max_mm,
                                    const uint32_t *weights, uint64_t *sums) {
-    if (!ix || !res) return fail(CRP_ERR_ARG, "NULL argument");
-    if (int rc = need_ctx()) return rc;
-    if (strand != '+' && strand != '-') return fail(CRP_ERR_ARG, "strand must be '+' or '-'");
-    if (max_mm > 3) return fail(CRP_ERR_ARG, "max_mm %u: at most 3 mismatches", max_mm);
-    if (res->guide_len != 20) return fail(CRP_ERR_STATE, "off-target scores are defined for guide_len 20 only");
-    const crp_genome *g = res->g;
-    if (std::find(ix->genomes.begin(), ix->genomes.end(), g) == ix->genomes.end())
-        return fail(CRP_ERR_STATE, "the result's genome has not been added to the index");
+    if (int rc = ot_check_candidates(ix, res, strand, max_mm, "scores", false)) return rc;
     if (int rc = ot_check_weights(max_mm, weights)) return rc;
     const int s = strand == '+' ? 0 : 1;
     const uint64_t n = s == 0 ? res->n_plus : res->n_minus;
     if (n == 0) return 0;
     if (!sums) return fail(CRP_ERR_ARG, "sums is NULL");
-    const uint32_t n_seg = (uint32_t)(s == 0 ? res->seg_plus : res->seg_minus).size();
-    const std::vector<uint32_t> seg = ot_segment_table(res, s);
     cudaStream_t st = ix->st;
-    CUDA_TRY(cudaEventRecord(ix->ev[4], res->st));             // the candidate streams are written on the scan's stream
-    CUDA_TRY(cudaStreamWaitEvent(st, ix->ev[4], 0));
-    uint32_t *d_seg = nullptr, *d_scratch = nullptr;
+    uint32_t *d_seg = nullptr;
     unsigned long long *d_keys = nullptr, *d_sums = nullptr;
-    if (dev_alloc(&d_seg, seg.size() * sizeof(uint32_t), st) != cudaSuccess ||
-        dev_alloc(&d_keys, n * sizeof(unsigned long long), st) != cudaSuccess ||
-        dev_alloc(&d_scratch, n * sizeof(uint32_t), st) != cudaSuccess ||
-        dev_alloc(&d_sums, n * sizeof(unsigned long long), st) != cudaSuccess) {
-        cudaGetLastError();
-        dev_free(d_seg, st);
-        dev_free(d_keys, st);
-        dev_free(d_scratch, st);
-        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu query rows failed", (unsigned long long)n);
-    }
     int rc = 0;
-    if (cudaMemcpyAsync(d_seg, seg.data(), seg.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
-        rc = fail(CRP_ERR_CUDA, "H2D of the segment table failed");
-    if (!rc) {                                                 // the query keys (counts to scratch), then the primed sums
-        OtQueryArgs a;
-        a.records = g->records;
-        a.pos = res->pos[s];
-        a.n = n;
-        a.seg_row = d_seg;
-        a.seg_tile = d_seg + n_seg + 1;
-        a.seg_begin = d_seg + 2 * (size_t)n_seg + 1;
-        a.n_seg = n_seg;
-        a.k1 = 1;
-        a.minus = s;
-        a.keys = d_keys;
-        a.counts = d_scratch;
-        k_ot_queries<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a);
-        k_ot_score_prime<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_keys, n, 0ull - weights[0], d_sums);
-        g_ctx.launches += 2;
-        if (cudaGetLastError() != cudaSuccess) rc = fail(CRP_ERR_CUDA, "off-target query keys failed");
+    if (dev_alloc(&d_sums, n * sizeof(unsigned long long), st) != cudaSuccess) {
+        cudaGetLastError();
+        rc = fail(CRP_ERR_NOMEM, "cudaMalloc of %llu query rows failed", (unsigned long long)n);
     }
-    if (!rc) rc = ot_score(ix, d_keys, n, max_mm, weights, d_sums);
-    if (!rc && (cudaMemcpyAsync(sums, d_sums, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-                cudaStreamSynchronize(st) != cudaSuccess))
-        rc = fail(CRP_ERR_CUDA, "D2H of the off-target scores failed");
+    if (!rc) rc = ot_candidate_keys(ix, res, s, nullptr, 0, &d_keys, &d_seg);
+    if (!rc) {                                                 // the query keys, then the primed sums
+        k_ot_score_prime<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_keys, n, 0ull - weights[0], d_sums);
+        g_ctx.launches++;
+        if (cudaGetLastError() != cudaSuccess) rc = fail(CRP_ERR_CUDA, "off-target score priming failed");
+    }
+    if (!rc) rc = ot_score(ix, d_keys, n, max_mm, weights, d_sums, sums);
     dev_free(d_seg, st);
     dev_free(d_keys, st);
-    dev_free(d_scratch, st);
     dev_free(d_sums, st);
     return rc;
 }
@@ -2761,26 +2682,18 @@ int crp_offtarget_score_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys
     if (max_mm > 3) return fail(CRP_ERR_ARG, "max_mm %u: at most 3 mismatches", max_mm);
     if (int rc = ot_check_weights(max_mm, weights)) return rc;
     if (n == 0) return 0;
-    if (!keys || !sums) return fail(CRP_ERR_ARG, "NULL argument");
-    if (n > 0xFFFFFFFFull) return fail(CRP_ERR_RANGE, "at most 2^32 - 1 keys per call");
-    for (uint64_t i = 0; i < n; ++i)
-        if (keys[i] >> 40) return fail(CRP_ERR_ARG, "key %llu has bits above bit 39", (unsigned long long)i);
+    if (!sums) return fail(CRP_ERR_ARG, "sums is NULL");
+    if (int rc = ot_check_keys(n, keys)) return rc;
     cudaStream_t st = ix->st;
     unsigned long long *d_keys = nullptr, *d_sums = nullptr;
-    if (dev_alloc(&d_keys, n * sizeof(unsigned long long), st) != cudaSuccess ||
-        dev_alloc(&d_sums, n * sizeof(unsigned long long), st) != cudaSuccess) {
+    int rc = ot_upload_keys(ix, n, keys, &d_keys);
+    if (!rc && dev_alloc(&d_sums, n * sizeof(unsigned long long), st) != cudaSuccess) {
         cudaGetLastError();
-        dev_free(d_keys, st);
-        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu keys failed", (unsigned long long)n);
+        rc = fail(CRP_ERR_NOMEM, "cudaMalloc of %llu keys failed", (unsigned long long)n);
     }
-    int rc = 0;
-    if (cudaMemcpyAsync(d_keys, keys, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemsetAsync(d_sums, 0, n * sizeof(unsigned long long), st) != cudaSuccess)
-        rc = fail(CRP_ERR_CUDA, "H2D of the keys failed");
-    if (!rc) rc = ot_score(ix, d_keys, n, max_mm, weights, d_sums);
-    if (!rc && (cudaMemcpyAsync(sums, d_sums, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-                cudaStreamSynchronize(st) != cudaSuccess))
-        rc = fail(CRP_ERR_CUDA, "D2H of the off-target scores failed");
+    if (!rc && cudaMemsetAsync(d_sums, 0, n * sizeof(unsigned long long), st) != cudaSuccess)
+        rc = fail(CRP_ERR_CUDA, "memset failed");
+    if (!rc) rc = ot_score(ix, d_keys, n, max_mm, weights, d_sums, sums);
     dev_free(d_keys, st);
     dev_free(d_sums, st);
     return rc;

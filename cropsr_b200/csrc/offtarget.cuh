@@ -24,11 +24,13 @@
 // 16-bit key of those 8 nt (a counting sort: histogram, scan, scatter) and compared within buckets on the
 // 24 bits of the other three parts.  A (query, site) pair is counted only at the pair (i, j) formed by
 // its two LOWEST exactly matching parts, so every pair with d <= k is counted exactly once; that test
-// runs only on the rare path d <= k.  The hot loop is XOR / SHF / LOP3 / POPC / compare.
+// runs only on the rare path d <= k.  The hot loop is XOR / SHF / LOP3 / POPC / compare.  One join kernel,
+// k_ot_join<Op>, serves counts, listings and scores: the mode's Op (OtCount, OtList, OtScore) decides what a pair
+// with d <= k does.
 //
 // Listing (an index built with loci): every site also has a 64-bit locus (ot_locus) at the slot of its key, and
-// k_ot_list walks the same work items as k_ot_count, storing the index of every site with d <= k in the query
-// row's slice of the output (sized by the caller from the counts) instead of counting it.
+// k_ot_join<OtList> stores the index of every site with d <= k in the query row's slice of the output (sized by
+// the caller from the counts) instead of counting it.
 //
 // Scores (oracle/offtarget_score_oracle.py states the same): the pairs are exactly those the counts count.  The
 // mismatch positions of a pair (0 = P[0], PAM-distal, .. 19) form a set of size d <= 3, ranked colexicographically:
@@ -47,7 +49,7 @@
 
 static constexpr uint32_t kOtBuckets = 1u << 16;           // 8 nt of a part pair
 static constexpr int kOtPairs = 10;
-static constexpr int kOtThreads = 128;                      // k_ot_count: CTA size = queries per work item
+static constexpr int kOtThreads = 128;                      // k_ot_join: CTA size = queries per work item
 static constexpr uint32_t kOtSiteTile = 2048;               // sites of a work item, staged in shared memory (8 KB)
 static constexpr uint32_t kOtNoCount = 0xFFFFFFFFu;         // counts of a candidate without a protospacer
 static constexpr unsigned long long kOtInvalid = 1ull << 63;   // query key: no protospacer
@@ -213,31 +215,23 @@ __global__ void __launch_bounds__(256) k_ot_sites(const OtSiteArgs a) {
     if (lane == 31 && incl) slot = atomicAdd(a.n, (unsigned long long)incl);
     slot = __shfl_sync(0xFFFFFFFFu, slot, 31) + incl - mine;
     if (!a.keys || !mine) return;
-    unsigned long long *out = a.keys + a.base + slot;
-    if constexpr (kLoci) {
-        unsigned long long *lout = a.loci + a.base + slot;
-        for (uint32_t m = plus; m; m &= m - 1)
-            if (ot_key<false>(prev, cur, next, __ffs(m) - 1, key)) {
-                *out++ = key;
-                *lout++ = ot_site_locus(desc, kw, __ffs(m) - 1, a.genome, false);
-            }
-        for (uint32_t m = minus; m; m &= m - 1)
-            if (ot_key<true>(prev, cur, next, __ffs(m) - 1, key)) {
-                *out++ = key;
-                *lout++ = ot_site_locus(desc, kw, __ffs(m) - 1, a.genome, true);
-            }
-    } else {
-        for (uint32_t m = plus; m; m &= m - 1)
-            if (ot_key<false>(prev, cur, next, __ffs(m) - 1, key)) *out++ = key;
-        for (uint32_t m = minus; m; m &= m - 1)
-            if (ot_key<true>(prev, cur, next, __ffs(m) - 1, key)) *out++ = key;
-    }
+    unsigned long long *out = a.keys + a.base + slot, *lout = kLoci ? a.loci + a.base + slot : nullptr;
+    for (uint32_t m = plus; m; m &= m - 1)
+        if (ot_key<false>(prev, cur, next, __ffs(m) - 1, key)) {
+            *out++ = key;
+            if constexpr (kLoci) *lout++ = ot_site_locus(desc, kw, __ffs(m) - 1, a.genome, false);
+        }
+    for (uint32_t m = minus; m; m &= m - 1)
+        if (ot_key<true>(prev, cur, next, __ffs(m) - 1, key)) {
+            *out++ = key;
+            if constexpr (kLoci) *lout++ = ot_site_locus(desc, kw, __ffs(m) - 1, a.genome, true);
+        }
 }
 
 // Query keys of one strand stream of a scan (rows in segment order): the protospacer is read from the tile
 // records at the candidate's (segment, t) -- not from the packed 30-mer, whose '+' windows hold the bases of
-// lower-case positions uncomplemented.  The counts row is primed: valid [-1, 0, ..] (the query's own site
-// brings mm0 to 0), invalid all kOtNoCount.
+// lower-case positions uncomplemented.  With counts, the counts row is primed: valid [-1, 0, ..] (the query's own
+// site brings mm0 to 0), invalid all kOtNoCount.
 struct OtQueryArgs {
     const uint4 *records;
     const uint32_t *pos;
@@ -247,7 +241,7 @@ struct OtQueryArgs {
     uint32_t n_seg, k1;                 // k1 = max_mm + 1 counts per query
     int minus;
     unsigned long long *keys;
-    uint32_t *counts;
+    uint32_t *counts;                   // [n][k1], or NULL
 };
 
 __global__ void k_ot_queries(const OtQueryArgs a) {
@@ -265,6 +259,7 @@ __global__ void k_ot_queries(const OtQueryArgs a) {
     const bool ok = a.minus ? ot_key<true>(rec[1 + k], rec[2 + k], rec[3 + k], b, key)
                             : ot_key<false>(rec[1 + k], rec[2 + k], rec[3 + k], b, key);
     a.keys[i] = ok ? key : kOtInvalid;
+    if (!a.counts) return;
     uint32_t *c = a.counts + i * a.k1;
     c[0] = ok ? 0xFFFFFFFFu : kOtNoCount;
     for (uint32_t d = 1; d < a.k1; ++d) c[d] = ok ? 0u : kOtNoCount;
@@ -398,24 +393,37 @@ __global__ void k_ot_scatter(const unsigned long long *__restrict__ keys, uint64
     }
 }
 
-// Work item = (query tile of <= 128 queries) x (site tile of <= 2048 sites) of one bucket, so that a bucket of
-// a repeat family (10^5 sites and more) spreads over many CTAs and an average bucket (~130 sites, configs[1])
-// is one item.  A persistent grid walks the items of the part pair; the site tile arrives by one bulk copy,
-// every thread holds one query and a slice of the tile (a tile with few queries gives each query several
-// threads), counts go to registers and are flushed with one atomic per non-zero count.
-struct OtCountArgs {
-    const uint32_t *sites;              // rest keys in bucket order
+// The join of one part pair.  Work item = (query tile of <= 128 queries) x (site tile of <= 2048 sites) of one
+// bucket, so that a bucket of a repeat family (10^5 sites and more) spreads over many CTAs and an average bucket
+// (~130 sites, configs[1]) is one item.  A persistent grid walks the items of the part pair; the site tile arrives by
+// one bulk copy, every thread holds one query and a slice of the tile (a tile with few queries gives each query
+// several threads).  What a pair with d <= k does is the mode's Op (OtCount, OtList, OtScore below):
+//   Op::Site                      the element of the site array: the rest key, or {rest key, site index}
+//   Op::Shared sh                 per CTA in shared memory, filled by op.setup(sh, tid) before the first item
+//   Op::Acc acc{}                 per thread and item
+//   op.visit(acc, sh, a, q, s, d) on the rare path d <= k
+//   op.flush(acc, a, q)           after the thread's slice of the tile
+struct OtJoin {
+    const void *sites;                  // Op::Site in bucket order
     const uint2 *queries;               // {rest key, row} in bucket order
     const uint32_t *soff, *qoff, *item_off;   // [kOtBuckets + 1]
-    uint32_t *counts;                   // [rows][k + 1]
     uint32_t k, jm1;
+    int pi, pj;                         // the part pair
 };
 
-__global__ void __launch_bounds__(kOtThreads) k_ot_count(const OtCountArgs a) {
-    __shared__ __align__(16) uint32_t s_sites[kOtSiteTile + 8];
+CRP_HD uint32_t ot_site_rest(uint32_t s) { return s; }
+CRP_HD uint32_t ot_site_rest(uint2 s) { return s.x; }
+
+template <class Op>
+__global__ void __launch_bounds__(kOtThreads) k_ot_join(const OtJoin a, const Op op) {
+    using Site = typename Op::Site;
+    constexpr uint32_t kAlign = 16 / sizeof(Site);                       // sites per 16 bytes of the bulk copy
+    __shared__ __align__(16) Site s_sites[kOtSiteTile + kAlign];         // the copy starts up to 16 bytes early
+    __shared__ typename Op::Shared sh;
     __shared__ __align__(8) unsigned long long bar;
     const uint32_t tid = threadIdx.x;
     const uint32_t total = a.item_off[kOtBuckets];
+    op.setup(sh, tid);
     if (tid == 0) {
         mbar_init(&bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -435,12 +443,12 @@ __global__ void __launch_bounds__(kOtThreads) k_ot_count(const OtCountArgs a) {
         const uint32_t qt = local / n_st, st = local % n_st;
         const uint32_t s0 = sb + st * kOtSiteTile, ns_t = min(kOtSiteTile, ns - st * kOtSiteTile);
         const uint32_t q0 = qb + qt * kOtThreads, nq_t = min((uint32_t)kOtThreads, nq - qt * kOtThreads);
-        const uint32_t a0 = s0 & ~3u;                                        // 16-byte aligned source
+        const uint32_t a0 = s0 & ~(kAlign - 1u);                             // 16-byte aligned source
         if (tid == 0) {
-            const uint32_t bytes = ((s0 + ns_t - a0) * 4u + 15u) & ~15u;
+            const uint32_t bytes = ((s0 + ns_t - a0) * (uint32_t)sizeof(Site) + 15u) & ~15u;
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // earlier generic reads of the tile come first
             mbar_expect(&bar, bytes);
-            bulk_copy(s_sites, a.sites + a0, bytes, &bar);
+            bulk_copy(s_sites, static_cast<const Site *>(a.sites) + a0, bytes, &bar);
         }
         const uint32_t g = kOtThreads / nq_t;                                // threads per query
         const bool active = tid < nq_t * g;
@@ -448,163 +456,93 @@ __global__ void __launch_bounds__(kOtThreads) k_ot_count(const OtCountArgs a) {
         mbar_wait(&bar, phase);
         phase ^= 1u;
         if (active) {
-            const uint32_t *S = s_sites + (s0 - a0);
-            uint32_t c0 = 0, c1 = 0, c2 = 0, c3 = 0;
+            const Site *S = s_sites + (s0 - a0);
+            typename Op::Acc acc{};
             for (uint32_t s = tid / nq_t; s < ns_t; s += g) {
-                const int d = ot_rest_mismatches(q.x, S[s], a.k, a.jm1);
+                const Site site = S[s];
+                const int d = ot_rest_mismatches(q.x, ot_site_rest(site), a.k, a.jm1);
                 if (d < 0) continue;
-                c0 += d == 0;
-                c1 += d == 1;
-                c2 += d == 2;
-                c3 += d == 3;
+                op.visit(acc, sh, a, q, site, d);
             }
-            uint32_t *c = a.counts + (size_t)q.y * (a.k + 1);
-            if (c0) atomicAdd(c, c0);
-            if (c1) atomicAdd(c + 1, c1);
-            if (c2) atomicAdd(c + 2, c2);
-            if (c3) atomicAdd(c + 3, c3);
+            op.flush(acc, a, q);
         }
         __syncthreads();                                                     // the tile is read before the next copy
     }
 }
 
-// Listing: the work items of k_ot_count with {rest key, site index} in the site tile (16 KB).  On the rare path
-// d <= k a thread takes a slot of the query row's slice with one atomic on the row's cursor and stores the site
-// index; a slot beyond the slice is never written -- the overflow flag is raised instead.  The query's own site
-// (d = 0, same locus) is left out.
-struct OtListArgs {
-    const uint2 *sites;                 // {rest key, site index} in bucket order
-    const uint2 *queries;               // {rest key, row} in bucket order
-    const uint32_t *soff, *qoff, *item_off;   // [kOtBuckets + 1]
+// Counts: per thread and item four register counts, flushed with one atomic per non-zero count.
+struct OtCount {
+    using Site = uint32_t;
+    struct Shared {};
+    struct Acc {
+        uint32_t c0, c1, c2, c3;
+    };
+    uint32_t *counts;                   // [rows][k + 1], primed by the caller
+    __device__ void setup(Shared &, uint32_t) const {}
+    __device__ void visit(Acc &acc, const Shared &, const OtJoin &, uint2, Site, int d) const {
+        acc.c0 += d == 0;
+        acc.c1 += d == 1;
+        acc.c2 += d == 2;
+        acc.c3 += d == 3;
+    }
+    __device__ void flush(const Acc &acc, const OtJoin &a, uint2 q) const {
+        uint32_t *c = counts + (size_t)q.y * (a.k + 1);
+        if (acc.c0) atomicAdd(c, acc.c0);
+        if (acc.c1) atomicAdd(c + 1, acc.c1);
+        if (acc.c2) atomicAdd(c + 2, acc.c2);
+        if (acc.c3) atomicAdd(c + 3, acc.c3);
+    }
+};
+
+// Listing: the sites carry their index (a 16 KB tile).  A pair takes a slot of the query row's slice with one atomic
+// on the row's cursor and stores the site index; a slot beyond the slice is never written -- the overflow flag is
+// raised instead.  The query's own site (d = 0, same locus) is left out.
+struct OtList {
+    using Site = uint2;                 // {rest key, site index}
+    struct Shared {};
+    struct Acc {};
     const unsigned long long *loci;     // [sites]
     const unsigned long long *own;      // [rows] locus of the row's own site, kOtNoLocus for none; NULL: no row has one
     const unsigned long long *first;    // [rows + 1] slice of every row in out
     uint32_t *cursor;                   // [rows] zeroed: sites found per row
     uint32_t *out;                      // [first[rows]] site indices
     unsigned int *overflow;
-    uint32_t k, jm1;
+    __device__ void setup(Shared &, uint32_t) const {}
+    __device__ void visit(Acc &, const Shared &, const OtJoin &, uint2 q, Site site, int d) const {
+        if (d == 0 && own && __ldg(loci + site.y) == __ldg(own + q.y)) return;
+        const unsigned long long b = __ldg(first + q.y), len = __ldg(first + q.y + 1) - b;
+        const uint32_t slot = atomicAdd(cursor + q.y, 1u);
+        if (slot < len) out[b + slot] = site.y;
+        else atomicOr(overflow, 1u);
+    }
+    __device__ void flush(const Acc &, const OtJoin &, uint2) const {}
 };
 
-__global__ void __launch_bounds__(kOtThreads) k_ot_list(const OtListArgs a) {
-    __shared__ __align__(16) uint2 s_sites[kOtSiteTile + 2];
-    __shared__ __align__(8) unsigned long long bar;
-    const uint32_t tid = threadIdx.x;
-    const uint32_t total = a.item_off[kOtBuckets];
-    if (tid == 0) {
-        mbar_init(&bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    uint32_t phase = 0;
-    for (uint32_t item = blockIdx.x; item < total; item += gridDim.x) {
-        uint32_t lo = 0, hi = kOtBuckets;      // bucket: last b with item_off[b] <= item
-        while (hi - lo > 1) {
-            const uint32_t mid = (lo + hi) >> 1;
-            if (__ldg(a.item_off + mid) <= item) lo = mid;
-            else hi = mid;
-        }
-        const uint32_t sb = __ldg(a.soff + lo), ns = __ldg(a.soff + lo + 1) - sb;
-        const uint32_t qb = __ldg(a.qoff + lo), nq = __ldg(a.qoff + lo + 1) - qb;
-        const uint32_t n_st = (ns + kOtSiteTile - 1) / kOtSiteTile, local = item - __ldg(a.item_off + lo);
-        const uint32_t qt = local / n_st, st = local % n_st;
-        const uint32_t s0 = sb + st * kOtSiteTile, ns_t = min(kOtSiteTile, ns - st * kOtSiteTile);
-        const uint32_t q0 = qb + qt * kOtThreads, nq_t = min((uint32_t)kOtThreads, nq - qt * kOtThreads);
-        const uint32_t a0 = s0 & ~1u;                                        // 16-byte aligned source
-        if (tid == 0) {
-            const uint32_t bytes = ((s0 + ns_t - a0) * 8u + 15u) & ~15u;
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // earlier generic reads of the tile come first
-            mbar_expect(&bar, bytes);
-            bulk_copy(s_sites, a.sites + a0, bytes, &bar);
-        }
-        const uint32_t g = kOtThreads / nq_t;                                // threads per query
-        const bool active = tid < nq_t * g;
-        const uint2 q = active ? a.queries[q0 + tid % nq_t] : make_uint2(0, 0);
-        mbar_wait(&bar, phase);
-        phase ^= 1u;
-        if (active) {
-            const uint2 *S = s_sites + (s0 - a0);
-            for (uint32_t s = tid / nq_t; s < ns_t; s += g) {
-                const uint2 site = S[s];
-                const int d = ot_rest_mismatches(q.x, site.x, a.k, a.jm1);
-                if (d < 0) continue;
-                if (d == 0 && a.own && __ldg(a.loci + site.y) == __ldg(a.own + q.y)) continue;
-                const unsigned long long b = __ldg(a.first + q.y), len = __ldg(a.first + q.y + 1) - b;
-                const uint32_t slot = atomicAdd(a.cursor + q.y, 1u);
-                if (slot < len) a.out[b + slot] = site.y;
-                else atomicOr(a.overflow, 1u);
-            }
-        }
-        __syncthreads();                                                     // the tile is read before the next copy
-    }
-}
-
-// Scores: the work items and site tiles of k_ot_count, and a copy of the weight table (5.4 KB) in shared memory.  On
-// the rare path d <= k a thread adds w[rank] of the pair's mismatch-position set to a uint64 in a register; a
-// non-zero sum is flushed with one 64-bit atomic per thread and item.  Rows are primed by the caller: a candidate
-// with -w[0] (its own site adds w[0]), a candidate without a protospacer with kOtNoScore (it joins no bucket), a
-// guide with 0.
-struct OtScoreArgs {
-    const uint32_t *sites;              // rest keys in bucket order
-    const uint2 *queries;               // {rest key, row} in bucket order
-    const uint32_t *soff, *qoff, *item_off;   // [kOtBuckets + 1]
+// Scores: a copy of the weight table (5.4 KB) in shared memory.  A pair adds w[rank] of its mismatch-position set to
+// a uint64 in a register; a non-zero sum is flushed with one 64-bit atomic per thread and item.  Rows are primed by
+// the caller: a candidate with -w[0] (its own site adds w[0]), a candidate without a protospacer with kOtNoScore (it
+// joins no bucket), a guide with 0.
+struct OtScore {
+    using Site = uint32_t;
+    struct Shared {
+        uint32_t w[kOtScoreSets];
+    };
+    struct Acc {
+        unsigned long long sum;
+    };
     const uint32_t *weights;            // [kOtScoreSets], by ot_mask_rank
     unsigned long long *sums;           // [rows]
-    uint32_t k, jm1;
-    int pi, pj;                         // the part pair
+    __device__ void setup(Shared &sh, uint32_t tid) const {
+        for (uint32_t r = tid; r < kOtScoreSets; r += kOtThreads) sh.w[r] = __ldg(weights + r);
+    }
+    __device__ void visit(Acc &acc, const Shared &sh, const OtJoin &a, uint2 q, Site site, int) const {
+        const uint32_t x = q.x ^ site;
+        acc.sum += sh.w[ot_mask_rank((x | x >> 1) & 0x555555u, a.pi, a.pj)];
+    }
+    __device__ void flush(const Acc &acc, const OtJoin &, uint2 q) const {
+        if (acc.sum) atomicAdd(sums + q.y, acc.sum);
+    }
 };
-
-__global__ void __launch_bounds__(kOtThreads) k_ot_score(const OtScoreArgs a) {
-    __shared__ __align__(16) uint32_t s_sites[kOtSiteTile + 8];
-    __shared__ uint32_t s_w[kOtScoreSets];
-    __shared__ __align__(8) unsigned long long bar;
-    const uint32_t tid = threadIdx.x;
-    const uint32_t total = a.item_off[kOtBuckets];
-    for (uint32_t r = tid; r < kOtScoreSets; r += kOtThreads) s_w[r] = __ldg(a.weights + r);
-    if (tid == 0) {
-        mbar_init(&bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    uint32_t phase = 0;
-    for (uint32_t item = blockIdx.x; item < total; item += gridDim.x) {
-        uint32_t lo = 0, hi = kOtBuckets;      // bucket: last b with item_off[b] <= item
-        while (hi - lo > 1) {
-            const uint32_t mid = (lo + hi) >> 1;
-            if (__ldg(a.item_off + mid) <= item) lo = mid;
-            else hi = mid;
-        }
-        const uint32_t sb = __ldg(a.soff + lo), ns = __ldg(a.soff + lo + 1) - sb;
-        const uint32_t qb = __ldg(a.qoff + lo), nq = __ldg(a.qoff + lo + 1) - qb;
-        const uint32_t n_st = (ns + kOtSiteTile - 1) / kOtSiteTile, local = item - __ldg(a.item_off + lo);
-        const uint32_t qt = local / n_st, st = local % n_st;
-        const uint32_t s0 = sb + st * kOtSiteTile, ns_t = min(kOtSiteTile, ns - st * kOtSiteTile);
-        const uint32_t q0 = qb + qt * kOtThreads, nq_t = min((uint32_t)kOtThreads, nq - qt * kOtThreads);
-        const uint32_t a0 = s0 & ~3u;                                        // 16-byte aligned source
-        if (tid == 0) {
-            const uint32_t bytes = ((s0 + ns_t - a0) * 4u + 15u) & ~15u;
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // earlier generic reads of the tile come first
-            mbar_expect(&bar, bytes);
-            bulk_copy(s_sites, a.sites + a0, bytes, &bar);
-        }
-        const uint32_t g = kOtThreads / nq_t;                                // threads per query
-        const bool active = tid < nq_t * g;
-        const uint2 q = active ? a.queries[q0 + tid % nq_t] : make_uint2(0, 0);
-        mbar_wait(&bar, phase);
-        phase ^= 1u;
-        if (active) {
-            const uint32_t *S = s_sites + (s0 - a0);
-            unsigned long long sum = 0;
-            for (uint32_t s = tid / nq_t; s < ns_t; s += g) {
-                const uint32_t site = S[s];
-                if (ot_rest_mismatches(q.x, site, a.k, a.jm1) < 0) continue;
-                const uint32_t x = q.x ^ site;
-                sum += s_w[ot_mask_rank((x | x >> 1) & 0x555555u, a.pi, a.pj)];
-            }
-            if (sum) atomicAdd(a.sums + q.y, sum);
-        }
-        __syncthreads();                                                     // the tile is read before the next copy
-    }
-}
 
 // The score rows of a candidate stream from the query keys k_ot_queries wrote: `own` (= -w[0]) or kOtNoScore.
 __global__ void k_ot_score_prime(const unsigned long long *__restrict__ keys, uint64_t n, unsigned long long own,

@@ -266,7 +266,21 @@ def write_gap_table(path, tokens, scan, min_len=10):
             w.writerows((key[1:], int(a), int(b)) for a, b in zip(start.tolist(), length.tolist()))
 
 
-_DNA = np.frombuffer(b"ATCG", dtype=np.uint8)
+_UPPER_DNA = np.frombuffer(b"ATCG", dtype=np.uint8)
+_COMPLEMENT = np.arange(256, dtype=np.uint8)
+_COMPLEMENT[list(b"ATCG")] = list(b"TAGC")
+
+
+def _protospacers(scan, first, seg, pos, strand):
+    """The protospacers of candidates with one, read from the host tokens: uint8 [n, 20], upper case, in the
+    orientation followed by the PAM -- '+' tok[t-20:t], '-' the reverse complement of tok[t+3:t+23].  seg: each
+    candidate's token within the part that starts at token `first`; pos: its pam_pos t."""
+    rows = []
+    for s, t in zip(seg.tolist(), pos.tolist()):
+        tok = scan.token_bytes[first + s]
+        rows.append(tok[t - 20:t] if strand == "+" else tok[t + 3:t + 23][::-1])
+    b = np.frombuffer(b"".join(rows), dtype=np.uint8).reshape(-1, 20) & 0xDF
+    return _COMPLEMENT[b] if strand == "-" else b
 
 
 def write_offtarget_table(path, tokens, scan, k=3, index=None, counts=None):
@@ -290,8 +304,8 @@ def write_offtarget_scores(path, tokens, scan, k=3, index=None):
     its order, with mit_hit_sum, the sum of the MIT hit scores (Hsu et al. 2013, CRISPOR's calcHitScore) of the
     candidate's OTHER NGG sites within k mismatches (.6f), and mit_specificity, 100 / (100 + mit_hit_sum) * 100
     rounded to an integer (CRISPOR's calcMitGuideScore); both blank where the candidate has no protospacer
-    (k_ot_score; semantics in oracle/offtarget_score_oracle.py).  CRISPOR also sums 4-mismatch and NAG / NGA sites,
-    so its numbers differ.  index: an index over the scan's genome handles, built by the caller (and not freed
+    (k_ot_join<OtScore>; semantics in oracle/offtarget_score_oracle.py).  CRISPOR also sums 4-mismatch and NAG / NGA
+    sites, so its numbers differ.  index: an index over the scan's genome handles, built by the caller (and not freed
     here), else built here."""
     weights = engine.mit_weights()
 
@@ -329,14 +343,7 @@ def _write_candidate_table(path, tokens, scan, value_columns, values, index=None
                     ok = np.zeros(0, bool)
                 proto = np.full(n, "", dtype=object)
                 if ok.any():
-                    # the protospacer from the host token: '+' tok[t-20:t], '-' the reverse complement of tok[t+3:t+23]
-                    rows = []
-                    for s, t in zip(seg_of[ok].tolist(), pos[ok].tolist()):
-                        tok = scan.token_bytes[first + s]
-                        rows.append(tok[t - 20:t] if strand == "+" else tok[t + 3:t + 23][::-1])
-                    b = np.frombuffer(b"".join(rows), dtype=np.uint8).reshape(-1, 20) & 0xDF   # upper case
-                    if strand == "-":
-                        b = np.select([b == 65, b == 84, b == 67, b == 71], [84, 65, 71, 67]).astype(np.uint8)
+                    b = _protospacers(scan, first, seg_of[ok], pos[ok], strand)
                     proto[ok] = b.view("S20").ravel().astype("U20").astype(object)
                 frame = {"chromosome": np.array([key[1:] for key in keys[first:first + cnt]], dtype=object)[seg_of]
                          if n else np.empty(0, object),
@@ -357,11 +364,6 @@ def offtarget_counts(index, scan, k=3):
     from one count per strand"""
     return {(part, strand): index.count_candidates(result, strand, k)
             for part, (_, result, _, _) in enumerate(scan.parts) for strand in "+-"}
-
-
-_UPPER_DNA = np.frombuffer(b"ATCG", dtype=np.uint8)
-_COMPLEMENT = np.arange(256, dtype=np.uint8)
-_COMPLEMENT[list(b"ATCG")] = list(b"TAGC")
 
 
 def write_offtarget_sites(path, tokens, scan, k=3, max_sites=1000, index=None, counts=None):
@@ -406,14 +408,7 @@ def write_offtarget_sites(path, tokens, scan, k=3, max_sites=1000, index=None, c
                 rows, lfirst, sites = index.list_candidates(result, strand, k, rows=rows, counts=c)
                 rows = rows.astype(np.int64)
                 pos = result.fetch(strand, want=("pos",))["pos"].astype(np.int64)
-                # the candidate's protospacer from the host token, as write_offtarget_table reads it
-                proto = []
-                for s, t in zip(seg_of[rows].tolist(), pos[rows].tolist()):
-                    tok = scan.token_bytes[first + s]
-                    proto.append(tok[t - 20:t] if strand == "+" else tok[t + 3:t + 23][::-1])
-                cb = np.frombuffer(b"".join(proto), dtype=np.uint8).reshape(-1, 20) & 0xDF
-                if strand == "-":
-                    cb = _COMPLEMENT[cb]
+                cb = _protospacers(scan, first, seg_of[rows], pos[rows], strand)
                 per = np.diff(lfirst).astype(np.int64)
                 cand = np.repeat(np.arange(len(rows)), per)
                 sk = site_keys[sites]

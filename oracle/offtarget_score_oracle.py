@@ -1,4 +1,4 @@
-"""CPU ORACLE for the opt-in off-target scores (csrc/offtarget.cuh k_ot_score, crp_offtarget_score_*,
+"""CPU ORACLE for the opt-in off-target scores (csrc/offtarget.cuh k_ot_join<OtScore>, crp_offtarget_score_*,
 engine.OffTargetIndex.score_candidates / score_guides, pipeline.write_offtarget_scores).  TEST INFRASTRUCTURE ONLY.
 
 Parity status: UNPINNED BY THE REFERENCE (it has no off-target search).  Written from the definition with Python

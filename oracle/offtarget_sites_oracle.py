@@ -1,4 +1,4 @@
-"""CPU ORACLE for the opt-in off-target listing and sites table (k_ot_list, crp_offtarget_list_*,
+"""CPU ORACLE for the opt-in off-target listing and sites table (k_ot_join<OtList>, crp_offtarget_list_*,
 engine.OffTargetIndex.list_candidates / list_guides, pipeline.write_offtarget_sites).  TEST INFRASTRUCTURE ONLY.
 
 Parity status: UNPINNED BY THE REFERENCE (it has no off-target search).  Written from the definition with Python

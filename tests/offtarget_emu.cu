@@ -3,7 +3,7 @@
 //   A  the site tests and the key builder of k_ot_sites / k_ot_queries (ot_pam_plus, ot_pam_minus, ot_key on the three
 //      record words around a position) equal a byte-by-byte reading of random tokens: every byte class, both strands,
 //      lower-case PAMs, sites straddling tile edges and token ends, segments that start or end inside a token;
-//   B  the pair rule of k_ot_count (ot_bucket, ot_rest, ot_rest_mismatches) counts a (query, site) pair with d <= 3
+//   B  the pair rule of k_ot_join (ot_bucket, ot_rest, ot_rest_mismatches) counts a (query, site) pair with d <= 3
 //      mismatches at exactly one of the 10 part pairs and a pair with d >= 4 at none: exhaustively over all 1,351
 //      mismatch-position sets of size <= 3 (random substitutions at those positions, random keys), for every k, and
 //      on a sample of larger sets.

@@ -1,7 +1,7 @@
-// TEST INFRASTRUCTURE: the rank of k_ot_score (csrc/offtarget.cuh: ot_mask_rank behind the pair rule ot_bucket /
-// ot_rest / ot_rest_mismatches of k_ot_count), run on the CPU from the SAME source.  For every part pair (i, j) and
-// every one of the 1,351 mismatch-position sets of size <= 3, query and site keys are built with substitutions at
-// exactly those positions (random keys and random substitute bases, several draws):
+// TEST INFRASTRUCTURE: the rank of k_ot_join<OtScore> (csrc/offtarget.cuh: ot_mask_rank behind the pair rule
+// ot_bucket / ot_rest / ot_rest_mismatches of k_ot_join), run on the CPU from the SAME source.  For every part pair
+// (i, j) and every one of the 1,351 mismatch-position sets of size <= 3, query and site keys are built with
+// substitutions at exactly those positions (random keys and random substitute bases, several draws):
 //   - where the pair rule keeps the set at (i, j) -- parts i and j match and no part below j other than i does --
 //     the bucket keys agree, ot_rest_mismatches returns |set| and ot_mask_rank returns the set's colex rank,
 //     computed here from binomials: {1, 21, 211}[|set| - 1] + C(a,1) + C(b,2) + C(c,3);

@@ -86,7 +86,7 @@ def test_vectorised_site_keys_equal_the_string_oracle(fasta):
 
 def test_offtarget_site_functions_and_pair_rule_on_the_cpu(tmp_path):
     """tests/offtarget_emu.cu compiles the per-site functions of k_ot_sites / k_ot_queries and the pair rule of
-    k_ot_count -- the SAME source -- for the host and checks them against byte-by-byte readings and all 1,351
+    k_ot_join -- the SAME source -- for the host and checks them against byte-by-byte readings and all 1,351
     mismatch-position sets of size <= 3."""
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
     if not os.path.exists(nvcc):

@@ -1,4 +1,4 @@
-"""Off-target scores (csrc/offtarget.cuh k_ot_score / ot_mask_rank, crp_offtarget_score_candidates / score_keys,
+"""Off-target scores (csrc/offtarget.cuh k_ot_join<OtScore> / ot_mask_rank, crp_offtarget_score_candidates / score_keys,
 engine.mit_weights / mit_specificity / OffTargetIndex.score_candidates / score_guides, pipeline.write_offtarget_scores,
 --offtarget-scores).
 
@@ -123,7 +123,7 @@ def test_hand_built_score_rows_are_what_the_definition_says():
 
 
 def test_score_rank_and_pair_rule_on_the_cpu(tmp_path):
-    """tests/offtarget_score_emu.cu compiles ot_mask_rank and the pair rule of k_ot_count / k_ot_score -- the SAME
+    """tests/offtarget_score_emu.cu compiles ot_mask_rank and the pair rule of k_ot_join -- the SAME
     source -- for the host and checks every part pair against all 1,351 mismatch-position sets of size <= 3."""
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
     if not os.path.exists(nvcc):

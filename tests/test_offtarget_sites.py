@@ -1,4 +1,4 @@
-"""Off-target loci and listing (csrc/offtarget.cuh k_ot_sites<true> / k_ot_list, crp_offtarget_new_with_loci /
+"""Off-target loci and listing (csrc/offtarget.cuh k_ot_sites<true> / k_ot_join<OtList>, crp_offtarget_new_with_loci /
 fetch_loci / list_candidates / list_keys, engine.OffTargetIndex(loci=True), pipeline.write_offtarget_sites,
 --offtarget-sites).
 

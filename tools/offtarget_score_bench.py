@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
-"""Cost of the off-target scores (csrc/offtarget.cuh: k_ot_score) next to the counts (k_ot_count) on the benchmark
-genomes:
+"""Cost of the off-target scores (csrc/offtarget.cuh: k_ot_join<OtScore>) next to the counts (k_ot_join<OtCount>) on
+the benchmark genomes:
 
     python tools/offtarget_score_bench.py [workload ...]     (default: arabidopsis maize)
 

@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""Cost of the off-target listing (csrc/offtarget.cuh: k_ot_sites<true>, k_ot_list) on the benchmark genomes:
+"""Cost of the off-target listing (csrc/offtarget.cuh: k_ot_sites<true>, k_ot_join<OtList>) on the benchmark genomes:
 
     python tools/offtarget_sites_bench.py [--tsv-max-mbp N] [workload ...]     (default: arabidopsis maize)
 
