@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # CROPSR_B200_LIB: another build of the same library (kernel experiments, tools/variants.sh)
 LIB_PATH = os.environ.get("CROPSR_B200_LIB") or os.path.join(_HERE, "libcropsr_b200.so")
 
-ABI_VERSION = 10
+ABI_VERSION = 11
 
 CRP_SCAN_DEFAULT = 0
 CRP_SCAN_NO_SCORE = 1
@@ -144,6 +144,7 @@ SIGNATURES = {
     "crp_offtarget_list_keys": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]),
     "crp_offtarget_score_candidates": (C.c_int, [C.c_void_p, C.c_void_p, C.c_char, C.c_uint32, C.c_void_p, C.c_void_p]),
     "crp_offtarget_score_keys": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]),
+    "crp_offtarget_new_pam": (C.c_int, [_vpp, C.c_char_p, C.c_int]),
     "crp_offtarget_timing": (C.c_int, [C.c_void_p, _f32p, _f32p, _u64p]),
     "crp_offtarget_free": (C.c_int, [C.c_void_p]),
 }

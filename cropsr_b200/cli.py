@@ -10,7 +10,8 @@ def build_parser():
     # line of this length (its own consistency assertion fails), and --help would crash
     p = argparse.ArgumentParser(prog="CROPSR.py", usage="CROPSR.py [-h] -f FASTA [-g GFF] [-p TXT] [-o CSV] [-l 20] [-L 200] --cas9 [-v]\n"
                                 "                 [--device N | --devices 0-7] [--side-output TSV] [--offtargets TSV] [--offtarget-sites TSV]\n"
-                                "                 [--offtarget-scores TSV] [--mismatches K] [--max-sites N] [--blas-threads N]")
+                                "                 [--offtarget-scores TSV] [--offtarget-pams NAG,NGA] [--mismatches K] [--max-sites N]\n"
+                                "                 [--blas-threads N]")
     p.add_argument("-f", "--fasta", metavar="", required=True, dest="f",
                    help="[required] path to input file in FASTA format")
     p.add_argument("-g", "--gff", metavar="", dest="g", help="path to input file in GFF format")
@@ -48,8 +49,14 @@ def build_parser():
                    help="also write a tab-separated table of off-target scores: per candidate its protospacer, the sum "
                         "of the MIT hit scores (Hsu et al. 2013, as CRISPOR computes them) of the other NGG sites of the "
                         "genome within K mismatches, and the MIT specificity 100 / (100 + sum) * 100; CRISPOR also "
-                        "counts 4-mismatch and NAG/NGA sites, so its numbers differ; -l 20 on one GPU only; the CSV is "
-                        "unaffected")
+                        "counts 4-mismatch sites, and NAG/NGA sites unless --offtarget-pams NAG,NGA is given, so its "
+                        "numbers differ; -l 20 on one GPU only; the CSV is unaffected")
+    p.add_argument("--offtarget-pams", metavar="", default=None,
+                   help="PAM patterns whose sites the off-target tables also read, besides NGG, e.g. NAG,NGA: N and "
+                        "two IUPAC letters (ACGTRYSWKMBDHV), disjoint from NGG and from each other.  --offtargets "
+                        "gains PAM_mm0 .. PAM_mmK per pattern, --offtarget-sites a site_pam column (the cap counts "
+                        "every pattern), --offtarget-scores PAM_mit_hit_sum per pattern and all_mit_specificity over "
+                        "all of them")
     p.add_argument("--mismatches", metavar="", type=int, default=3,
                    help="K of --offtargets, --offtarget-sites and --offtarget-scores: 0 to 3, default = 3")
     p.add_argument("--max-sites", metavar="", type=int, default=1000,
@@ -99,15 +106,19 @@ def main(argv=None):
     if args.verbose:
         print(banner(args))
     devices = parse_devices(args.devices) if args.devices else [args.device]
+    pams = args.offtarget_pams.split(",") if args.offtarget_pams is not None else []
     if args.offtargets is not None or args.offtarget_sites is not None or args.offtarget_scores is not None:
         from .pipeline import check_offtarget_args
         try:
             check_offtarget_args(args.l, devices, args.mismatches,
-                                 args.max_sites if args.offtarget_sites is not None else None)
+                                 args.max_sites if args.offtarget_sites is not None else None, pams)
         except ValueError as e:
             flag = ("--offtarget-sites" if args.offtarget_sites is not None else
                     "--offtargets" if args.offtargets is not None else "--offtarget-scores")
             sys.exit(f"CROPSR.py: error: {flag}: {e}")
+    elif args.offtarget_pams is not None:
+        sys.exit("CROPSR.py: error: --offtarget-pams: no off-target table asked for (--offtargets, --offtarget-sites, "
+                 "--offtarget-scores)")
     if args.side_output is not None:
         from .pipeline import check_side_output_args
         try:
@@ -120,5 +131,5 @@ def main(argv=None):
                       side_output=args.side_output, flank=args.L, annotation_info=args.p, devices=devices,
                       offtargets=args.offtargets, max_mismatches=args.mismatches,
                       offtarget_sites=args.offtarget_sites, max_sites=args.max_sites,
-                      offtarget_scores=args.offtarget_scores)
+                      offtarget_scores=args.offtarget_scores, offtarget_pams=pams)
     return 0

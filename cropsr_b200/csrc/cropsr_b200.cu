@@ -32,7 +32,7 @@
 #include "extras.cuh"
 #include "offtarget.cuh"
 
-#define CRP_ABI_VERSION 10
+#define CRP_ABI_VERSION 11
 
 static constexpr size_t kScanSmemFixed = (size_t)kStages * kRecBytes + 2 * (size_t)kListCap * sizeof(uint16_t);
 
@@ -2106,6 +2106,8 @@ struct crp_offtarget {
     unsigned long long *keys = nullptr;        // site keys of every genome added, any order
     unsigned long long *loci = nullptr;        // crp_offtarget_new_with_loci: the locus of every site, at its key's slot
     bool with_loci = false;
+    uint32_t s2 = 8, s3 = 8;                   // code sets of PAM letters 2 and 3 (ot_pam_plus_sets): {G}, {G} is NGG
+    bool own_site = true;                      // a candidate's own site is a site of the index: G in s2 and in s3
     uint64_t n_sites = 0;
     float ms_sites = 0.f, ms_count = 0.f;      // summed over add_genome / of the last count, list or score call
     uint64_t comparisons = 0;
@@ -2239,6 +2241,7 @@ static int ot_candidate_keys(crp_offtarget *ix, const crp_result *res, int s, ui
     a.minus = s;
     a.keys = *d_keys;
     a.counts = d_counts;
+    a.own = ix->own_site ? 0xFFFFFFFFu : 0u;
     k_ot_queries<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a);
     g_ctx.launches++;
     if (cudaGetLastError() != cudaSuccess) return fail(CRP_ERR_CUDA, "off-target query keys failed");
@@ -2303,6 +2306,28 @@ int crp_offtarget_new_with_loci(crp_offtarget **ix) {
     return 0;
 }
 
+int crp_offtarget_new_pam(crp_offtarget **ix, const char *pam, int with_loci) {
+    if (!ix || !pam) return fail(CRP_ERR_ARG, "NULL argument");
+    // code sets (bit c = code c, A0 T1 C2 G3) of the IUPAC letters for one to three bases
+    auto set_of = [](char ch) -> uint32_t {
+        switch (ch & ~0x20) {
+        case 'A': return 1; case 'T': return 2; case 'C': return 4; case 'G': return 8;
+        case 'R': return 9; case 'Y': return 6; case 'S': return 12; case 'W': return 3;
+        case 'K': return 10; case 'M': return 5; case 'B': return 14; case 'D': return 11;
+        case 'H': return 7; case 'V': return 13;
+        default: return 0;
+        }
+    };
+    uint32_t s2 = 0, s3 = 0;
+    if ((pam[0] & ~0x20) != 'N' || !(s2 = set_of(pam[1])) || !(s3 = set_of(pam[2])) || pam[3])
+        return fail(CRP_ERR_ARG, "PAM pattern \"%.8s\": N and two of ACGTRYSWKMBDHV expected", pam);
+    if (int rc = with_loci ? crp_offtarget_new_with_loci(ix) : crp_offtarget_new(ix)) return rc;
+    (*ix)->s2 = s2;
+    (*ix)->s3 = s3;
+    (*ix)->own_site = (s2 & 8u) && (s3 & 8u);
+    return 0;
+}
+
 int crp_offtarget_add_genome(crp_offtarget *ix, const crp_genome *g) {
     if (!ix || !g) return fail(CRP_ERR_ARG, "NULL argument");
     if (int rc = need_ctx()) return rc;
@@ -2328,15 +2353,23 @@ int crp_offtarget_add_genome(crp_offtarget *ix, const crp_genome *g) {
     a.n = d_n;
     a.loci = nullptr;
     a.genome = (uint32_t)ix->genomes.size();
+    a.s2 = ix->s2;
+    a.s3 = ix->s3;
+    const bool ngg = ix->s2 == 8u && ix->s3 == 8u;          // the NGG kernels, as before patterns existed
+    auto launch = [&](bool loci) {
+        const unsigned blocks = (unsigned)((items + 255) / 256);
+        if (loci && ngg) k_ot_sites<true, false><<<blocks, 256, 0, st>>>(a);
+        else if (loci) k_ot_sites<true, true><<<blocks, 256, 0, st>>>(a);
+        else if (ngg) k_ot_sites<false, false><<<blocks, 256, 0, st>>>(a);
+        else k_ot_sites<false, true><<<blocks, 256, 0, st>>>(a);
+        g_ctx.launches++;
+    };
     int rc = 0;
     *h_n = 0;
     // pass 1 counts, pass 2 appends behind the sites already held (the key and locus arrays grow by one copy)
     if (cudaEventRecord(ix->ev[0], st) != cudaSuccess || cudaMemsetAsync(d_n, 0, sizeof *d_n, st) != cudaSuccess)
         rc = fail(CRP_ERR_CUDA, "off-target setup failed");
-    if (!rc && items) {
-        k_ot_sites<false><<<(unsigned)((items + 255) / 256), 256, 0, st>>>(a);
-        g_ctx.launches++;
-    }
+    if (!rc && items) launch(false);
     if (!rc && (cudaMemcpyAsync(h_n, d_n, sizeof *d_n, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
                 cudaStreamSynchronize(st) != cudaSuccess))
         rc = fail(CRP_ERR_CUDA, "site count failed: %s", cudaGetErrorString(cudaGetLastError()));
@@ -2363,13 +2396,7 @@ int crp_offtarget_add_genome(crp_offtarget *ix, const crp_genome *g) {
             a.keys = keys;
             a.loci = loci;
             if (!rc && cudaMemsetAsync(d_n, 0, sizeof *d_n, st) != cudaSuccess) rc = fail(CRP_ERR_CUDA, "memset failed");
-            if (!rc) {
-                if (loci)
-                    k_ot_sites<true><<<(unsigned)((items + 255) / 256), 256, 0, st>>>(a);
-                else
-                    k_ot_sites<false><<<(unsigned)((items + 255) / 256), 256, 0, st>>>(a);
-                g_ctx.launches++;
-            }
+            if (!rc) launch(loci != nullptr);
             if (!rc && (cudaMemcpyAsync(h_n, d_n, sizeof *d_n, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
                         cudaEventRecord(ix->ev[1], st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess))
                 rc = fail(CRP_ERR_CUDA, "site keys failed: %s", cudaGetErrorString(cudaGetLastError()));
@@ -2664,7 +2691,8 @@ int crp_offtarget_score_candidates(crp_offtarget *ix, const crp_result *res, cha
     }
     if (!rc) rc = ot_candidate_keys(ix, res, s, nullptr, 0, &d_keys, &d_seg);
     if (!rc) {                                                 // the query keys, then the primed sums
-        k_ot_score_prime<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_keys, n, 0ull - weights[0], d_sums);
+        k_ot_score_prime<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_keys, n, ix->own_site ? 0ull - weights[0] : 0ull,
+                                                                      d_sums);
         g_ctx.launches++;
         if (cudaGetLastError() != cudaSuccess) rc = fail(CRP_ERR_CUDA, "off-target score priming failed");
     }

@@ -19,6 +19,15 @@
 //                   nothing subtracted.
 //   output          mm_d = number of (other) sites at exactly d mismatches, d = 0 .. k, k <= 3.
 //
+// Other PAMs (crp_offtarget_new_pam, oracle/offtarget_pam_oracle.py): an index holds the sites of one pattern N S2 S3,
+// S2 and S3 sets of codes given by the IUPAC letters A C G T R Y S W K M B D H V (N refused).  With comp(S) =
+// {c ^ 1 : c in S}:
+//   site '+' at t   tok[t+1] a base in S2, tok[t+2] a base in S3, t >= 20, tok[t-20 .. t) all bases
+//   site '-' at t   tok[t] a base in comp(S3), tok[t+1] a base in comp(S2), t + 23 <= L, tok[t+3 .. t+23) all bases
+// NGG is the definition above.  Key, mismatches and loci are unchanged.  A candidate's own site is a site of the index
+// exactly when G is in S2 and in S3; only then is it subtracted (counts, scores) -- otherwise a candidate row starts at
+// 0, as a guide's does.  The listing leaves out a site at the candidate's own locus in either case.
+//
 // Algorithm: exact pigeonhole filtering.  P is cut into 5 parts of 4 nt; with <= 3 mismatches at least
 // two parts match exactly.  For each of the 10 part pairs (i, j) sites and queries are bucketed by the
 // 16-bit key of those 8 nt (a counting sort: histogram, scan, scatter) and compared within buckets on the
@@ -42,8 +51,8 @@
 // w[rank] over its pairs (the candidate's own site, rank 0, subtracted; nothing subtracted for guides).  With the
 // table of the MIT specificity score (Hsu et al. 2013, as CRISPOR's calcHitScore computes it: score1 * score2 *
 // score3 * 100 in IEEE double, stored as round(hit * 2^24)) the sum over a candidate's NGG sites within k <= 3
-// mismatches is H * 2^24, and its specificity 100 / (100 + H) * 100.  CRISPOR sums over 4 mismatches and NAG / NGA
-// sites as well, so its numbers are not these.  Integer atomics make the sum independent of the order of the pairs.
+// mismatches is H * 2^24, and its specificity 100 / (100 + H) * 100.  CRISPOR sums over 4 mismatches as well, so its
+// numbers are not these.  Integer atomics make the sum independent of the order of the pairs.
 #pragma once
 #include "scan.cuh"
 
@@ -93,6 +102,25 @@ CRP_HD uint32_t ot_pam_plus(uint4 cur, uint4 next) {
 CRP_HD uint32_t ot_pam_minus(uint4 cur, uint4 next) {
     const uint32_t c = ~cur.x & cur.y & ~cur.w, cn = ~next.x & next.y & ~next.w;
     return c & crp_funnel_r(c, cn, 1);
+}
+
+// The same for a PAM pattern N S2 S3 (crp_offtarget_new_pam): s2, s3 are the code sets of letters 2 and 3, bit c set
+// for code c (A0 T1 C2 G3; {G} = 8 is NGG).  A letter matches a base of its set; never a non-base.
+CRP_HD uint32_t ot_pam_letter(uint4 w, uint32_t set) {
+    const uint32_t m = ((~w.x & ~w.y) & (0u - (set & 1u))) | ((w.x & ~w.y) & (0u - (set >> 1 & 1u))) |
+                       ((~w.x & w.y) & (0u - (set >> 2 & 1u))) | ((w.x & w.y) & (0u - (set >> 3 & 1u)));
+    return m & ~w.w;
+}
+// {c ^ 1 : c in set}: the letters of the '-' strand
+CRP_HD uint32_t ot_pam_comp(uint32_t set) { return (set & 5u) << 1 | (set >> 1 & 5u); }
+// '+' a letter of s2 at p0+b+1 and of s3 at p0+b+2; '-' a letter of comp(s3) at p0+b and of comp(s2) at p0+b+1
+CRP_HD uint32_t ot_pam_plus_sets(uint4 cur, uint4 next, uint32_t s2, uint32_t s3) {
+    return crp_funnel_r(ot_pam_letter(cur, s2), ot_pam_letter(next, s2), 1) &
+           crp_funnel_r(ot_pam_letter(cur, s3), ot_pam_letter(next, s3), 2);
+}
+CRP_HD uint32_t ot_pam_minus_sets(uint4 cur, uint4 next, uint32_t s2, uint32_t s3) {
+    const uint32_t c2 = ot_pam_comp(s2), c3 = ot_pam_comp(s3);
+    return ot_pam_letter(cur, c3) & crp_funnel_r(ot_pam_letter(cur, c2), ot_pam_letter(next, c2), 1);
 }
 
 // Key of the site at bit b of word `cur` from the three words around it (positions p0-32 .. p0+63):
@@ -167,7 +195,8 @@ __device__ __forceinline__ uint32_t ot_lanemask_lt() {
 // words cover the 20 positions to the left and the 23 to the right of every owned position).  keys == NULL:
 // count only.  Otherwise keys[base + slot] for an unordered slot per site, and with kLoci its locus at
 // loci[base + slot] (ot_site_locus: t and segment from the tile's descriptor word); the instantiation without loci reads
-// neither field.
+// neither field.  kSets: the sites of the PAM pattern N s2 s3 (ot_pam_plus_sets); without it NGG (ot_pam_plus), and
+// s2 / s3 are not read.
 struct OtSiteArgs {
     const uint4 *records;
     uint32_t n_tiles;
@@ -176,9 +205,10 @@ struct OtSiteArgs {
     unsigned long long *n;              // counter
     unsigned long long *loci;           // kLoci only
     uint32_t genome;                    // kLoci only: ordinal of the genome handle in the index
+    uint32_t s2, s3;                    // kSets only: code sets of PAM letters 2 and 3
 };
 
-template <bool kLoci>
+template <bool kLoci, bool kSets>
 __global__ void __launch_bounds__(256) k_ot_sites(const OtSiteArgs a) {
     const uint64_t it = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const uint32_t lane = threadIdx.x & 31;
@@ -193,8 +223,13 @@ __global__ void __launch_bounds__(256) k_ot_sites(const OtSiteArgs a) {
         if (p0 < n_owned) {
             const uint32_t own = n_owned - p0 >= 32u ? 0xFFFFFFFFu : (1u << (n_owned - p0)) - 1u;
             prev = rec[1 + k], cur = rec[2 + k], next = rec[3 + k];
-            plus = ot_pam_plus(cur, next) & own;
-            minus = ot_pam_minus(cur, next) & own;
+            if constexpr (kSets) {
+                plus = ot_pam_plus_sets(cur, next, a.s2, a.s3) & own;
+                minus = ot_pam_minus_sets(cur, next, a.s2, a.s3) & own;
+            } else {
+                plus = ot_pam_plus(cur, next) & own;
+                minus = ot_pam_minus(cur, next) & own;
+            }
             if constexpr (kLoci) {
                 desc = rec[0];
                 kw = k;
@@ -230,8 +265,8 @@ __global__ void __launch_bounds__(256) k_ot_sites(const OtSiteArgs a) {
 
 // Query keys of one strand stream of a scan (rows in segment order): the protospacer is read from the tile
 // records at the candidate's (segment, t) -- not from the packed 30-mer, whose '+' windows hold the bases of
-// lower-case positions uncomplemented.  With counts, the counts row is primed: valid [-1, 0, ..] (the query's own
-// site brings mm0 to 0), invalid all kOtNoCount.
+// lower-case positions uncomplemented.  With counts, the counts row is primed: valid [own, 0, ..], invalid all
+// kOtNoCount.  own is 0xFFFFFFFF (-1) when the query's own site is a site of the index (it brings mm0 to 0), else 0.
 struct OtQueryArgs {
     const uint4 *records;
     const uint32_t *pos;
@@ -242,6 +277,7 @@ struct OtQueryArgs {
     int minus;
     unsigned long long *keys;
     uint32_t *counts;                   // [n][k1], or NULL
+    uint32_t own;                       // mm0 of a valid row before the join
 };
 
 __global__ void k_ot_queries(const OtQueryArgs a) {
@@ -261,7 +297,7 @@ __global__ void k_ot_queries(const OtQueryArgs a) {
     a.keys[i] = ok ? key : kOtInvalid;
     if (!a.counts) return;
     uint32_t *c = a.counts + i * a.k1;
-    c[0] = ok ? 0xFFFFFFFFu : kOtNoCount;
+    c[0] = ok ? a.own : kOtNoCount;
     for (uint32_t d = 1; d < a.k1; ++d) c[d] = ok ? 0u : kOtNoCount;
 }
 

@@ -630,22 +630,55 @@ def _weights(weights):
     return w
 
 
+# PAM patterns N + two IUPAC letters (crp_offtarget_new_pam): the bases each letter stands for; N is refused there
+PAM_LETTERS = {"A": "A", "C": "C", "G": "G", "T": "T", "R": "AG", "Y": "CT", "S": "CG", "W": "AT", "K": "GT",
+               "M": "AC", "B": "CGT", "D": "AGT", "H": "ACT", "V": "ACG"}
+
+
+def parse_pam(text):
+    """A PAM pattern, upper case ('nag' -> 'NAG'): ValueError unless it is N followed by two of A C G T R Y S W K M B
+    D H V (IUPAC letters for one to three bases)."""
+    pam = str(text).upper()
+    if len(pam) != 3 or pam[0] != "N" or pam[1] not in PAM_LETTERS or pam[2] not in PAM_LETTERS:
+        raise ValueError(f"PAM pattern {text!r}: N followed by two of {''.join(PAM_LETTERS)} expected")
+    return pam
+
+
+def pams_overlap(a, b):
+    """True if a base triple matches both patterns: N a2 a3 and N b2 b3 overlap iff a2, b2 and a3, b3 share a base"""
+    a, b = parse_pam(a), parse_pam(b)
+    return all(set(PAM_LETTERS[x]) & set(PAM_LETTERS[y]) for x, y in zip(a[1:], b[1:]))
+
+
+def pam_has_own_site(pam):
+    """True if a scan candidate's own site (its NGG) is a site of the pattern: G in letters 2 and 3.  Only then do
+    its counts and score leave the site out."""
+    pam = parse_pam(pam)
+    return "G" in PAM_LETTERS[pam[1]] and "G" in PAM_LETTERS[pam[2]]
+
+
 class OffTargetIndex:
-    """NGG sites (both strands, case-insensitive) of one or more committed genomes, resident in HBM:
-    counts of sites within 0 .. k <= 3 mismatches of every scan candidate or of arbitrary guides, and with
-    loci=True the sites themselves (semantics: include/cropsr_b200.h, csrc/offtarget.cuh)."""
+    """The sites of one PAM pattern (NGG by default; both strands, case-insensitive) of one or more committed genomes,
+    resident in HBM: counts of sites within 0 .. k <= 3 mismatches of every scan candidate or of arbitrary guides,
+    their weighted scores, and with loci=True the sites themselves (semantics: include/cropsr_b200.h,
+    csrc/offtarget.cuh)."""
 
     NO_COUNT = N.OFFTARGET_NO_COUNT
     NO_SCORE = N.OFFTARGET_NO_SCORE
 
-    def __init__(self, genomes=(), loci=False):
+    def __init__(self, genomes=(), loci=False, pam="NGG"):
         """loci=True: the index also keeps every site's locus (8 bytes per site more), which site_loci and the
-        listings (list_candidates, list_guides) need."""
+        listings (list_candidates, list_guides) need.  pam: the PAM pattern (parse_pam) whose sites the index holds;
+        a candidate's own site is left out of its counts and score only where pam_has_own_site(pam)."""
+        self.pam = parse_pam(pam)
         if _device is None:
             init(0)
         self._h = C.c_void_p()
         self.loci = bool(loci)
-        check((lib.crp_offtarget_new_with_loci if self.loci else lib.crp_offtarget_new)(C.byref(self._h)))
+        if self.pam == "NGG":
+            check((lib.crp_offtarget_new_with_loci if self.loci else lib.crp_offtarget_new)(C.byref(self._h)))
+        else:
+            check(lib.crp_offtarget_new_pam(C.byref(self._h), self.pam.encode(), int(self.loci)))
         for g in genomes:
             self.add_genome(g)
 
@@ -748,7 +781,7 @@ class OffTargetIndex:
         """uint64[n_strand]: per candidate of one strand stream (stream order) the sum of weights[rank] over the
         sites its counts count (its own site not included), rank being that of the pair's mismatch-position set
         (score_sets order); NO_SCORE where the candidate has no protospacer.  weights: uint32[SCORE_SETS], each
-        < 2**31 (default mit_weights(): sums of MIT hit scores * 2**24 over NGG sites within k mismatches)."""
+        < 2**31 (default mit_weights(): sums of MIT hit scores * 2**24 over the sites within k mismatches)."""
         w = _weights(weights)
         n = int(result.n_plus if strand == "+" else result.n_minus)
         out = np.empty(n, dtype=np.uint64)

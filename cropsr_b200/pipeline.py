@@ -283,7 +283,7 @@ def _protospacers(scan, first, seg, pos, strand):
     return _COMPLEMENT[b] if strand == "-" else b
 
 
-def write_offtarget_table(path, tokens, scan, k=3, index=None, counts=None):
+def write_offtarget_table(path, tokens, scan, k=3, index=None, counts=None, extra=()):
     """Opt-in off-target table (not part of the reference's output): one row per unique candidate in
     reference order (token by token, '+' then '-', ascending t) with its protospacer as upper-case DNA
     in the orientation followed by the PAM, and the numbers of OTHER NGG sites of the whole genome at
@@ -291,31 +291,56 @@ def write_offtarget_table(path, tokens, scan, k=3, index=None, counts=None):
     and counts are blank where the candidate has none (cut off by the token end, or a byte outside
     ACGTacgt).  One index is built from every genome handle of the scan before anything is counted:
     handles split at MAX_POSITIONS_PER_GENOME see each other's sites.  index: such an index, built by the
-    caller (and not freed here); counts: offtarget_counts(index, scan, k), computed here when not given."""
+    caller (and not freed here); counts: offtarget_counts(index, scan, k), computed here when not given.
+    extra: (pam, index, counts or None) of further PAM patterns (--offtarget-pams), each adding the columns
+    {pam}_mm0 .. {pam}_mmk of the sites of its index after mm0 .. mmk, in the order given."""
+    groups = [("", index, counts)] + [(f"{pam}_", ix, c) for pam, ix, c in extra]
+
     def values(index, part, result, strand):
-        c = index.count_candidates(result, strand, k) if counts is None else counts[(part, strand)]
-        ok = c[:, 0] != index.NO_COUNT
-        return ok, {f"mm{d}": c[:, d].astype(np.int64).astype(str).astype(object) for d in range(k + 1)}
-    _write_candidate_table(path, tokens, scan, [f"mm{d}" for d in range(k + 1)], values, index)
+        out = {}
+        for prefix, ix, cnt in groups:
+            ix = index if ix is None else ix
+            c = ix.count_candidates(result, strand, k) if cnt is None else cnt[(part, strand)]
+            if not prefix:
+                ok = c[:, 0] != index.NO_COUNT
+            out.update({f"{prefix}mm{d}": c[:, d].astype(np.int64).astype(str).astype(object) for d in range(k + 1)})
+        return ok, out
+    _write_candidate_table(path, tokens, scan, [f"{prefix}mm{d}" for prefix, _, _ in groups for d in range(k + 1)],
+                           values, index)
 
 
-def write_offtarget_scores(path, tokens, scan, k=3, index=None):
+def write_offtarget_scores(path, tokens, scan, k=3, index=None, extra=()):
     """Opt-in off-target score table (not part of the reference's output): the rows of write_offtarget_table, in
     its order, with mit_hit_sum, the sum of the MIT hit scores (Hsu et al. 2013, CRISPOR's calcHitScore) of the
     candidate's OTHER NGG sites within k mismatches (.6f), and mit_specificity, 100 / (100 + mit_hit_sum) * 100
     rounded to an integer (CRISPOR's calcMitGuideScore); both blank where the candidate has no protospacer
-    (k_ot_join<OtScore>; semantics in oracle/offtarget_score_oracle.py).  CRISPOR also sums 4-mismatch and NAG / NGA
-    sites, so its numbers differ.  index: an index over the scan's genome handles, built by the caller (and not freed
-    here), else built here."""
+    (k_ot_join<OtScore>; semantics in oracle/offtarget_score_oracle.py).  CRISPOR also sums 4-mismatch sites, so its
+    numbers differ.  index: an index over the scan's genome handles, built by the caller (and not freed here), else
+    built here.  extra: (pam, index) of further PAM patterns (--offtarget-pams): one {pam}_mit_hit_sum column each, in
+    the order given, then all_mit_specificity from the exact sum of the integer sums of all patterns."""
     weights = engine.mit_weights()
+
+    def hit_sum(sums, ok):
+        hit = np.zeros(len(sums), dtype=object)
+        hit[ok] = np.char.mod("%.6f", sums[ok].astype(np.float64) / engine.SCORE_ONE).astype(object)
+        return hit
 
     def values(index, part, result, strand):
         sums = index.score_candidates(result, strand, k, weights)
         ok = sums != np.uint64(index.NO_SCORE)
-        hit = np.zeros(len(sums), dtype=object)
-        hit[ok] = np.char.mod("%.6f", sums[ok].astype(np.float64) / engine.SCORE_ONE).astype(object)
-        return ok, {"mit_hit_sum": hit, "mit_specificity": engine.mit_specificity(sums).astype(str).astype(object)}
-    _write_candidate_table(path, tokens, scan, ["mit_hit_sum", "mit_specificity"], values, index)
+        out = {"mit_hit_sum": hit_sum(sums, ok), "mit_specificity": engine.mit_specificity(sums).astype(str).astype(object)}
+        if extra:
+            total = sums.copy()
+            for pam, ix in extra:
+                s = ix.score_candidates(result, strand, k, weights)
+                out[f"{pam}_mit_hit_sum"] = hit_sum(s, ok)
+                total[ok] += s[ok]
+            out["all_mit_specificity"] = engine.mit_specificity(total).astype(str).astype(object)
+        return ok, out
+    columns = ["mit_hit_sum", "mit_specificity"]
+    if extra:
+        columns += [f"{pam}_mit_hit_sum" for pam, _ in extra] + ["all_mit_specificity"]
+    _write_candidate_table(path, tokens, scan, columns, values, index)
 
 
 def _write_candidate_table(path, tokens, scan, value_columns, values, index=None):
@@ -366,7 +391,7 @@ def offtarget_counts(index, scan, k=3):
             for part, (_, result, _, _) in enumerate(scan.parts) for strand in "+-"}
 
 
-def write_offtarget_sites(path, tokens, scan, k=3, max_sites=1000, index=None, counts=None):
+def write_offtarget_sites(path, tokens, scan, k=3, max_sites=1000, index=None, counts=None, extra=()):
     """Opt-in off-target sites table (not part of the reference's output): one row per (candidate, other NGG
     site of the genome within k mismatches), candidates in the order of write_offtarget_table, and within a
     candidate by mismatches, then the site's token (file order), site_pam_pos, '+' before '-'.  site_protospacer
@@ -374,13 +399,16 @@ def write_offtarget_sites(path, tokens, scan, k=3, max_sites=1000, index=None, c
     candidate's protospacer in lower case (semantics in oracle/offtarget_sites_oracle.py).  A candidate with no
     other site, or with more than max_sites, writes no rows: its counts are in the --offtargets table.
     index: an index with loci over the scan's genome handles in scan.parts order, built by the caller (and not
-    freed here); counts: offtarget_counts(index, scan, k).  Returns (pairs written, candidates left out by the cap)."""
+    freed here); counts: offtarget_counts(index, scan, k).  extra: (pam, index with loci, counts or None) of further PAM
+    patterns (--offtarget-pams), disjoint from NGG and from each other: their sites join the listing, a last column
+    site_pam names the pattern of each row's site, and max_sites caps a candidate's total over all patterns.  Returns
+    (pairs written, candidates left out by the cap)."""
     import csv
     import pandas as pd
     keys = list(tokens.keys())
     names = np.array([key[1:] for key in keys], dtype=object)
     columns = ["chromosome", "strand", "pam_pos", "protospacer", "site_chromosome", "site_strand", "site_pam_pos",
-               "site_protospacer", "mismatches"]
+               "site_protospacer", "mismatches"] + (["site_pam"] if extra else [])
     with open(path, "w", newline="") as f:
         csv.writer(f, delimiter="\t").writerow(columns)
     own_index = index is None
@@ -388,48 +416,56 @@ def write_offtarget_sites(path, tokens, scan, k=3, max_sites=1000, index=None, c
         index = engine.OffTargetIndex([g for g, _, _, _ in scan.parts], loci=True)
     pairs = capped = 0
     try:
-        site_keys = index.sites()
-        s_gen, s_seg, s_t, s_strand = index.site_loci()
         part_first = np.array([first for _, _, first, _ in scan.parts], dtype=np.int64)
-        s_tok = part_first[s_gen.astype(np.int64)] + s_seg.astype(np.int64) if len(site_keys) else np.zeros(0, np.int64)
+        groups = []                                     # (pam, index, counts, site keys, site token, t, strand)
+        for pam, ix, cnt in [("NGG", index, counts)] + list(extra):
+            site_keys = ix.sites()
+            s_gen, s_seg, s_t, s_strand = ix.site_loci()
+            s_tok = part_first[s_gen.astype(np.int64)] + s_seg.astype(np.int64) if len(site_keys) else np.zeros(0, np.int64)
+            groups.append((pam, ix, cnt, site_keys, s_tok, s_t.astype(np.int64), s_strand.astype(np.int64)))
         for part, (genome, result, first, cnt) in enumerate(scan.parts):
             chunks = []
             for si, (strand, seg_cnt) in enumerate((("+", result.seg_plus), ("-", result.seg_minus))):
                 seg_of = np.repeat(np.arange(cnt, dtype=np.int64), seg_cnt.astype(np.int64))
                 if not len(seg_of):
                     continue
-                c = index.count_candidates(result, strand, k) if counts is None else counts[(part, strand)]
-                ok = c[:, 0] != index.NO_COUNT
-                total = np.where(ok, c[:, :k + 1].astype(np.int64).sum(axis=1), 0)
+                cs = [ix.count_candidates(result, strand, k) if c is None else c[(part, strand)]
+                      for _, ix, c, *_ in groups]
+                ok = cs[0][:, 0] != index.NO_COUNT
+                total = np.where(ok, sum(c[:, :k + 1].astype(np.int64).sum(axis=1) for c in cs), 0)
                 capped += int((total > max_sites).sum())
                 rows = np.nonzero((total > 0) & (total <= max_sites))[0]
                 if not len(rows):
                     continue
-                rows, lfirst, sites = index.list_candidates(result, strand, k, rows=rows, counts=c)
-                rows = rows.astype(np.int64)
                 pos = result.fetch(strand, want=("pos",))["pos"].astype(np.int64)
-                cb = _protospacers(scan, first, seg_of[rows], pos[rows], strand)
-                per = np.diff(lfirst).astype(np.int64)
-                cand = np.repeat(np.arange(len(rows)), per)
-                sk = site_keys[sites]
-                sb = _UPPER_DNA[((sk[:, None] >> (2 * np.arange(20, dtype=np.uint64))) & np.uint64(3)).astype(np.intp)]
-                differ = sb != cb[cand]
-                sb = sb | (differ.astype(np.uint8) << 5)                  # lower case where the bases differ
-                mm = differ.sum(axis=1)
-                row = rows[cand]
-                site = sites.astype(np.int64)
-                chunks.append((seg_of[row], np.full(len(row), si), row, mm, s_tok[site], s_t[site].astype(np.int64),
-                               s_strand[site].astype(np.int64), pos, cb[cand], sb, strand))
+                for (pam, ix, _, site_keys, s_tok, s_t, s_strand), c in zip(groups, cs):
+                    lrows, lfirst, sites = ix.list_candidates(result, strand, k, rows=rows, counts=c)
+                    lrows = lrows.astype(np.int64)
+                    cb = _protospacers(scan, first, seg_of[lrows], pos[lrows], strand)
+                    per = np.diff(lfirst).astype(np.int64)
+                    cand = np.repeat(np.arange(len(lrows)), per)
+                    sk = site_keys[sites]
+                    sb = _UPPER_DNA[((sk[:, None] >> (2 * np.arange(20, dtype=np.uint64))) & np.uint64(3)).astype(np.intp)]
+                    differ = sb != cb[cand]
+                    sb = sb | (differ.astype(np.uint8) << 5)              # lower case where the bases differ
+                    mm = differ.sum(axis=1)
+                    row = lrows[cand]
+                    site = sites.astype(np.int64)
+                    chunks.append((seg_of[row], np.full(len(row), si), row, mm, s_tok[site], s_t[site], s_strand[site],
+                                   pos, cb[cand], sb, strand, pam))
             if not chunks:
                 continue
             frames, sort_keys = [], []
-            for seg, sidx, row, mm, tok_i, site_t, site_s, pos, cb, sb, strand in chunks:
-                frames.append(pd.DataFrame({
+            for seg, sidx, row, mm, tok_i, site_t, site_s, pos, cb, sb, strand, pam in chunks:
+                frame = {
                     "chromosome": names[first + seg], "strand": strand, "pam_pos": pos[row],
                     "protospacer": cb.view("S20").ravel().astype("U20").astype(object),
                     "site_chromosome": names[tok_i], "site_strand": np.array(["+", "-"], dtype=object)[site_s],
                     "site_pam_pos": site_t, "site_protospacer": sb.view("S20").ravel().astype("U20").astype(object),
-                    "mismatches": mm}, columns=columns))
+                    "mismatches": mm}
+                if extra:
+                    frame["site_pam"] = pam
+                frames.append(pd.DataFrame(frame, columns=columns))
                 sort_keys.append(np.stack((seg, sidx, row, mm, tok_i, site_t, site_s)))
             frame = pd.concat(frames, ignore_index=True)
             key = np.concatenate(sort_keys, axis=1)
@@ -442,9 +478,11 @@ def write_offtarget_sites(path, tokens, scan, k=3, max_sites=1000, index=None, c
     return pairs, capped
 
 
-def check_offtarget_args(guide_len, devices, max_mismatches, max_sites=None):
+def check_offtarget_args(guide_len, devices, max_mismatches, max_sites=None, pams=()):
     """The off-target tables' limits, checked before any device work: ValueError with the reason.
-    max_sites: the cap of the sites table (write_offtarget_sites), at least 1."""
+    max_sites: the cap of the sites table (write_offtarget_sites), at least 1.  pams: PAM patterns whose sites are
+    counted besides NGG (--offtarget-pams): each a pattern of engine.parse_pam, none of them overlapping NGG or
+    another (a base triple matches at most one pattern, so no site is found twice).  Returns them upper case."""
     if int(guide_len) != 20:
         raise ValueError(f"off-target counts are defined for 20-base guides, not -l {guide_len}")
     if devices is not None and len(devices) > 1:
@@ -454,6 +492,24 @@ def check_offtarget_args(guide_len, devices, max_mismatches, max_sites=None):
         raise ValueError(f"--mismatches {max_mismatches}: 0 to 3 mismatches are supported")
     if max_sites is not None and int(max_sites) < 1:
         raise ValueError(f"--max-sites {max_sites}: at least 1")
+    out = []
+    for text in pams:
+        try:
+            pam = engine.parse_pam(text)
+        except ValueError as e:
+            raise ValueError(f"--offtarget-pams: {e}") from None
+        if pam == "NGG":
+            raise ValueError("--offtarget-pams: NGG sites are always counted; list the other patterns only")
+        if engine.pams_overlap(pam, "NGG"):
+            raise ValueError(f"--offtarget-pams {pam}: it overlaps NGG, whose sites are always counted; list the bases "
+                             f"outside NGG instead (NAG instead of NRG)")
+        for other in out:
+            if other == pam:
+                raise ValueError(f"--offtarget-pams: {pam} is listed twice")
+            if engine.pams_overlap(pam, other):
+                raise ValueError(f"--offtarget-pams: {other} and {pam} overlap; the patterns must be disjoint")
+        out.append(pam)
+    return out
 
 
 def check_side_output_args(flank):
@@ -466,7 +522,7 @@ def check_side_output_args(flank):
 def run_cas9(fasta, gff, output="data.csv", guide_len=20, verbose=False, blas_threads=1,
              time_path="time.txt", out=print, side_output=None, flank=200, device_ingest=True, annotation_info=None,
              chunk_rows=None, devices=None, handle_limit=None, offtargets=None, max_mismatches=3,
-             offtarget_sites=None, max_sites=1000, offtarget_scores=None):
+             offtarget_sites=None, max_sites=1000, offtarget_scores=None, offtarget_pams=()):
     """devices: CUDA ordinals; more than one shards the genome over one process per GPU
     (cropsr_b200/multi.py) and writes the same CSV.  handle_limit: positions per genome handle
     (tests shrink it to walk the several-handles path on small inputs).  offtargets: path of the opt-in
@@ -475,9 +531,17 @@ def run_cas9(fasta, gff, output="data.csv", guide_len=20, verbose=False, blas_th
     (write_offtarget_sites: every other site within max_mismatches of every candidate with at most max_sites
     of them); with both tables one index serves both and every strand is counted once.  offtarget_scores: path of
     the opt-in off-target score table (write_offtarget_scores: MIT hit-score sum and specificity over the NGG sites
-    within max_mismatches); one index, with loci only when the sites table needs them, serves every table."""
+    within max_mismatches); one index, with loci only when the sites table needs them, serves every table.
+    offtarget_pams: PAM patterns whose sites every off-target table also reads (NAG, NGA, ...: disjoint from NGG and
+    from each other, check_offtarget_args), one index each after the NGG index; without them every table is as
+    before."""
+    pams = []
+    if offtarget_pams and offtargets is None and offtarget_sites is None and offtarget_scores is None:
+        raise ValueError("--offtarget-pams: no off-target table asked for (--offtargets, --offtarget-sites, "
+                         "--offtarget-scores)")
     if offtargets is not None or offtarget_sites is not None or offtarget_scores is not None:
-        check_offtarget_args(guide_len, devices, max_mismatches, max_sites if offtarget_sites is not None else None)
+        pams = check_offtarget_args(guide_len, devices, max_mismatches, max_sites if offtarget_sites is not None else None,
+                                    offtarget_pams)
     if side_output:
         check_side_output_args(flank)
     begin = time.time()
@@ -534,22 +598,32 @@ def run_cas9(fasta, gff, output="data.csv", guide_len=20, verbose=False, blas_th
         write_gap_table(side_output + ".gaps.tsv", tokens, scan)
     ot_stats = {}
     if offtargets is not None or offtarget_sites is not None or offtarget_scores is not None:
-        index = engine.OffTargetIndex([g for g, _, _, _ in scan.parts], loci=offtarget_sites is not None)
+        handles = [g for g, _, _, _ in scan.parts]
+        indexes = []                                    # NGG first, then the extra patterns in the order given
         try:
+            for pam in ["NGG"] + pams:
+                indexes.append(engine.OffTargetIndex(handles, loci=offtarget_sites is not None, pam=pam))
+            index = indexes[0]
             # with the sites table, each strand is counted once for both count-driven tables
-            counts = offtarget_counts(index, scan, max_mismatches) if offtarget_sites is not None else None
+            counts = [offtarget_counts(ix, scan, max_mismatches) if offtarget_sites is not None else None
+                      for ix in indexes]
+            extra = [(pam, ix, c) for pam, ix, c in zip(pams, indexes[1:], counts[1:])]
             if offtargets is not None:
-                write_offtarget_table(offtargets, tokens, scan, max_mismatches, index=index, counts=counts)
+                write_offtarget_table(offtargets, tokens, scan, max_mismatches, index=index, counts=counts[0],
+                                      extra=extra)
             if offtarget_sites is not None:
                 pairs, capped = write_offtarget_sites(offtarget_sites, tokens, scan, max_mismatches, max_sites,
-                                                      index=index, counts=counts)
+                                                      index=index, counts=counts[0], extra=extra)
                 ot_stats = {"offtarget_pairs": pairs, "offtarget_capped": capped}
             if offtarget_scores is not None:
-                write_offtarget_scores(offtarget_scores, tokens, scan, max_mismatches, index=index)
+                write_offtarget_scores(offtarget_scores, tokens, scan, max_mismatches, index=index,
+                                       extra=[(pam, ix) for pam, ix, _ in extra])
         finally:
-            index.free()
+            for ix in indexes:
+                ix.free()
         if verbose and offtarget_sites is not None:
-            out(f"{pairs:n} off-target sites listed in {offtarget_sites}; {capped:n} candidates with more than "
+            at = f" at {', '.join(['NGG'] + pams)} PAMs" if pams else ""
+            out(f"{pairs:n} off-target sites{at} listed in {offtarget_sites}; {capped:n} candidates with more than "
                 f"{max_sites:n} left out")
     stats = {"tokens": len(tokens), "candidates": len(table), "rows": rows_written,
              "scan_ms": scan.scan_ms(), **scan.timing(), **ot_stats}

@@ -378,6 +378,19 @@ int crp_offtarget_count_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys
  * add_genome of such an index answers CRP_ERR_RANGE for a handle of 2^24 segments or more and for a 128th
  * handle.  An index made by crp_offtarget_new behaves as before and keeps no loci. */
 int crp_offtarget_new_with_loci(crp_offtarget **ix);
+/* ---- other PAMs.  An index made by crp_offtarget_new_pam holds the sites of the PAM pattern `pam` instead of NGG
+ * (with loci when with_loci is non-zero): three characters, any case, N followed by two IUPAC letters for one to three
+ * bases, A C G T R Y S W K M B D H V (N is refused there).  With S2, S3 the code sets of letters 2 and 3 and
+ * comp(S) = {c ^ 1 : c in S}:
+ *   site '+' at t   tok[t+1] a base in S2, tok[t+2] a base in S3, tok[t-20 .. t) all of ACGTacgt; P = tok[t-20 .. t)
+ *   site '-' at t   tok[t] a base in comp(S3), tok[t+1] a base in comp(S2), tok[t+3 .. t+23) all of ACGTacgt;
+ *                   P = revcomp(tok[t+3 .. t+23))
+ * Keys, loci and every count, list and score call work on such an index as on an NGG one (crp_offtarget_new and
+ * crp_offtarget_new_with_loci are "NGG"), with one rule for scan candidates: their own site is a site of the index
+ * exactly when G is in S2 and in S3 (NGG, NRG, NKG, ...), and only then is it subtracted from the counts and the
+ * score.  Otherwise a candidate's row starts at 0, as a key's does.  A listing leaves out a site at the candidate's
+ * own locus either way.  CRP_ERR_ARG for NULL or a pattern outside this definition. */
+int crp_offtarget_new_pam(crp_offtarget **ix, const char *pam, int with_loci);
 /* The loci in crp_offtarget_fetch_sites order; CRP_ERR_STATE on an index without loci, CRP_ERR_RANGE (and *n)
  * if capacity is too small. */
 int crp_offtarget_fetch_loci(const crp_offtarget *ix, uint64_t capacity, uint64_t *loci, uint64_t *n);
@@ -403,8 +416,9 @@ int crp_offtarget_list_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys,
  * Entries for sets larger than max_mm are not read; an entry >= 2^31 among the others is CRP_ERR_ARG, so that no sum
  * can overflow.  A candidate without a protospacer gets CRP_OT_NO_SCORE.  The sum does not depend on the order in
  * which pairs are found.  With round(hit * 2^24) of the MIT hit score (Hsu et al. 2013, CRISPOR's calcHitScore) as
- * weights, sum / 2^24 is the MIT hit-score sum over NGG sites within max_mm <= 3 mismatches -- CRISPOR also sums
- * 4-mismatch and NAG / NGA sites, so its score is not this one.  Other refusals as for the count calls. */
+ * weights, sum / 2^24 is the MIT hit-score sum over the index's sites (NGG, or its PAM pattern) within max_mm <= 3
+ * mismatches -- CRISPOR also sums 4-mismatch sites, so its score is not this one.  Other refusals as for the count
+ * calls. */
 #define CRP_OT_SCORE_SETS 1351
 #define CRP_OT_NO_SCORE 0xFFFFFFFFFFFFFFFFull
 int crp_offtarget_score_candidates(crp_offtarget *ix, const crp_result *res, char strand, uint32_t max_mm,
