@@ -783,11 +783,8 @@ int crp_genome_add_fasta_record(crp_genome *g, uint32_t token_id, const uint8_t 
     if (!g) return fail(CRP_ERR_ARG, "g is NULL");
     if (g->committed) return fail(CRP_ERR_STATE, "genome already committed");
     if (!seq_bytes || !n_bytes || !line_width) return fail(CRP_ERR_FORMAT, "empty FASTA record");
-    // bytes = bases + one line end per full line, the last one optional
-    const uint64_t body = seq_bytes[n_bytes - 1] == '\n' ? n_bytes - 1 : n_bytes;
-    const uint64_t k = body / ((uint64_t)line_width + 1), r = body % ((uint64_t)line_width + 1);
-    if (r == 0) return fail(CRP_ERR_FORMAT, "FASTA record is not made of %u-base lines", line_width);
-    const uint64_t n_bases = k * line_width + r, token_len = n_bases + 4;
+    const uint64_t n_bases = fasta_record_bases(n_bytes, seq_bytes[n_bytes - 1], line_width), token_len = n_bases + 4;
+    if (!n_bases) return fail(CRP_ERR_FORMAT, "FASTA record is not made of %u-base lines", line_width);
     if (token_len >= (1ull << 31) - (1ull << 15))
         return fail(CRP_ERR_RANGE, "token of %llu positions exceeds the 31-bit position range",
                     (unsigned long long)token_len);

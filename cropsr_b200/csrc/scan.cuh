@@ -262,6 +262,58 @@ struct FastaRec {
     uint32_t last, pad;   // last: last record of the file (its token ends in ')]', not '),')
 };
 
+// Bases of a record of n_bytes > 0 sequence bytes ending in last_byte, in lines of width > 0 bases: one line end per
+// full line, the last one optional.  0 when no such lines give that byte count (a whole number of width + 1 byte lines).
+inline uint64_t fasta_record_bases(uint64_t n_bytes, uint8_t last_byte, uint32_t width) {
+    const uint64_t body = last_byte == '\n' ? n_bytes - 1 : n_bytes;
+    const uint64_t k = body / ((uint64_t)width + 1), r = body % ((uint64_t)width + 1);
+    return r ? k * width + r : 0;
+}
+
+// the byte loads of k_fasta_strip, with a host twin: tests/fasta_strip_emu.cu runs fasta_strip_group on the CPU
+CRP_HD uint32_t crp_ldg_u8(const uint8_t *p) {
+#ifdef __CUDA_ARCH__
+    return __ldg(p);
+#else
+    return *p;
+#endif
+}
+
+// One item of k_fasta_strip: the 16 token bytes of record r from token position p0 (a multiple of 16) into w[4],
+// four per word, little-endian.  Returns 1 if a byte it reads breaks the record's plainness.
+CRP_HD unsigned int fasta_strip_group(const uint8_t *__restrict__ raw, const FastaRec &r, uint64_t p0, uint32_t w[4]) {
+    const uint64_t n = r.n_bases, L = n + 4;
+    uint64_t b = p0 ? p0 - 1 : 0;                  // base index of the first base byte of the group
+    uint64_t line = b / r.width;
+    uint32_t col = (uint32_t)(b - line * r.width);
+    const uint8_t *src = raw + r.raw_off + b + line;
+    if (b && !col) {                               // the group starts a line: the line end before it is this group's
+        col = r.width;                             // to check (the group before stops at the last base of the line)
+        --src;
+    }
+    unsigned int err = 0;
+#pragma unroll
+    for (int i = 0; i < 16; ++i) {
+        const uint64_t p = p0 + i;
+        uint32_t c = 0;
+        if (p == 0 || p == n + 1) c = '\'';
+        else if (p == n + 2) c = ')';
+        else if (p == n + 3) c = r.last ? ']' : ',';
+        else if (p < L) {
+            if (col == r.width) {                  // a line end is due here
+                if (crp_ldg_u8(src) != '\n') err = 1;
+                ++src;
+                col = 0;
+            }
+            c = crp_ldg_u8(src++);
+            ++col;
+            if (c <= 0x20 || c >= 0x7F || c == '\'' || c == '"' || c == '\\' || c == '>') err = 1;
+        }
+        w[i >> 2] |= c << (8 * (i & 3));
+    }
+    return err;
+}
+
 __global__ void __launch_bounds__(256)
 k_fasta_strip(const uint8_t *__restrict__ raw, const FastaRec *__restrict__ recs, uint32_t n_recs, uint64_t n_items,
               uint8_t *__restrict__ ascii, unsigned int *__restrict__ bad) {
@@ -275,32 +327,8 @@ k_fasta_strip(const uint8_t *__restrict__ raw, const FastaRec *__restrict__ recs
         }
         const FastaRec r = recs[lo];
         const uint64_t p0 = (it - r.first_item) * 16;  // token position of output byte 0
-        const uint64_t n = r.n_bases, L = n + 4;
-        uint64_t b = p0 ? p0 - 1 : 0;                  // base index of the first base byte of the group
-        uint64_t line = b / r.width;
-        uint32_t col = (uint32_t)(b - line * r.width);
-        const uint8_t *src = raw + r.raw_off + b + line;
         uint32_t w[4] = {0, 0, 0, 0};
-        unsigned int err = 0;
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-            const uint64_t p = p0 + i;
-            uint32_t c = 0;
-            if (p == 0 || p == n + 1) c = '\'';
-            else if (p == n + 2) c = ')';
-            else if (p == n + 3) c = r.last ? ']' : ',';
-            else if (p < L) {
-                if (col == r.width) {                  // a line end is due here
-                    if (__ldg(src) != '\n') err = 1;
-                    ++src;
-                    col = 0;
-                }
-                c = __ldg(src++);
-                ++col;
-                if (c <= 0x20 || c >= 0x7F || c == '\'' || c == '"' || c == '\\' || c == '>') err = 1;
-            }
-            w[i >> 2] |= c << (8 * (i & 3));
-        }
+        const unsigned int err = fasta_strip_group(raw, r, p0, w);
         *reinterpret_cast<uint4 *>(ascii + r.ascii_off + p0) = make_uint4(w[0], w[1], w[2], w[3]);
         if (err) atomicOr(bad, 1u);
     }

@@ -408,8 +408,12 @@ def test_device_fasta_ingest_refuses_text_that_is_not_plain(eng, tmp_path):
     """Ragged lines, blanks or quotes inside the sequence: the device validation answers
     CRP_ERR_FORMAT and the pipeline falls back to the literal host ingest."""
     from cropsr_b200 import pipeline
+    # width 61, the line end after line 11 replaced by a base: line 12 starts at base 671, the first base of the
+    # 16-byte group of k_fasta_strip at token position 672
+    rows = [(b"ACGGTCCATTGA" * 6)[k % 12:k % 12 + 61] for k in range(20)]
+    merged = b">a\n" + b"\n".join(rows[:10]) + b"\n" + rows[10] + b"A" + rows[11] + b"\n" + b"\n".join(rows[12:]) + b"\n"
     for k, data in enumerate((b">a\nACGTACGT\nACGT\nACGTACGT\n", b">a\nACGTACGT\nAC GTACG\nAC\n", b">a\nACGTACGT\nAC'TACGT\nAC\n",
-                              b">a\nACGTACGT\nACGTACGT\n\n", b">a\nACGTACGT\n\nACGTACGT\n")):
+                              b">a\nACGTACGT\nACGTACGT\n\n", b">a\nACGTACGT\n\nACGTACGT\n", merged)):
         path = tmp_path / f"bad{k}.fa"
         path.write_bytes(data)
         assert pipeline.scan_fasta_file(str(path), 20) is None, data
