@@ -2123,7 +2123,7 @@ static int ot_join(crp_offtarget *ix, const unsigned long long *d_keys, uint64_t
     uint2 *d_q = nullptr;
     unsigned long long *d_misc = nullptr;      // [0] comparisons, [1] overflow flag
     if (dev_alloc(&d_tbl, 7 * tbl * sizeof(uint32_t), st) != cudaSuccess ||
-        dev_alloc(&d_sites, (ix->n_sites + 8) * sizeof(Site), st) != cudaSuccess ||
+        dev_alloc(&d_sites, (ix->n_sites + kOtSitePad) * sizeof(Site), st) != cudaSuccess ||
         dev_alloc(&d_q, (n + 1) * sizeof(uint2), st) != cudaSuccess ||
         dev_alloc(&d_misc, 2 * sizeof(unsigned long long), st) != cudaSuccess) {
         cudaGetLastError();

@@ -331,6 +331,67 @@ __global__ void k_ot_gather(const OtGatherArgs a) {
     a.own[i] = ot_locus(a.pos[r], lo, a.genome, a.minus != 0);
 }
 
+// ---- geometry of a work item of k_ot_join (host and device: tests/offtarget_join_emu.cu checks it exhaustively)
+// Sites allocated past the last one of a part pair's site array: the bulk copy of a tile rounds its source down to 16
+// bytes and its length up to 16, so it reads up to 12 bytes (3 uint32 sites, 1.5 uint2 sites) past the last site.
+static constexpr uint32_t kOtSitePad = 8;
+
+CRP_HD uint32_t crp_ldg_u32(const uint32_t *p) {
+#ifdef __CUDA_ARCH__
+    return __ldg(p);
+#else
+    return *p;
+#endif
+}
+// work items of a bucket of ns sites and nq queries (k_ot_scan): query tiles x site tiles, 0 unless both are present.
+// 64-bit: one bucket of 2^32 - 1 queries and sites has 2^46 items, which k_ot_scan's check of the part pair's total
+// (< 2^32) then catches; in 32 bits the product, and the tile counts near 2^32, would wrap unseen.
+CRP_HD unsigned long long ot_bucket_items(uint32_t ns, uint32_t nq) {
+    return ns && nq ? ((unsigned long long)nq + kOtThreads - 1) / kOtThreads *
+                          (((unsigned long long)ns + kOtSiteTile - 1) / kOtSiteTile)
+                    : 0ull;
+}
+// the bucket of work item `item` (< item_off[kOtBuckets]): the last b with item_off[b] <= item.  Empty buckets repeat
+// the offset of the bucket after them, so the last such b is the one with items.
+CRP_HD uint32_t ot_item_bucket(const uint32_t *item_off, uint32_t item) {
+    uint32_t lo = 0, hi = kOtBuckets;
+    while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (crp_ldg_u32(item_off + mid) <= item) lo = mid;
+        else hi = mid;
+    }
+    return lo;
+}
+// the tiles of work item `item` of bucket b: queries [q0, q0 + nq_t) and sites [s0, s0 + ns_t) of the bucket-ordered
+// arrays; item - item_off[b] = qt * n_st + st over the bucket's n_st site tiles
+struct OtItem {
+    uint32_t q0, nq_t, s0, ns_t;
+};
+CRP_HD OtItem ot_item(const uint32_t *soff, const uint32_t *qoff, const uint32_t *item_off, uint32_t b, uint32_t item) {
+    const uint32_t sb = crp_ldg_u32(soff + b), ns = crp_ldg_u32(soff + b + 1) - sb;
+    const uint32_t qb = crp_ldg_u32(qoff + b), nq = crp_ldg_u32(qoff + b + 1) - qb;
+    const uint32_t n_st = (ns + kOtSiteTile - 1) / kOtSiteTile, local = item - crp_ldg_u32(item_off + b);
+    const uint32_t qt = local / n_st, st = local % n_st;
+    OtItem it;
+    it.s0 = sb + st * kOtSiteTile;
+    it.ns_t = min(kOtSiteTile, ns - st * kOtSiteTile);
+    it.q0 = qb + qt * kOtThreads;
+    it.nq_t = min((uint32_t)kOtThreads, nq - qt * kOtThreads);
+    return it;
+}
+// The bulk copy of the tile [s0, s0 + ns_t) of site elements of kSize bytes: from element ot_copy_first (16-byte
+// aligned), ot_copy_bytes (a multiple of 16, at most (kOtSiteTile + 16 / kSize) elements) into the shared tile, where
+// site s0 is element s0 - a0.
+template <uint32_t kSize>
+CRP_HD uint32_t ot_copy_first(uint32_t s0) { return s0 & ~(16u / kSize - 1u); }
+template <uint32_t kSize>
+CRP_HD uint32_t ot_copy_bytes(uint32_t s0, uint32_t ns_t, uint32_t a0) { return ((s0 + ns_t - a0) * kSize + 15u) & ~15u; }
+CRP_HD uint32_t ot_copy_offset(uint32_t s0, uint32_t a0) { return s0 - a0; }
+// The split of a tile's queries over the CTA: g threads per query; thread tid < nq_t * g holds query tid % nq_t and
+// visits the sites tid / nq_t, + g, ...; the others are idle.
+CRP_HD uint32_t ot_threads_per_query(uint32_t nq_t) { return kOtThreads / nq_t; }
+CRP_HD bool ot_thread_active(uint32_t tid, uint32_t nq_t, uint32_t g) { return tid < nq_t * g; }
+
 // ---- counting sort by the bucket of part pair (i, j): histogram, scan, scatter.  Warps aggregate their
 // atomics per bucket (__match_any_sync): a repeat family puts whole warps into one bucket.
 __global__ void k_ot_hist(const unsigned long long *__restrict__ keys, uint64_t n, int pi, int pj, uint32_t *hist) {
@@ -360,10 +421,9 @@ __global__ void __launch_bounds__(kOtScanThreads) k_ot_scan(const OtScanArgs a) 
     constexpr uint32_t per = kOtBuckets / kOtScanThreads;
     __shared__ unsigned long long s_warp[kOtScanThreads / 32];
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, which = blockIdx.x;
-    auto value = [&](uint32_t b) -> uint32_t {
+    auto value = [&](uint32_t b) -> unsigned long long {
         if (which < 2) return a.hist[which][b];
-        const uint32_t ns = a.hist[0][b], nq = a.hist[1][b];
-        return ns && nq ? ((nq + kOtThreads - 1) / kOtThreads) * ((ns + kOtSiteTile - 1) / kOtSiteTile) : 0u;
+        return ot_bucket_items(a.hist[0][b], a.hist[1][b]);
     };
     unsigned long long sum = 0, cmp = 0;
     for (uint32_t e = 0; e < per; ++e) {
@@ -453,8 +513,7 @@ CRP_HD uint32_t ot_site_rest(uint2 s) { return s.x; }
 template <class Op>
 __global__ void __launch_bounds__(kOtThreads) k_ot_join(const OtJoin a, const Op op) {
     using Site = typename Op::Site;
-    constexpr uint32_t kAlign = 16 / sizeof(Site);                       // sites per 16 bytes of the bulk copy
-    __shared__ __align__(16) Site s_sites[kOtSiteTile + kAlign];         // the copy starts up to 16 bytes early
+    __shared__ __align__(16) Site s_sites[kOtSiteTile + 16 / sizeof(Site)];   // the copy starts up to 16 bytes early
     __shared__ typename Op::Shared sh;
     __shared__ __align__(8) unsigned long long bar;
     const uint32_t tid = threadIdx.x;
@@ -467,32 +526,22 @@ __global__ void __launch_bounds__(kOtThreads) k_ot_join(const OtJoin a, const Op
     __syncthreads();
     uint32_t phase = 0;
     for (uint32_t item = blockIdx.x; item < total; item += gridDim.x) {
-        uint32_t lo = 0, hi = kOtBuckets;      // bucket: last b with item_off[b] <= item
-        while (hi - lo > 1) {
-            const uint32_t mid = (lo + hi) >> 1;
-            if (__ldg(a.item_off + mid) <= item) lo = mid;
-            else hi = mid;
-        }
-        const uint32_t sb = __ldg(a.soff + lo), ns = __ldg(a.soff + lo + 1) - sb;
-        const uint32_t qb = __ldg(a.qoff + lo), nq = __ldg(a.qoff + lo + 1) - qb;
-        const uint32_t n_st = (ns + kOtSiteTile - 1) / kOtSiteTile, local = item - __ldg(a.item_off + lo);
-        const uint32_t qt = local / n_st, st = local % n_st;
-        const uint32_t s0 = sb + st * kOtSiteTile, ns_t = min(kOtSiteTile, ns - st * kOtSiteTile);
-        const uint32_t q0 = qb + qt * kOtThreads, nq_t = min((uint32_t)kOtThreads, nq - qt * kOtThreads);
-        const uint32_t a0 = s0 & ~(kAlign - 1u);                             // 16-byte aligned source
+        const OtItem it = ot_item(a.soff, a.qoff, a.item_off, ot_item_bucket(a.item_off, item), item);
+        const uint32_t s0 = it.s0, ns_t = it.ns_t, nq_t = it.nq_t;
+        const uint32_t a0 = ot_copy_first<sizeof(Site)>(s0);
         if (tid == 0) {
-            const uint32_t bytes = ((s0 + ns_t - a0) * (uint32_t)sizeof(Site) + 15u) & ~15u;
+            const uint32_t bytes = ot_copy_bytes<sizeof(Site)>(s0, ns_t, a0);
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // earlier generic reads of the tile come first
             mbar_expect(&bar, bytes);
             bulk_copy(s_sites, static_cast<const Site *>(a.sites) + a0, bytes, &bar);
         }
-        const uint32_t g = kOtThreads / nq_t;                                // threads per query
-        const bool active = tid < nq_t * g;
-        const uint2 q = active ? a.queries[q0 + tid % nq_t] : make_uint2(0, 0);
+        const uint32_t g = ot_threads_per_query(nq_t);
+        const bool active = ot_thread_active(tid, nq_t, g);
+        const uint2 q = active ? a.queries[it.q0 + tid % nq_t] : make_uint2(0, 0);
         mbar_wait(&bar, phase);
         phase ^= 1u;
         if (active) {
-            const Site *S = s_sites + (s0 - a0);
+            const Site *S = s_sites + ot_copy_offset(s0, a0);
             typename Op::Acc acc{};
             for (uint32_t s = tid / nq_t; s < ns_t; s += g) {
                 const Site site = S[s];
