@@ -132,6 +132,26 @@ CRP_HD double rs1_canonical(const double *__restrict__ T, uint32_t s0, uint32_t 
     return rs1_canonical_masks(T, ~s1 & ~s0 & valid, ~s1 & s0 & valid, s1 & ~s0 & valid, s1 & s0 & valid);
 }
 
+// Host side: the table slot (relative to ln.offset) of lane ln when exactly the table entries in `on`
+// match (bit i = entries[i]; forced entries carry no match bit and are ignored).  *outside is set if a
+// match bit falls outside its group's mask, which the lane's select masks would drop.  The hash that
+// RS1_LANE_SUMS computes on the device; build_rs1_tables and tests/rs1_lanes_emu.cu share it.
+static uint32_t rs1_table_slot(const Rs1Lane &ln, uint32_t on, bool *outside) {
+    uint32_t h = 0;
+    for (int g = 0; g < ln.n_groups; ++g) {
+        uint32_t x = 0;                           // match bits of this first-base group
+        for (int i = 0; i < ln.n_table; ++i) {
+            const Rs1Entry &e = ln.entries[i];
+            if (!e.forced && (on >> i & 1) && ln.groups[g].first_base == e.first_base) x |= 1u << e.bit;
+        }
+        if (outside && (x & ~ln.groups[g].mask)) *outside = true;
+        h += x * ln.groups[g].magic;
+    }
+    uint32_t slot = ln.bits ? h >> (32 - ln.bits) : 0u;
+    if (ln.swizzle) slot = (uint32_t)(((unsigned long long)h * (unsigned)ln.swizzle) >> 32);   // RS1_SWZ
+    return slot;
+}
+
 // Host side: exact sequential sums of every valid subset of each lane's table entries
 // (forced entries -- the PAM bases -- are part of every sum).
 static int build_rs1_tables(std::vector<double> &tab, char *err, size_t errlen) {
@@ -149,26 +169,20 @@ static int build_rs1_tables(std::vector<double> &tab, char *err, size_t errlen) 
                     if ((sub >> i & 1) && (sub >> j & 1) && ln.entries[free_idx[i]].pos == ln.entries[free_idx[j]].pos)
                         ok = false;
             if (!ok) continue;
-            uint32_t h = 0;
-            for (int g = 0; g < ln.n_groups; ++g) {
-                uint32_t x = 0;                   // match bits of this first-base group
-                for (int i = 0; i < n_free; ++i) {
-                    const Rs1Entry &e = ln.entries[free_idx[i]];
-                    if ((sub >> i & 1) && ln.groups[g].first_base == e.first_base) x |= 1u << e.bit;
-                }
-                if (x & ~ln.groups[g].mask) {
-                    snprintf(err, errlen, "rs1 lane %s: entry outside its group mask", ln.name);
-                    return -1;
-                }
-                h += x * ln.groups[g].magic;
+            uint32_t on = 0;                      // the subset as entry bits
+            for (int i = 0; i < n_free; ++i)
+                if (sub >> i & 1) on |= 1u << free_idx[i];
+            bool outside = false;
+            const uint32_t slot = rs1_table_slot(ln, on, &outside);
+            if (outside) {
+                snprintf(err, errlen, "rs1 lane %s: entry outside its group mask", ln.name);
+                return -1;
             }
             volatile double sum = 0.0;            // one IEEE add per entry, in ascending column order
             for (int i = 0, f = 0; i < ln.n_table; ++i) {
-                const bool on = ln.entries[i].forced ? true : ((sub >> f++) & 1);
-                if (on) sum = sum + ln.entries[i].weight;
+                const bool on_i = ln.entries[i].forced ? true : ((sub >> f++) & 1);
+                if (on_i) sum = sum + ln.entries[i].weight;
             }
-            uint32_t slot = ln.bits ? h >> (32 - ln.bits) : 0u;
-            if (ln.swizzle) slot = (uint32_t)(((unsigned long long)h * (unsigned)ln.swizzle) >> 32);   // RS1_SWZ
             const uint32_t idx = ln.offset + slot;
             if (idx >= RS1_TABLE_DOUBLES || used[idx]) {
                 snprintf(err, errlen, "rs1 table hash of lane %s is not injective", ln.name);

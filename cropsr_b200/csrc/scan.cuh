@@ -708,6 +708,9 @@ __device__ __forceinline__ void emit_one(const ScanArgs &a, const double *__rest
             const Window w = extract_window<kMinus>(rec, ws + (kMinus ? 0u : 2u), t, L);
             CRP_CHECK(a, w.packed == word, 14);
             CRP_CHECK(a, __double_as_longlong(rs1_canonical(tab, w.s0, w.s1, w.valid)) == __double_as_longlong(x), 15);
+            // and the lane tables must agree with the column-by-column replay, which reads no table
+            CRP_CHECK(a, __double_as_longlong(rs1_dense(w.s0, w.s1, w.valid, CRP_CLASS_CANONICAL, CRP_CLASS_CANONICAL)) ==
+                             __double_as_longlong(x), 16);
         }
 #endif
         __stcs(packed + row, word);
