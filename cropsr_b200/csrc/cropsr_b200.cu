@@ -75,86 +75,7 @@ struct Perf {
 };
 static Perf g_perf;
 
-// ------------------------------------------------------------------ host objects
-struct Segment {
-    uint32_t token_id;
-    const uint8_t *token;
-    uint64_t token_len, begin, end;
-    uint64_t stage_begin, stage_end;   // token positions copied to the device
-    uint32_t first_tile, n_tiles;
-    // FASTA record ingested on the device (crp_genome_add_fasta_record): token == NULL
-    const uint8_t *raw = nullptr;      // first sequence byte of the record, as in the file
-    uint64_t raw_bytes = 0;
-    uint32_t width = 0, last = 0;
-    uint64_t ascii_off = 0;            // token position stage_begin in the ASCII buffer kept on the device
-};
-
-struct crp_genome {
-    std::vector<Segment> segs;
-    cudaStream_t st = nullptr;         // every operation on this genome and its results is ordered on this stream
-    cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};   // commit timing: start, H2D done, pack done
-    bool committed = false;
-    uint64_t n_positions = 0;          // owned positions
-    uint4 *records = nullptr;          // n_tiles tile records (scan.cuh)
-    unsigned char *pam = nullptr;      // n_tiles PAM records (count phase of the scan: tiles at the ends of a token)
-    TileHdr *hdr = nullptr;            // n_tiles tile headers (count phase of the scan: descriptor + chunk counts)
-    uint32_t n_tiles = 0;
-    uint32_t *d_seg_first = nullptr, *d_seg_count = nullptr;
-    float ms_h2d = 0.f, ms_pack = 0.f;
-    uint8_t *d_ascii = nullptr;                // ASCII tokens, kept after the pack only for device-ingested FASTA records
-    bool fasta = false;
-    unsigned int *h_bad = nullptr;             // pinned: non-zero after the commit if a FASTA record was not plain
-};
-
-struct crp_result {
-    const crp_genome *g = nullptr;
-    cudaStream_t st = nullptr;
-    cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};   // scan start, scan (+ all-gather) end, counts on the host
-    cudaEvent_t ev_kernel = nullptr;           // sharded scans: between the kernel and the all-gather
-    unsigned long long *h_counts = nullptr;    // pinned, [2*stride]: counts land here when the scan has run
-    uint32_t stride = 0;                       // count slots per strand: n_seg, or the `slots` of a sharded scan
-    unsigned long long *d_gather = nullptr;    // sharded scans: [world][2*stride] counts of every rank (NCCL all-gather)
-    unsigned long long *h_gather = nullptr;    // pinned copy
-    bool fused = false;                        // counts exchanged by the kernel itself (peer stores), not by NCCL
-    uint32_t epoch = 0;
-    unsigned int *h_xchg_error = nullptr;      // pinned
-    float ms_kernel = 0.f;
-    int guide_len = 0;
-    uint32_t flags = 0;
-    uint64_t capacity = 0;
-    uint64_t n_plus = 0, n_minus = 0;
-    bool scored = false;
-    uint32_t *pos[2] = {nullptr, nullptr};
-    unsigned long long *packed[2] = {nullptr, nullptr};
-    double *x[2] = {nullptr, nullptr};
-    unsigned char *state = nullptr;            // warp_pref | cta_tot | segment counts | tickets, one allocation
-    size_t state_bytes = 0, zero_offset = 0;   // segment counts and tickets start at zero_offset
-    unsigned long long *d_counts = nullptr;    // [2*stride], inside state
-    std::vector<uint64_t> seg_plus, seg_minus;
-    float ms_scan = 0.f;                       // every launch of this scan, a capacity rerun included
-    uint32_t n_launches = 0;
-};
-
-// CRP_TRACE=1: host-side wall time of every stage of the big calls, on stderr
-#include <chrono>
-struct Trace {
-    const char *what;
-    bool on;
-    std::chrono::steady_clock::time_point t0;
-    explicit Trace(const char *w) : what(w), on(getenv("CRP_TRACE") != nullptr), t0(std::chrono::steady_clock::now()) {}
-    void lap(const char *stage) {
-        if (!on) return;
-        const auto t1 = std::chrono::steady_clock::now();
-        fprintf(stderr, "[crp] %s: %s %.3f ms\n", what, stage, std::chrono::duration<double, std::milli>(t1 - t0).count());
-        t0 = t1;
-    }
-};
-
-static int need_ctx() {
-    if (!g_ctx.ready) return fail(CRP_ERR_STATE, "crp_init has not been called");
-    return 0;
-}
-
+// ------------------------------------------------------------------ device and pinned blocks
 // Device memory comes from a block cache of this library: cudaMalloc / cudaFree cost 10-70 ms per
 // call on a 180 GB part and the driver's stream-ordered pool grows for milliseconds whenever the
 // set of live sizes changes, while a genome commit and a scan allocate ~1 GB between them.  A freed
@@ -169,8 +90,16 @@ struct DevBlock {
 static std::vector<DevBlock> g_dev_free;                       // idle blocks
 static std::vector<DevBlock> g_dev_live;                       // blocks handed out
 static std::mutex g_mem_mu;                                    // guards both block lists and the pinned list
-template <typename T>
-static cudaError_t dev_alloc(T **ptr, size_t bytes, cudaStream_t st) {
+// Blocks of both caches are handed out only to their owners, DevBuf and PinnedBuf (below).
+class BlockCache {
+    template <typename T> friend class DevBuf;
+    template <typename T> friend class PinnedBuf;
+    static cudaError_t dev_alloc(void **ptr, size_t bytes, cudaStream_t st);
+    static void dev_free(void *ptr, cudaStream_t st);
+    static void *pinned_get(size_t bytes);
+    static void pinned_put(void *p);
+};
+cudaError_t BlockCache::dev_alloc(void **ptr, size_t bytes, cudaStream_t st) {
     std::lock_guard<std::mutex> lock(g_mem_mu);
     const size_t want = (bytes ? bytes : 16) + 255 & ~(size_t)255;
     // best fit among the idle blocks whose last user has FINISHED: a block that is still in use on another
@@ -225,10 +154,10 @@ static cudaError_t dev_alloc(T **ptr, size_t bytes, cudaStream_t st) {
         }
     }
     g_dev_live.push_back(blk);
-    *ptr = reinterpret_cast<T *>(blk.ptr);
+    *ptr = blk.ptr;
     return cudaSuccess;
 }
-static void dev_free(void *ptr, cudaStream_t st) {
+void BlockCache::dev_free(void *ptr, cudaStream_t st) {
     if (!ptr) return;
     std::lock_guard<std::mutex> lock(g_mem_mu);
     for (size_t i = g_dev_live.size(); i-- > 0;)
@@ -251,27 +180,175 @@ static void dev_cache_release() {
 
 // Small pinned host blocks (the per-scan counts) are recycled: cudaHostAlloc takes ~0.1 ms.
 static std::vector<std::pair<size_t, void *>> g_pinned_free;
-static void *pinned_get(size_t bytes) {
+static size_t g_pinned_live = 0;                               // pinned blocks handed out
+void *BlockCache::pinned_get(size_t bytes) {
     std::lock_guard<std::mutex> lock(g_mem_mu);
     for (size_t i = 0; i < g_pinned_free.size(); ++i)
         if (g_pinned_free[i].first >= bytes) {
             void *p = g_pinned_free[i].second;
             g_pinned_free.erase(g_pinned_free.begin() + i);
+            g_pinned_live++;
             return p;
         }
     const size_t want = bytes < 4096 ? 4096 : bytes;
     void *p = nullptr;
     if (cudaHostAlloc(&p, want + sizeof(size_t) * 2, cudaHostAllocMapped) != cudaSuccess) return nullptr;   // kernels may store into it
     *reinterpret_cast<size_t *>(p) = want;
+    g_pinned_live++;
     return reinterpret_cast<char *>(p) + sizeof(size_t) * 2;
 }
-static void pinned_put(void *p) {
+void BlockCache::pinned_put(void *p) {
     if (!p) return;
     std::lock_guard<std::mutex> lock(g_mem_mu);
     const size_t cap = *reinterpret_cast<size_t *>(reinterpret_cast<char *>(p) - sizeof(size_t) * 2);
     g_pinned_free.emplace_back(cap, p);
+    g_pinned_live--;
 }
 
+// The owners of those blocks: a DevBuf holds one device block of n elements and gives it back to the cache on the
+// stream it was allocated on, when reset or destroyed; a PinnedBuf does the same for a pinned block.  alloc() first
+// gives back any block the buffer holds, and on failure returns CRP_ERR_NOMEM with `what` in the message.
+template <typename T>
+class DevBuf {
+  public:
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(DevBuf &&o) noexcept {
+        if (this != &o) {
+            reset();
+            std::swap(p_, o.p_);
+            std::swap(st_, o.st_);
+        }
+        return *this;
+    }
+    ~DevBuf() { reset(); }
+    int alloc(size_t n, cudaStream_t st, const char *what) {
+        reset();
+        void *p = nullptr;
+        if (BlockCache::dev_alloc(&p, n * sizeof(T), st) != cudaSuccess) {
+            cudaGetLastError();
+            return fail(CRP_ERR_NOMEM, "cudaMalloc of %s (%zu bytes) failed", what, n * sizeof(T));
+        }
+        p_ = static_cast<T *>(p);
+        st_ = st;
+        return 0;
+    }
+    void reset() {
+        BlockCache::dev_free(p_, st_);
+        p_ = nullptr;
+    }
+    T *get() const { return p_; }
+
+  private:
+    T *p_ = nullptr;
+    cudaStream_t st_ = nullptr;
+};
+
+template <typename T>
+class PinnedBuf {
+  public:
+    PinnedBuf() = default;
+    PinnedBuf(const PinnedBuf &) = delete;
+    PinnedBuf &operator=(const PinnedBuf &) = delete;
+    ~PinnedBuf() { reset(); }
+    int alloc(size_t n, const char *what) {
+        reset();
+        p_ = static_cast<T *>(BlockCache::pinned_get(n * sizeof(T)));
+        if (!p_) {
+            cudaGetLastError();
+            return fail(CRP_ERR_NOMEM, "cudaHostAlloc of %s (%zu bytes) failed", what, n * sizeof(T));
+        }
+        return 0;
+    }
+    void reset() {
+        BlockCache::pinned_put(p_);
+        p_ = nullptr;
+    }
+    T *get() const { return p_; }
+
+  private:
+    T *p_ = nullptr;
+};
+
+// ------------------------------------------------------------------ host objects
+struct Segment {
+    uint32_t token_id;
+    const uint8_t *token;
+    uint64_t token_len, begin, end;
+    uint64_t stage_begin, stage_end;   // token positions copied to the device
+    uint32_t first_tile, n_tiles;
+    // FASTA record ingested on the device (crp_genome_add_fasta_record): token == NULL
+    const uint8_t *raw = nullptr;      // first sequence byte of the record, as in the file
+    uint64_t raw_bytes = 0;
+    uint32_t width = 0, last = 0;
+    uint64_t ascii_off = 0;            // token position stage_begin in the ASCII buffer kept on the device
+};
+
+struct crp_genome {
+    std::vector<Segment> segs;
+    cudaStream_t st = nullptr;         // every operation on this genome and its results is ordered on this stream
+    cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};   // commit timing: start, H2D done, pack done
+    bool committed = false;
+    uint64_t n_positions = 0;          // owned positions
+    DevBuf<uint4> records;             // n_tiles tile records (scan.cuh)
+    DevBuf<unsigned char> pam;         // n_tiles PAM records (count phase of the scan: tiles at the ends of a token)
+    DevBuf<TileHdr> hdr;               // n_tiles tile headers (count phase of the scan: descriptor + chunk counts)
+    uint32_t n_tiles = 0;
+    DevBuf<uint32_t> d_seg_first, d_seg_count;
+    float ms_h2d = 0.f, ms_pack = 0.f;
+    DevBuf<uint8_t> d_ascii;                   // ASCII tokens, kept after the pack only for device-ingested FASTA records
+    bool fasta = false;
+    PinnedBuf<unsigned int> h_bad;             // non-zero after the commit if a FASTA record was not plain
+};
+
+struct crp_result {
+    const crp_genome *g = nullptr;
+    cudaStream_t st = nullptr;
+    cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};   // scan start, scan (+ all-gather) end, counts on the host
+    cudaEvent_t ev_kernel = nullptr;           // sharded scans: between the kernel and the all-gather
+    PinnedBuf<unsigned long long> h_counts;    // [2*stride]: counts land here when the scan has run
+    uint32_t stride = 0;                       // count slots per strand: n_seg, or the `slots` of a sharded scan
+    DevBuf<unsigned long long> d_gather;       // sharded scans: [world][2*stride] counts of every rank (NCCL all-gather)
+    PinnedBuf<unsigned long long> h_gather;    // its copy on the host
+    bool fused = false;                        // counts exchanged by the kernel itself (peer stores), not by NCCL
+    uint32_t epoch = 0;
+    PinnedBuf<unsigned int> h_xchg_error;
+    float ms_kernel = 0.f;
+    int guide_len = 0;
+    uint32_t flags = 0;
+    uint64_t capacity = 0;
+    uint64_t n_plus = 0, n_minus = 0;
+    bool scored = false;
+    DevBuf<uint32_t> pos[2];
+    DevBuf<unsigned long long> packed[2];
+    DevBuf<double> x[2];
+    DevBuf<unsigned char> state;               // warp_pref | cta_tot | segment counts | tickets, one allocation
+    size_t state_bytes = 0, zero_offset = 0;   // segment counts and tickets start at zero_offset
+    unsigned long long *d_counts = nullptr;    // [2*stride], inside state
+    std::vector<uint64_t> seg_plus, seg_minus;
+    float ms_scan = 0.f;                       // every launch of this scan, a capacity rerun included
+    uint32_t n_launches = 0;
+};
+
+// CRP_TRACE=1: host-side wall time of every stage of the big calls, on stderr
+#include <chrono>
+struct Trace {
+    const char *what;
+    bool on;
+    std::chrono::steady_clock::time_point t0;
+    explicit Trace(const char *w) : what(w), on(getenv("CRP_TRACE") != nullptr), t0(std::chrono::steady_clock::now()) {}
+    void lap(const char *stage) {
+        if (!on) return;
+        const auto t1 = std::chrono::steady_clock::now();
+        fprintf(stderr, "[crp] %s: %s %.3f ms\n", what, stage, std::chrono::duration<double, std::milli>(t1 - t0).count());
+        t0 = t1;
+    }
+};
+
+static int need_ctx() {
+    if (!g_ctx.ready) return fail(CRP_ERR_STATE, "crp_init has not been called");
+    return 0;
+}
 
 // ------------------------------------------------------------------ NCCL (one process per GPU)
 // The library talks to NCCL through dlopen: a single-GPU run needs no NCCL at all, and inside a
@@ -446,10 +523,11 @@ int crp_shutdown(void) {
 /* JSON object with the library's counters since crp_init (SURVEY.md section 5: perf report) */
 int crp_perf_report(char *buf, uint64_t capacity, uint64_t *needed) {
     char tmp[1536];
-    size_t live = 0, idle = 0, live_bytes = 0, idle_bytes = 0;
+    size_t live = 0, idle = 0, live_bytes = 0, idle_bytes = 0, pinned_live = 0;
     {
         std::lock_guard<std::mutex> lock(g_mem_mu);
         live = g_dev_live.size();
+        pinned_live = g_pinned_live;
         idle = g_dev_free.size();
         for (const DevBlock &b : g_dev_live) live_bytes += b.bytes;
         for (const DevBlock &b : g_dev_free) idle_bytes += b.bytes;
@@ -461,7 +539,7 @@ int crp_perf_report(char *buf, uint64_t capacity, uint64_t *needed) {
         "\"positions_packed\": %llu, \"candidates\": %llu, \"h2d_token_bytes\": %llu, \"d2h_row_bytes\": %llu, "
         "\"ms_h2d\": %.4f, \"ms_pack\": %.4f, \"ms_scan\": %.4f, \"ms_scan_kernels\": %.4f, "
         "\"comm\": {\"rank\": %d, \"world\": %d, \"fused_exchange\": %s}, "
-        "\"block_cache\": {\"live_blocks\": %zu, \"live_bytes\": %zu, \"idle_blocks\": %zu, \"idle_bytes\": %zu, \"hits\": %llu, \"misses\": %llu}}",
+        "\"block_cache\": {\"live_blocks\": %zu, \"live_bytes\": %zu, \"idle_blocks\": %zu, \"idle_bytes\": %zu, \"hits\": %llu, \"misses\": %llu, \"pinned_live_blocks\": %zu}}",
         CRP_ABI_VERSION, crp_checked_build(), g_ctx.device, g_ctx.sm_count, (unsigned long long)g_ctx.launches.load(),
         (unsigned long long)g_perf.commits.load(), (unsigned long long)g_perf.scans.load(),
         (unsigned long long)g_perf.sharded_scans.load(), (unsigned long long)g_perf.fused_exchanges.load(),
@@ -469,7 +547,7 @@ int crp_perf_report(char *buf, uint64_t capacity, uint64_t *needed) {
         (unsigned long long)g_perf.candidates.load(), (unsigned long long)g_perf.h2d_bytes.load(),
         (unsigned long long)g_perf.d2h_bytes.load(), g_perf.ms_h2d, g_perf.ms_pack, g_perf.ms_scan, g_perf.ms_kernel,
         g_comm.comm ? g_comm.rank : 0, g_comm.comm ? g_comm.world : 1, g_comm.comm && g_comm.fused && g_comm.mode == 0 ? "true" : "false",
-        live, live_bytes, idle, idle_bytes, (unsigned long long)g_perf.cache_hits.load(), (unsigned long long)g_perf.cache_misses.load());
+        live, live_bytes, idle, idle_bytes, (unsigned long long)g_perf.cache_hits.load(), (unsigned long long)g_perf.cache_misses.load(), pinned_live);
     if (needed) *needed = (uint64_t)n + 1;
     if (!buf || capacity < (uint64_t)n + 1) return fail(CRP_ERR_RANGE, "perf report needs %d bytes", n + 1);
     memcpy(buf, tmp, (size_t)n + 1);
@@ -528,13 +606,12 @@ int crp_comm_init(int rank, int world, const uint8_t *id) {
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
     std::vector<uint64_t> handles((size_t)world * 8);
     {
-        unsigned long long *d = nullptr;
-        CUDA_TRY(cudaMalloc(&d, ((size_t)world + 1) * 64));
-        CUDA_TRY(cudaMemcpy(d, &mine, 64, cudaMemcpyHostToDevice));
-        NCCL_TRY(g_comm.AllGather(d, d + 8, 8, ncclUint64, g_comm.comm, g_ctx.stream));
+        DevBuf<unsigned long long> d;
+        if (int rc = d.alloc(((size_t)world + 1) * 8, g_ctx.stream, "the IPC handles")) return rc;
+        CUDA_TRY(cudaMemcpyAsync(d.get(), &mine, 64, cudaMemcpyHostToDevice, g_ctx.stream));
+        NCCL_TRY(g_comm.AllGather(d.get(), d.get() + 8, 8, ncclUint64, g_comm.comm, g_ctx.stream));
         CUDA_TRY(cudaStreamSynchronize(g_ctx.stream));
-        CUDA_TRY(cudaMemcpy(handles.data(), d + 8, (size_t)world * 64, cudaMemcpyDeviceToHost));
-        cudaFree(d);
+        CUDA_TRY(cudaMemcpy(handles.data(), d.get() + 8, (size_t)world * 64, cudaMemcpyDeviceToHost));
     }
     for (int q = 0; q < world && ok; ++q) {
         if (q == rank) {
@@ -602,13 +679,12 @@ int crp_comm_max_f64(double *v, uint32_t n) {
     if (int rc = need_ctx()) return rc;
     if (!v && n) return fail(CRP_ERR_ARG, "v is NULL");
     if (!g_comm.comm || n == 0) return 0;
-    double *d = nullptr;
-    CUDA_TRY(dev_alloc(&d, n * sizeof(double), g_ctx.stream));
-    CUDA_TRY(cudaMemcpyAsync(d, v, n * sizeof(double), cudaMemcpyHostToDevice, g_ctx.stream));
-    NCCL_TRY(g_comm.AllReduce(d, d, n, ncclDouble, ncclMax, g_comm.comm, g_ctx.stream));
-    CUDA_TRY(cudaMemcpyAsync(v, d, n * sizeof(double), cudaMemcpyDeviceToHost, g_ctx.stream));
+    DevBuf<double> d;
+    if (int rc = d.alloc(n, g_ctx.stream, "the reduction")) return rc;
+    CUDA_TRY(cudaMemcpyAsync(d.get(), v, n * sizeof(double), cudaMemcpyHostToDevice, g_ctx.stream));
+    NCCL_TRY(g_comm.AllReduce(d.get(), d.get(), n, ncclDouble, ncclMax, g_comm.comm, g_ctx.stream));
+    CUDA_TRY(cudaMemcpyAsync(v, d.get(), n * sizeof(double), cudaMemcpyDeviceToHost, g_ctx.stream));
     CUDA_TRY(cudaStreamSynchronize(g_ctx.stream));
-    dev_free(d, g_ctx.stream);
     return 0;
 }
 
@@ -616,13 +692,12 @@ int crp_comm_sum_f64(double *v, uint32_t n) {
     if (int rc = need_ctx()) return rc;
     if (!v && n) return fail(CRP_ERR_ARG, "v is NULL");
     if (!g_comm.comm || n == 0) return 0;
-    double *d = nullptr;
-    CUDA_TRY(dev_alloc(&d, n * sizeof(double), g_ctx.stream));
-    CUDA_TRY(cudaMemcpyAsync(d, v, n * sizeof(double), cudaMemcpyHostToDevice, g_ctx.stream));
-    NCCL_TRY(g_comm.AllReduce(d, d, n, ncclDouble, ncclSum, g_comm.comm, g_ctx.stream));
-    CUDA_TRY(cudaMemcpyAsync(v, d, n * sizeof(double), cudaMemcpyDeviceToHost, g_ctx.stream));
+    DevBuf<double> d;
+    if (int rc = d.alloc(n, g_ctx.stream, "the reduction")) return rc;
+    CUDA_TRY(cudaMemcpyAsync(d.get(), v, n * sizeof(double), cudaMemcpyHostToDevice, g_ctx.stream));
+    NCCL_TRY(g_comm.AllReduce(d.get(), d.get(), n, ncclDouble, ncclSum, g_comm.comm, g_ctx.stream));
+    CUDA_TRY(cudaMemcpyAsync(v, d.get(), n * sizeof(double), cudaMemcpyDeviceToHost, g_ctx.stream));
     CUDA_TRY(cudaStreamSynchronize(g_ctx.stream));
-    dev_free(d, g_ctx.stream);
     return 0;
 }
 
@@ -635,17 +710,13 @@ int crp_comm_allgather_u64(const uint64_t *in, uint32_t n, uint64_t *out) {
         memcpy(out, in, n * sizeof(uint64_t));
         return 0;
     }
-    unsigned long long *d = nullptr;
     const size_t w = (size_t)g_comm.world;
-    CUDA_TRY(dev_alloc(&d, (w + 1) * n * sizeof(uint64_t), g_ctx.stream));
-    CUDA_TRY(cudaMemcpyAsync(d, in, n * sizeof(uint64_t), cudaMemcpyHostToDevice, g_ctx.stream));
-    if (int rc = comm_allgather_u64(d, d + n, n, g_ctx.stream)) {
-        dev_free(d, g_ctx.stream);
-        return rc;
-    }
-    CUDA_TRY(cudaMemcpyAsync(out, d + n, w * n * sizeof(uint64_t), cudaMemcpyDeviceToHost, g_ctx.stream));
+    DevBuf<unsigned long long> d;
+    if (int rc = d.alloc((w + 1) * n, g_ctx.stream, "the all-gather")) return rc;
+    CUDA_TRY(cudaMemcpyAsync(d.get(), in, n * sizeof(uint64_t), cudaMemcpyHostToDevice, g_ctx.stream));
+    if (int rc = comm_allgather_u64(d.get(), d.get() + n, n, g_ctx.stream)) return rc;
+    CUDA_TRY(cudaMemcpyAsync(out, d.get() + n, w * n * sizeof(uint64_t), cudaMemcpyDeviceToHost, g_ctx.stream));
     CUDA_TRY(cudaStreamSynchronize(g_ctx.stream));
-    dev_free(d, g_ctx.stream);
     return 0;
 }
 
@@ -656,7 +727,7 @@ int crp_link_probe(uint64_t h2d_bytes, uint64_t d2h_bytes, uint32_t reps, float 
     if (int rc = need_ctx()) return rc;
     if (!ms || !reps) return fail(CRP_ERR_ARG, "bad argument");
     void *h_in = nullptr, *h_out = nullptr;
-    unsigned char *d_in = nullptr, *d_out = nullptr;
+    DevBuf<unsigned char> d_in, d_out;
     cudaStream_t s2 = nullptr;
     int rc = 0;
     do {
@@ -667,17 +738,19 @@ int crp_link_probe(uint64_t h2d_bytes, uint64_t d2h_bytes, uint32_t reps, float 
         }
         memset(h_in, 1, h2d_bytes + 16);
         memset(h_out, 1, d2h_bytes + 16);
-        if (dev_alloc(&d_in, h2d_bytes + 16, g_ctx.stream) != cudaSuccess || dev_alloc(&d_out, d2h_bytes + 16, g_ctx.stream) != cudaSuccess ||
-            cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking) != cudaSuccess) {
-            rc = fail(CRP_ERR_NOMEM, "device buffers of the link probe failed");
+        if ((rc = d_in.alloc(h2d_bytes + 16, g_ctx.stream, "the link probe's input")) ||
+            (rc = d_out.alloc(d2h_bytes + 16, g_ctx.stream, "the link probe's output")))
+            break;
+        if (cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking) != cudaSuccess) {
+            rc = fail(CRP_ERR_CUDA, "cudaStreamCreate failed");
             break;
         }
         cudaStreamSynchronize(g_ctx.stream);
         double total = 0.0;
         for (uint32_t i = 0; i <= reps; ++i) {            // round 0 warms up
             const auto t0 = std::chrono::steady_clock::now();
-            cudaMemcpyAsync(d_in, h_in, h2d_bytes, cudaMemcpyHostToDevice, g_ctx.stream);
-            cudaMemcpyAsync(h_out, d_out, d2h_bytes, cudaMemcpyDeviceToHost, s2);
+            cudaMemcpyAsync(d_in.get(), h_in, h2d_bytes, cudaMemcpyHostToDevice, g_ctx.stream);
+            cudaMemcpyAsync(h_out, d_out.get(), d2h_bytes, cudaMemcpyDeviceToHost, s2);
             cudaStreamSynchronize(g_ctx.stream);
             cudaStreamSynchronize(s2);
             if (i) total += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -686,8 +759,6 @@ int crp_link_probe(uint64_t h2d_bytes, uint64_t d2h_bytes, uint32_t reps, float 
         *ms = (float)(total / reps);
     } while (0);
     if (s2) cudaStreamDestroy(s2);
-    dev_free(d_in, g_ctx.stream);
-    dev_free(d_out, g_ctx.stream);
     if (h_in) cudaFreeHost(h_in);
     if (h_out) cudaFreeHost(h_out);
     return rc;
@@ -718,12 +789,10 @@ int crp_comm_shutdown(void) {
 /* Evict the L2 cache (benchmarks: between timed scans): a memset larger than L2, on the library stream. */
 int crp_flush_l2(void) {
     if (int rc = need_ctx()) return rc;
-    unsigned char *buf = nullptr;                    // from the block cache: allocated once, reused by every call
+    DevBuf<unsigned char> buf;                       // from the block cache: allocated once, reused by every call
     const size_t bytes = 512ull << 20;
-    CUDA_TRY(dev_alloc(&buf, bytes, g_ctx.stream));
-    cudaError_t e = cudaMemsetAsync(buf, 0, bytes, g_ctx.stream);
-    dev_free(buf, g_ctx.stream);
-    CUDA_TRY(e);
+    if (int rc = buf.alloc(bytes, g_ctx.stream, "the L2 flush")) return rc;
+    CUDA_TRY(cudaMemsetAsync(buf.get(), 0, bytes, g_ctx.stream));
     CUDA_TRY(cudaStreamSynchronize(g_ctx.stream));
     return 0;
 }
@@ -813,21 +882,20 @@ int crp_genome_token_length(const crp_genome *g, uint32_t segment, uint64_t *tok
 int crp_genome_fetch_token(const crp_genome *g, uint32_t segment, uint8_t *dst, uint64_t capacity) {
     if (!g || !dst) return fail(CRP_ERR_ARG, "NULL argument");
     if (int rc = need_ctx()) return rc;
-    if (!g->committed || !g->d_ascii) return fail(CRP_ERR_STATE, "the genome keeps no tokens on the device");
+    if (!g->committed || !g->d_ascii.get()) return fail(CRP_ERR_STATE, "the genome keeps no tokens on the device");
     if (segment >= g->segs.size()) return fail(CRP_ERR_ARG, "segment %u out of range", segment);
     const Segment &s = g->segs[segment];
     if (!s.raw) return fail(CRP_ERR_STATE, "segment %u was not ingested from FASTA bytes", segment);
     if (capacity < s.token_len) return fail(CRP_ERR_RANGE, "token needs %llu bytes", (unsigned long long)s.token_len);
     cudaStream_t st = g->st ? g->st : g_ctx.stream;
-    CUDA_TRY(cudaMemcpyAsync(dst, g->d_ascii + s.ascii_off, s.token_len, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(dst, g->d_ascii.get() + s.ascii_off, s.token_len, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return 0;
 }
 
 int crp_genome_release_tokens(crp_genome *g) {
     if (!g) return fail(CRP_ERR_ARG, "g is NULL");
-    dev_free(g->d_ascii, g->st ? g->st : g_ctx.stream);
-    g->d_ascii = nullptr;
+    g->d_ascii.reset();
     return 0;
 }
 
@@ -889,26 +957,21 @@ static int commit_enqueue(crp_genome *g) {
     g_perf.positions += g->n_positions;
     g_perf.h2d_bytes += ascii_bytes;
 
-    uint8_t *d_ascii = nullptr;
-    PackDesc *d_descs = nullptr;
-    const size_t rec_bytes = (size_t)g->n_tiles * kRecBytes;
-    if (dev_alloc(&d_ascii, ascii_bytes + 64, st) != cudaSuccess ||
-        (!one && dev_alloc(&d_descs, (descs.size() + 1) * sizeof(PackDesc), st) != cudaSuccess) ||
-        dev_alloc(&g->records, rec_bytes + 16, st) != cudaSuccess ||
-        dev_alloc(&g->pam, (size_t)g->n_tiles * kPamBytes + 16, st) != cudaSuccess ||
-        dev_alloc(&g->hdr, ((size_t)g->n_tiles + 1) * sizeof(TileHdr), st) != cudaSuccess) {
-        cudaGetLastError();
-        dev_free(d_ascii, st);
-        dev_free(d_descs, st);
-        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu record bytes + %llu staging bytes failed",
-                    (unsigned long long)rec_bytes, (unsigned long long)ascii_bytes);
-    }
+    DevBuf<PackDesc> d_descs;             // staging: both go back at the end, behind the pack kernel in stream order
+    DevBuf<uint8_t> d_ascii;
+    int rc;
+    if ((rc = d_ascii.alloc(ascii_bytes + 64, st, "the token staging")) ||
+        (!one && (rc = d_descs.alloc(descs.size() + 1, st, "the pack descriptors"))) ||
+        (rc = g->records.alloc((size_t)g->n_tiles * (kRecBytes / sizeof(uint4)) + 1, st, "the tile records")) ||
+        (rc = g->pam.alloc((size_t)g->n_tiles * kPamBytes + 16, st, "the PAM records")) ||
+        (rc = g->hdr.alloc((size_t)g->n_tiles + 1, st, "the tile headers")))
+        return rc;
     for (int i = 0; i < 3; ++i)
         if (!g->ev[i]) CUDA_TRY(cudaEventCreate(&g->ev[i]));
     CUDA_TRY(cudaEventRecord(g->ev[0], st));
-    uint8_t *d_raw = nullptr;
-    FastaRec *d_recs = nullptr;
-    unsigned int *d_bad = nullptr;
+    DevBuf<uint8_t> d_raw;
+    DevBuf<FastaRec> d_recs;
+    DevBuf<unsigned int> d_bad;
     std::vector<FastaRec> frecs;
     uint64_t raw_total = 0, strip_items = 0;
     for (size_t si = 0; si < g->segs.size(); ++si) {
@@ -927,62 +990,58 @@ static int commit_enqueue(crp_genome *g) {
         strip_items += (s.token_len + 15) / 16;
     }
     if (!frecs.empty()) {
-        if (dev_alloc(&d_raw, raw_total + 64, st) != cudaSuccess ||
-            dev_alloc(&d_recs, frecs.size() * sizeof(FastaRec), st) != cudaSuccess ||
-            dev_alloc(&d_bad, sizeof(unsigned int), st) != cudaSuccess) {
-            cudaGetLastError();
-            return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu FASTA bytes failed", (unsigned long long)raw_total);
-        }
-        CUDA_TRY(cudaMemsetAsync(d_bad, 0, sizeof(unsigned int), st));
+        if ((rc = d_raw.alloc(raw_total + 64, st, "the FASTA bytes")) ||
+            (rc = d_recs.alloc(frecs.size(), st, "the FASTA records")) || (rc = d_bad.alloc(1, st, "the FASTA flag")))
+            return rc;
+        CUDA_TRY(cudaMemsetAsync(d_bad.get(), 0, sizeof(unsigned int), st));
     }
     for (size_t si = 0, fi = 0; si < g->segs.size(); ++si) {
         const Segment &s = g->segs[si];
         if (s.raw) {
-            CUDA_TRY(cudaMemcpyAsync(d_raw + frecs[fi++].raw_off, s.raw, s.raw_bytes, cudaMemcpyHostToDevice, st));
+            CUDA_TRY(cudaMemcpyAsync(d_raw.get() + frecs[fi++].raw_off, s.raw, s.raw_bytes, cudaMemcpyHostToDevice, st));
         } else if (s.stage_end > s.stage_begin && s.n_tiles) {
-            CUDA_TRY(cudaMemcpyAsync(d_ascii + seg_ascii[si], s.token + s.stage_begin, s.stage_end - s.stage_begin,
+            CUDA_TRY(cudaMemcpyAsync(d_ascii.get() + seg_ascii[si], s.token + s.stage_begin, s.stage_end - s.stage_begin,
                                      cudaMemcpyHostToDevice, st));
         }
     }
     if (!frecs.empty()) {
-        CUDA_TRY(cudaMemcpyAsync(d_recs, frecs.data(), frecs.size() * sizeof(FastaRec), cudaMemcpyHostToDevice, st));
+        CUDA_TRY(cudaMemcpyAsync(d_recs.get(), frecs.data(), frecs.size() * sizeof(FastaRec), cudaMemcpyHostToDevice, st));
         const uint64_t want = (strip_items + 255) / 256, cap = (uint64_t)g_ctx.sm_count * 16;
-        k_fasta_strip<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(d_raw, d_recs, (uint32_t)frecs.size(),
-                                                                           strip_items, d_ascii, d_bad);
+        k_fasta_strip<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(d_raw.get(), d_recs.get(), (uint32_t)frecs.size(),
+                                                                           strip_items, d_ascii.get(), d_bad.get());
         g_ctx.launches++;
         CUDA_TRY(cudaGetLastError());
-        if (!g->h_bad) g->h_bad = static_cast<unsigned int *>(pinned_get(sizeof(unsigned int)));
-        if (!g->h_bad) return fail(CRP_ERR_NOMEM, "cudaHostAlloc failed");
-        *g->h_bad = 0;
-        CUDA_TRY(cudaMemcpyAsync(g->h_bad, d_bad, sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
-        dev_free(d_raw, st);
-        dev_free(d_recs, st);
-        dev_free(d_bad, st);
+        if (!g->h_bad.get() && (rc = g->h_bad.alloc(1, "the FASTA flag"))) return rc;
+        *g->h_bad.get() = 0;
+        CUDA_TRY(cudaMemcpyAsync(g->h_bad.get(), d_bad.get(), sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
+        d_raw.reset();                    // before the pack kernel in stream order
+        d_recs.reset();
+        d_bad.reset();
     }
     if (!one && !descs.empty())
-        CUDA_TRY(cudaMemcpyAsync(d_descs, descs.data(), descs.size() * sizeof(PackDesc), cudaMemcpyHostToDevice, st));
+        CUDA_TRY(cudaMemcpyAsync(d_descs.get(), descs.data(), descs.size() * sizeof(PackDesc), cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaEventRecord(g->ev[1], st));
     const uint64_t n_items = (uint64_t)g->n_tiles * kPackItems;
     if (n_items) {
         PackDesc first = descs[0];
         if (one) first.td.n = (uint32_t)(g->segs[0].end - g->segs[0].begin);     // positions of the whole segment
         const uint64_t want = (n_items + 255) / 256, cap = (uint64_t)g_ctx.sm_count * 16;
-        CUDA_TRY(cudaMemsetAsync(g->hdr, 0, (size_t)g->n_tiles * sizeof(TileHdr), st));      // chunk counts are accumulated
-        k_pack<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(d_ascii, d_descs, first, n_items, g->records, g->pam, g->hdr);
+        CUDA_TRY(cudaMemsetAsync(g->hdr.get(), 0, (size_t)g->n_tiles * sizeof(TileHdr), st));      // chunk counts are accumulated
+        k_pack<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(d_ascii.get(), d_descs.get(), first, n_items, g->records.get(),
+                                                                    g->pam.get(), g->hdr.get());
         g_ctx.launches++;
         CUDA_TRY(cudaGetLastError());
     }
     CUDA_TRY(cudaEventRecord(g->ev[2], st));
     if (!one && !g->segs.empty()) {
         const size_t nb = g->segs.size() * sizeof(uint32_t);
-        CUDA_TRY(dev_alloc(&g->d_seg_first, nb, st));
-        CUDA_TRY(dev_alloc(&g->d_seg_count, nb, st));
-        CUDA_TRY(cudaMemcpyAsync(g->d_seg_first, seg_first.data(), nb, cudaMemcpyHostToDevice, st));
-        CUDA_TRY(cudaMemcpyAsync(g->d_seg_count, seg_count.data(), nb, cudaMemcpyHostToDevice, st));
+        if ((rc = g->d_seg_first.alloc(g->segs.size(), st, "the segment table")) ||
+            (rc = g->d_seg_count.alloc(g->segs.size(), st, "the segment table")))
+            return rc;
+        CUDA_TRY(cudaMemcpyAsync(g->d_seg_first.get(), seg_first.data(), nb, cudaMemcpyHostToDevice, st));
+        CUDA_TRY(cudaMemcpyAsync(g->d_seg_count.get(), seg_count.data(), nb, cudaMemcpyHostToDevice, st));
     }
-    if (g->fasta) g->d_ascii = d_ascii;   // kept: the host fetches the tokens it formats rows from
-    else dev_free(d_ascii, st);           // stream ordered: after the pack kernel
-    dev_free(d_descs, st);
+    if (g->fasta) g->d_ascii = std::move(d_ascii);   // kept: the host fetches the tokens it formats rows from
     g->committed = true;
     return 0;
 }
@@ -1001,7 +1060,7 @@ int crp_genome_commit(crp_genome *g) {
     g_perf.ms_h2d += g->ms_h2d;
     g_perf.ms_pack += g->ms_pack;
     for (Segment &s : g->segs) s.token = nullptr;   // host tokens may be released now
-    if (g->h_bad && *g->h_bad)
+    if (g->h_bad.get() && *g->h_bad.get())
         return fail(CRP_ERR_FORMAT, "a FASTA record is not plain fixed-width text; use the host ingest for this file");
     return 0;
 }
@@ -1015,47 +1074,23 @@ int crp_genome_timing(const crp_genome *g, float *ms_h2d, float *ms_pack) {
 
 int crp_genome_free(crp_genome *g) {
     if (!g) return 0;
-    cudaStream_t st = stream_of(g);
-    dev_free(g->records, st);
-    dev_free(g->pam, st);
-    dev_free(g->hdr, st);
-    dev_free(g->d_ascii, st);
-    pinned_put(g->h_bad);
-    dev_free(g->d_seg_first, st);
-    dev_free(g->d_seg_count, st);
     for (cudaEvent_t e : g->ev)
         if (e) cudaEventDestroy(e);
     delete g;
     return 0;
 }
 
-static void free_streams(crp_result *r) {
-    for (int s = 0; s < 2; ++s) {
-        dev_free(r->pos[s], r->st);
-        dev_free(r->packed[s], r->st);
-        dev_free(r->x[s], r->st);
-        r->pos[s] = nullptr;
-        r->packed[s] = nullptr;
-        r->x[s] = nullptr;
-    }
-}
-
 static int alloc_streams(crp_result *r, uint64_t cap, bool scored) {
     r->capacity = cap;
     const uint64_t n = cap ? cap : 1;
     for (int s = 0; s < 2; ++s) {
-        if (dev_alloc(&r->pos[s], n * sizeof(uint32_t), r->st) != cudaSuccess) goto oom;
+        if (int rc = r->pos[s].alloc(n, r->st, "a candidate stream")) return rc;
         if (scored) {
-            if (dev_alloc(&r->packed[s], n * sizeof(unsigned long long), r->st) != cudaSuccess) goto oom;
-            if (dev_alloc(&r->x[s], n * sizeof(double), r->st) != cudaSuccess) goto oom;
+            if (int rc = r->packed[s].alloc(n, r->st, "a candidate stream")) return rc;
+            if (int rc = r->x[s].alloc(n, r->st, "a candidate stream")) return rc;
         }
     }
     return 0;
-oom:
-    cudaGetLastError();
-    free_streams(r);
-    return fail(CRP_ERR_NOMEM, "cudaMalloc of candidate streams (%llu entries per strand) failed",
-                (unsigned long long)cap);
 }
 
 // Launch geometry of the cooperative scan kernel for a genome of n_tiles tiles.
@@ -1094,9 +1129,9 @@ static int plan_scan(const crp_genome *g, bool scored, ScanPlan *p) {
 static int launch_scan(const crp_genome *g, crp_result *r, const ScanPlan &p) {
     cudaStream_t st = r->st;
     ScanArgs a;
-    a.records = g->records;
-    a.pam = g->pam;
-    a.hdr = g->hdr;
+    a.records = g->records.get();
+    a.pam = g->pam.get();
+    a.hdr = g->hdr.get();
     a.n_tiles = g->n_tiles;
     a.static_eighths = 4;
     if (const char *e = getenv("CRP_STATIC_EIGHTHS")) a.static_eighths = (uint32_t)atoi(e) > 8 ? 8 : (uint32_t)atoi(e);
@@ -1104,23 +1139,23 @@ static int launch_scan(const crp_genome *g, crp_result *r, const ScanPlan &p) {
     a.flags = r->flags;
     a.tables = g_ctx.d_tables;
     a.capacity = r->capacity < 0xFFFFFFFFull ? r->capacity : 0xFFFFFFFFull;   // rows are 32-bit in the kernel (counts are packed 32 | 32)
-    a.pos_plus = r->pos[0];
-    a.pos_minus = r->pos[1];
-    a.packed_plus = r->packed[0];
-    a.packed_minus = r->packed[1];
-    a.x_plus = r->x[0];
-    a.x_minus = r->x[1];
+    a.pos_plus = r->pos[0].get();
+    a.pos_minus = r->pos[1].get();
+    a.packed_plus = r->packed[0].get();
+    a.packed_minus = r->packed[1].get();
+    a.x_plus = r->x[0].get();
+    a.x_minus = r->x[1].get();
     const uint32_t n_seg = (uint32_t)g->segs.size();
-    unsigned long long *s64 = reinterpret_cast<unsigned long long *>(r->state);
+    unsigned long long *s64 = reinterpret_cast<unsigned long long *>(r->state.get());
     a.warp_pref = s64;
     a.cta_tot = s64 + (size_t)g->n_tiles * kPrefWords;
     a.seg_counts = r->d_counts;
     a.tickets = reinterpret_cast<unsigned int *>(r->d_counts + 2 * (size_t)r->stride);
     a.n_seg = n_seg;
     a.seg_stride = r->stride;
-    a.seg_first_tile = g->d_seg_first;      // NULL for a single-segment genome
-    a.seg_tile_count = g->d_seg_count;
-    a.seg_counts_host = r->h_counts;        // mapped pinned memory: the kernel stores the counts there itself
+    a.seg_first_tile = g->d_seg_first.get();   // NULL for a single-segment genome
+    a.seg_tile_count = g->d_seg_count.get();
+    a.seg_counts_host = r->h_counts.get();     // mapped pinned memory: the kernel stores the counts there itself
     a.fault = g_ctx.d_fault;
     a.world = 1;
     a.rank = 0;
@@ -1131,7 +1166,7 @@ static int launch_scan(const crp_genome *g, crp_result *r, const ScanPlan &p) {
         a.peer_gather[q] = nullptr;
         a.peer_flags[q] = nullptr;
     }
-    const unsigned long long *gathered = r->d_gather;       // where the blocks of all ranks end up
+    const unsigned long long *gathered = r->d_gather.get();   // where the blocks of all ranks end up
     if (r->fused) {
         // Fused exchange: the kernel stores this rank's counts into every rank's buffer right after its
         // count phase and leaves once all blocks are in its own -- no collective launch behind the kernel.
@@ -1158,21 +1193,21 @@ static int launch_scan(const crp_genome *g, crp_result *r, const ScanPlan &p) {
         CUDA_TRY(cudaGetLastError());
     } else if (r->stride) {
         CUDA_TRY(cudaMemsetAsync(r->d_counts, 0, 2 * (size_t)r->stride * sizeof(unsigned long long), st));
-        memset(r->h_counts, 0, 2 * (size_t)r->stride * sizeof(unsigned long long));
+        memset(r->h_counts.get(), 0, 2 * (size_t)r->stride * sizeof(unsigned long long));
     }
     if (r->ev_kernel) CUDA_TRY(cudaEventRecord(r->ev_kernel, st));
-    if (r->d_gather && !r->fused) {
+    if (r->d_gather.get() && !r->fused) {
         // NCCL exchange: every rank's per-segment counts to every rank, right behind the kernel on the
         // same stream, so the CUDA events bracket kernel + collective
-        if (int rc = comm_allgather_u64(r->d_counts, r->d_gather, 2 * (size_t)r->stride, st)) return rc;
+        if (int rc = comm_allgather_u64(r->d_counts, r->d_gather.get(), 2 * (size_t)r->stride, st)) return rc;
     }
     CUDA_TRY(cudaEventRecord(r->ev[1], st));
     // (the per-segment counts are already in r->h_counts: the kernel stored them into mapped host memory)
-    if (r->h_gather && gathered)
-        CUDA_TRY(cudaMemcpyAsync(r->h_gather, gathered, (size_t)g_comm.world * 2 * r->stride * sizeof(unsigned long long),
+    if (r->h_gather.get() && gathered)
+        CUDA_TRY(cudaMemcpyAsync(r->h_gather.get(), gathered, (size_t)g_comm.world * 2 * r->stride * sizeof(unsigned long long),
                                  cudaMemcpyDeviceToHost, st));
     if (r->fused)
-        CUDA_TRY(cudaMemcpyAsync(r->h_xchg_error, xchg_error(g_comm.xchg), sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaMemcpyAsync(r->h_xchg_error.get(), xchg_error(g_comm.xchg), sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaEventRecord(r->ev[2], st));
     return 0;
 }
@@ -1198,24 +1233,19 @@ static int scan_enqueue(crp_genome *g, int guide_len, uint32_t flags, crp_result
     r->zero_offset = ((size_t)g->n_tiles * kPrefWords + (size_t)plan.grid) * sizeof(unsigned long long);
     r->state_bytes = r->zero_offset + 2 * (size_t)r->stride * sizeof(unsigned long long) +
                      4 * sizeof(unsigned int);
-    if (dev_alloc(&r->state, r->state_bytes, r->st) != cudaSuccess)
-        return bail(fail(CRP_ERR_NOMEM, "cudaMalloc of scan state failed"));
-    r->d_counts = reinterpret_cast<unsigned long long *>(r->state + r->zero_offset);
-    r->h_counts = static_cast<unsigned long long *>(pinned_get((2 * (size_t)r->stride + 1) * sizeof(unsigned long long)));
-    if (!r->h_counts) return bail(fail(CRP_ERR_NOMEM, "cudaHostAlloc of the counts failed"));
+    if ((rc = r->state.alloc(r->state_bytes, r->st, "the scan state"))) return bail(rc);
+    r->d_counts = reinterpret_cast<unsigned long long *>(r->state.get() + r->zero_offset);
+    if ((rc = r->h_counts.alloc(2 * (size_t)r->stride + 1, "the counts"))) return bail(rc);
     if (slots) {
-        const size_t gb = (size_t)g_comm.world * 2 * slots * sizeof(unsigned long long);
+        const size_t gn = (size_t)g_comm.world * 2 * slots;
         r->fused = g_comm.fused && g_comm.mode == 0 && slots <= kXchgSlots;
         r->epoch = ++g_comm.epoch;
         if (r->fused) {
-            r->h_xchg_error = static_cast<unsigned int *>(pinned_get(sizeof(unsigned int)));
-            if (!r->h_xchg_error) return bail(fail(CRP_ERR_NOMEM, "cudaHostAlloc failed"));
-            *r->h_xchg_error = 0;
+            if ((rc = r->h_xchg_error.alloc(1, "the exchange error"))) return bail(rc);
+            *r->h_xchg_error.get() = 0;
         }
-        if (dev_alloc(&r->d_gather, gb, r->st) != cudaSuccess)
-            return bail(fail(CRP_ERR_NOMEM, "cudaMalloc of the gathered counts failed"));
-        r->h_gather = static_cast<unsigned long long *>(pinned_get(gb));
-        if (!r->h_gather) return bail(fail(CRP_ERR_NOMEM, "cudaHostAlloc of the gathered counts failed"));
+        if ((rc = r->d_gather.alloc(gn, r->st, "the gathered counts"))) return bail(rc);
+        if ((rc = r->h_gather.alloc(gn, "the gathered counts"))) return bail(rc);
         if (cudaEventCreate(&r->ev_kernel) != cudaSuccess) return bail(fail(CRP_ERR_CUDA, "cudaEventCreate failed"));
     }
     if (cudaEventCreate(&r->ev[0]) != cudaSuccess || cudaEventCreate(&r->ev[1]) != cudaSuccess ||
@@ -1243,8 +1273,8 @@ static int scan_finish(crp_genome *g, crp_result *r, cudaStream_t post = nullptr
         r->seg_plus.assign(n_seg, 0);
         r->seg_minus.assign(n_seg, 0);
         for (uint32_t s = 0; s < n_seg; ++s) {
-            r->seg_plus[s] = r->h_counts[s];
-            r->seg_minus[s] = r->h_counts[r->stride + s];
+            r->seg_plus[s] = r->h_counts.get()[s];
+            r->seg_minus[s] = r->h_counts.get()[r->stride + s];
             r->n_plus += r->seg_plus[s];
             r->n_minus += r->seg_minus[s];
         }
@@ -1266,25 +1296,26 @@ static int scan_finish(crp_genome *g, crp_result *r, cudaStream_t post = nullptr
             }
         }
 #endif
-        if (r->fused && *r->h_xchg_error)
-            return fail(CRP_ERR_CUDA, "sharded scan: the counts of rank %u did not arrive (peer not scanning?)", *r->h_xchg_error - 1);
+        if (r->fused && *r->h_xchg_error.get())
+            return fail(CRP_ERR_CUDA, "sharded scan: the counts of rank %u did not arrive (peer not scanning?)", *r->h_xchg_error.get() - 1);
         const uint64_t need = r->n_plus > r->n_minus ? r->n_plus : r->n_minus;
         if (need <= r->capacity) break;
         if (attempt == 1) return fail(CRP_ERR_STATE, "candidate streams overflowed twice");
         // the rerun is local: the counts are already exchanged, the second launch only fills the streams
         r->fused = false;
-        if (r->d_gather) {
-            dev_free(r->d_gather, r->st);
-            r->d_gather = nullptr;               // keeps h_gather of the first launch
+        r->d_gather.reset();                     // keeps h_gather of the first launch
+        for (int s = 0; s < 2; ++s) {
+            r->pos[s].reset();
+            r->packed[s].reset();
+            r->x[s].reset();
         }
-        free_streams(r);
         if (int rc = alloc_streams(r, need, r->scored)) return rc;
         ScanPlan plan = {};
         if (int rc = plan_scan(g, r->scored, &plan)) return rc;
         if (int rc = launch_scan(g, r, plan)) return rc;
     }
     g_perf.scans++;
-    if (r->stride != (uint32_t)g->segs.size() || r->h_gather) g_perf.sharded_scans++;
+    if (r->stride != (uint32_t)g->segs.size() || r->h_gather.get()) g_perf.sharded_scans++;
     if (r->epoch && g_comm.fused && g_comm.mode == 0) g_perf.fused_exchanges++;
     g_perf.capacity_reruns += r->n_launches - 1;
     g_perf.candidates += r->n_plus + r->n_minus;
@@ -1295,7 +1326,7 @@ static int scan_finish(crp_genome *g, crp_result *r, cudaStream_t post = nullptr
         for (int s = 0; s < 2; ++s)
             if (n[s]) {
                 const uint64_t want = (n[s] + 255) / 256, cap = (uint64_t)g_ctx.sm_count * 16;
-                k_logistic<<<(unsigned)(want < cap ? want : cap), 256, 0, post ? post : r->st>>>(r->x[s], n[s]);
+                k_logistic<<<(unsigned)(want < cap ? want : cap), 256, 0, post ? post : r->st>>>(r->x[s].get(), n[s]);
                 g_ctx.launches++;
             }
         CUDA_TRY(cudaGetLastError());
@@ -1343,8 +1374,8 @@ int crp_scan_score_sharded(crp_genome *g, int guide_len, uint32_t flags, uint32_
 
 int crp_result_gathered_counts(const crp_result *res, uint64_t *counts) {
     if (!res || !counts) return fail(CRP_ERR_ARG, "NULL argument");
-    if (!res->h_gather) return fail(CRP_ERR_STATE, "not the result of a sharded scan");
-    memcpy(counts, res->h_gather, (size_t)g_comm.world * 2 * res->stride * sizeof(uint64_t));
+    if (!res->h_gather.get()) return fail(CRP_ERR_STATE, "not the result of a sharded scan");
+    memcpy(counts, res->h_gather.get(), (size_t)g_comm.world * 2 * res->stride * sizeof(uint64_t));
     return 0;
 }
 
@@ -1360,21 +1391,16 @@ static int rs1_rows(uint64_t n, const uint8_t *rows, const uint8_t *cls, double 
     if (int rc = need_ctx()) return rc;
     if (!n) return 0;
     cudaStream_t st = g_ctx.stream;
-    uint8_t *d_rows = nullptr;
-    double *d_out = nullptr;
-    if (dev_alloc(&d_rows, 31 * n, st) != cudaSuccess || dev_alloc(&d_out, n * sizeof(double), st) != cudaSuccess) {
-        cudaGetLastError();
-        dev_free(d_rows, st);
-        return fail(CRP_ERR_NOMEM, "cudaMalloc for %llu rows failed", (unsigned long long)n);
-    }
-    CUDA_TRY(cudaMemcpyAsync(d_rows, rows, 30 * n, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(d_rows + 30 * n, cls, n, cudaMemcpyHostToDevice, st));
-    k_rs1_rows<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(d_rows, d_rows + 30 * n, n, d_out, logistic);
+    DevBuf<double> d_out;
+    DevBuf<uint8_t> d_rows;
+    int rc;
+    if ((rc = d_rows.alloc(31 * n, st, "the rows")) || (rc = d_out.alloc(n, st, "the scores"))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(d_rows.get(), rows, 30 * n, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(d_rows.get() + 30 * n, cls, n, cudaMemcpyHostToDevice, st));
+    k_rs1_rows<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(d_rows.get(), d_rows.get() + 30 * n, n, d_out.get(), logistic);
     g_ctx.launches++;
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(score, d_out, n * sizeof(double), cudaMemcpyDeviceToHost, st));
-    dev_free(d_rows, st);
-    dev_free(d_out, st);
+    CUDA_TRY(cudaMemcpyAsync(score, d_out.get(), n * sizeof(double), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return 0;
 }
@@ -1384,18 +1410,14 @@ int crp_logistic(uint64_t n, const double *x, double *score) {
     if (int rc = need_ctx()) return rc;
     if (!n) return 0;
     cudaStream_t st = g_ctx.stream;
-    double *d = nullptr;
-    if (dev_alloc(&d, n * sizeof(double), st) != cudaSuccess) {
-        cudaGetLastError();
-        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu doubles failed", (unsigned long long)n);
-    }
-    CUDA_TRY(cudaMemcpyAsync(d, x, n * sizeof(double), cudaMemcpyHostToDevice, st));
+    DevBuf<double> d;
+    if (int rc = d.alloc(n, st, "the logistic's input")) return rc;
+    CUDA_TRY(cudaMemcpyAsync(d.get(), x, n * sizeof(double), cudaMemcpyHostToDevice, st));
     const uint64_t want = (n + 255) / 256, cap = (uint64_t)g_ctx.sm_count * 16;
-    k_logistic<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(d, n);
+    k_logistic<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(d.get(), n);
     g_ctx.launches++;
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(score, d, n * sizeof(double), cudaMemcpyDeviceToHost, st));
-    dev_free(d, st);
+    CUDA_TRY(cudaMemcpyAsync(score, d.get(), n * sizeof(double), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return 0;
 }
@@ -1428,10 +1450,10 @@ static int fetch_enqueue(const crp_result *res, int s, uint64_t first, uint64_t 
     if (!st) st = res->st;
     g_perf.d2h_bytes += count * ((pos ? 4 : 0) + (packed ? 8 : 0) + (x ? 8 : 0));
     if (count) {
-        if (pos) CUDA_TRY(cudaMemcpyAsync(pos, res->pos[s] + first, count * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        if (pos) CUDA_TRY(cudaMemcpyAsync(pos, res->pos[s].get() + first, count * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
         if (packed)
-            CUDA_TRY(cudaMemcpyAsync(packed, res->packed[s] + first, count * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-        if (x) CUDA_TRY(cudaMemcpyAsync(x, res->x[s] + first, count * sizeof(double), cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(cudaMemcpyAsync(packed, res->packed[s].get() + first, count * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+        if (x) CUDA_TRY(cudaMemcpyAsync(x, res->x[s].get() + first, count * sizeof(double), cudaMemcpyDeviceToHost, st));
     }
     return 0;
 }
@@ -1469,12 +1491,6 @@ int crp_result_timing_detail(const crp_result *res, float *ms_kernels, float *ms
 
 int crp_result_free(crp_result *r) {
     if (!r) return 0;
-    free_streams(r);
-    dev_free(r->state, r->st);
-    dev_free(r->d_gather, r->st);
-    pinned_put(r->h_counts);
-    pinned_put(r->h_gather);
-    pinned_put(r->h_xchg_error);
     if (r->ev_kernel) cudaEventDestroy(r->ev_kernel);
     for (cudaEvent_t e : r->ev)
         if (e) cudaEventDestroy(e);
@@ -1656,31 +1672,27 @@ int crp_result_extras(const crp_result *res, uint32_t segment, char strand, uint
     const Segment &sg = g->segs[segment];
     cudaStream_t st = res->st;
     const int s = strand == '+' ? 0 : 1;
-    uint8_t *d8 = nullptr;
-    uint32_t *d32 = nullptr;
-    CUDA_TRY(dev_alloc(&d8, 3 * n, st));
-    if (dev_alloc(&d32, 3 * n * sizeof(uint32_t), st) != cudaSuccess) {
-        dev_free(d8, st);
-        return fail(CRP_ERR_NOMEM, "cudaMalloc failed");
-    }
+    DevBuf<uint32_t> d32;
+    DevBuf<uint8_t> d8;
+    int rc;
+    if ((rc = d8.alloc(3 * n, st, "the extras")) || (rc = d32.alloc(3 * n, st, "the extras"))) return rc;
     ExtrasArgs a;
-    a.records = g->records;
-    a.pos = res->pos[s] + first;
+    a.records = g->records.get();
+    a.pos = res->pos[s].get() + first;
     a.n = n;
     a.first_tile = sg.first_tile;
     a.seg_begin = (uint32_t)sg.begin;
     a.L = (uint32_t)sg.token_len;
     a.flank = flank;
     a.minus = s;
-    a.gc = d8;
-    a.flags = d8 + n;
-    a.run = d8 + 2 * n;
-    a.cut = d32;
-    a.flank_lo = d32 + n;
-    a.flank_hi = d32 + 2 * n;
+    a.gc = d8.get();
+    a.flags = d8.get() + n;
+    a.run = d8.get() + 2 * n;
+    a.cut = d32.get();
+    a.flank_lo = d32.get() + n;
+    a.flank_hi = d32.get() + 2 * n;
     k_extras<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a);
     g_ctx.launches++;
-    int rc = 0;
     auto back = [&](void *dst, const void *src, size_t bytes) {
         if (dst && !rc && cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st) != cudaSuccess)
             rc = fail(CRP_ERR_CUDA, "D2H of extras failed");
@@ -1693,8 +1705,6 @@ int crp_result_extras(const crp_result *res, uint32_t segment, char strand, uint
     back(flank_hi, a.flank_hi, n * 4);
     if (!rc && cudaStreamSynchronize(st) != cudaSuccess)
         rc = fail(CRP_ERR_CUDA, "extras kernel failed: %s", cudaGetErrorString(cudaGetLastError()));
-    dev_free(d8, st);
-    dev_free(d32, st);
     return rc;
 }
 
@@ -1713,53 +1723,47 @@ int crp_result_extras_strand(const crp_result *res, char strand, uint32_t flank,
     const crp_genome *g = res->g;
     const std::vector<uint64_t> &cnt = s == 0 ? res->seg_plus : res->seg_minus;
     cudaStream_t st = res->st;
-    uint8_t *d8 = nullptr;
-    uint32_t *d32 = nullptr;
-    CUDA_TRY(dev_alloc(&d8, 3 * n, st));
-    if (dev_alloc(&d32, 3 * n * sizeof(uint32_t), st) != cudaSuccess) {
-        dev_free(d8, st);
-        return fail(CRP_ERR_NOMEM, "cudaMalloc failed");
-    }
+    DevBuf<uint32_t> d32;
+    DevBuf<uint8_t> d8;
+    int rc;
+    if ((rc = d8.alloc(3 * n, st, "the extras")) || (rc = d32.alloc(3 * n, st, "the extras"))) return rc;
     uint64_t first = 0;
     for (size_t sgi = 0; sgi < cnt.size(); ++sgi) {
         const uint64_t m = cnt[sgi];
         if (m) {
             const Segment &sg = g->segs[sgi];
             ExtrasArgs a;
-            a.records = g->records;
-            a.pos = res->pos[s] + first;
+            a.records = g->records.get();
+            a.pos = res->pos[s].get() + first;
             a.n = m;
             a.first_tile = sg.first_tile;
             a.seg_begin = (uint32_t)sg.begin;
             a.L = (uint32_t)sg.token_len;
             a.flank = flank;
             a.minus = s;
-            a.gc = d8 + first;
-            a.flags = d8 + n + first;
-            a.run = d8 + 2 * n + first;
-            a.cut = d32 + first;
-            a.flank_lo = d32 + n + first;
-            a.flank_hi = d32 + 2 * n + first;
+            a.gc = d8.get() + first;
+            a.flags = d8.get() + n + first;
+            a.run = d8.get() + 2 * n + first;
+            a.cut = d32.get() + first;
+            a.flank_lo = d32.get() + n + first;
+            a.flank_hi = d32.get() + 2 * n + first;
             k_extras<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(a);
             g_ctx.launches++;
         }
         first += m;
     }
-    int rc = 0;
     auto back = [&](void *dst, const void *src, size_t bytes) {
         if (dst && !rc && cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st) != cudaSuccess)
             rc = fail(CRP_ERR_CUDA, "D2H of extras failed");
     };
-    back(gc, d8, n);
-    back(flags, d8 + n, n);
-    back(run, d8 + 2 * n, n);
-    back(cut, d32, n * 4);
-    back(flank_lo, d32 + n, n * 4);
-    back(flank_hi, d32 + 2 * n, n * 4);
+    back(gc, d8.get(), n);
+    back(flags, d8.get() + n, n);
+    back(run, d8.get() + 2 * n, n);
+    back(cut, d32.get(), n * 4);
+    back(flank_lo, d32.get() + n, n * 4);
+    back(flank_hi, d32.get() + 2 * n, n * 4);
     if (!rc && cudaStreamSynchronize(st) != cudaSuccess)
         rc = fail(CRP_ERR_CUDA, "extras kernels failed: %s", cudaGetErrorString(cudaGetLastError()));
-    dev_free(d8, st);
-    dev_free(d32, st);
     return rc;
 }
 
@@ -1791,34 +1795,29 @@ int crp_result_annotate_strand(const crp_result *res, char strand, const uint64_
         }
     }
     cudaStream_t st = res->st;
-    uint32_t *d_iv = nullptr;
-    int32_t *d_f = nullptr;
-    CUDA_TRY(dev_alloc(&d_iv, host.size() * sizeof(uint32_t), st));
-    if (dev_alloc(&d_f, n * sizeof(int32_t), st) != cudaSuccess) {
-        dev_free(d_iv, st);
-        return fail(CRP_ERR_NOMEM, "cudaMalloc failed");
-    }
-    int rc = 0;
-    if (cudaMemcpyAsync(d_iv, host.data(), host.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
-        rc = fail(CRP_ERR_CUDA, "H2D of intervals failed");
+    DevBuf<int32_t> d_f;
+    DevBuf<uint32_t> d_iv;
+    int rc;
+    if ((rc = d_iv.alloc(host.size(), st, "the intervals")) || (rc = d_f.alloc(n, st, "the features"))) return rc;
+    if (cudaMemcpyAsync(d_iv.get(), host.data(), host.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "H2D of intervals failed");
+    const uint32_t *iv = d_iv.get();
     uint64_t first = 0;
-    for (size_t sgi = 0; sgi < cnt.size() && !rc; ++sgi) {
+    for (size_t sgi = 0; sgi < cnt.size(); ++sgi) {
         const uint64_t m = cnt[sgi];
         if (m) {
             const uint64_t o = iv_offset[sgi];
-            k_annotate<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(res->pos[s] + first, m, s, d_iv + o, d_iv + n_iv + o,
-                                                                   d_iv + 2 * (size_t)n_iv + o,
-                                                                   (uint32_t)(iv_offset[sgi + 1] - o), d_f + first);
+            k_annotate<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(res->pos[s].get() + first, m, s, iv + o, iv + n_iv + o,
+                                                                   iv + 2 * (size_t)n_iv + o,
+                                                                   (uint32_t)(iv_offset[sgi + 1] - o), d_f.get() + first);
             g_ctx.launches++;
         }
         first += m;
     }
-    if (!rc && (cudaMemcpyAsync(feature, d_f, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-                cudaStreamSynchronize(st) != cudaSuccess))
-        rc = fail(CRP_ERR_CUDA, "annotate failed: %s", cudaGetErrorString(cudaGetLastError()));
-    dev_free(d_iv, st);
-    dev_free(d_f, st);
-    return rc;
+    if (cudaMemcpyAsync(feature, d_f.get(), n * sizeof(int32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "annotate failed: %s", cudaGetErrorString(cudaGetLastError()));
+    return 0;
 }
 
 /* Runs of bytes that are not A C G T a c g t inside one segment (the gaps of an assembly: N, IUPAC codes,
@@ -1838,47 +1837,38 @@ int crp_genome_other_runs(const crp_genome *g, uint32_t segment, uint32_t min_le
     uint32_t cap = 1u << 16;
     std::vector<uint32_t> hs, he;
     for (int attempt = 0; attempt < 2; ++attempt) {
-        uint32_t *d = nullptr;
-        unsigned int *d_n = nullptr;
-        CUDA_TRY(dev_alloc(&d, 2 * (size_t)cap * sizeof(uint32_t), st));
-        if (dev_alloc(&d_n, 2 * sizeof(unsigned int), st) != cudaSuccess) {
-            dev_free(d, st);
-            return fail(CRP_ERR_NOMEM, "cudaMalloc failed");
-        }
+        DevBuf<unsigned int> d_n;
+        DevBuf<uint32_t> d;
+        int rc;
+        if ((rc = d.alloc(2 * (size_t)cap, st, "the run boundaries")) || (rc = d_n.alloc(2, st, "the run counts"))) return rc;
         RunArgs a;
-        a.records = g->records;
+        a.records = g->records.get();
         a.first_tile = sg.first_tile;
         a.n_tiles = sg.n_tiles;
         a.seg_begin = (uint32_t)sg.begin;
         a.seg_end = (uint32_t)sg.end;
-        a.starts = d;
-        a.ends = d + cap;
-        a.n_starts = d_n;
-        a.n_ends = d_n + 1;
+        a.starts = d.get();
+        a.ends = d.get() + cap;
+        a.n_starts = d_n.get();
+        a.n_ends = d_n.get() + 1;
         a.capacity = cap;
         unsigned int n[2] = {0, 0};
-        int rc = 0;
         const uint64_t items = (uint64_t)sg.n_tiles * kTileWords;
-        if (cudaMemsetAsync(d_n, 0, 2 * sizeof(unsigned int), st) != cudaSuccess) rc = fail(CRP_ERR_CUDA, "memset failed");
-        if (!rc) {
-            k_other_runs<<<(unsigned)((items + 255) / 256), 256, 0, st>>>(a);
-            g_ctx.launches++;
-            if (cudaMemcpyAsync(n, d_n, sizeof n, cudaMemcpyDeviceToHost, st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess)
-                rc = fail(CRP_ERR_CUDA, "run kernel failed: %s", cudaGetErrorString(cudaGetLastError()));
-        }
-        if (!rc && n[0] != n[1]) rc = fail(CRP_ERR_STATE, "run boundaries do not pair up (%u starts, %u ends)", n[0], n[1]);
-        if (!rc && n[0] <= cap) {
+        if (cudaMemsetAsync(d_n.get(), 0, 2 * sizeof(unsigned int), st) != cudaSuccess) return fail(CRP_ERR_CUDA, "memset failed");
+        k_other_runs<<<(unsigned)((items + 255) / 256), 256, 0, st>>>(a);
+        g_ctx.launches++;
+        if (cudaMemcpyAsync(n, d_n.get(), sizeof n, cudaMemcpyDeviceToHost, st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess)
+            return fail(CRP_ERR_CUDA, "run kernel failed: %s", cudaGetErrorString(cudaGetLastError()));
+        if (n[0] != n[1]) return fail(CRP_ERR_STATE, "run boundaries do not pair up (%u starts, %u ends)", n[0], n[1]);
+        if (n[0] <= cap) {
             hs.resize(n[0]);
             he.resize(n[0]);
             if (n[0] && (cudaMemcpyAsync(hs.data(), a.starts, n[0] * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
                          cudaMemcpyAsync(he.data(), a.ends, n[0] * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
                          cudaStreamSynchronize(st) != cudaSuccess))
-                rc = fail(CRP_ERR_CUDA, "D2H of run boundaries failed");
+                return fail(CRP_ERR_CUDA, "D2H of run boundaries failed");
+            break;
         }
-        dev_free(d, st);
-        dev_free(d_n, st);
-        if (rc) return rc;
-        if (n[0] <= cap) break;
         if (attempt == 1) return fail(CRP_ERR_RANGE, "more than %u runs in one segment", cap);
         cap = n[0];
     }
@@ -1928,59 +1918,47 @@ int crp_primer_windows(const crp_genome *g, uint64_t n, const uint32_t *segment,
         h[3 * n + i] = hi[i];
     }
     cudaStream_t st = stream_of(g);
-    uint32_t *d_in = nullptr, *d_cnt = nullptr;
-    unsigned long long *d_pairs = nullptr;
-    uint16_t *d_first = nullptr;
-    uint8_t *d_status = nullptr;
-    PrimerClasses *d_cls = nullptr;
-    int rc = 0;
-    if (dev_alloc(&d_in, 4 * n * sizeof(uint32_t), st) || dev_alloc(&d_cnt, 2 * n * sizeof(uint32_t), st) ||
-        dev_alloc(&d_pairs, n * sizeof(unsigned long long), st) || dev_alloc(&d_first, 4 * n * sizeof(uint16_t), st) ||
-        dev_alloc(&d_status, n, st) || dev_alloc(&d_cls, sizeof(PrimerClasses), st)) {
-        cudaGetLastError();
-        rc = fail(CRP_ERR_NOMEM, "cudaMalloc of primer buffers failed");
-    }
-    if (!rc) {
-        PrimerArgs a;
-        a.records = g->records;
-        a.cls = d_cls;
-        a.first_tile = d_in;
-        a.seg_begin = d_in + n;
-        a.lo = d_in + 2 * n;
-        a.hi = d_in + 3 * n;
-        a.n = n;
-        a.e = prm->e;
-        a.n_fwd = d_cnt;
-        a.n_rev = d_cnt + n;
-        a.n_pairs = d_pairs;
-        a.first = d_first;
-        a.status = d_status;
-        const uint64_t want = (n + 7) / 8, cap = (uint64_t)g_ctx.sm_count * 8;
-        if (cudaMemcpyAsync(d_in, h.data(), 4 * n * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-            cudaMemcpyAsync(d_cls, &pc, sizeof pc, cudaMemcpyHostToDevice, st) != cudaSuccess)
-            rc = fail(CRP_ERR_CUDA, "H2D of primer windows failed");
-        if (!rc) {
-            k_primers<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(a);
-            g_ctx.launches++;
-            auto back = [&](void *dst, const void *src, size_t bytes) {
-                if (dst && !rc && cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st) != cudaSuccess)
-                    rc = fail(CRP_ERR_CUDA, "D2H of primer results failed");
-            };
-            back(n_fwd, a.n_fwd, n * 4);
-            back(n_rev, a.n_rev, n * 4);
-            back(n_pairs, a.n_pairs, n * 8);
-            back(first, a.first, n * 8);
-            back(status, a.status, n);
-            if (!rc && cudaStreamSynchronize(st) != cudaSuccess)
-                rc = fail(CRP_ERR_CUDA, "primer kernel failed: %s", cudaGetErrorString(cudaGetLastError()));
-        }
-    }
-    dev_free(d_in, st);
-    dev_free(d_cnt, st);
-    dev_free(d_pairs, st);
-    dev_free(d_first, st);
-    dev_free(d_status, st);
-    dev_free(d_cls, st);
+    DevBuf<PrimerClasses> d_cls;
+    DevBuf<uint8_t> d_status;
+    DevBuf<uint16_t> d_first;
+    DevBuf<unsigned long long> d_pairs;
+    DevBuf<uint32_t> d_cnt, d_in;
+    int rc;
+    if ((rc = d_in.alloc(4 * n, st, "the primer windows")) || (rc = d_cnt.alloc(2 * n, st, "the primer counts")) ||
+        (rc = d_pairs.alloc(n, st, "the primer pairs")) || (rc = d_first.alloc(4 * n, st, "the first primers")) ||
+        (rc = d_status.alloc(n, st, "the primer status")) || (rc = d_cls.alloc(1, st, "the primer classes")))
+        return rc;
+    PrimerArgs a;
+    a.records = g->records.get();
+    a.cls = d_cls.get();
+    a.first_tile = d_in.get();
+    a.seg_begin = d_in.get() + n;
+    a.lo = d_in.get() + 2 * n;
+    a.hi = d_in.get() + 3 * n;
+    a.n = n;
+    a.e = prm->e;
+    a.n_fwd = d_cnt.get();
+    a.n_rev = d_cnt.get() + n;
+    a.n_pairs = d_pairs.get();
+    a.first = d_first.get();
+    a.status = d_status.get();
+    const uint64_t want = (n + 7) / 8, cap = (uint64_t)g_ctx.sm_count * 8;
+    if (cudaMemcpyAsync(d_in.get(), h.data(), 4 * n * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemcpyAsync(d_cls.get(), &pc, sizeof pc, cudaMemcpyHostToDevice, st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "H2D of primer windows failed");
+    k_primers<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(a);
+    g_ctx.launches++;
+    auto back = [&](void *dst, const void *src, size_t bytes) {
+        if (dst && !rc && cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st) != cudaSuccess)
+            rc = fail(CRP_ERR_CUDA, "D2H of primer results failed");
+    };
+    back(n_fwd, a.n_fwd, n * 4);
+    back(n_rev, a.n_rev, n * 4);
+    back(n_pairs, a.n_pairs, n * 8);
+    back(first, a.first, n * 8);
+    back(status, a.status, n);
+    if (!rc && cudaStreamSynchronize(st) != cudaSuccess)
+        rc = fail(CRP_ERR_CUDA, "primer kernel failed: %s", cudaGetErrorString(cudaGetLastError()));
     return rc;
 }
 
@@ -2003,28 +1981,21 @@ int crp_result_annotate(const crp_result *res, uint32_t segment, char strand, ui
         host[2 * (size_t)n_intervals + j] = running;
     }
     cudaStream_t st = res->st;
-    uint32_t *d_iv = nullptr;
-    int32_t *d_f = nullptr;
-    CUDA_TRY(dev_alloc(&d_iv, host.size() * sizeof(uint32_t), st));
-    if (dev_alloc(&d_f, n * sizeof(int32_t), st) != cudaSuccess) {
-        dev_free(d_iv, st);
-        return fail(CRP_ERR_NOMEM, "cudaMalloc failed");
-    }
-    int rc = 0;
+    DevBuf<int32_t> d_f;
+    DevBuf<uint32_t> d_iv;
+    int rc;
+    if ((rc = d_iv.alloc(host.size(), st, "the intervals")) || (rc = d_f.alloc(n, st, "the features"))) return rc;
     const int s = strand == '+' ? 0 : 1;
-    if (cudaMemcpyAsync(d_iv, host.data(), host.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
-        rc = fail(CRP_ERR_CUDA, "H2D of intervals failed");
-    if (!rc) {
-        k_annotate<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(res->pos[s] + first, n, s, d_iv, d_iv + n_intervals,
-                                                               d_iv + 2 * (size_t)n_intervals, n_intervals, d_f);
-        g_ctx.launches++;
-        if (cudaMemcpyAsync(feature, d_f, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-            cudaStreamSynchronize(st) != cudaSuccess)
-            rc = fail(CRP_ERR_CUDA, "annotate failed: %s", cudaGetErrorString(cudaGetLastError()));
-    }
-    dev_free(d_iv, st);
-    dev_free(d_f, st);
-    return rc;
+    if (cudaMemcpyAsync(d_iv.get(), host.data(), host.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "H2D of intervals failed");
+    const uint32_t *iv = d_iv.get();
+    k_annotate<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(res->pos[s].get() + first, n, s, iv, iv + n_intervals,
+                                                           iv + 2 * (size_t)n_intervals, n_intervals, d_f.get());
+    g_ctx.launches++;
+    if (cudaMemcpyAsync(feature, d_f.get(), n * sizeof(int32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "annotate failed: %s", cudaGetErrorString(cudaGetLastError()));
+    return 0;
 }
 
 int crp_rescore(const crp_genome *g, uint64_t n, const uint32_t *segment, const uint32_t *t, const char *strand,
@@ -2049,30 +2020,18 @@ int crp_rescore(const crp_genome *g, uint64_t n, const uint32_t *segment, const 
         items[i].cls = cls[i];
     }
     cudaStream_t st = stream_of(g);
-    RescoreItem *d_items = nullptr;
-    double *d_x = nullptr;
-    CUDA_TRY(dev_alloc(&d_items, n * sizeof(RescoreItem), st));
-    if (dev_alloc(&d_x, n * sizeof(double), st) != cudaSuccess) {
-        dev_free(d_items, st);
-        return fail(CRP_ERR_NOMEM, "cudaMalloc failed");
-    }
-    int rc = 0;
-    do {
-        if (cudaMemcpyAsync(d_items, items.data(), n * sizeof(RescoreItem), cudaMemcpyHostToDevice, st) != cudaSuccess) {
-            rc = fail(CRP_ERR_CUDA, "H2D of rescore items failed");
-            break;
-        }
-        k_rescore<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(g->records, d_items, n, d_x);
-        g_ctx.launches++;
-        if (cudaMemcpyAsync(x_out, d_x, n * sizeof(double), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-            cudaStreamSynchronize(st) != cudaSuccess) {
-            rc = fail(CRP_ERR_CUDA, "rescore failed: %s", cudaGetErrorString(cudaGetLastError()));
-            break;
-        }
-    } while (0);
-    dev_free(d_items, st);
-    dev_free(d_x, st);
-    return rc;
+    DevBuf<double> d_x;
+    DevBuf<RescoreItem> d_items;
+    int rc;
+    if ((rc = d_items.alloc(n, st, "the rescore items")) || (rc = d_x.alloc(n, st, "the rescores"))) return rc;
+    if (cudaMemcpyAsync(d_items.get(), items.data(), n * sizeof(RescoreItem), cudaMemcpyHostToDevice, st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "H2D of rescore items failed");
+    k_rescore<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(g->records.get(), d_items.get(), n, d_x.get());
+    g_ctx.launches++;
+    if (cudaMemcpyAsync(x_out, d_x.get(), n * sizeof(double), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "rescore failed: %s", cudaGetErrorString(cudaGetLastError()));
+    return 0;
 }
 
 }  // extern "C"
@@ -2100,8 +2059,8 @@ struct crp_offtarget {
     cudaStream_t st = nullptr;                 // own stream, ordered behind each genome's stream by an event
     cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};   // sites start / end, count start / end, genome ready
     std::vector<const crp_genome *> genomes;
-    unsigned long long *keys = nullptr;        // site keys of every genome added, any order
-    unsigned long long *loci = nullptr;        // crp_offtarget_new_with_loci: the locus of every site, at its key's slot
+    DevBuf<unsigned long long> keys;           // site keys of every genome added, any order
+    DevBuf<unsigned long long> loci;           // crp_offtarget_new_with_loci: the locus of every site, at its key's slot
     bool with_loci = false;
     uint32_t s2 = 8, s3 = 8;                   // code sets of PAM letters 2 and 3 (ot_pam_plus_sets): {G}, {G} is NGG
     bool own_site = true;                      // a candidate's own site is a site of the index: G in s2 and in s3
@@ -2118,78 +2077,66 @@ static int ot_join(crp_offtarget *ix, const unsigned long long *d_keys, uint64_t
     using Site = typename Op::Site;
     cudaStream_t st = ix->st;
     const size_t tbl = kOtBuckets + 1;
-    uint32_t *d_tbl = nullptr;
-    Site *d_sites = nullptr;
-    uint2 *d_q = nullptr;
-    unsigned long long *d_misc = nullptr;      // [0] comparisons, [1] overflow flag
-    if (dev_alloc(&d_tbl, 7 * tbl * sizeof(uint32_t), st) != cudaSuccess ||
-        dev_alloc(&d_sites, (ix->n_sites + kOtSitePad) * sizeof(Site), st) != cudaSuccess ||
-        dev_alloc(&d_q, (n + 1) * sizeof(uint2), st) != cudaSuccess ||
-        dev_alloc(&d_misc, 2 * sizeof(unsigned long long), st) != cudaSuccess) {
-        cudaGetLastError();
-        dev_free(d_tbl, st);
-        dev_free(d_sites, st);
-        dev_free(d_q, st);
-        return fail(CRP_ERR_NOMEM, "cudaMalloc of the off-target work buffers failed");
-    }
-    uint32_t *hist_s = d_tbl, *hist_q = d_tbl + tbl;
+    DevBuf<unsigned long long> d_misc;         // [0] comparisons, [1] overflow flag
+    DevBuf<uint2> d_q;
+    DevBuf<Site> d_sites;
+    DevBuf<uint32_t> d_tbl;
+    int rc;
+    if ((rc = d_tbl.alloc(7 * tbl, st, "the off-target tables")) ||
+        (rc = d_sites.alloc(ix->n_sites + kOtSitePad, st, "the off-target sites")) ||
+        (rc = d_q.alloc(n + 1, st, "the off-target queries")) || (rc = d_misc.alloc(2, st, "the off-target counters")))
+        return rc;
+    uint32_t *hist_s = d_tbl.get(), *hist_q = d_tbl.get() + tbl;
     OtScanArgs sa;
     sa.hist[0] = hist_s;
     sa.hist[1] = hist_q;
-    sa.off[0] = d_tbl + 2 * tbl;
-    sa.off[1] = d_tbl + 3 * tbl;
-    sa.cursor[0] = d_tbl + 4 * tbl;
-    sa.cursor[1] = d_tbl + 5 * tbl;
-    sa.item_off = d_tbl + 6 * tbl;
-    sa.comparisons = d_misc;
-    sa.overflow = reinterpret_cast<unsigned int *>(d_misc + 1);
+    sa.off[0] = d_tbl.get() + 2 * tbl;
+    sa.off[1] = d_tbl.get() + 3 * tbl;
+    sa.cursor[0] = d_tbl.get() + 4 * tbl;
+    sa.cursor[1] = d_tbl.get() + 5 * tbl;
+    sa.item_off = d_tbl.get() + 6 * tbl;
+    sa.comparisons = d_misc.get();
+    sa.overflow = reinterpret_cast<unsigned int *>(d_misc.get() + 1);
     OtJoin ja;
-    ja.sites = d_sites;
-    ja.queries = d_q;
+    ja.sites = d_sites.get();
+    ja.queries = d_q.get();
     ja.soff = sa.off[0];
     ja.qoff = sa.off[1];
     ja.item_off = sa.item_off;
     ja.k = k;
     auto grid = [](uint64_t items) { return (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((items + 255) / 256, (uint64_t)g_ctx.sm_count * 16)); };
-    int rc = 0;
     unsigned long long misc[2] = {0, 0};
-    if (cudaMemsetAsync(d_misc, 0, 2 * sizeof(unsigned long long), st) != cudaSuccess ||
+    if (cudaMemsetAsync(d_misc.get(), 0, 2 * sizeof(unsigned long long), st) != cudaSuccess ||
         cudaEventRecord(ix->ev[2], st) != cudaSuccess)
-        rc = fail(CRP_ERR_CUDA, "off-target setup failed");
-    for (int p = 0; p < kOtPairs && !rc && n && ix->n_sites; ++p) {
+        return fail(CRP_ERR_CUDA, "off-target setup failed");
+    const unsigned long long *keys = ix->keys.get();
+    for (int p = 0; p < kOtPairs && n && ix->n_sites; ++p) {
         int i = 0, j = 0;
         ot_pair(p, i, j);
         ja.jm1 = (uint32_t)(j - 1);
         ja.pi = i;
         ja.pj = j;
-        if (cudaMemsetAsync(d_tbl, 0, 2 * tbl * sizeof(uint32_t), st) != cudaSuccess) {
-            rc = fail(CRP_ERR_CUDA, "memset failed");
-            break;
-        }
-        k_ot_hist<<<grid(ix->n_sites), 256, 0, st>>>(ix->keys, ix->n_sites, i, j, hist_s);
+        if (cudaMemsetAsync(d_tbl.get(), 0, 2 * tbl * sizeof(uint32_t), st) != cudaSuccess)
+            return fail(CRP_ERR_CUDA, "memset failed");
+        k_ot_hist<<<grid(ix->n_sites), 256, 0, st>>>(keys, ix->n_sites, i, j, hist_s);
         k_ot_hist<<<grid(n), 256, 0, st>>>(d_keys, n, i, j, hist_q);
         k_ot_scan<<<3, kOtScanThreads, 0, st>>>(sa);
         if constexpr (std::is_same_v<Site, uint2>)   // {rest key, site index}: the query form of the scatter
-            k_ot_scatter<<<grid(ix->n_sites), 256, 0, st>>>(ix->keys, ix->n_sites, i, j, sa.cursor[0], nullptr, d_sites);
+            k_ot_scatter<<<grid(ix->n_sites), 256, 0, st>>>(keys, ix->n_sites, i, j, sa.cursor[0], nullptr, d_sites.get());
         else
-            k_ot_scatter<<<grid(ix->n_sites), 256, 0, st>>>(ix->keys, ix->n_sites, i, j, sa.cursor[0], d_sites, nullptr);
-        k_ot_scatter<<<grid(n), 256, 0, st>>>(d_keys, n, i, j, sa.cursor[1], nullptr, d_q);
+            k_ot_scatter<<<grid(ix->n_sites), 256, 0, st>>>(keys, ix->n_sites, i, j, sa.cursor[0], d_sites.get(), nullptr);
+        k_ot_scatter<<<grid(n), 256, 0, st>>>(d_keys, n, i, j, sa.cursor[1], nullptr, d_q.get());
         k_ot_join<Op><<<(unsigned)g_ctx.sm_count * 8, kOtThreads, 0, st>>>(ja, op);
         g_ctx.launches += 6;
-        if (cudaGetLastError() != cudaSuccess) rc = fail(CRP_ERR_CUDA, "off-target launch failed");
+        if (cudaGetLastError() != cudaSuccess) return fail(CRP_ERR_CUDA, "off-target launch failed");
     }
-    if (!rc && (cudaEventRecord(ix->ev[3], st) != cudaSuccess ||
-                cudaMemcpyAsync(misc, d_misc, sizeof misc, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-                cudaStreamSynchronize(st) != cudaSuccess ||
-                cudaEventElapsedTime(&ix->ms_count, ix->ev[2], ix->ev[3]) != cudaSuccess))
-        rc = fail(CRP_ERR_CUDA, "off-target join failed: %s", cudaGetErrorString(cudaGetLastError()));
-    if (!rc && misc[1]) rc = fail(CRP_ERR_RANGE, "a part pair needs 2^32 work items or more");
-    if (!rc) ix->comparisons = misc[0];
-    dev_free(d_tbl, st);
-    dev_free(d_sites, st);
-    dev_free(d_q, st);
-    dev_free(d_misc, st);
-    return rc;
+    if (cudaEventRecord(ix->ev[3], st) != cudaSuccess ||
+        cudaMemcpyAsync(misc, d_misc.get(), sizeof misc, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess || cudaEventElapsedTime(&ix->ms_count, ix->ev[2], ix->ev[3]) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "off-target join failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (misc[1]) return fail(CRP_ERR_RANGE, "a part pair needs 2^32 work items or more");
+    ix->comparisons = misc[0];
+    return 0;
 }
 
 // The checks of a *_candidates call, in this order: CRP_ERR_ARG for a NULL index or result, a strand other than '+' /
@@ -2208,35 +2155,32 @@ static int ot_check_candidates(const crp_offtarget *ix, const crp_result *res, c
     return 0;
 }
 
-// The query keys of strand stream s of a checked result into *d_keys [n] (k_ot_queries), on ix->st behind the scan's
-// stream.  d_counts [n][k1], when not NULL, gets every row's primed counts.  *d_seg keeps the segment table
-// (ot_segment_table) for k_ot_gather.  The caller frees *d_keys and *d_seg, also after a failure.
+// The query keys of strand stream s of a checked result into d_keys [n] (k_ot_queries), on ix->st behind the scan's
+// stream.  d_counts [n][k1], when not NULL, gets every row's primed counts.  d_seg keeps the segment table
+// (ot_segment_table) for k_ot_gather.
 static int ot_candidate_keys(crp_offtarget *ix, const crp_result *res, int s, uint32_t *d_counts, uint32_t k1,
-                             unsigned long long **d_keys, uint32_t **d_seg) {
+                             DevBuf<unsigned long long> &d_keys, DevBuf<uint32_t> &d_seg) {
     const uint64_t n = s == 0 ? res->n_plus : res->n_minus;
     const uint32_t n_seg = (uint32_t)(s == 0 ? res->seg_plus : res->seg_minus).size();
     const std::vector<uint32_t> seg = ot_segment_table(res, s);
     cudaStream_t st = ix->st;
     CUDA_TRY(cudaEventRecord(ix->ev[4], res->st));             // the candidate streams are written on the scan's stream
     CUDA_TRY(cudaStreamWaitEvent(st, ix->ev[4], 0));
-    if (dev_alloc(d_seg, seg.size() * sizeof(uint32_t), st) != cudaSuccess ||
-        dev_alloc(d_keys, n * sizeof(unsigned long long), st) != cudaSuccess) {
-        cudaGetLastError();
-        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu query rows failed", (unsigned long long)n);
-    }
-    if (cudaMemcpyAsync(*d_seg, seg.data(), seg.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
+    int rc;
+    if ((rc = d_seg.alloc(seg.size(), st, "the segment table")) || (rc = d_keys.alloc(n, st, "the query keys"))) return rc;
+    if (cudaMemcpyAsync(d_seg.get(), seg.data(), seg.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
         return fail(CRP_ERR_CUDA, "H2D of the segment table failed");
     OtQueryArgs a;
-    a.records = res->g->records;
-    a.pos = res->pos[s];
+    a.records = res->g->records.get();
+    a.pos = res->pos[s].get();
     a.n = n;
-    a.seg_row = *d_seg;
-    a.seg_tile = *d_seg + n_seg + 1;
-    a.seg_begin = *d_seg + 2 * (size_t)n_seg + 1;
+    a.seg_row = d_seg.get();
+    a.seg_tile = d_seg.get() + n_seg + 1;
+    a.seg_begin = d_seg.get() + 2 * (size_t)n_seg + 1;
     a.n_seg = n_seg;
     a.k1 = k1;
     a.minus = s;
-    a.keys = *d_keys;
+    a.keys = d_keys.get();
     a.counts = d_counts;
     a.own = ix->own_site ? 0xFFFFFFFFu : 0u;
     k_ot_queries<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a);
@@ -2255,13 +2199,10 @@ static int ot_check_keys(uint64_t n, const uint64_t *keys) {
     return 0;
 }
 
-// Checked keys into *d_keys [n] on ix->st; the caller frees *d_keys, also after a failure.
-static int ot_upload_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys, unsigned long long **d_keys) {
-    if (dev_alloc(d_keys, n * sizeof(unsigned long long), ix->st) != cudaSuccess) {
-        cudaGetLastError();
-        return fail(CRP_ERR_NOMEM, "cudaMalloc of %llu keys failed", (unsigned long long)n);
-    }
-    if (cudaMemcpyAsync(*d_keys, keys, n * sizeof(uint64_t), cudaMemcpyHostToDevice, ix->st) != cudaSuccess)
+// Checked keys into d_keys [n] on ix->st.
+static int ot_upload_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys, DevBuf<unsigned long long> &d_keys) {
+    if (int rc = d_keys.alloc(n, ix->st, "the query keys")) return rc;
+    if (cudaMemcpyAsync(d_keys.get(), keys, n * sizeof(uint64_t), cudaMemcpyHostToDevice, ix->st) != cudaSuccess)
         return fail(CRP_ERR_CUDA, "H2D of the keys failed");
     return 0;
 }
@@ -2339,15 +2280,16 @@ int crp_offtarget_add_genome(crp_offtarget *ix, const crp_genome *g) {
     CUDA_TRY(cudaEventRecord(ix->ev[4], stream_of(g)));        // the records are written on the genome's stream
     CUDA_TRY(cudaStreamWaitEvent(st, ix->ev[4], 0));
     const uint64_t items = (uint64_t)g->n_tiles * kTileWords;
-    unsigned long long *d_n = nullptr, *h_n = static_cast<unsigned long long *>(pinned_get(sizeof(unsigned long long)));
-    if (!h_n) return fail(CRP_ERR_NOMEM, "cudaHostAlloc failed");
-    CUDA_TRY(dev_alloc(&d_n, sizeof(unsigned long long), st));
+    PinnedBuf<unsigned long long> h_n;
+    DevBuf<unsigned long long> d_n;
+    if (int rc = h_n.alloc(1, "the site count")) return rc;
+    if (int rc = d_n.alloc(1, st, "the site count")) return rc;
     OtSiteArgs a;
-    a.records = g->records;
+    a.records = g->records.get();
     a.n_tiles = g->n_tiles;
     a.keys = nullptr;
     a.base = ix->n_sites;
-    a.n = d_n;
+    a.n = d_n.get();
     a.loci = nullptr;
     a.genome = (uint32_t)ix->genomes.size();
     a.s2 = ix->s2;
@@ -2361,65 +2303,52 @@ int crp_offtarget_add_genome(crp_offtarget *ix, const crp_genome *g) {
         else k_ot_sites<false, true><<<blocks, 256, 0, st>>>(a);
         g_ctx.launches++;
     };
-    int rc = 0;
-    *h_n = 0;
+    unsigned long long *h = h_n.get();
+    *h = 0;
     // pass 1 counts, pass 2 appends behind the sites already held (the key and locus arrays grow by one copy)
-    if (cudaEventRecord(ix->ev[0], st) != cudaSuccess || cudaMemsetAsync(d_n, 0, sizeof *d_n, st) != cudaSuccess)
-        rc = fail(CRP_ERR_CUDA, "off-target setup failed");
-    if (!rc && items) launch(false);
-    if (!rc && (cudaMemcpyAsync(h_n, d_n, sizeof *d_n, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-                cudaStreamSynchronize(st) != cudaSuccess))
-        rc = fail(CRP_ERR_CUDA, "site count failed: %s", cudaGetErrorString(cudaGetLastError()));
-    const uint64_t add = *h_n, total = ix->n_sites + add;
-    if (!rc && total > 0xFFFFFFFFull) rc = fail(CRP_ERR_RANGE, "%llu sites exceed 2^32 - 1", (unsigned long long)total);
-    if (!rc && add) {
-        unsigned long long *keys = nullptr, *loci = nullptr;
-        if (dev_alloc(&keys, total * sizeof(unsigned long long), st) != cudaSuccess ||
-            (ix->with_loci && dev_alloc(&loci, total * sizeof(unsigned long long), st) != cudaSuccess)) {
-            cudaGetLastError();
-            dev_free(keys, st);
-            rc = fail(CRP_ERR_NOMEM, "cudaMalloc of %llu site keys failed", (unsigned long long)total);
-        } else {
-            if (ix->n_sites && cudaMemcpyAsync(keys, ix->keys, ix->n_sites * sizeof(unsigned long long), cudaMemcpyDeviceToDevice,
-                                               st) != cudaSuccess)
-                rc = fail(CRP_ERR_CUDA, "copy of the site keys failed");
-            if (!rc && loci && ix->n_sites &&
-                cudaMemcpyAsync(loci, ix->loci, ix->n_sites * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, st) != cudaSuccess)
-                rc = fail(CRP_ERR_CUDA, "copy of the site loci failed");
-            dev_free(ix->keys, st);
-            dev_free(ix->loci, st);
-            ix->keys = keys;
-            ix->loci = loci;
-            a.keys = keys;
-            a.loci = loci;
-            if (!rc && cudaMemsetAsync(d_n, 0, sizeof *d_n, st) != cudaSuccess) rc = fail(CRP_ERR_CUDA, "memset failed");
-            if (!rc) launch(loci != nullptr);
-            if (!rc && (cudaMemcpyAsync(h_n, d_n, sizeof *d_n, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-                        cudaEventRecord(ix->ev[1], st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess))
-                rc = fail(CRP_ERR_CUDA, "site keys failed: %s", cudaGetErrorString(cudaGetLastError()));
-            if (!rc && *h_n != add) rc = fail(CRP_ERR_STATE, "site passes disagree (%llu, %llu)", (unsigned long long)add, *h_n);
-            if (rc) {                          // the old keys went with the old array: the index is emptied
-                dev_free(ix->keys, st);
-                dev_free(ix->loci, st);
-                ix->keys = nullptr;
-                ix->loci = nullptr;
-                ix->n_sites = 0;
-                ix->genomes.clear();
-            }
-        }
-    } else if (!rc) {
-        rc = cudaEventRecord(ix->ev[1], st) == cudaSuccess && cudaEventSynchronize(ix->ev[1]) == cudaSuccess
-                 ? 0 : fail(CRP_ERR_CUDA, "event failed");
+    if (cudaEventRecord(ix->ev[0], st) != cudaSuccess || cudaMemsetAsync(a.n, 0, sizeof *h, st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "off-target setup failed");
+    if (items) launch(false);
+    if (cudaMemcpyAsync(h, a.n, sizeof *h, cudaMemcpyDeviceToHost, st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "site count failed: %s", cudaGetErrorString(cudaGetLastError()));
+    const uint64_t add = *h, total = ix->n_sites + add;
+    if (total > 0xFFFFFFFFull) return fail(CRP_ERR_RANGE, "%llu sites exceed 2^32 - 1", (unsigned long long)total);
+    if (add) {
+        DevBuf<unsigned long long> keys, loci;
+        if (int rc = keys.alloc(total, st, "the site keys")) return rc;
+        if (ix->with_loci)
+            if (int rc = loci.alloc(total, st, "the site loci")) return rc;
+        auto lost = [ix](int rc) {                 // the old keys went with the old array: the index is emptied
+            ix->keys.reset();
+            ix->loci.reset();
+            ix->n_sites = 0;
+            ix->genomes.clear();
+            return rc;
+        };
+        if (ix->n_sites && cudaMemcpyAsync(keys.get(), ix->keys.get(), ix->n_sites * sizeof(unsigned long long),
+                                           cudaMemcpyDeviceToDevice, st) != cudaSuccess)
+            return lost(fail(CRP_ERR_CUDA, "copy of the site keys failed"));
+        if (loci.get() && ix->n_sites &&
+            cudaMemcpyAsync(loci.get(), ix->loci.get(), ix->n_sites * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, st) != cudaSuccess)
+            return lost(fail(CRP_ERR_CUDA, "copy of the site loci failed"));
+        ix->keys = std::move(keys);                // the old arrays go back here, behind the copies
+        ix->loci = std::move(loci);
+        a.keys = ix->keys.get();
+        a.loci = ix->loci.get();
+        if (cudaMemsetAsync(a.n, 0, sizeof *h, st) != cudaSuccess) return lost(fail(CRP_ERR_CUDA, "memset failed"));
+        launch(a.loci != nullptr);
+        if (cudaMemcpyAsync(h, a.n, sizeof *h, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+            cudaEventRecord(ix->ev[1], st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess)
+            return lost(fail(CRP_ERR_CUDA, "site keys failed: %s", cudaGetErrorString(cudaGetLastError())));
+        if (*h != add) return lost(fail(CRP_ERR_STATE, "site passes disagree (%llu, %llu)", (unsigned long long)add, *h));
+    } else if (cudaEventRecord(ix->ev[1], st) != cudaSuccess || cudaEventSynchronize(ix->ev[1]) != cudaSuccess) {
+        return fail(CRP_ERR_CUDA, "event failed");
     }
     float ms = 0.f;
-    if (!rc && cudaEventElapsedTime(&ms, ix->ev[0], ix->ev[1]) == cudaSuccess) ix->ms_sites += ms;
-    if (!rc) {
-        ix->n_sites = total;
-        ix->genomes.push_back(g);
-    }
-    dev_free(d_n, st);
-    pinned_put(h_n);
-    return rc;
+    if (cudaEventElapsedTime(&ms, ix->ev[0], ix->ev[1]) == cudaSuccess) ix->ms_sites += ms;
+    ix->n_sites = total;
+    ix->genomes.push_back(g);
+    return 0;
 }
 
 int crp_offtarget_num_sites(const crp_offtarget *ix, uint64_t *n) {
@@ -2435,7 +2364,7 @@ int crp_offtarget_fetch_sites(const crp_offtarget *ix, uint64_t capacity, uint64
                                             (unsigned long long)capacity);
     if (!ix->n_sites) return 0;
     if (!keys) return fail(CRP_ERR_ARG, "keys is NULL");
-    CUDA_TRY(cudaMemcpyAsync(keys, ix->keys, ix->n_sites * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->st));
+    CUDA_TRY(cudaMemcpyAsync(keys, ix->keys.get(), ix->n_sites * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->st));
     CUDA_TRY(cudaStreamSynchronize(ix->st));
     return 0;
 }
@@ -2446,21 +2375,13 @@ int crp_offtarget_count_candidates(crp_offtarget *ix, const crp_result *res, cha
     const uint64_t n = s == 0 ? res->n_plus : res->n_minus;
     if (n == 0) return 0;
     if (!counts) return fail(CRP_ERR_ARG, "counts is NULL");
-    cudaStream_t st = ix->st;
     const uint32_t k1 = max_mm + 1;
-    uint32_t *d_seg = nullptr, *d_counts = nullptr;
-    unsigned long long *d_keys = nullptr;
-    int rc = 0;
-    if (dev_alloc(&d_counts, n * k1 * sizeof(uint32_t), st) != cudaSuccess) {
-        cudaGetLastError();
-        rc = fail(CRP_ERR_NOMEM, "cudaMalloc of %llu query rows failed", (unsigned long long)n);
-    }
-    if (!rc) rc = ot_candidate_keys(ix, res, s, d_counts, k1, &d_keys, &d_seg);
-    if (!rc) rc = ot_count(ix, d_keys, n, max_mm, d_counts, counts);
-    dev_free(d_seg, st);
-    dev_free(d_keys, st);
-    dev_free(d_counts, st);
-    return rc;
+    DevBuf<uint32_t> d_counts;
+    DevBuf<unsigned long long> d_keys;
+    DevBuf<uint32_t> d_seg;
+    if (int rc = d_counts.alloc(n * k1, ix->st, "the off-target counts")) return rc;
+    if (int rc = ot_candidate_keys(ix, res, s, d_counts.get(), k1, d_keys, d_seg)) return rc;
+    return ot_count(ix, d_keys.get(), n, max_mm, d_counts.get(), counts);
 }
 
 int crp_offtarget_count_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys, uint32_t max_mm, uint32_t *counts) {
@@ -2472,19 +2393,12 @@ int crp_offtarget_count_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys
     if (int rc = ot_check_keys(n, keys)) return rc;
     cudaStream_t st = ix->st;
     const uint32_t k1 = max_mm + 1;
-    unsigned long long *d_keys = nullptr;
-    uint32_t *d_counts = nullptr;
-    int rc = ot_upload_keys(ix, n, keys, &d_keys);
-    if (!rc && dev_alloc(&d_counts, n * k1 * sizeof(uint32_t), st) != cudaSuccess) {
-        cudaGetLastError();
-        rc = fail(CRP_ERR_NOMEM, "cudaMalloc of %llu keys failed", (unsigned long long)n);
-    }
-    if (!rc && cudaMemsetAsync(d_counts, 0, n * k1 * sizeof(uint32_t), st) != cudaSuccess)
-        rc = fail(CRP_ERR_CUDA, "memset failed");
-    if (!rc) rc = ot_count(ix, d_keys, n, max_mm, d_counts, counts);
-    dev_free(d_keys, st);
-    dev_free(d_counts, st);
-    return rc;
+    DevBuf<uint32_t> d_counts;
+    DevBuf<unsigned long long> d_keys;
+    if (int rc = ot_upload_keys(ix, n, keys, d_keys)) return rc;
+    if (int rc = d_counts.alloc(n * k1, st, "the off-target counts")) return rc;
+    if (cudaMemsetAsync(d_counts.get(), 0, n * k1 * sizeof(uint32_t), st) != cudaSuccess) return fail(CRP_ERR_CUDA, "memset failed");
+    return ot_count(ix, d_keys.get(), n, max_mm, d_counts.get(), counts);
 }
 
 int crp_offtarget_fetch_loci(const crp_offtarget *ix, uint64_t capacity, uint64_t *loci, uint64_t *n) {
@@ -2495,7 +2409,7 @@ int crp_offtarget_fetch_loci(const crp_offtarget *ix, uint64_t capacity, uint64_
                                             (unsigned long long)capacity);
     if (!ix->n_sites) return 0;
     if (!loci) return fail(CRP_ERR_ARG, "loci is NULL");
-    CUDA_TRY(cudaMemcpyAsync(loci, ix->loci, ix->n_sites * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->st));
+    CUDA_TRY(cudaMemcpyAsync(loci, ix->loci.get(), ix->n_sites * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->st));
     CUDA_TRY(cudaStreamSynchronize(ix->st));
     return 0;
 }
@@ -2509,44 +2423,34 @@ static int ot_list(crp_offtarget *ix, const unsigned long long *d_keys, const un
                    uint32_t k, const uint64_t *first, uint32_t *sites) {
     cudaStream_t st = ix->st;
     const uint64_t total = first[n];
-    unsigned long long *d_first = nullptr;
-    uint32_t *d_cursor = nullptr, *d_out = nullptr;
-    unsigned int *d_flag = nullptr;
-    if (dev_alloc(&d_first, (n + 1) * sizeof(unsigned long long), st) != cudaSuccess ||
-        dev_alloc(&d_cursor, n * sizeof(uint32_t), st) != cudaSuccess ||
-        dev_alloc(&d_out, std::max<uint64_t>(total, 1) * sizeof(uint32_t), st) != cudaSuccess ||
-        dev_alloc(&d_flag, sizeof(unsigned int), st) != cudaSuccess) {
-        cudaGetLastError();
-        dev_free(d_first, st);
-        dev_free(d_cursor, st);
-        dev_free(d_out, st);
-        return fail(CRP_ERR_NOMEM, "cudaMalloc of a listing of %llu sites failed", (unsigned long long)total);
-    }
-    int rc = 0;
-    if (cudaMemcpyAsync(d_first, first, (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemsetAsync(d_cursor, 0, n * sizeof(uint32_t), st) != cudaSuccess ||
-        cudaMemsetAsync(d_flag, 0, sizeof(unsigned int), st) != cudaSuccess)
-        rc = fail(CRP_ERR_CUDA, "listing setup failed");
-    if (!rc) rc = ot_join(ix, d_keys, n, k, OtList{ix->loci, d_own, d_first, d_cursor, d_out, d_flag});
-    std::vector<uint32_t> found(rc ? 0 : n);
+    DevBuf<unsigned int> d_flag;
+    DevBuf<uint32_t> d_out, d_cursor;
+    DevBuf<unsigned long long> d_first;
+    int rc;
+    if ((rc = d_first.alloc(n + 1, st, "the listing slices")) || (rc = d_cursor.alloc(n, st, "the listing cursors")) ||
+        (rc = d_out.alloc(std::max<uint64_t>(total, 1), st, "the listing")) || (rc = d_flag.alloc(1, st, "the listing flag")))
+        return rc;
+    if (cudaMemcpyAsync(d_first.get(), first, (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemsetAsync(d_cursor.get(), 0, n * sizeof(uint32_t), st) != cudaSuccess ||
+        cudaMemsetAsync(d_flag.get(), 0, sizeof(unsigned int), st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "listing setup failed");
+    if ((rc = ot_join(ix, d_keys, n, k, OtList{ix->loci.get(), d_own, d_first.get(), d_cursor.get(), d_out.get(), d_flag.get()})))
+        return rc;
+    std::vector<uint32_t> found(n);
     unsigned int flag = 0;
-    if (!rc && (cudaMemcpyAsync(found.data(), d_cursor, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-                cudaMemcpyAsync(&flag, d_flag, sizeof flag, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-                cudaStreamSynchronize(st) != cudaSuccess))
-        rc = fail(CRP_ERR_CUDA, "D2H of the listing cursors failed");
-    for (uint64_t i = 0; i < n && !rc; ++i)
+    if (cudaMemcpyAsync(found.data(), d_cursor.get(), n * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaMemcpyAsync(&flag, d_flag.get(), sizeof flag, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "D2H of the listing cursors failed");
+    for (uint64_t i = 0; i < n; ++i)
         if (found[i] != first[i + 1] - first[i])
-            rc = fail(CRP_ERR_STATE, "row %llu: %u sites found, its slice holds %llu", (unsigned long long)i, found[i],
-                      (unsigned long long)(first[i + 1] - first[i]));
-    if (!rc && flag) rc = fail(CRP_ERR_STATE, "a row found more sites than its slice holds");
-    if (!rc && total && (cudaMemcpyAsync(sites, d_out, total * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-                         cudaStreamSynchronize(st) != cudaSuccess))
-        rc = fail(CRP_ERR_CUDA, "D2H of the listing failed");
-    dev_free(d_first, st);
-    dev_free(d_cursor, st);
-    dev_free(d_out, st);
-    dev_free(d_flag, st);
-    return rc;
+            return fail(CRP_ERR_STATE, "row %llu: %u sites found, its slice holds %llu", (unsigned long long)i, found[i],
+                        (unsigned long long)(first[i + 1] - first[i]));
+    if (flag) return fail(CRP_ERR_STATE, "a row found more sites than its slice holds");
+    if (total && (cudaMemcpyAsync(sites, d_out.get(), total * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+                  cudaStreamSynchronize(st) != cudaSuccess))
+        return fail(CRP_ERR_CUDA, "D2H of the listing failed");
+    return 0;
 }
 
 // first [n + 1] of a listing call: CRP_ERR_ARG unless it starts at 0 and never decreases
@@ -2575,48 +2479,40 @@ int crp_offtarget_list_candidates(crp_offtarget *ix, const crp_result *res, char
             return fail(CRP_ERR_ARG, "rows[%llu] = %u: rows must be ascending, distinct and below %llu", (unsigned long long)i,
                         rows[i], (unsigned long long)n);
     cudaStream_t st = ix->st;
-    uint32_t *d_seg = nullptr, *d_rows = nullptr;
-    unsigned long long *d_keys = nullptr, *d_sel = nullptr;   // d_sel: [n_rows] keys, [n_rows] own loci
-    unsigned int *d_invalid = nullptr;
-    int rc = ot_candidate_keys(ix, res, s, nullptr, 0, &d_keys, &d_seg);   // every row's key, then the selected rows
-    if (!rc && (dev_alloc(&d_rows, n_rows * sizeof(uint32_t), st) != cudaSuccess ||
-                dev_alloc(&d_sel, 2 * n_rows * sizeof(unsigned long long), st) != cudaSuccess ||
-                dev_alloc(&d_invalid, sizeof(unsigned int), st) != cudaSuccess)) {
-        cudaGetLastError();
-        rc = fail(CRP_ERR_NOMEM, "cudaMalloc of %llu selected rows failed", (unsigned long long)n_rows);
-    }
-    if (!rc && (cudaMemcpyAsync(d_rows, rows, n_rows * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-                cudaMemsetAsync(d_invalid, 0, sizeof(unsigned int), st) != cudaSuccess))
-        rc = fail(CRP_ERR_CUDA, "H2D of the listing rows failed");
+    DevBuf<unsigned int> d_invalid;
+    DevBuf<unsigned long long> d_sel;          // [n_rows] keys, [n_rows] own loci
+    DevBuf<uint32_t> d_rows;
+    DevBuf<unsigned long long> d_keys;
+    DevBuf<uint32_t> d_seg;
+    int rc;
+    if ((rc = ot_candidate_keys(ix, res, s, nullptr, 0, d_keys, d_seg))) return rc;   // every row's key, then the selected rows
+    if ((rc = d_rows.alloc(n_rows, st, "the selected rows")) || (rc = d_sel.alloc(2 * n_rows, st, "the selected keys")) ||
+        (rc = d_invalid.alloc(1, st, "the row flag")))
+        return rc;
+    if (cudaMemcpyAsync(d_rows.get(), rows, n_rows * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemsetAsync(d_invalid.get(), 0, sizeof(unsigned int), st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "H2D of the listing rows failed");
+    OtGatherArgs ga;
+    ga.keys = d_keys.get();
+    ga.pos = res->pos[s].get();
+    ga.rows = d_rows.get();
+    ga.seg_row = d_seg.get();
+    ga.n = n_rows;
+    ga.n_seg = (uint32_t)(s == 0 ? res->seg_plus : res->seg_minus).size();
+    ga.genome = (uint32_t)(std::find(ix->genomes.begin(), ix->genomes.end(), res->g) - ix->genomes.begin());
+    ga.minus = s;
+    ga.sel_keys = d_sel.get();
+    ga.own = d_sel.get() + n_rows;
+    ga.invalid = d_invalid.get();
+    k_ot_gather<<<(unsigned)((n_rows + 255) / 256), 256, 0, st>>>(ga);
+    g_ctx.launches++;
     unsigned int invalid = 0;
-    if (!rc) {
-        OtGatherArgs ga;
-        ga.keys = d_keys;
-        ga.pos = res->pos[s];
-        ga.rows = d_rows;
-        ga.seg_row = d_seg;
-        ga.n = n_rows;
-        ga.n_seg = (uint32_t)(s == 0 ? res->seg_plus : res->seg_minus).size();
-        ga.genome = (uint32_t)(std::find(ix->genomes.begin(), ix->genomes.end(), res->g) - ix->genomes.begin());
-        ga.minus = s;
-        ga.sel_keys = d_sel;
-        ga.own = d_sel + n_rows;
-        ga.invalid = d_invalid;
-        k_ot_gather<<<(unsigned)((n_rows + 255) / 256), 256, 0, st>>>(ga);
-        g_ctx.launches++;
-        if (cudaGetLastError() != cudaSuccess ||
-            cudaMemcpyAsync(&invalid, d_invalid, sizeof invalid, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-            cudaStreamSynchronize(st) != cudaSuccess)
-            rc = fail(CRP_ERR_CUDA, "off-target query keys failed: %s", cudaGetErrorString(cudaGetLastError()));
-    }
-    if (!rc && invalid) rc = fail(CRP_ERR_ARG, "a selected row has no protospacer (its counts are 0xFFFFFFFF)");
-    if (!rc) rc = ot_list(ix, d_sel, d_sel + n_rows, n_rows, max_mm, first, sites);
-    dev_free(d_seg, st);
-    dev_free(d_keys, st);
-    dev_free(d_rows, st);
-    dev_free(d_sel, st);
-    dev_free(d_invalid, st);
-    return rc;
+    if (cudaGetLastError() != cudaSuccess ||
+        cudaMemcpyAsync(&invalid, d_invalid.get(), sizeof invalid, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "off-target query keys failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (invalid) return fail(CRP_ERR_ARG, "a selected row has no protospacer (its counts are 0xFFFFFFFF)");
+    return ot_list(ix, ga.sel_keys, ga.own, n_rows, max_mm, first, sites);
 }
 
 int crp_offtarget_list_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys, uint32_t max_mm, const uint64_t *first,
@@ -2629,11 +2525,9 @@ int crp_offtarget_list_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys,
     if (int rc = ot_check_keys(n, keys)) return rc;
     if (int rc = ot_check_first(n, first)) return rc;
     if (first[n] && !sites) return fail(CRP_ERR_ARG, "sites is NULL");
-    unsigned long long *d_keys = nullptr;
-    int rc = ot_upload_keys(ix, n, keys, &d_keys);
-    if (!rc) rc = ot_list(ix, d_keys, nullptr, n, max_mm, first, sites);
-    dev_free(d_keys, ix->st);
-    return rc;
+    DevBuf<unsigned long long> d_keys;
+    if (int rc = ot_upload_keys(ix, n, keys, d_keys)) return rc;
+    return ot_list(ix, d_keys.get(), nullptr, n, max_mm, first, sites);
 }
 
 }  // extern "C"
@@ -2652,20 +2546,15 @@ static int ot_check_weights(uint32_t k, const uint32_t *weights) {
 static int ot_score(crp_offtarget *ix, const unsigned long long *d_keys, uint64_t n, uint32_t k, const uint32_t *weights,
                     unsigned long long *d_sums, uint64_t *sums) {
     cudaStream_t st = ix->st;
-    uint32_t *d_w = nullptr;
-    if (dev_alloc(&d_w, kOtScoreSets * sizeof(uint32_t), st) != cudaSuccess) {
-        cudaGetLastError();
-        return fail(CRP_ERR_NOMEM, "cudaMalloc of the weight table failed");
-    }
-    int rc = 0;
-    if (cudaMemcpyAsync(d_w, weights, kOtScoreSets * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
-        rc = fail(CRP_ERR_CUDA, "H2D of the weight table failed");
-    if (!rc) rc = ot_join(ix, d_keys, n, k, OtScore{d_w, d_sums});
-    if (!rc && (cudaMemcpyAsync(sums, d_sums, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-                cudaStreamSynchronize(st) != cudaSuccess))
-        rc = fail(CRP_ERR_CUDA, "D2H of the off-target scores failed");
-    dev_free(d_w, st);
-    return rc;
+    DevBuf<uint32_t> d_w;
+    if (int rc = d_w.alloc(kOtScoreSets, st, "the weight table")) return rc;
+    if (cudaMemcpyAsync(d_w.get(), weights, kOtScoreSets * sizeof(uint32_t), cudaMemcpyHostToDevice, st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "H2D of the weight table failed");
+    if (int rc = ot_join(ix, d_keys, n, k, OtScore{d_w.get(), d_sums})) return rc;
+    if (cudaMemcpyAsync(sums, d_sums, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess)
+        return fail(CRP_ERR_CUDA, "D2H of the off-target scores failed");
+    return 0;
 }
 
 extern "C" {
@@ -2679,25 +2568,16 @@ int crp_offtarget_score_candidates(crp_offtarget *ix, const crp_result *res, cha
     if (n == 0) return 0;
     if (!sums) return fail(CRP_ERR_ARG, "sums is NULL");
     cudaStream_t st = ix->st;
-    uint32_t *d_seg = nullptr;
-    unsigned long long *d_keys = nullptr, *d_sums = nullptr;
-    int rc = 0;
-    if (dev_alloc(&d_sums, n * sizeof(unsigned long long), st) != cudaSuccess) {
-        cudaGetLastError();
-        rc = fail(CRP_ERR_NOMEM, "cudaMalloc of %llu query rows failed", (unsigned long long)n);
-    }
-    if (!rc) rc = ot_candidate_keys(ix, res, s, nullptr, 0, &d_keys, &d_seg);
-    if (!rc) {                                                 // the query keys, then the primed sums
-        k_ot_score_prime<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_keys, n, ix->own_site ? 0ull - weights[0] : 0ull,
-                                                                      d_sums);
-        g_ctx.launches++;
-        if (cudaGetLastError() != cudaSuccess) rc = fail(CRP_ERR_CUDA, "off-target score priming failed");
-    }
-    if (!rc) rc = ot_score(ix, d_keys, n, max_mm, weights, d_sums, sums);
-    dev_free(d_seg, st);
-    dev_free(d_keys, st);
-    dev_free(d_sums, st);
-    return rc;
+    DevBuf<unsigned long long> d_sums, d_keys;
+    DevBuf<uint32_t> d_seg;
+    if (int rc = d_sums.alloc(n, st, "the off-target sums")) return rc;
+    if (int rc = ot_candidate_keys(ix, res, s, nullptr, 0, d_keys, d_seg)) return rc;
+    // the query keys, then the primed sums
+    k_ot_score_prime<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_keys.get(), n, ix->own_site ? 0ull - weights[0] : 0ull,
+                                                                  d_sums.get());
+    g_ctx.launches++;
+    if (cudaGetLastError() != cudaSuccess) return fail(CRP_ERR_CUDA, "off-target score priming failed");
+    return ot_score(ix, d_keys.get(), n, max_mm, weights, d_sums.get(), sums);
 }
 
 int crp_offtarget_score_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys, uint32_t max_mm, const uint32_t *weights,
@@ -2710,18 +2590,11 @@ int crp_offtarget_score_keys(crp_offtarget *ix, uint64_t n, const uint64_t *keys
     if (!sums) return fail(CRP_ERR_ARG, "sums is NULL");
     if (int rc = ot_check_keys(n, keys)) return rc;
     cudaStream_t st = ix->st;
-    unsigned long long *d_keys = nullptr, *d_sums = nullptr;
-    int rc = ot_upload_keys(ix, n, keys, &d_keys);
-    if (!rc && dev_alloc(&d_sums, n * sizeof(unsigned long long), st) != cudaSuccess) {
-        cudaGetLastError();
-        rc = fail(CRP_ERR_NOMEM, "cudaMalloc of %llu keys failed", (unsigned long long)n);
-    }
-    if (!rc && cudaMemsetAsync(d_sums, 0, n * sizeof(unsigned long long), st) != cudaSuccess)
-        rc = fail(CRP_ERR_CUDA, "memset failed");
-    if (!rc) rc = ot_score(ix, d_keys, n, max_mm, weights, d_sums, sums);
-    dev_free(d_keys, st);
-    dev_free(d_sums, st);
-    return rc;
+    DevBuf<unsigned long long> d_sums, d_keys;
+    if (int rc = ot_upload_keys(ix, n, keys, d_keys)) return rc;
+    if (int rc = d_sums.alloc(n, st, "the off-target sums")) return rc;
+    if (cudaMemsetAsync(d_sums.get(), 0, n * sizeof(unsigned long long), st) != cudaSuccess) return fail(CRP_ERR_CUDA, "memset failed");
+    return ot_score(ix, d_keys.get(), n, max_mm, weights, d_sums.get(), sums);
 }
 
 int crp_offtarget_timing(const crp_offtarget *ix, float *ms_sites, float *ms_count, uint64_t *comparisons) {
@@ -2735,8 +2608,8 @@ int crp_offtarget_timing(const crp_offtarget *ix, float *ms_sites, float *ms_cou
 int crp_offtarget_free(crp_offtarget *ix) {
     if (!ix) return 0;
     if (ix->st) {
-        dev_free(ix->keys, ix->st);
-        dev_free(ix->loci, ix->st);
+        ix->keys.reset();                      // they record on ix->st: back before it is destroyed
+        ix->loci.reset();
         cudaStreamSynchronize(ix->st);
     }
     for (cudaEvent_t e : ix->ev)
